@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- payload GB/s of the KMP packet-matching hot path on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2]): synthetic UDP stream, 10 M packets x 1400-byte payloads per GPU
@@ -452,6 +452,14 @@ def h2d_peak(D, nbytes, reps=3):
     return D.sum_over_ranks(float(nbytes)) * reps / dt / 1e9
 
 
+def dump_outputs(out_dir, **arrays):
+    """DIR/<name>.npy for each array, as float64: exact for integer counts below 2**53, so that the outputs of two
+    builds on the same seeded stream can be compared value for value."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def oracle_prefix_ok(kmp, m, patterns, data, offsets, n):
     """counts of the first n packets through the C ABI's host form == the oracle's (bit-exact)"""
     from oracle import oracle_py
@@ -549,6 +557,8 @@ def ours(args, kmp, patterns):
     ms_step = max_over_ranks(e0.elapsed_time(e1)) / args.steps
     launches = m.launches - launches0  # partition + union + count expansion per step (libkmpb200's own counter)
     counts_resident = d_counts.cpu().numpy().copy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, counts=counts_resident)
 
     # ---- the dominant kernel alone (roofline) -----------------------------------------------------
     m.set_profile(True)
@@ -1015,7 +1025,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-sweep", action="store_true", help="skip the small forms of configs 4 and 5 on the default line")
     ap.add_argument("--no-parity", action="store_true", help="skip the full-size cross-check against the per-pattern engine")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (the count vector) as DIR/counts.npy, float64")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config != "c3"):
+        ap.error("--dump-outputs writes the outputs of the default configuration (--impl ours --config c3)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     # stdout carries the one JSON line and nothing else: whatever libraries write to file descriptor 1 in the

@@ -140,6 +140,23 @@ def test_cli_output_is_the_reference_output(strings):
             assert b"".join(lines[:-1]) == expected, (pcap, argv)
 
 
+def test_bench_dump_outputs_are_the_stream_counts(oracle, strings, tmp_path):
+    """bench.py --dump-outputs: the count vector of the last timed step as float64, equal to the oracle's counts on the
+    same seeded stream, which bench.py's numpy generator rebuilds on the host."""
+    import sys
+    import bench
+
+    n = 20_000
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "0", "--packets", str(n),
+                        "--no-e2e", "--no-cpu", "--no-sweep", "--no-parity", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout)["steps"] == 2
+    got = np.load(str(tmp_path / "counts.npy"))
+    data, off = bench.synth_stream(bench.SEED, 0, n, 1400, 2, strings)
+    assert got.dtype == np.float64 and got.tolist() == oracle.count_csr(data, off, strings)
+
+
 def test_integration_snippet_counts(tmp_path):
     """INTEGRATION.md section 1 as a C program (tests/c/integration_snippet.c): overlapping "aa" in "aaaa" = 3, the
     text of a payload ends at its NUL."""

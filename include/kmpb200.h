@@ -147,6 +147,46 @@ uint64_t kmpb_launch_count(const kmpb_ctx *ctx);
  * the context's streams: [0] whole call (H2D + kernels + D2H), [1] match kernels only. */
 int kmpb_last_timing(const kmpb_ctx *ctx, double *ms_out, int n);
 
+/* ---- finding: where the patterns occur ----------------------------------------------------- */
+/* The count entry points say how often each pattern occurs; the find entry points say where.  A match is one
+ * occurrence that the count forms count, no more and no less: it lies inside one packet, no NUL byte comes before its
+ * end in that packet (serial.c:191), and overlapping occurrences are separate matches.  Each match is one record:
+ *   packet   index of the packet in the caller's batch (kmpb_find_pcap: among the accepted packets, the numbering of
+ *            kmpb_pcap_packets and of kmpb_count_pcap's first / count);
+ *   offset   byte offset of the match's first byte inside that packet's payload;
+ *   pattern  the lowest file-order index among the patterns equal to the matched one (a token listed three times
+ *            yields one record per occurrence, carrying the index of its first listing).
+ * So for every pattern i, the count kmpb_count_host reports for i on the same batch equals the number of records whose
+ * pattern is the first index of i's token.  "Sorted" means ordered by (packet, offset, pattern).
+ * Finding always runs the union engine, whatever kmpb_set_engine selected (the per-pattern engine only counts).
+ * n_pat == 0 or an empty batch is valid and yields 0 matches.  Errors: KMPB_ESTATE before kmpb_set_patterns,
+ * KMPB_EINVAL for a NULL pointer or an unknown flag, KMPB_ENODEVICE without a B200. */
+typedef struct kmpb_match {
+    uint64_t packet;
+    uint32_t offset;
+    uint32_t pattern;
+} kmpb_match; /* 16 bytes */
+
+#define KMPB_FIND_SORTED 1u /* kmpb_find_device_span: sort the records (device radix sort, scratch owned by the context) */
+
+/* Device form, asynchronous on `stream` like kmpb_count_device_span and with its preconditions and limits (d_bytes
+ * 32-byte aligned, at most 2^31-1 packets, offsets below 2^56, at most 64 GiB in one batch).  d_out (device,
+ * kmpb_match[capacity]) receives records [0, min(total, capacity)); *d_n_found (device, uint64) is OVERWRITTEN with the
+ * total number of matches, which may exceed capacity.  With KMPB_FIND_SORTED and no overflow the records are sorted;
+ * the sort costs time in proportion to `capacity`, so size the buffer close to the total (the sum of the kmpb_count_*
+ * counts of the batch is exact).  On overflow the records written are an unspecified subset of the matches, in no
+ * particular order: run again with a larger buffer.  Unsorted, the records come in an unspecified order.  One call in
+ * flight per context; it shares scratch buffers with the count forms. */
+int kmpb_find_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets, uint64_t n_packets,
+                          uint64_t first_byte, uint64_t end_byte, kmpb_match *d_out, uint64_t capacity,
+                          uint64_t *d_n_found, uint32_t flags, void *stream);
+/* Host form: synchronous, chunked and overlapped like kmpb_count_host (KMPB_CHUNK_MB sets the chunk size), always
+ * sorted.  out (host, kmpb_match[capacity]) receives the first min(total, capacity) records in sorted order and
+ * *n_found the total.  The device record buffers grow as needed; a chunk whose records overflowed them is matched
+ * again from the copy already on the device. */
+int kmpb_find_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, uint64_t n_packets,
+                   kmpb_match *out, uint64_t capacity, uint64_t *n_found);
+
 /* ---- the data-parallel split of the MPI variant -------------------------------------------- */
 /* mpi_dumping.c:149-157: every rank gets n_packets / world packets, rank 0 also the remainder;
  * slices are contiguous in packet order.  Pure arithmetic, usable without a GPU. */
@@ -207,6 +247,14 @@ int kmpb_count_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t
  * defaults of kmpb_count_pcap) -- e.g. while another thread is still reading the savefile (serial.c:91-141); pinned
  * allocations take a few hundred milliseconds.  The counting calls grow the buffers themselves when they must. */
 int kmpb_reserve_staging(kmpb_ctx *ctx, uint64_t max_batch_bytes, uint64_t max_packets);
+/* kmpb_find_host for accepted packets [first, first+count) of a savefile, through kmpb_count_pcap's packing pipeline:
+ * always sorted, `packet` is the accepted-packet index (first + position in the slice). */
+int kmpb_find_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count, kmpb_match *out, uint64_t capacity,
+                   uint64_t *n_found);
+/* The capture record number (0-based, counting every record of the file, accepted or not) of accepted packets
+ * [first, first+count) into frames_out[count]: the frame a match's packet came from (Wireshark numbers frames from 1).
+ * Savefiles of 2^32 records or more are outside the documented limits. */
+int kmpb_pcap_frame_index(const kmpb_pcap *pc, uint64_t first, uint64_t count, uint64_t *frames_out);
 
 /* Frames arriving one at a time (live_openmp_task.c:160-217: pcap_next in a loop, batches handed to
  * tasks while the capture goes on).  kmpb_stream_push runs the extractor on one captured frame and

@@ -77,6 +77,14 @@ SIGNATURES = {
     "kmpb_pcap_bytes": (ctypes.c_uint64, [ctypes.c_void_p]),
     "kmpb_count_pcap": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64, c_u64p]),
     "kmpb_reserve_staging": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64]),
+    "kmpb_find_device_span": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64,
+                                             ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64,
+                                             ctypes.c_void_p, ctypes.c_uint32, ctypes.c_void_p]),
+    "kmpb_find_host": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64,
+                                      ctypes.c_void_p, ctypes.c_uint64, c_u64p]),
+    "kmpb_find_pcap": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64,
+                                      ctypes.c_void_p, ctypes.c_uint64, c_u64p]),
+    "kmpb_pcap_frame_index": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p]),
     "kmpb_stream_open": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.POINTER(ctypes.c_void_p)]),
     "kmpb_stream_push": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_uint32]),
     "kmpb_stream_flush": (ctypes.c_int, [ctypes.c_void_p, c_u64p]),

@@ -133,6 +133,51 @@ int finish_chunked(kmpb_ctx *ctx, int n_slots, uint64_t *counts_out)
     return KMPB_OK;
 }
 
+// bytes per chunk of the chunked forms: 64 MiB, or KMPB_CHUNK_MB
+uint64_t chunk_bytes_setting()
+{
+    uint64_t chunk_bytes = 64ull << 20;
+    if (const char *env = getenv("KMPB_CHUNK_MB")) {
+        long mb = atol(env);
+        if (mb > 0) chunk_bytes = (uint64_t)mb << 20;
+    }
+    return chunk_bytes;
+}
+
+// every offset, not a sample: a decreasing pair anywhere would size a copy wrongly (one pass over 8 bytes per packet,
+// all host threads; nothing next to copying the packets themselves)
+int check_offsets(const uint64_t *offsets, uint64_t n_packets)
+{
+    int64_t bad = -1;
+#pragma omp parallel for schedule(static) reduction(max : bad)
+    for (int64_t k = 0; k < (int64_t)n_packets; k++)
+        if (offsets[k + 1] < offsets[k] && k > bad) bad = k;
+    if (bad >= 0) return kmpb_fail(KMPB_EINVAL, "offsets decrease at packet %lld", (long long)bad);
+    return KMPB_OK;
+}
+
+// chunk plan of a host batch: whole packets, ~chunk_bytes each; the largest chunk's bytes (from its 512-byte aligned
+// base) and packets
+struct host_chunk { uint64_t k0, k1; };
+std::vector<host_chunk> plan_host_chunks(const uint64_t *offsets, uint64_t n_packets, uint64_t chunk_bytes, uint64_t &max_bytes,
+                                         uint64_t &max_pkts)
+{
+    std::vector<host_chunk> plan;
+    max_bytes = max_pkts = 0;
+    for (uint64_t k0 = 0; k0 < n_packets;) {
+        const uint64_t want = offsets[k0] + chunk_bytes;
+        uint64_t k1 = (uint64_t)(std::lower_bound(offsets + k0 + 1, offsets + n_packets, want) - offsets);
+        if (k1 > n_packets) k1 = n_packets;
+        k1 = std::min<uint64_t>(k1, k0 + ((1ull << 31) - 2));
+        plan.push_back({k0, k1});
+        const uint64_t base = offsets[k0] & ~511ull;
+        max_bytes = std::max(max_bytes, offsets[k1] - base);
+        max_pkts = std::max(max_pkts, k1 - k0);
+        k0 = k1;
+    }
+    return plan;
+}
+
 int init_context(kmpb_ctx *ctx)
 {
     const int device = ctx->device;
@@ -166,6 +211,86 @@ int device_flags(kmpb_ctx *ctx, int n_slots)
     KMPB_CUDA(cudaMemcpy(work, ctx->d_work, sizeof work, cudaMemcpyDeviceToHost));
     for (int s = 0; s < n_slots; s++)
         if (work[s * 4 + 1]) return kmpb_fail(KMPB_ELIMIT, "a packet of 2 GiB or more is not supported (its work item was skipped)");
+    return KMPB_OK;
+}
+
+// the record buffer of a stream slot of the chunked find forms, at least `records` long (grown by an eighth more)
+int ensure_find_rec(kmpb_ctx *ctx, int slot, uint64_t records)
+{
+    if (!ctx->d_find_found) KMPB_CUDA(cudaMalloc((void **)&ctx->d_find_found, KMPB_COPY_STREAMS * sizeof(unsigned long long)));
+    if (records <= ctx->find_rec_cap[slot] && ctx->d_find_rec[slot]) return KMPB_OK;
+    const uint64_t cap = records + records / 8 + 1024;
+    cudaFree(ctx->d_find_rec[slot]);
+    ctx->d_find_rec[slot] = nullptr;
+    ctx->find_rec_cap[slot] = 0;
+    KMPB_CUDA(cudaMalloc((void **)&ctx->d_find_rec[slot], cap * sizeof(kmpb_match)));
+    ctx->find_rec_cap[slot] = cap;
+    return KMPB_OK;
+}
+
+// The chunk pipeline of the host find forms.  stage(c, slot, batch, packet_base) puts chunk c on the device in the
+// slot's staging buffers (copies on the slot's stream) -- kmpb_count_host's or kmpb_count_pcap's way; the find kernel
+// follows on the same stream.  Chunk c is finished (its match count read, its records sorted and copied out) just
+// before its slot takes chunk c + KMPB_COPY_STREAMS, so the copies and kernels of the chunks in between keep the device
+// busy meanwhile.  A chunk whose records overflowed the slot's buffer is matched again, from the copy still on the
+// device, into a buffer of the exact size; once `capacity` records are out, later chunks are only counted.
+template <class Stage>
+int find_chunks(kmpb_ctx *ctx, uint64_t n_chunks, uint64_t guess, Stage &&stage, kmpb_match *out, uint64_t capacity,
+                uint64_t *n_found)
+{
+    kmpb_batch batch[KMPB_COPY_STREAMS] = {};
+    uint64_t base[KMPB_COPY_STREAMS] = {};
+    uint64_t total = 0, written = 0;
+    int rc;
+    auto finish = [&](uint64_t c) -> int {
+        const int slot = (int)(c % KMPB_COPY_STREAMS);
+        cudaStream_t s = ctx->copy_stream[slot];
+        unsigned long long n = 0;
+        KMPB_CUDA_Q(ctx, cudaMemcpyAsync(&n, ctx->d_find_found + slot, sizeof n, cudaMemcpyDeviceToHost, s));
+        KMPB_CUDA_Q(ctx, cudaStreamSynchronize(s));
+        const uint64_t take = std::min<uint64_t>(n, capacity - written);
+        if (take) {
+            int rc2;
+            if (n > ctx->find_rec_cap[slot]) {
+                if ((rc2 = ensure_find_rec(ctx, slot, n)) || (rc2 = kmpb_find_match(ctx, batch[slot], slot, ctx->d_find_rec[slot], n,
+                                                                                     ctx->d_find_found + slot, s))) {
+                    quiesce(ctx);
+                    return rc2;
+                }
+            }
+            if ((rc2 = kmpb_find_finish(ctx, batch[slot], base[slot], ctx->d_find_rec[slot], n, ctx->d_find_found + slot, true, s))) {
+                quiesce(ctx);
+                return rc2;
+            }
+            KMPB_CUDA_Q(ctx, cudaMemcpyAsync(out + written, ctx->d_find_rec[slot], take * sizeof(kmpb_match), cudaMemcpyDeviceToHost, s));
+            KMPB_CUDA_Q(ctx, cudaStreamSynchronize(s));
+        }
+        total += n;
+        written += take;
+        return KMPB_OK;
+    };
+    for (uint64_t c = 0; c < n_chunks; c++) {
+        const int slot = (int)(c % KMPB_COPY_STREAMS);
+        if (c >= (uint64_t)KMPB_COPY_STREAMS && (rc = finish(c - KMPB_COPY_STREAMS))) return rc;
+        if ((rc = ensure_find_rec(ctx, slot, guess))) { quiesce(ctx); return rc; }
+        if ((rc = stage(c, slot, batch[slot], base[slot])) ||
+            (rc = kmpb_find_match(ctx, batch[slot], slot, ctx->d_find_rec[slot], ctx->find_rec_cap[slot], ctx->d_find_found + slot,
+                                  ctx->copy_stream[slot]))) {
+            quiesce(ctx);
+            return rc;
+        }
+    }
+    for (uint64_t c = n_chunks > (uint64_t)KMPB_COPY_STREAMS ? n_chunks - KMPB_COPY_STREAMS : 0; c < n_chunks; c++)
+        if ((rc = finish(c))) return rc;
+    *n_found = total;
+    return device_flags(ctx, (int)std::min<uint64_t>(KMPB_COPY_STREAMS, n_chunks));
+}
+
+// the argument checks every find form starts with
+int find_args(kmpb_ctx *ctx, const void *out, uint64_t capacity, const void *n_found)
+{
+    if (ctx == nullptr || n_found == nullptr || (out == nullptr && capacity)) return kmpb_fail(KMPB_EINVAL, "NULL argument");
+    if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "find before kmpb_set_patterns");
     return KMPB_OK;
 }
 
@@ -233,7 +358,12 @@ void kmpb_destroy(kmpb_ctx *ctx)
     kmpb_release_tables(ctx);
     cudaFree(ctx->d_work);
     cudaFree(ctx->d_items);
+    cudaFree(ctx->d_find_found);
+    cudaFree(ctx->d_sort_keys[0]);
+    cudaFree(ctx->d_sort_keys[1]);
+    cudaFree(ctx->d_sort_temp);
     for (int i = 0; i < KMPB_COPY_STREAMS; i++) {
+        cudaFree(ctx->d_find_rec[i]);
         cudaFree(ctx->d_stage_bytes[i]);
         cudaFree(ctx->d_stage_off[i]);
         cudaFreeHost(ctx->h_stage_bytes[i]);
@@ -403,37 +533,12 @@ int kmpb_count_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets
     memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
     if (n_packets == 0) return KMPB_OK;
     if (bytes == nullptr || offsets == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL batch pointer");
-    {   // every offset, not a sample: a decreasing pair anywhere would size a copy wrongly (one pass over 8 bytes per
-        // packet, all host threads; nothing next to copying the packets themselves)
-        int64_t bad = -1;
-#pragma omp parallel for schedule(static) reduction(max : bad)
-        for (int64_t k = 0; k < (int64_t)n_packets; k++)
-            if (offsets[k + 1] < offsets[k] && k > bad) bad = k;
-        if (bad >= 0) return kmpb_fail(KMPB_EINVAL, "offsets decrease at packet %lld", (long long)bad);
-    }
-    int rc = use_device(ctx);
+    int rc = check_offsets(offsets, n_packets);
     if (rc) return rc;
+    if ((rc = use_device(ctx))) return rc;
 
-    // chunk plan: whole packets, ~chunk_bytes each
-    uint64_t chunk_bytes = 64ull << 20;
-    if (const char *env = getenv("KMPB_CHUNK_MB")) {
-        long mb = atol(env);
-        if (mb > 0) chunk_bytes = (uint64_t)mb << 20;
-    }
-    struct chunk { uint64_t k0, k1; };
-    std::vector<chunk> plan;
     uint64_t max_bytes = 0, max_pkts = 0;
-    for (uint64_t k0 = 0; k0 < n_packets;) {
-        const uint64_t want = offsets[k0] + chunk_bytes;
-        uint64_t k1 = (uint64_t)(std::lower_bound(offsets + k0 + 1, offsets + n_packets, want) - offsets);
-        if (k1 > n_packets) k1 = n_packets;
-        k1 = std::min<uint64_t>(k1, k0 + ((1ull << 31) - 2));
-        plan.push_back({k0, k1});
-        const uint64_t base = offsets[k0] & ~511ull;
-        max_bytes = std::max(max_bytes, offsets[k1] - base);
-        max_pkts = std::max(max_pkts, k1 - k0);
-        k0 = k1;
-    }
+    const std::vector<host_chunk> plan = plan_host_chunks(offsets, n_packets, chunk_bytes_setting(), max_bytes, max_pkts);
     const int n_slots = (int)std::min<size_t>(KMPB_COPY_STREAMS, plan.size());
     if ((rc = ensure_staging(ctx, max_bytes, max_pkts))) return rc;
     if ((rc = kmpb_union_scratch(ctx, max_bytes))) return rc;
@@ -483,11 +588,7 @@ int kmpb_count_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t
     if (count == 0) return KMPB_OK;
     int rc = use_device(ctx);
     if (rc) return rc;
-    uint64_t chunk_bytes = 64ull << 20;
-    if (const char *env = getenv("KMPB_CHUNK_MB")) {
-        long mb = atol(env);
-        if (mb > 0) chunk_bytes = (uint64_t)mb << 20;
-    }
+    const uint64_t chunk_bytes = chunk_bytes_setting();
     const uint64_t max_pkts = 1ull << 22, last = first + count;
     // a packet larger than a chunk still travels whole: size the slots for the largest chunk of the plan
     uint64_t max_bytes = 0, max_n = 0, n_chunks = 0;
@@ -536,6 +637,96 @@ int kmpb_count_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t
         fprintf(stderr, "kmpb_count_pcap: %llu chunks; waiting for a free slot %.3f s, packing %.3f s, issuing copies and kernels %.3f s\n",
                 (unsigned long long)c, t_wait, t_pack, t_issue);
     return finish_chunked(ctx, n_slots, counts_out);
+}
+
+// ---- find: where the patterns occur (include/kmpb200.h; kernels in union_kernel.cu and find.cu) ----------------
+int kmpb_find_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets, uint64_t n_packets,
+                          uint64_t first_byte, uint64_t end_byte, kmpb_match *d_out, uint64_t capacity,
+                          uint64_t *d_n_found, uint32_t flags, void *stream_v)
+{
+    int rc = find_args(ctx, d_out, capacity, d_n_found);
+    if (rc) return rc;
+    if (flags & ~KMPB_FIND_SORTED) return kmpb_fail(KMPB_EINVAL, "unknown find flags 0x%x", flags);
+    if (n_packets && (d_bytes == nullptr || d_offsets == nullptr)) return kmpb_fail(KMPB_EINVAL, "NULL device pointer");
+    if (end_byte < first_byte) return kmpb_fail(KMPB_EINVAL, "offsets decrease");
+    if ((rc = use_device(ctx))) return rc;
+    cudaStream_t stream = (cudaStream_t)stream_v;
+    if ((rc = kmpb_union_scratch(ctx, end_byte - first_byte))) return rc;
+    const kmpb_batch b{d_bytes, 0, d_offsets, n_packets, first_byte, end_byte};
+    unsigned long long *found = reinterpret_cast<unsigned long long *>(d_n_found);
+    if ((rc = kmpb_find_match(ctx, b, 0, d_out, capacity, found, stream))) return rc;
+    return kmpb_find_finish(ctx, b, 0, d_out, capacity, found, (flags & KMPB_FIND_SORTED) != 0, stream);
+}
+
+int kmpb_find_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, uint64_t n_packets,
+                   kmpb_match *out, uint64_t capacity, uint64_t *n_found)
+{
+    int rc = find_args(ctx, out, capacity, n_found);
+    if (rc) return rc;
+    *n_found = 0;
+    if (ctx->host.n_pat == 0 || n_packets == 0) return KMPB_OK;
+    if (bytes == nullptr || offsets == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL batch pointer");
+    if ((rc = check_offsets(offsets, n_packets))) return rc;
+    if ((rc = use_device(ctx))) return rc;
+    uint64_t max_bytes = 0, max_pkts = 0;
+    const std::vector<host_chunk> plan = plan_host_chunks(offsets, n_packets, chunk_bytes_setting(), max_bytes, max_pkts);
+    if ((rc = ensure_staging(ctx, max_bytes, max_pkts))) return rc;
+    if ((rc = kmpb_union_scratch(ctx, max_bytes))) return rc;
+    auto stage = [&](uint64_t c, int slot, kmpb_batch &b, uint64_t &base) -> int {
+        cudaStream_t s = ctx->copy_stream[slot];
+        const uint64_t k0 = plan[c].k0, k1 = plan[c].k1;
+        const uint64_t abs_base = offsets[k0] & ~511ull;
+        KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_bytes[slot], bytes + abs_base, offsets[k1] - abs_base, cudaMemcpyHostToDevice, s));
+        KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_off[slot], offsets + k0, (k1 - k0 + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+        b = kmpb_batch{ctx->d_stage_bytes[slot], abs_base, ctx->d_stage_off[slot], k1 - k0, offsets[k0], offsets[k1]};
+        base = k0;
+        return KMPB_OK;
+    };
+    return find_chunks(ctx, plan.size(), max_bytes / 256, stage, out, capacity, n_found);
+}
+
+int kmpb_find_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count, kmpb_match *out, uint64_t capacity,
+                   uint64_t *n_found)
+{
+    if (pc == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
+    int rc = find_args(ctx, out, capacity, n_found);
+    if (rc) return rc;
+    *n_found = 0;
+    if (ctx->host.n_pat == 0) return KMPB_OK;
+    const uint64_t total = kmpb_pcap_packets(pc);
+    if (first > total || count > total - first) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
+    if (count == 0) return KMPB_OK;
+    if ((rc = use_device(ctx))) return rc;
+    const uint64_t chunk_bytes = chunk_bytes_setting();
+    const uint64_t max_pkts = 1ull << 22, last = first + count;
+    std::vector<uint64_t> starts; // first packet of every chunk, then `last`
+    uint64_t max_bytes = 0, max_n = 0;
+    for (uint64_t k0 = first; k0 < last;) {
+        uint64_t nb = 0;
+        const uint64_t k1 = kmpb_pcap_chunk_end(pc, k0, last, chunk_bytes, max_pkts, &nb);
+        starts.push_back(k0);
+        max_bytes = std::max(max_bytes, nb);
+        max_n = std::max(max_n, k1 - k0);
+        k0 = k1;
+    }
+    starts.push_back(last);
+    if ((rc = ensure_staging(ctx, max_bytes, max_n))) return rc;
+    if ((rc = ensure_host_staging(ctx, max_bytes, max_n))) return rc;
+    if ((rc = kmpb_union_scratch(ctx, max_bytes))) return rc;
+    // (a slot's pinned buffers are free again: its previous chunk has been finished, which waited for its stream)
+    auto stage = [&](uint64_t c, int slot, kmpb_batch &b, uint64_t &base) -> int {
+        cudaStream_t s = ctx->copy_stream[slot];
+        const uint64_t k0 = starts[c], k1 = starts[c + 1];
+        kmpb_pcap_pack(pc, k0, k1 - k0, ctx->h_stage_bytes[slot], ctx->h_stage_off[slot]);
+        const uint64_t nbytes = ctx->h_stage_off[slot][k1 - k0];
+        memset(ctx->h_stage_bytes[slot] + nbytes, 0, 64);
+        KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_bytes[slot], ctx->h_stage_bytes[slot], nbytes + 64, cudaMemcpyHostToDevice, s));
+        KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_off[slot], ctx->h_stage_off[slot], (k1 - k0 + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+        b = kmpb_batch{ctx->d_stage_bytes[slot], 0, ctx->d_stage_off[slot], k1 - k0, 0, nbytes};
+        base = k0;
+        return KMPB_OK;
+    };
+    return find_chunks(ctx, starts.size() - 1, max_bytes / 256, stage, out, capacity, n_found);
 }
 
 // ---- frames pushed one at a time (the live-capture shape) ----------------------------------------

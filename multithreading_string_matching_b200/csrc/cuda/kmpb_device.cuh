@@ -31,6 +31,7 @@ struct kmpb_device_tables {
     // union engine
     uint32_t *vtab = nullptr;       // [vtab_words] start-anchored verification tables (automaton.c)
     uint32_t *filter = nullptr;     // [256]
+    uint32_t *uniq_first = nullptr; // [n_uniq] lowest file-order index of each distinct pattern (the find records' pattern)
 };
 
 struct kmpb_ctx {
@@ -60,6 +61,14 @@ struct kmpb_ctx {
     size_t h_stage_bytes_cap = 0, h_stage_off_cap = 0;
     cudaEvent_t ev_h2d[KMPB_COPY_STREAMS] = {};
     uint64_t *d_counts = nullptr;        // [n_pat] result of kmpb_count_host
+    // find: record buffers and found counters of the chunked forms (per stream slot), the sort's keys and CUB scratch
+    kmpb_match *d_find_rec[KMPB_COPY_STREAMS] = {};
+    uint64_t find_rec_cap[KMPB_COPY_STREAMS] = {};
+    unsigned long long *d_find_found = nullptr; // [KMPB_COPY_STREAMS]
+    uint64_t *d_sort_keys[2] = {};
+    uint64_t sort_cap = 0;
+    void *d_sort_temp = nullptr;
+    size_t sort_temp_bytes = 0;
     bool attr_union_set = false, attr_perpat_set = false; // per-device function attributes
     uint64_t launches = 0;
     double last_ms[2] = {0, 0};
@@ -83,6 +92,14 @@ struct kmpb_fused_out {
     uint32_t n = 0;
 };
 
+// Where the find kernel writes its records: rec[capacity] of {absolute position, 0, distinct id} (find.cu turns them
+// into kmpb_match), *found counts every match, also those past the capacity.
+struct kmpb_find_out {
+    kmpb_match *rec = nullptr;
+    uint64_t capacity = 0;
+    unsigned long long *found = nullptr;
+};
+
 // tables.cu
 int kmpb_upload_tables(kmpb_ctx *ctx);
 void kmpb_release_tables(kmpb_ctx *ctx);
@@ -90,7 +107,13 @@ void kmpb_release_tables(kmpb_ctx *ctx);
 int kmpb_launch_perpat(kmpb_ctx *ctx, const kmpb_batch &b, uint64_t *d_uniq_counts, cudaStream_t stream);
 // union_kernel.cu
 int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_uniq_counts, cudaStream_t stream,
-                      const kmpb_fused_out &out = kmpb_fused_out());
+                      const kmpb_fused_out &out = kmpb_fused_out(), const kmpb_find_out *find = nullptr);
 int kmpb_union_scratch(kmpb_ctx *ctx, uint64_t max_batch_bytes);
+// find.cu: the find kernel into d_rec[capacity] (*d_found = every match of the batch), then the records turned into
+// kmpb_match (packet index + packet_base), sorted or not
+int kmpb_find_match(kmpb_ctx *ctx, const kmpb_batch &b, int slot, kmpb_match *d_rec, uint64_t capacity, unsigned long long *d_found,
+                    cudaStream_t stream);
+int kmpb_find_finish(kmpb_ctx *ctx, const kmpb_batch &b, uint64_t packet_base, kmpb_match *d_rec, uint64_t capacity,
+                     const unsigned long long *d_found, bool sorted, cudaStream_t stream);
 // api.cu
 int kmpb_launch_expand(kmpb_ctx *ctx, const uint64_t *d_uniq_counts, uint64_t *d_counts, cudaStream_t stream);

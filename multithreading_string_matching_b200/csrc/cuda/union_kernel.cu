@@ -60,6 +60,7 @@
 //  counted exactly once.  Counts go to shared-memory counters and leave the block as one atomic per
 //  distinct pattern.  No separators, no padding and no second pass over the payload.
 #include <algorithm>
+#include <cooperative_groups.h>
 #include <type_traits>
 
 #include "kmpb_device.cuh"
@@ -346,6 +347,9 @@ enum { DC_TEXT_LO = 0, DC_TEXT_HI,   // p.bytes - p.abs_base: absolute byte 0
        DC_SLOTS_A, DC_SHIFT_A, DC_SLOTS_B, DC_SHIFT_B, DC_ONE, DC_REC, DC_BLOB,
        DC_MUL4096, DC_VTAB_SA,     // shared address of the probe tables, 0 = they are in global memory
        DC_COUNTS_SA,             // shared address of the counters, 0 = global atomics
+       DC_REC_LO = 18, DC_REC_HI, // find kernel: the record buffer (kmpb_match[capacity])
+       DC_CAP_LO, DC_CAP_HI,     // ... its capacity in records
+       DC_FOUND_LO, DC_FOUND_HI, // ... the uint64 counter of every match found (also those past the capacity)
        DC_LAST = 31 };           // "I am the last block" flag
 
 // The scratch words of a warp (128 bytes): two sets of 32 bytes, one per item parity --
@@ -390,6 +394,31 @@ __device__ __forceinline__ void count_hit(const drain_args &d, uint32_t u)
     else atomicAdd(reinterpret_cast<unsigned long long *>(const_cast<uint8_t *>(dc_ptr(DC_CNT_LO))) + u, 1ull);
 }
 
+// The find kernel's hit (after count_hit): one 16-byte record {absolute position, distinct id} that the locate kernel
+// (find.cu) turns into {packet, offset, pattern}.  Slots are reserved by one atomic per group of lanes that hit
+// together: a single counter takes every match of the batch (C3: 33.8 M per pass), one atomic per hit would serialise
+// on it.  Every match is counted; those whose slot lies past the capacity are not written.
+__device__ __forceinline__ void emit_hit(const uint64_t pos, const uint32_t u)
+{
+    namespace cg = cooperative_groups;
+    const cg::coalesced_group g = cg::coalesced_threads();
+    unsigned long long base = 0;
+    if (g.thread_rank() == 0)
+        base = atomicAdd(reinterpret_cast<unsigned long long *>(const_cast<uint8_t *>(dc_ptr(DC_FOUND_LO))), (unsigned long long)g.size());
+    const uint64_t slot = g.shfl(base, 0) + g.thread_rank();
+    const uint2 cap = lds64(smem_sa() + UN_OFF_MISC + 4u * DC_CAP_LO);
+    if (slot < (((uint64_t)cap.y << 32) | cap.x)) {
+        uint4 *rec = reinterpret_cast<uint4 *>(const_cast<uint8_t *>(dc_ptr(DC_REC_LO))) + slot;
+        __stcs(rec, make_uint4((uint32_t)pos, (uint32_t)(pos >> 32), 0u, u));
+    }
+}
+template <bool EMIT>
+__device__ __forceinline__ void hit(const drain_args &d, const uint32_t u, const uint64_t pos)
+{
+    count_hit(d, u);
+    if (EMIT) emit_hit(pos, u);
+}
+
 // 4 text bytes starting at g, of which the first `need` (>= 1) matter: never read past the word that holds the last
 // needed byte, which lies inside the packet.
 __device__ __forceinline__ uint32_t text_window(const uint8_t *g, uint32_t need)
@@ -411,7 +440,7 @@ struct probe_consts {
 // table B (the longer ones); the slots' records carry the pattern's first 8 bytes and their masks, so a record costs one
 // 16-byte load and one masked compare, and only a record that agrees on those bytes is looked at further (patterns of
 // more than 8 bytes: word by word against the text in global memory -- L2, the row was read a moment ago).
-template <bool VS>
+template <bool VS, bool EMIT>
 __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_consts &pc, const uint32_t x0, const uint32_t x1,
                                             const uint32_t room, const uint64_t pos)
 {
@@ -426,7 +455,7 @@ __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_con
     const uint32_t vt_one = pc.one, vt_slots_a = pc.slots_a, vt_slots_b = pc.slots_b;
     if (vt_one) { // one-byte patterns: a direct table (room >= 1 always holds)
         const uint32_t u = vt(vt_one + (x0 & 0xffu));
-        if (u != 0xffffffffu) count_hit(d, u);
+        if (u != 0xffffffffu) hit<EMIT>(d, u, pos);
     }
     if (room < 2) return;
     uint2 ea = make_uint2(0, 0), eb = make_uint2(0, 0); // {first record, records}
@@ -454,7 +483,7 @@ __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_con
                 same = (rem >= 4 ? diff : diff & ((1u << (8 * rem)) - 1u)) == 0;
             }
         }
-        if (same) count_hit(d, b.y);
+        if (same) hit<EMIT>(d, b.y, pos);
     }
 }
 
@@ -464,6 +493,7 @@ __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_con
 // free-running counters, slots handed out and slots verified.
 __device__ __forceinline__ uint32_t warp_c_sa() { return smem_sa() + UN_OFF_C + (threadIdx.x >> 5) * (UN_CCAP * UN_C_BYTES1); }
 // verify the n (<= 32) candidates from slot `head` on, one per lane
+template <bool EMIT>
 __device__ __forceinline__ void verify_round(const drain_args &d, const uint32_t head, const uint32_t n)
 {
     const uint32_t lane = threadIdx.x & 31;
@@ -474,12 +504,13 @@ __device__ __forceinline__ void verify_round(const drain_args &d, const uint32_t
         pc.slots_a = c0.x; pc.shift_a = c0.y; pc.slots_b = c0.z; pc.shift_b = c0.w; pc.one = c1.x; pc.rec = c1.y;
         const uint4 e = lds128v(warp_c_sa() + ((head + lane) & (UN_CCAP - 1)) * UN_C_BYTES1);
         const uint64_t pos = ((uint64_t)(e.w >> 8) << 32) | e.z;
-        if (d.vtab_sa) verify_cand<true>(d, pc, e.x, e.y, e.w & 0xffu, pos);
-        else verify_cand<false>(d, pc, e.x, e.y, e.w & 0xffu, pos);
+        if (d.vtab_sa) verify_cand<true, EMIT>(d, pc, e.x, e.y, e.w & 0xffu, pos);
+        else verify_cand<false, EMIT>(d, pc, e.x, e.y, e.w & 0xffu, pos);
     }
 }
 // the candidates still waiting at the end of a batch
-__device__ __noinline__ void flush_candidates()
+template <bool EMIT>
+__device__ __forceinline__ void flush_body()
 {
     drain_args d;
     d.q_sa = warp_q_sa();
@@ -488,11 +519,13 @@ __device__ __noinline__ void flush_candidates()
     d.counts_sa = dc(DC_COUNTS_SA);
     __syncwarp();
     const uint2 cs = lds64v(d.scratch_sa + SC_CAND); // {handed out, verified}: fewer than 32 apart between resolve steps
-    verify_round(d, cs.y, cs.x - cs.y);
+    verify_round<EMIT>(d, cs.y, cs.x - cs.y);
     __syncwarp();
     if ((threadIdx.x & 31) == 0) sts32v(d.scratch_sa + SC_CAND + 4, cs.x);
     __syncwarp();
 }
+__device__ __noinline__ void flush_candidates() { flush_body<false>(); }
+__device__ __noinline__ void flush_candidates_find() { flush_body<true>(); }
 
 // Phase 0 of a resolve step, on its own so that the row loop can issue it a row or two ahead: the n (<= 32) oldest
 // events' groups (32 B + 8 B lookahead), one per lane, from L2 (the rows were read a few microseconds ago) straight
@@ -532,6 +565,7 @@ __device__ __forceinline__ void drain_fetch(const uint32_t head, const uint32_t 
 // event carries its item's parity, and what the resolve step has to know about either item waits in the warp's
 // scratch words, where the warp put it when it took the item: no lane has to look anything up in global memory for
 // it, and the row loop does not keep it in registers.  Positions are relative to the item's row0 (32 bits).
+template <bool EMIT>
 __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n)
 {
     drain_args d;
@@ -718,14 +752,14 @@ __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n
             ctail += __popc(any);
             __syncwarp();
             if (ctail - chead >= 32u) {
-                verify_round(d, chead, 32u);
+                verify_round<EMIT>(d, chead, 32u);
                 chead += 32u;
                 __syncwarp();
             }
         }
     }
     while (ctail - chead >= 32u) {
-        verify_round(d, chead, 32u);
+        verify_round<EMIT>(d, chead, 32u);
         chead += 32u;
     }
     __syncwarp();
@@ -738,7 +772,12 @@ __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n
 __device__ __noinline__ void drain_events(const uint32_t head, const uint32_t n)
 {
     drain_fetch(head, n);
-    drain_body(head, n);
+    drain_body<false>(head, n);
+}
+__device__ __noinline__ void drain_events_find(const uint32_t head, const uint32_t n)
+{
+    drain_fetch(head, n);
+    drain_body<true>(head, n);
 }
 
 // NUL-dense row.  An event without candidates exists only to tell later candidates where the last NUL before them
@@ -759,12 +798,16 @@ __device__ __forceinline__ uint32_t uni(uint32_t v) { return __shfl_sync(FULL, v
 __device__ __forceinline__ uint64_t uni(uint64_t v) { return __shfl_sync(FULL, v, 0); }
 #undef DP_SEL
 #define DP_SEL(k) p.sel[k]
-__global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_kernel(const __grid_constant__ union_params p)
+// The kernel body, in two instantiations: the count kernel (EMIT = false) and the find kernel (EMIT = true), which
+// also writes a record per match; what it needs of the record buffer waits in the DC_* words, not in registers.
+template <bool EMIT>
+__device__ __forceinline__ void union_body(const union_params &__restrict__ p, const kmpb_find_out &__restrict__ fo)
 {
     uint32_t *lut = reinterpret_cast<uint32_t *>(smem);                      // L, then G
     uint32_t *s_misc = reinterpret_cast<uint32_t *>(smem + UN_OFF_MISC);
     uint32_t *s_counts = reinterpret_cast<uint32_t *>(smem + UN_OFF_COUNTS);
-    const uint32_t counts_bytes = p.counts_in_smem ? ((4u * p.n_uniq + 15u) & ~15u) : 0u;
+    const uint32_t n_uniq = p.n_uniq; // read unconditionally: p is a reference here, a load under the condition would branch
+    const uint32_t counts_bytes = p.counts_in_smem ? ((4u * n_uniq + 15u) & ~15u) : 0u;
     uint32_t *s_vtab = reinterpret_cast<uint32_t *>(smem + UN_OFF_COUNTS + counts_bytes);
 
     for (uint32_t i = threadIdx.x; i < 256 * 32; i += UN_THREADS) {
@@ -791,6 +834,12 @@ __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_kernel(const __grid_
         s_misc[DC_MUL4096] = p.mul4096;
         s_misc[DC_VTAB_SA] = p.vtab_in_smem ? saddr_of(s_vtab) : 0u;
         s_misc[DC_COUNTS_SA] = p.counts_in_smem ? saddr_of(s_counts) : 0u;
+        if (EMIT) {
+            const uint64_t rec = reinterpret_cast<uint64_t>(fo.rec), found = reinterpret_cast<uint64_t>(fo.found);
+            s_misc[DC_REC_LO] = (uint32_t)rec; s_misc[DC_REC_HI] = (uint32_t)(rec >> 32);
+            s_misc[DC_CAP_LO] = (uint32_t)fo.capacity; s_misc[DC_CAP_HI] = (uint32_t)(fo.capacity >> 32);
+            s_misc[DC_FOUND_LO] = (uint32_t)found; s_misc[DC_FOUND_HI] = (uint32_t)(found >> 32);
+        }
     }
     const uint32_t lane = threadIdx.x & 31;
     __syncthreads();
@@ -815,7 +864,8 @@ __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_kernel(const __grid_
     // resolve the oldest min(pending, 32) events (out of line: the rare places)
     auto resolve_oldest = [&]() {
         const uint32_t qn = pending(), n = qn < UN_QDRAIN ? qn : UN_QDRAIN;
-        drain_events(oldest(), n);
+        if (EMIT) drain_events_find(oldest(), n);
+        else drain_events(oldest(), n);
         qs -= n;
     };
 
@@ -978,7 +1028,7 @@ __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_kernel(const __grid_
             // loop, inlined (one copy of the code, and no call whose register needs the loop would have to respect).
             while ((qs & QS_FETCHED) || pending() >= 2 * UN_QDRAIN) {
                 if (!(qs & QS_FETCHED)) drain_fetch(oldest(), UN_QDRAIN);
-                drain_body(oldest(), UN_QDRAIN);
+                drain_body<EMIT>(oldest(), UN_QDRAIN);
                 qs = (qs & ~QS_FETCHED) - UN_QDRAIN;
                 if (lane == 0) { // that many fewer events of older items
                     const uint32_t older = lds32v(warp_scratch_sa() + SC_STATE + 4);
@@ -1017,7 +1067,8 @@ __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_kernel(const __grid_
     }
     // leftovers
     while (pending()) resolve_oldest();
-    flush_candidates();
+    if (EMIT) flush_candidates_find();
+    else flush_candidates();
 
     __syncthreads();
     if (p.counts_in_smem)
@@ -1044,6 +1095,17 @@ __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_kernel(const __grid_
     }
 }
 
+__global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_kernel(const __grid_constant__ union_params p)
+{
+    union_body<false>(p, kmpb_find_out());
+}
+
+__global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_find_kernel(const __grid_constant__ union_params p,
+                                                                        const __grid_constant__ kmpb_find_out fo)
+{
+    union_body<true>(p, fo);
+}
+
 // ---- host side ------------------------------------------------------------------------------------
 
 // scratch for batches of up to max_batch_bytes: work counters and the item table, one set per slot
@@ -1061,7 +1123,7 @@ int kmpb_union_scratch(kmpb_ctx *ctx, uint64_t max_batch_bytes)
 }
 
 int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_uniq_counts, cudaStream_t stream,
-                      const kmpb_fused_out &out)
+                      const kmpb_fused_out &out, const kmpb_find_out *find)
 {
     const kmpb_tables &h = ctx->host;
     if (h.n_uniq == 0 || b.n_packets == 0 || b.end_byte == b.first_byte) return KMPB_OK;
@@ -1097,6 +1159,7 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     const size_t smem_bytes = UN_SMEM_FIXED + counts_bytes + (vtab_in_smem ? 4ull * h.vtab_words : 0);
     if (!ctx->attr_union_set) {
         KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
+        KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_find_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
         ctx->attr_union_set = true;
     }
     kmpb_union_partition_kernel<<<(n_items + 1 + 255) / 256, 256, 0, stream>>>(b.d_offsets, (uint32_t)b.n_packets, n_items,
@@ -1130,7 +1193,8 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     int grid = (int)std::min<uint32_t>((uint32_t)ctx->sm_count, (warps_needed + UN_WARPS - 1) / UN_WARPS);
     if (grid < 1) grid = 1;
     if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[0], stream));
-    kmpb_union_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p);
+    if (find) kmpb_union_find_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, *find);
+    else kmpb_union_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p);
     if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[1], stream));
     ctx->launches += 2;
     KMPB_CUDA(cudaGetLastError());

@@ -43,6 +43,7 @@ static uint32_t load32(const uint8_t *p, int swapped)
 typedef struct {
     uint64_t at;  /* file offset of the payload's first byte */
     uint32_t len;
+    uint32_t frame; /* its capture record number, from 0 (a savefile of 2^32 records or more is outside the limits) */
 } payload_ref;
 
 /* Growing list of accepted payloads. */
@@ -56,7 +57,7 @@ typedef struct {
 static int take_frame(ref_list *l, const uint8_t *file, size_t at, uint32_t caplen, extract_fn extract)
 {
     uint32_t off, len;
-    l->frames++;
+    const uint64_t frame = l->frames++;
     if (!extract(file + at, caplen, &off, &len)) return KMPB_OK;
     if (l->packets == l->cap) {
         size_t cap = l->cap ? 2 * l->cap : (size_t)1 << 16;
@@ -67,6 +68,7 @@ static int take_frame(ref_list *l, const uint8_t *file, size_t at, uint32_t capl
     }
     l->refs[l->packets].at = at + off;
     l->refs[l->packets].len = len;
+    l->refs[l->packets].frame = (uint32_t)frame;
     l->bytes += len;
     l->packets++;
     return KMPB_OK;
@@ -280,6 +282,14 @@ void kmpb_pcap_close(kmpb_pcap *pc)
 uint64_t kmpb_pcap_packets(const kmpb_pcap *pc) { return pc ? pc->n_packets : 0; }
 uint64_t kmpb_pcap_frames(const kmpb_pcap *pc) { return pc ? pc->n_frames : 0; }
 uint64_t kmpb_pcap_bytes(const kmpb_pcap *pc) { return pc ? pc->total_bytes : 0; }
+
+int kmpb_pcap_frame_index(const kmpb_pcap *pc, uint64_t first, uint64_t count, uint64_t *frames_out)
+{
+    if (pc == NULL || (frames_out == NULL && count)) return kmpb_fail(KMPB_EINVAL, "kmpb_pcap_frame_index: NULL argument");
+    if (first > pc->n_packets || count > pc->n_packets - first) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
+    for (uint64_t k = 0; k < count; k++) frames_out[k] = pc->refs[first + k].frame;
+    return KMPB_OK;
+}
 
 uint64_t kmpb_pcap_chunk_end(const kmpb_pcap *pc, uint64_t first, uint64_t last, uint64_t max_bytes, uint64_t max_packets,
                              uint64_t *bytes_out)

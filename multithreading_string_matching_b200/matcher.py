@@ -18,6 +18,9 @@ from ._lib import CCsr, CPatterns, CSynth, KmpbError, c_i32p, c_u8p, c_u32p, c_u
 ENGINE_AUTO, ENGINE_PERPAT, ENGINE_UNION = 0, 1, 2
 PROTO_UDP, PROTO_TCP = 0, 1
 _PROTO = {"udp": PROTO_UDP, "tcp": PROTO_TCP, PROTO_UDP: PROTO_UDP, PROTO_TCP: PROTO_TCP}
+FIND_SORTED = 1
+# one kmpb_match record (include/kmpb200.h): where a pattern occurs
+MATCH_DTYPE = np.dtype([("packet", "<u8"), ("offset", "<u4"), ("pattern", "<u4")])
 _ENGINE = {"auto": ENGINE_AUTO, "perpat": ENGINE_PERPAT, "union": ENGINE_UNION,
            ENGINE_AUTO: ENGINE_AUTO, ENGINE_PERPAT: ENGINE_PERPAT, ENGINE_UNION: ENGINE_UNION}
 
@@ -209,6 +212,54 @@ class Matcher:
             return counts[: len(self.patterns)].tolist()
         finally:
             lib().kmpb_pcap_close(pc)
+
+    def _find(self, call, capacity):
+        """call(out_ptr, capacity, n_found_ref) once with a guessed capacity, once more with the exact total if the
+        guess was short -> sorted records"""
+        total = ctypes.c_uint64(0)
+        for _ in range(2):
+            out = np.zeros(max(capacity, 1), dtype=MATCH_DTYPE)
+            check(call(out.ctypes.data, capacity, ctypes.byref(total)))
+            if total.value <= capacity:
+                return out[: total.value]
+            capacity = total.value
+        raise AssertionError("the match count changed between two runs on the same input")
+
+    def find_host(self, data, offsets):
+        """Every match in a host CSR batch (kmpb_find_host): a structured array (packet u8, offset u4, pattern u4)
+        sorted by (packet, offset, pattern); pattern is the lowest index among equal patterns."""
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        data = _as_u8(data)
+        n = len(offsets) - 1
+        guess = (int(offsets[-1]) - int(offsets[0])) // 256 + 1024 if n > 0 else 0
+        return self._find(lambda out, cap, nf: lib().kmpb_find_host(self._ctx, data.ctypes.data, offsets.ctypes.data, n,
+                                                                    out, cap, nf), guess)
+
+    def find_pcap(self, path, proto="udp", first=0, count=None):
+        """Every match in accepted packets [first, first+count) of a savefile (kmpb_find_pcap), sorted; `packet` is the
+        accepted-packet index and the added field `frame` (u8) the 0-based capture record number it came from."""
+        pc = ctypes.c_void_p()
+        check(lib().kmpb_pcap_open(os.fsencode(path), _PROTO[proto], ctypes.byref(pc)))
+        try:
+            n = lib().kmpb_pcap_packets(pc)
+            count = n - first if count is None else count
+            guess = lib().kmpb_pcap_bytes(pc) // 256 + 1024
+            rec = self._find(lambda out, cap, nf: lib().kmpb_find_pcap(self._ctx, pc, first, count, out, cap, nf), guess)
+            frames = np.zeros(max(count, 1), dtype=np.uint64)
+            check(lib().kmpb_pcap_frame_index(pc, first, count, frames.ctypes.data))
+        finally:
+            lib().kmpb_pcap_close(pc)
+        out = np.zeros(len(rec), dtype=MATCH_DTYPE.descr + [("frame", "<u8")])
+        for f in ("packet", "offset", "pattern"):
+            out[f] = rec[f]
+        out["frame"] = frames[(rec["packet"] - first).astype(np.int64)]
+        return out
+
+    def find_device(self, d_bytes, d_offsets, n_packets, d_out, capacity, d_n_found, span, sorted=False, stream=None):
+        """kmpb_find_device_span: asynchronous; d_out (kmpb_match[capacity]) and d_n_found (uint64, overwritten with
+        the total) are device pointers."""
+        check(lib().kmpb_find_device_span(self._ctx, d_bytes, d_offsets, n_packets, span[0], span[1], d_out, capacity,
+                                          d_n_found, FIND_SORTED if sorted else 0, stream))
 
     def stream(self, proto="udp", batch_bytes=0):
         """Frames one at a time (the live_openmp_task.c shape): returns a FrameStream."""

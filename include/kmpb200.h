@@ -51,6 +51,9 @@ extern "C" {
 #define KMPB_ELIMIT (-8)    /* a documented limit was exceeded (see DESIGN.md section 7) */
 
 #define KMPB_MAX_PATTERN_LEN 99 /* char str[100] + fscanf("%s"), serial.c:64-66 */
+/* Every packet of a batch must be shorter than this: 2 GiB - 1 MiB.  (The union engine's work items then always span
+ * less than 2^31 bytes, which its 32-bit item-relative positions need.) */
+#define KMPB_PACKET_LIMIT ((1ull << 31) - (1ull << 20))
 
 #define KMPB_PROTO_UDP 0 /* dump_UDP_packet, packet_dumping.h:87-139 (default, serial.c:31) */
 #define KMPB_PROTO_TCP 1 /* dump_TCP_packet, packet_dumping.h:150-188 */
@@ -98,7 +101,10 @@ int kmpb_get_prefix(kmpb_ctx *ctx, uint32_t pattern_index, int32_t *pi_out, uint
 /* serial.c:153-155 / openmp_data.c:157-175 / mpi_dumping.c:198-200:
  *     for k in packets: for i in patterns: count[i] += kmp_matcher(payload[k], pattern[i], pi[i])
  * The payloads come as one flat CSR batch instead of N malloc'd buffers (serial.c:124-137):
- * packet k is bytes[offsets[k] .. offsets[k+1]), offsets has n_packets+1 non-decreasing entries.
+ * packet k is bytes[offsets[k] .. offsets[k+1]), offsets has n_packets+1 non-decreasing entries, and every
+ * packet is shorter than KMPB_PACKET_LIMIT.  Every host form -- kmpb_count_host, kmpb_find_host, the savefile forms
+ * (a payload is its frame's captured length less the headers) and kmpb_stream_push -- checks each packet before
+ * anything runs and returns KMPB_ELIMIT naming it.
  *
  * Host form: bytes / offsets are host memory (pinned memory from kmpb_host_alloc is copied
  * asynchronously in chunks on several streams, overlapped with the match kernels; pageable memory
@@ -128,9 +134,10 @@ int kmpb_count_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t
 int kmpb_count_device_span_peers(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets,
                                  uint64_t n_packets, uint64_t first_byte, uint64_t end_byte,
                                  uint64_t *const *d_counts_all, uint32_t n_vectors, void *stream);
-/* The device forms never wait, so they cannot report what only the device knows: a packet of 2 GiB or more (outside
- * the documented limits; its work item is skipped).  This call waits for the context's device and returns KMPB_ELIMIT
- * if any device-form call since the last check met one (the host forms check by themselves). */
+/* The device forms never wait, so they cannot report what only the device knows: a packet of KMPB_PACKET_LIMIT bytes or
+ * more (outside the documented limits: the union engine's counts and records of that batch are unspecified).  This call
+ * waits for the context's device and returns KMPB_ELIMIT if any union-engine device-form call since the last check met
+ * one; the check clears what it reports.  (The host forms check every packet before anything runs: they never set it.) */
 int kmpb_check_device_errors(kmpb_ctx *ctx);
 /* Device copy of the per-pattern counts of the last kmpb_count_host call (uint64[n_pat] on the
  * context's GPU), for callers that combine several GPUs with a collective (mpi_dumping.c:202). */

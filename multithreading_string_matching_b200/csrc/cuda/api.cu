@@ -23,7 +23,6 @@
 namespace {
 
 void quiesce(kmpb_ctx *ctx);
-int device_flags(kmpb_ctx *ctx, int n_slots);
 
 int use_device(const kmpb_ctx *ctx)
 {
@@ -128,9 +127,8 @@ int finish_chunked(kmpb_ctx *ctx, int n_slots, uint64_t *counts_out)
     KMPB_CUDA(cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[1]));
     ctx->last_ms[0] = ms;
     ctx->last_ms[1] = 0;
-    // device-side error flags of the union engine (oversized packets)
-    if (ctx->engine != KMPB_ENGINE_PERPAT) return device_flags(ctx, n_slots);
-    return KMPB_OK;
+    return KMPB_OK; // (no device-side flags to read: check_offsets, check_pcap_lengths or kmpb_stream_push checked
+                    // every packet's size before anything ran)
 }
 
 // bytes per chunk of the chunked forms: 64 MiB, or KMPB_CHUNK_MB
@@ -144,16 +142,31 @@ uint64_t chunk_bytes_setting()
     return chunk_bytes;
 }
 
-// every offset, not a sample: a decreasing pair anywhere would size a copy wrongly (one pass over 8 bytes per packet,
-// all host threads; nothing next to copying the packets themselves)
+// every offset, not a sample: a decreasing pair anywhere would size a copy wrongly, a packet of KMPB_PACKET_LIMIT bytes
+// or more would be skipped by the union engine (one pass over 8 bytes per packet, all host threads; nothing next to
+// copying the packets themselves)
 int check_offsets(const uint64_t *offsets, uint64_t n_packets)
 {
-    int64_t bad = -1;
-#pragma omp parallel for schedule(static) reduction(max : bad)
-    for (int64_t k = 0; k < (int64_t)n_packets; k++)
-        if (offsets[k + 1] < offsets[k] && k > bad) bad = k;
+    int64_t bad = -1, big = -1;
+#pragma omp parallel for schedule(static) reduction(max : bad, big)
+    for (int64_t k = 0; k < (int64_t)n_packets; k++) {
+        if (offsets[k + 1] < offsets[k]) bad = k > bad ? k : bad;
+        else if (offsets[k + 1] - offsets[k] >= KMPB_PACKET_LIMIT) big = k > big ? k : big;
+    }
     if (bad >= 0) return kmpb_fail(KMPB_EINVAL, "offsets decrease at packet %lld", (long long)bad);
+    if (big >= 0)
+        return kmpb_fail(KMPB_ELIMIT, "packet %lld is %llu bytes long; packets must be shorter than %llu (2 GiB - 1 MiB)",
+                         (long long)big, (unsigned long long)(offsets[big + 1] - offsets[big]), KMPB_PACKET_LIMIT);
     return KMPB_OK;
+}
+
+// the savefile forms' twin of check_offsets' size check, over accepted packets [first, first+count)
+int check_pcap_lengths(const kmpb_pcap *pc, uint64_t first, uint64_t count)
+{
+    const uint64_t k = kmpb_pcap_first_long(pc, first, count, KMPB_PACKET_LIMIT);
+    if (k == first + count) return KMPB_OK;
+    return kmpb_fail(KMPB_ELIMIT, "packet %llu has a payload of %llu bytes (2 GiB - 1 MiB) or more; packets must be shorter",
+                     (unsigned long long)k, KMPB_PACKET_LIMIT);
 }
 
 // chunk plan of a host batch: whole packets, ~chunk_bytes each; the largest chunk's bytes (from its 512-byte aligned
@@ -201,17 +214,6 @@ void quiesce(kmpb_ctx *ctx)
         if (s) cudaStreamSynchronize(s);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     cudaGetLastError();
-}
-
-// the union engine's device-side error flags of scratch slots [0, n_slots)
-int device_flags(kmpb_ctx *ctx, int n_slots)
-{
-    if (ctx->d_work == nullptr) return KMPB_OK;
-    uint32_t work[KMPB_COPY_STREAMS * 4];
-    KMPB_CUDA(cudaMemcpy(work, ctx->d_work, sizeof work, cudaMemcpyDeviceToHost));
-    for (int s = 0; s < n_slots; s++)
-        if (work[s * 4 + 1]) return kmpb_fail(KMPB_ELIMIT, "a packet of 2 GiB or more is not supported (its work item was skipped)");
-    return KMPB_OK;
 }
 
 // the record buffer of a stream slot of the chunked find forms, at least `records` long (grown by an eighth more)
@@ -283,7 +285,7 @@ int find_chunks(kmpb_ctx *ctx, uint64_t n_chunks, uint64_t guess, Stage &&stage,
     for (uint64_t c = n_chunks > (uint64_t)KMPB_COPY_STREAMS ? n_chunks - KMPB_COPY_STREAMS : 0; c < n_chunks; c++)
         if ((rc = finish(c))) return rc;
     *n_found = total;
-    return device_flags(ctx, (int)std::min<uint64_t>(KMPB_COPY_STREAMS, n_chunks));
+    return KMPB_OK; // (as in finish_chunked: the stage's caller checked every packet's size first)
 }
 
 // the argument checks every find form starts with
@@ -321,7 +323,16 @@ int kmpb_check_device_errors(kmpb_ctx *ctx)
     int rc = use_device(ctx);
     if (rc) return rc;
     KMPB_CUDA(cudaDeviceSynchronize());
-    return device_flags(ctx, KMPB_COPY_STREAMS);
+    if (ctx->d_work == nullptr) return KMPB_OK;
+    // the union engine's error flags, word 1 of every slot's work counters: set by its kernels, cleared only here
+    uint32_t work[KMPB_COPY_STREAMS * 4];
+    KMPB_CUDA(cudaMemcpy(work, ctx->d_work, sizeof work, cudaMemcpyDeviceToHost));
+    bool flagged = false;
+    for (int s = 0; s < KMPB_COPY_STREAMS; s++) flagged |= work[s * 4 + 1] != 0;
+    if (!flagged) return KMPB_OK;
+    KMPB_CUDA(cudaMemset(ctx->d_work, 0, sizeof work));
+    return kmpb_fail(KMPB_ELIMIT, "a device-form batch held a packet of %llu bytes (2 GiB - 1 MiB) or more: its results are "
+                     "unspecified", KMPB_PACKET_LIMIT);
 }
 
 int kmpb_create(kmpb_ctx **out, int device)
@@ -586,7 +597,9 @@ int kmpb_count_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t
     const uint64_t total = kmpb_pcap_packets(pc);
     if (first > total || count > total - first) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
     if (count == 0) return KMPB_OK;
-    int rc = use_device(ctx);
+    int rc = check_pcap_lengths(pc, first, count);
+    if (rc) return rc;
+    if ((rc = use_device(ctx))) return rc;
     if (rc) return rc;
     const uint64_t chunk_bytes = chunk_bytes_setting();
     const uint64_t max_pkts = 1ull << 22, last = first + count;
@@ -696,6 +709,7 @@ int kmpb_find_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t 
     const uint64_t total = kmpb_pcap_packets(pc);
     if (first > total || count > total - first) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
     if (count == 0) return KMPB_OK;
+    if ((rc = check_pcap_lengths(pc, first, count))) return rc;
     if ((rc = use_device(ctx))) return rc;
     const uint64_t chunk_bytes = chunk_bytes_setting();
     const uint64_t max_pkts = 1ull << 22, last = first + count;
@@ -796,6 +810,9 @@ int kmpb_stream_push(kmpb_stream *st, const uint8_t *frame, uint32_t captured_le
     uint32_t off = 0, len = 0;
     st->frames++;
     if (!st->extract(frame, captured_len, &off, &len)) return KMPB_OK;
+    if (len >= KMPB_PACKET_LIMIT)
+        return kmpb_fail(KMPB_ELIMIT, "packet %llu has a payload of %u bytes; packets must be shorter than %llu (2 GiB - 1 MiB)",
+                         (unsigned long long)st->packets, len, KMPB_PACKET_LIMIT);
     if (len > st->batch_bytes) return kmpb_fail(KMPB_ELIMIT, "a %u-byte payload does not fit a %llu-byte batch", len, (unsigned long long)st->batch_bytes);
     int rc = use_device(st->ctx);
     if (rc) return rc;

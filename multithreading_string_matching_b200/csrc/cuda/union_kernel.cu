@@ -135,7 +135,7 @@ struct union_params {
     uint32_t n_packets;
     const uint32_t *items; // [n_items+1] first packet of each work item
     uint32_t n_items;
-    uint32_t *work;         // [0] next item, [1] error flags, [2] blocks that have finished
+    uint32_t *work;         // [0] next item, [1] error flags (until kmpb_check_device_errors), [2] blocks that have finished
     const uint32_t *filter; // [256] filter words in 6-bit fields
     uint32_t n_uniq;
     uint32_t counts_in_smem; // counters live in shared memory
@@ -156,13 +156,15 @@ struct union_params {
 };
 
 // ---- work partition: item i = packets [items[i], items[i+1]) ---------------------------------
+// It also flags (work[1]) every packet of KMPB_PACKET_LIMIT bytes or more: such a packet runs across some item's target,
+// as targets lie at most an item apart, and it is the packet just before that item's first.
 __global__ void kmpb_union_partition_kernel(const uint64_t *__restrict__ offsets, uint32_t n_packets,
                                             uint32_t n_items, uint32_t n_big, uint64_t item_bytes, uint64_t small_bytes,
                                             uint32_t *__restrict__ items,
                                             uint32_t *__restrict__ work)
 {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i == 0) { work[0] = 0; work[1] = 0; work[2] = 0; }
+    if (i == 0) { work[0] = 0; work[2] = 0; }
     if (i > n_items) return;
     if (i == n_items) { items[i] = n_packets; return; }
     // first packet whose start is >= the item's target byte: n_big items of item_bytes, then small
@@ -200,6 +202,7 @@ __global__ void kmpb_union_partition_kernel(const uint64_t *__restrict__ offsets
         if (offsets[mid] < target) lo = mid + 1; else hi = mid;
     }
     items[i] = lo;
+    if (lo > 0 && offsets[lo] - offsets[lo - 1] >= KMPB_PACKET_LIMIT) atomicOr(work + 1, 1u);
 }
 
 // ---- helpers -----------------------------------------------------------------------------------
@@ -878,7 +881,7 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
         if (ks >= ke) continue;
         const uint64_t b_abs = uni(p.offsets[ks]), e_abs = uni(p.offsets[ke]);
         if (b_abs == e_abs) continue;
-        if (e_abs - b_abs >= (1ull << 31) - 4096) { // a packet of about 2 GiB: outside the documented limits
+        if (e_abs - b_abs >= (1ull << 31) - 4096) { // only past KMPB_PACKET_LIMIT (the partition has flagged the packet)
             if (lane == 0) atomicOr(&p.work[1], 1u);
             continue;
         }
@@ -1116,7 +1119,10 @@ int kmpb_union_scratch(kmpb_ctx *ctx, uint64_t max_batch_bytes)
     cudaFree(ctx->d_items);
     ctx->d_items = nullptr;
     ctx->items_cap = 0;
-    if (!ctx->d_work) KMPB_CUDA(cudaMalloc((void **)&ctx->d_work, KMPB_COPY_STREAMS * 4 * sizeof(uint32_t)));
+    if (!ctx->d_work) {
+        KMPB_CUDA(cudaMalloc((void **)&ctx->d_work, KMPB_COPY_STREAMS * 4 * sizeof(uint32_t)));
+        KMPB_CUDA(cudaMemset(ctx->d_work, 0, KMPB_COPY_STREAMS * 4 * sizeof(uint32_t))); // no error flags yet
+    }
     KMPB_CUDA(cudaMalloc((void **)&ctx->d_items, (size_t)KMPB_COPY_STREAMS * need * sizeof(uint32_t)));
     ctx->items_cap = need;
     return KMPB_OK;

@@ -73,6 +73,9 @@ typedef struct kmpb_tables {
 uint64_t kmpb_pcap_chunk_end(const kmpb_pcap *pc, uint64_t first, uint64_t last, uint64_t max_bytes, uint64_t max_packets,
                              uint64_t *bytes_out);
 void kmpb_pcap_pack(const kmpb_pcap *pc, uint64_t first, uint64_t count, uint8_t *dst, uint64_t *offsets);
+/* the first accepted packet in [first, first+count) whose payload is min_len bytes or longer, else first+count (a
+ * payload is its frame's captured length less the headers: a savefile can hold one of any size up to 4 GiB) */
+uint64_t kmpb_pcap_first_long(const kmpb_pcap *pc, uint64_t first, uint64_t count, uint64_t min_len);
 
 /* slot of a key (a text position's first two or three bytes) in a probe table (the device uses the same expression) */
 uint32_t kmpb_vtab_slot(uint32_t key, uint32_t shift);

@@ -300,6 +300,13 @@ uint64_t kmpb_pcap_chunk_end(const kmpb_pcap *pc, uint64_t first, uint64_t last,
     return k;
 }
 
+uint64_t kmpb_pcap_first_long(const kmpb_pcap *pc, uint64_t first, uint64_t count, uint64_t min_len)
+{
+    for (uint64_t k = first; k < first + count; k++)
+        if (pc->refs[k].len >= min_len) return k;
+    return first + count;
+}
+
 void kmpb_pcap_pack(const kmpb_pcap *pc, uint64_t first, uint64_t count, uint8_t *dst, uint64_t *offsets)
 {
     pack_payloads(pc->file, pc->refs + first, count, dst, offsets);

@@ -235,6 +235,11 @@ class Matcher:
         return self._find(lambda out, cap, nf: lib().kmpb_find_host(self._ctx, data.ctypes.data, offsets.ctypes.data, n,
                                                                     out, cap, nf), guess)
 
+    def find_host_ptr(self, bytes_ptr, offsets_ptr, n_packets, capacity_guess):
+        """find_host over raw host pointers (bytes_ptr is absolute byte 0 of the offsets), like count_host_ptr"""
+        return self._find(lambda out, cap, nf: lib().kmpb_find_host(self._ctx, bytes_ptr, offsets_ptr, n_packets, out, cap, nf),
+                          capacity_guess)
+
     def find_pcap(self, path, proto="udp", first=0, count=None):
         """Every match in accepted packets [first, first+count) of a savefile (kmpb_find_pcap), sorted; `packet` is the
         accepted-packet index and the added field `frame` (u8) the 0-based capture record number it came from."""

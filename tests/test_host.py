@@ -147,6 +147,32 @@ def test_packer_savefile_variants(oracle, tmp_path):
     assert e.value.code == -5
 
 
+def test_savefile_payload_length_scan(tmp_path):
+    """kmpb_pcap_first_long: the scan the savefile forms run over the accepted packets before anything else, to refuse
+    a payload of KMPB_PACKET_LIMIT bytes or more (a payload is the captured length less the headers: any size)."""
+    p = str(tmp_path / "lens.pcap")
+    _write_pcap(p, [_udp_frame(b"x" * 10), b"not udp", _udp_frame(b"y" * 300), _udp_frame(b""), _udp_frame(b"z" * 5000),
+                    _udp_frame(b"w" * 7)])
+    lib = kmp.lib()
+    fn = lib.kmpb_pcap_first_long
+    fn.restype = ctypes.c_uint64
+    fn.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_uint64]
+    pc = ctypes.c_void_p()
+    kmp.matcher.check(lib.kmpb_pcap_open(os.fsencode(p), kmp.PROTO_UDP, ctypes.byref(pc)))
+    try:
+        assert lib.kmpb_pcap_packets(pc) == 5  # payloads 10, 300, 0, 5000, 7
+        assert fn(pc, 0, 5, 300) == 1
+        assert fn(pc, 0, 5, 301) == 3
+        assert fn(pc, 2, 3, 300) == 3
+        assert fn(pc, 2, 1, 300) == 3  # none in [2, 3): first + count
+        assert fn(pc, 4, 1, 8) == 5
+        assert fn(pc, 4, 1, 7) == 4
+        assert fn(pc, 0, 5, 5001) == 5
+        assert fn(pc, 5, 0, 0) == 5
+    finally:
+        lib.kmpb_pcap_close(pc)
+
+
 def _pcapng(frames, big_endian=False, simple_from=None, second_section_at=None):
     """A pcapng file by hand: SHB, IDB, one packet block per frame (Enhanced; Simple from index `simple_from`
     on), a name-resolution block in the middle, optionally a second section in the other byte order."""

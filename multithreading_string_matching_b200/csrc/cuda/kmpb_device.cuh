@@ -31,6 +31,7 @@ struct kmpb_device_tables {
     // union engine
     uint32_t *vtab = nullptr;       // [vtab_words] start-anchored verification tables (automaton.c)
     uint32_t *filter = nullptr;     // [256]
+    uint32_t *gate = nullptr;       // [host.gate_words] prefix gate (automaton.c build_gate), null when there is none
     uint32_t *uniq_first = nullptr; // [n_uniq] lowest file-order index of each distinct pattern (the find records' pattern)
 };
 

@@ -39,8 +39,11 @@
 //  per event completing on a per-warp mbarrier was measured in its place: 13 % slower, 48-byte copies are not what that
 //  engine is for.)
 //  Phase 1:
-//    - the lane re-runs the filter over the quarter that reported (two bytes per update, like the row loop), this time
-//      recording which start positions fired and which bytes are NUL;
+//    - the lane tests the start positions of the quarter that reported against the PREFIX GATE (automaton.c
+//      build_gate: a hashed bitmap, word by a position's first two bytes, bit by its third), which every true start
+//      passes and most of the filter's false ones fail, and finds the quarter's NULs by a zero-byte test of its words;
+//      a pattern set without a gate (a one-byte pattern, very many keys) re-runs the filter over the quarter instead
+//      (two bytes per update, like the row loop), recording which start positions fired and which bytes are NUL;
 //    - it finds the packet that holds its first candidate: a division when all the item's packets have the same size,
 //      else a search in the item's slice of `offsets` (interpolation guess, then binary search); the item's packet and
 //      byte range waits in the warp's scratch words;
@@ -153,6 +156,9 @@ struct union_params {
     const uint32_t *pat_to_uniq;
     uint32_t n_pat, n_out;
     unsigned long long *out[KMPB_MAX_OUT];
+    const uint32_t *gate;   // prefix gate (automaton.c build_gate), gate_words words; copied to shared memory after
+    uint32_t gate_words;    // the probe tables when gate_in_smem, else not used (the resolve step re-runs the filter)
+    uint32_t gate_shift, gate_in_smem;
 };
 
 // ---- work partition: item i = packets [items[i], items[i+1]) ---------------------------------
@@ -353,6 +359,7 @@ enum { DC_TEXT_LO = 0, DC_TEXT_HI,   // p.bytes - p.abs_base: absolute byte 0
        DC_REC_LO = 18, DC_REC_HI, // find kernel: the record buffer (kmpb_match[capacity])
        DC_CAP_LO, DC_CAP_HI,     // ... its capacity in records
        DC_FOUND_LO, DC_FOUND_HI, // ... the uint64 counter of every match found (also those past the capacity)
+       DC_GATE_SA, DC_GATE_SHIFT, // shared address of the prefix gate (0 = none: phase 1 re-runs the filter), its hash shift
        DC_LAST = 31 };           // "I am the last block" flag
 
 // The scratch words of a warp (128 bytes): two sets of 32 bytes, one per item parity --
@@ -390,6 +397,19 @@ struct drain_args {
     uint32_t vtab_sa;    // the probe tables in shared memory, 0 = in global memory
     uint32_t counts_sa;  // the shared counters, or 0
 };
+
+// Diagnostic build (EXTRA_NVFLAGS=-DKMPB_UN_STATS, scripts/event_counts.py): what the resolve steps do, counted per warp
+// by lane 0 -- events resolved, resolve steps, candidates appended to the candidate ring, verification rounds.  The
+// production build has none of it.
+#ifdef KMPB_UN_STATS
+__device__ unsigned long long kmpb_un_stats[4];
+#define UN_STAT(i, v)                                                                                 \
+    do {                                                                                              \
+        if ((threadIdx.x & 31) == 0) atomicAdd(&kmpb_un_stats[i], (unsigned long long)(v));          \
+    } while (0)
+#else
+#define UN_STAT(i, v) do { } while (0)
+#endif
 
 __device__ __forceinline__ void count_hit(const drain_args &d, uint32_t u)
 {
@@ -500,6 +520,7 @@ template <bool EMIT>
 __device__ __forceinline__ void verify_round(const drain_args &d, const uint32_t head, const uint32_t n)
 {
     const uint32_t lane = threadIdx.x & 31;
+    UN_STAT(3, 1);
     if (lane < n) {
         probe_consts pc;
         const uint4 c0 = lds128(smem_sa() + UN_OFF_MISC + 4u * DC_SLOTS_A);
@@ -578,6 +599,8 @@ __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n
     d.counts_sa = dc(DC_COUNTS_SA);
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t lutL = smem_sa() + (lane << 2), mul2 = dc(DC_MUL4096);
+    const uint2 gate_c = lds64(smem_sa() + UN_OFF_MISC + 4u * DC_GATE_SA);
+    const uint32_t gate_sa = gate_c.x, gate_sh = gate_c.y;
     uint32_t lt;
     asm("mov.u32 %0, %%lanemask_lt;" : "=r"(lt));
     cp_async_wait_all(); // phase 0 (drain_fetch): my event's bytes are in its slot
@@ -594,34 +617,74 @@ __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n
         const uint4 s0 = lds128v(set_sa), s1 = lds128v(set_sa + 16);
         ks = s0.x; ke = s0.y; b_rel = s0.z; e_rel = s0.w;
         row0_lo = s1.x; row0_hi = s1.y; carry = s1.z; psize = s1.w;
-        // Re-run the filter over the quarters that reported (usually one), one byte per update, this time recording
-        // which start positions fired and which bytes are NUL.  Quarter k: bytes 8k..8k+11 -- three bytes of run-in,
-        // then the starts 8k..8k+8 report at the bytes 8k+3..8k+11, and so do the NULs among the bytes 8k..8k+8 (the
-        // quarters of the row loop overlap by one start; OR-ing a bit twice changes nothing).
         uint32_t quarters = (((t.y & 0x7f7f7f7fu) + 0x7f7f7f7fu) | t.y) & 0x80808080u; // bit 8k+7: quarter k
-        while (quarters) {
-            const uint32_t k8 = (__ffs(quarters) - 1) & ~7u; // 8k
-            quarters &= quarters - 1;
-            const uint2 w01 = lds64v(entry_sa + k8);
-            const uint32_t w0 = w01.x, w1 = w01.y, w2 = lds32v(entry_sa + k8 + 8);
-            uint32_t S = 0, cmr = 0, zr = 0;
-            // Two bytes per update, as in the row loop; after an update bits 24..28 / 18..22 hold the candidate buckets of
-            // the start three before b0 / b1, bits 29 / 23 "that byte is NUL".  Adding 0x1f to a 5-bit field carries into
-            // the bit above it iff the field is not zero, and x * 132 moves bits 29 and 23 of x to bits 31 and 30: two
-            // report bits per update and kind, shifted into cmr / zr from below (nothing can report before byte 3).
+        if (gate_sa) {
+            // The prefix gate: start s passes when bit 31 - (byte s+2 & 31) of word gate[hash(bytes s, s+1)] is set, which
+            // holds at every true start (automaton.c build_gate), and fails at most of the filter's false ones -- the
+            // short patterns' bucket unions admit byte combinations no pattern begins with.  The starts of a quarter that
+            // reported are all tested: the gate takes the place of the filter re-run below, is tighter and costs less (about 85
+            // instructions per quarter against 103).
+            // NULs: an exact zero-byte test of the quarter's bytes (every NUL raises its quarter's report).
+            while (quarters) {
+                const uint32_t k8 = (__ffs(quarters) - 1) & ~7u; // 8k
+                quarters &= quarters - 1;
+                const uint2 w01 = lds64v(entry_sa + k8);
+                const uint32_t w0 = w01.x, w1 = w01.y, w2 = lds32v(entry_sa + k8 + 8);
+                uint32_t g = 0; // bit j: start 8k + 1 + j passes (quarter 0: 8k + j), filled from the top start down
+                // x: the start's text word (its first two bytes pick the word), xb: the word two bytes on (its low 5 bits
+                // pick the bit; a rotate takes its shift amount modulo 32); the bit is rotated to bit 31 and shifted into g
+                auto probe = [&](const uint32_t x, const uint32_t xb) {
+                    const uint32_t w = lds32(gate_sa + 4u * ((x * KMPB_GATE_MUL) >> gate_sh));
+                    g = __funnelshift_l(__funnelshift_l(w, w, xb), g, 1);
+                };
+                const uint32_t x5 = __funnelshift_r(w1, w2, 8), x6 = __funnelshift_r(w1, w2, 16);
+                const uint32_t x7 = __funnelshift_r(w1, w2, 24), x9 = w2 >> 8, x10 = w2 >> 16;
+                const uint32_t x1 = __funnelshift_r(w0, w1, 8), x2 = __funnelshift_r(w0, w1, 16), x3 = __funnelshift_r(w0, w1, 24);
+                // the row loop's quarter 0 holds the starts 0..8, quarter k > 0 the starts 8k+1..8k+8: 8k is quarter k-1's
+                probe(w2, x10); probe(x7, x9); probe(x6, w2); probe(x5, x7); probe(w1, x6);
+                probe(x3, x5); probe(x2, w1); probe(x1, x3);
+                if (k8 == 0) probe(w0, x2);
+                cm |= g << (k8 == 0 ? 0u : k8 + 1u);
+                // NULs: only if the quarter's report can hold one (bit 5: b0's NUL -- or b1's bucket 3 --, bit 7: b1's
+                // NUL).  Bit 7 of every zero byte of w0, w1 (exact: no borrow runs from byte to byte); the multiply
+                // gathers the eight bits, moved to bits 0, 8, 16, 24 (w0) and 4, 12, 20, 28 (w1), into bits 21..28
+                // without carries; the ninth byte is w2's first.
+                if ((t.y >> k8) & 0xa0u) {
+                    const uint32_t z0 = ~(((w0 & 0x7f7f7f7fu) + 0x7f7f7f7fu) | w0) & 0x80808080u;
+                    const uint32_t z1 = ~(((w1 & 0x7f7f7f7fu) + 0x7f7f7f7fu) | w1) & 0x80808080u;
+                    const uint32_t z8 = ((((z0 >> 7) | (z1 >> 3)) * 0x00204081u) >> 21) & 0xffu;
+                    zm |= (z8 | ((w2 & 0xffu) == 0u ? 0x100u : 0u)) << k8;
+                }
+            }
+        } else {
+            // No gate: re-run the filter over the quarters that reported (usually one), this time recording which start
+            // positions fired and which bytes are NUL.  Quarter k: bytes 8k..8k+11 -- three bytes of run-in, then the
+            // starts 8k..8k+8 report at the bytes 8k+3..8k+11, and so do the NULs among the bytes 8k..8k+8 (the
+            // quarters of the row loop overlap by one start; OR-ing a bit twice changes nothing).
+            while (quarters) {
+                const uint32_t k8 = (__ffs(quarters) - 1) & ~7u; // 8k
+                quarters &= quarters - 1;
+                const uint2 w01 = lds64v(entry_sa + k8);
+                const uint32_t w0 = w01.x, w1 = w01.y, w2 = lds32v(entry_sa + k8 + 8);
+                uint32_t S = 0, cmr = 0, zr = 0;
+                // Two bytes per update, as in the row loop; after an update bits 24..28 / 18..22 hold the candidate buckets
+                // of the start three before b0 / b1, bits 29 / 23 "that byte is NUL".  Adding 0x1f to a 5-bit field carries
+                // into the bit above it iff the field is not zero, and x * 132 moves bits 29 and 23 of x to bits 31 and 30:
+                // two report bits per update and kind, shifted into cmr / zr from below (nothing can report before byte 3).
 #define SV2(word, k0)                                                                                           \
     do {                                                                                                        \
         SA2(word, k0);                                                                                          \
         zr = __funnelshift_l((S & 0x20800000u) * 132u, zr, 2);                                                  \
         cmr = __funnelshift_l((((S & 0x1f7c0000u) + 0x1f7c0000u) & 0x20800000u) * 132u, cmr, 2);               \
     } while (0)
-            SA2(w0, 0);
-            SV2(w0, 2);
-            SV2(w1, 0); SV2(w1, 2);
-            SV2(w2, 0); SV2(w2, 2);
+                SA2(w0, 0);
+                SV2(w0, 2);
+                SV2(w1, 0); SV2(w1, 2);
+                SV2(w2, 0); SV2(w2, 2);
 #undef SV2
-            cm |= (__brev(cmr) >> 23) << k8; // the first report is the highest of the 9 bits
-            zm |= (__brev(zr) >> 23) << k8;
+                cm |= (__brev(cmr) >> 23) << k8; // the first report is the highest of the 9 bits
+                zm |= (__brev(zr) >> 23) << k8;
+            }
         }
         // the item's first and last rows overhang it: starts count inside [b_rel, e_rel) only, and bytes
         // past e_rel may be anything, so NULs count below e_rel only
@@ -739,6 +802,9 @@ __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n
                      : "+r"(incl)
                      : "r"(dd));
     const uint32_t total = __shfl_sync(FULL, incl, 31);
+    UN_STAT(0, n);
+    UN_STAT(1, 1);
+    UN_STAT(2, total);
     if (ctail - chead + total <= UN_CCAP) {
         // The ring takes them all: every lane fills its run at its own pace -- no trips in step with the lane that has
         // the most.  (The order of the candidates in the ring does not matter.)
@@ -822,6 +888,9 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
         for (uint32_t i = threadIdx.x; i < p.n_uniq; i += UN_THREADS) s_counts[i] = 0;
     if (p.vtab_in_smem)
         for (uint32_t i = threadIdx.x; i < p.vtab_words; i += UN_THREADS) s_vtab[i] = p.vtab[i];
+    uint32_t *s_gate = s_vtab + (p.vtab_in_smem ? p.vtab_words : 0u);
+    if (p.gate_in_smem)
+        for (uint32_t i = threadIdx.x; i < p.gate_words; i += UN_THREADS) s_gate[i] = p.gate[i];
     for (uint32_t i = threadIdx.x; i < UN_SCRATCH_BYTES / 4; i += UN_THREADS)
         reinterpret_cast<uint32_t *>(smem + UN_OFF_SCRATCH)[i] = 0; // item parity, pending flag, carries
     if (threadIdx.x == 0) {
@@ -837,6 +906,8 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
         s_misc[DC_MUL4096] = p.mul4096;
         s_misc[DC_VTAB_SA] = p.vtab_in_smem ? saddr_of(s_vtab) : 0u;
         s_misc[DC_COUNTS_SA] = p.counts_in_smem ? saddr_of(s_counts) : 0u;
+        s_misc[DC_GATE_SA] = p.gate_in_smem ? saddr_of(s_gate) : 0u;
+        s_misc[DC_GATE_SHIFT] = p.gate_shift;
         if (EMIT) {
             const uint64_t rec = reinterpret_cast<uint64_t>(fo.rec), found = reinterpret_cast<uint64_t>(fo.found);
             s_misc[DC_REC_LO] = (uint32_t)rec; s_misc[DC_REC_HI] = (uint32_t)(rec >> 32);
@@ -1128,6 +1199,20 @@ int kmpb_union_scratch(kmpb_ctx *ctx, uint64_t max_batch_bytes)
     return KMPB_OK;
 }
 
+#ifdef KMPB_UN_STATS
+// the diagnostic counters: copied to out[4] (events, resolve steps, candidates, verification rounds), zeroed if reset
+extern "C" int kmpb_union_stats(uint64_t out[4], int reset)
+{
+    KMPB_CUDA(cudaDeviceSynchronize());
+    KMPB_CUDA(cudaMemcpyFromSymbol(out, kmpb_un_stats, 4 * sizeof(uint64_t)));
+    if (reset) {
+        const unsigned long long zero[4] = {0, 0, 0, 0};
+        KMPB_CUDA(cudaMemcpyToSymbol(kmpb_un_stats, zero, sizeof zero));
+    }
+    return KMPB_OK;
+}
+#endif
+
 int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_uniq_counts, cudaStream_t stream,
                       const kmpb_fused_out &out, const kmpb_find_out *find)
 {
@@ -1162,7 +1247,10 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     const bool counts_in_smem = UN_SMEM_FIXED + 4ull * h.n_uniq + 16 <= UN_SMEM_MAX - 8192;
     const size_t counts_bytes = counts_in_smem ? ((4ull * h.n_uniq + 15) & ~15ull) : 0;
     const bool vtab_in_smem = UN_SMEM_FIXED + counts_bytes + 4ull * h.vtab_words <= UN_SMEM_MAX;
-    const size_t smem_bytes = UN_SMEM_FIXED + counts_bytes + (vtab_in_smem ? 4ull * h.vtab_words : 0);
+    const size_t vtab_bytes = vtab_in_smem ? 4ull * h.vtab_words : 0;
+    // the prefix gate after them, if there is one and it fits; without it the resolve step re-runs the filter
+    const bool gate_in_smem = h.gate_words && UN_SMEM_FIXED + counts_bytes + vtab_bytes + 4ull * h.gate_words <= UN_SMEM_MAX;
+    const size_t smem_bytes = UN_SMEM_FIXED + counts_bytes + vtab_bytes + (gate_in_smem ? 4ull * h.gate_words : 0);
     if (!ctx->attr_union_set) {
         KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
         KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_find_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
@@ -1195,6 +1283,10 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     p.n_pat = h.n_pat;
     p.n_out = out.n;
     for (int r = 0; r < KMPB_MAX_OUT; r++) p.out[r] = out.vec[r];
+    p.gate = ctx->dev.gate;
+    p.gate_words = h.gate_words;
+    p.gate_shift = h.gate_shift;
+    p.gate_in_smem = gate_in_smem ? 1u : 0u;
     const uint32_t warps_needed = n_items;
     int grid = (int)std::min<uint32_t>((uint32_t)ctx->sm_count, (warps_needed + UN_WARPS - 1) / UN_WARPS);
     if (grid < 1) grid = 1;

@@ -478,6 +478,54 @@ static int build_verify_tables(kmpb_tables *t)
     return KMPB_OK;
 }
 
+/* ---- prefix gate ------------------------------------------------------------------------------ */
+
+#define GATE_MIN_WORDS 32u
+#define GATE_MAX_WORDS 1024u /* 4 KB: what is left of the block's shared memory next to the probe tables of a small set */
+#define GATE_WORDS_PER_KEY 16u
+
+uint32_t kmpb_gate_slot(uint32_t x, uint32_t shift) { return (x * KMPB_GATE_MUL) >> shift; }
+
+/* The resolve step's test of a start position before it becomes a candidate (union_kernel.cu, phase 1): the position's
+ * first two bytes pick a word, its third byte a bit.  Every pattern sets the bit of its own start, so the gate lets
+ * every true start through; what it rejects are the filter's false starts (the short patterns' buckets admit byte
+ * combinations no pattern has).  One word per 16 distinct two-byte keys or more (a one-byte pattern is 256 keys); when
+ * more than an eighth of the bits end up set, the gate would reject too little and is not built. */
+static int build_gate(kmpb_tables *t)
+{
+    uint32_t keys = 0, last = 0xffffffffu; /* distinct patterns are in content order: equal first two bytes are adjacent */
+    for (uint32_t u = 0; u < t->n_uniq; u++) {
+        const uint8_t *p = t->uniq_blob + t->uniq_off[u];
+        if (t->uniq_len[u] == 1) { keys += 256; continue; }
+        const uint32_t k = p[0] | (uint32_t)p[1] << 8;
+        keys += k != last;
+        last = k;
+    }
+    uint32_t log_w = 5;
+    while ((1u << log_w) < GATE_MAX_WORDS && (1u << log_w) < GATE_WORDS_PER_KEY * keys) log_w++;
+    const uint32_t words = 1u << log_w, shift = 32 - log_w;
+    uint32_t *g = calloc(words, sizeof *g);
+    if (!g) return kmpb_fail(KMPB_ENOMEM, "out of memory building the prefix gate");
+    for (uint32_t u = 0; u < t->n_uniq; u++) {
+        const uint8_t *p = t->uniq_blob + t->uniq_off[u];
+        const uint32_t len = t->uniq_len[u];
+        if (len == 1)
+            for (uint32_t c = 0; c < 256; c++) g[kmpb_gate_slot(p[0] | c << 8, shift)] = 0xffffffffu;
+        else
+            g[kmpb_gate_slot(p[0] | (uint32_t)p[1] << 8, shift)] |= len == 2 ? 0xffffffffu : 0x80000000u >> (p[2] & 31);
+    }
+    uint64_t set = 0;
+    for (uint32_t i = 0; i < words; i++) set += (uint64_t)__builtin_popcount(g[i]);
+    if (t->n_uniq == 0 || 8 * set > 32ull * words) {
+        free(g);
+        return KMPB_OK;
+    }
+    t->gate = g;
+    t->gate_words = words;
+    t->gate_shift = shift;
+    return KMPB_OK;
+}
+
 /* ---- entry points ----------------------------------------------------------------------------- */
 
 int kmpb_tables_build(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat)
@@ -546,6 +594,7 @@ int kmpb_tables_build_ex(kmpb_tables *t, const uint8_t *blob, const uint32_t *pa
 
     int rc = with_dfa ? build_dfa(t) : KMPB_OK;
     if (rc == KMPB_OK) rc = build_verify_tables(t);
+    if (rc == KMPB_OK) rc = build_gate(t);
     if (rc == KMPB_OK) rc = kmpb_filter6_build(t, t->filter6, &t->filter6_fp_estimate);
     free(uniq);
     if (rc != KMPB_OK) kmpb_tables_free(t);
@@ -564,5 +613,6 @@ void kmpb_tables_free(kmpb_tables *t)
     free(t->out_head);
     free(t->out_id);
     free(t->vtab);
+    free(t->gate);
     memset(t, 0, sizeof *t);
 }

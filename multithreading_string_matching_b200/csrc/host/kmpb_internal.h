@@ -65,6 +65,13 @@ typedef struct kmpb_tables {
      *   pattern words: every pattern zero-padded to a multiple of 4 bytes */
     uint32_t *vtab;
     uint32_t vtab_words;
+
+    /* prefix gate (automaton.c build_gate): a hashed bitmap that every position at which some pattern starts passes.
+     * Word kmpb_gate_slot(first two bytes, gate_shift) of a position; in it, a pattern of three and more bytes sets bit
+     * 31 - (third byte & 31), a two-byte pattern every bit, a one-byte pattern every bit of the words of all 256 second
+     * bytes.  gate_words = 0: no gate (too full to be worth its lookups: the resolve step re-runs the filter instead). */
+    uint32_t *gate;
+    uint32_t gate_words, gate_shift;
 } kmpb_tables;
 
 /* pcap_csr.c, used by the streamed savefile path (api.cu): end of the chunk of whole packets that starts at
@@ -79,6 +86,10 @@ uint64_t kmpb_pcap_first_long(const kmpb_pcap *pc, uint64_t first, uint64_t coun
 
 /* slot of a key (a text position's first two or three bytes) in a probe table (the device uses the same expression) */
 uint32_t kmpb_vtab_slot(uint32_t key, uint32_t shift);
+/* word of the prefix gate for a text position whose first bytes are the low bytes of x (only the low two matter: the
+ * multiplier's low 16 bits are zero, so the device hashes a whole text word without masking it) */
+#define KMPB_GATE_MUL 0x79b10000u
+uint32_t kmpb_gate_slot(uint32_t x, uint32_t shift);
 int kmpb_tables_build(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat);
 /* ... and, with_dfa != 0, the merged automaton of all patterns the table tests compare against (never uploaded) */
 int kmpb_tables_build_ex(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, int with_dfa);

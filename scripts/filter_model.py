@@ -1,7 +1,10 @@
 #!/usr/bin/env python3
 """CPU model of the union engine's prefilter: candidate and event rates of different filter geometries on
 the BASELINE workloads (no GPU).  A geometry = (depth, pattern buckets); a bucket's stage d passes the byte
-values some member has at depth d (every value when a member is shorter).  Usage: scripts/filter_model.py"""
+values some member has at depth d (every value when a member is shorter).  Usage: scripts/filter_model.py
+scripts/filter_model.py gate: the resolve step's prefix gate (automaton.c build_gate) on the C3 text -- candidates and
+verification rounds per resolve step with the filter re-run, with the gate in its place, and with both (compare with
+scripts/event_counts.py, which counts the same on a B200)."""
 import sys, os, itertools, random
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -166,3 +169,81 @@ def main2():
 
 if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "2":
     main2()
+
+
+GATE_MUL = 0x79B10000
+
+
+def gate_table(pats):
+    """automaton.c build_gate: (words, shift), or None when the gate would be too full to be built"""
+    u = sorted(set(pats))
+    keys = 256 * sum(len(p) == 1 for p in u) + len({p[:2] for p in u if len(p) >= 2})
+    log_w = 5
+    while (1 << log_w) < 1024 and (1 << log_w) < 16 * keys:
+        log_w += 1
+    shift = 32 - log_w
+    g = np.zeros(1 << log_w, dtype=np.uint64)
+    slot = lambda x: ((x * GATE_MUL) & 0xFFFFFFFF) >> shift
+    for p in u:
+        if len(p) == 1:
+            for c in range(256):
+                g[slot(p[0] | c << 8)] = 0xFFFFFFFF
+        else:
+            g[slot(p[0] | p[1] << 8)] |= 0xFFFFFFFF if len(p) == 2 else 0x80000000 >> (p[2] & 31)
+    if 8 * sum(bin(int(w)).count("1") for w in g) > 32 * len(g):
+        return None
+    return g.astype(np.uint32), shift
+
+
+def gate_model(text, A, depth, pats, gate):
+    """per KB: events, candidates of the filter re-run / of the gate on the reported quarters / of both, true starts;
+    verification rounds per resolve step (32 events, rounds of 32 candidates) = candidates per event"""
+    words, shift = gate
+    n = (len(text) - 40) // 32 * 32
+    t = text.astype(np.uint32)
+    c = A[0][text[:n]]
+    for d in range(1, depth):
+        c = c & A[d][text[d:d + n]]
+    cand = (c != 0).reshape(-1, 32)
+    nul = (text[:n] == 0).reshape(-1, 32)
+    rep = cand | nul
+    # the row loop's quarters: starts 0..8, 9..16, 17..24, 25..31; the gate tests those of each quarter that reported
+    qrep = np.stack([rep[:, 0:9].any(1), rep[:, 9:17].any(1), rep[:, 17:25].any(1), rep[:, 25:32].any(1)], 1)
+    win = np.zeros_like(cand)
+    for k in range(4):
+        win[:, (8 * k + 1 if k else 0):min(8 * k + 9, 32)] |= qrep[:, k:k + 1]
+    key = t[:n] | t[1:n + 1] << 8
+    slot = ((key.astype(np.uint64) * GATE_MUL) & 0xFFFFFFFF) >> shift
+    gate_ok = ((words[slot.astype(np.int64)] >> (31 - (t[2:n + 2] & 31))) & 1).astype(bool).reshape(-1, 32)
+    kb = n / 1024.0
+    ev = rep.any(1).sum()
+    now = (cand & win).sum()
+    alone = (gate_ok & win).sum()
+    both = (gate_ok & cand & win).sum()
+    import re
+    rx = re.compile(b"(?=(" + b"|".join(re.escape(p) for p in sorted(set(pats), key=len, reverse=True)) + b"))")
+    true = len({m.start() for m in rx.finditer(text[:n].tobytes())})
+    return dict(events=ev / kb, cand_rerun=now / kb, cand_gate=alone / kb, cand_both=both / kb, true_starts=true / kb,
+                rounds_rerun=now / ev, rounds_gate=alone / ev, rounds_both=both / ev)
+
+
+def main_gate(packets=8000):
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+    pats = [bytes(p) for p in M.load_patterns(os.path.join(root, "tests", "golden", "data", "strings.txt"))]
+    data, offsets = bench.synth_stream(0xB200, 0, packets, 1400, 2, pats)
+    text = np.frombuffer(bytes(data), dtype=np.uint8)
+    sp, bucket, _ = optimise(pats, 4, 5)
+    A = stage_tables(sp, bucket, 4, 5)
+    g = gate_table(pats)
+    print("gate: %d words, shift %d" % (len(g[0]), g[1]))
+    r = gate_model(text, A, 4, pats, g)
+    print("C3 (%d packets), per KB: events %.2f | candidates: filter re-run %.2f, gate %.2f, both %.2f, true starts %.2f"
+          % (packets, r["events"], r["cand_rerun"], r["cand_gate"], r["cand_both"], r["true_starts"]))
+    print("verification rounds per resolve step: filter re-run %.3f, gate %.3f, both %.3f"
+          % (r["rounds_rerun"], r["rounds_gate"], r["rounds_both"]))
+
+
+if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "gate":
+    main_gate()

@@ -25,6 +25,7 @@
  *   - a packet's text is payload[0 .. min(first NUL byte, payload_len))        serial.c:191
  *   - occurrences are counted with overlaps ("aa" in "aaaa" = 3)               serial.c:203-206
  *   - patterns are counted independently; duplicated patterns each get the count
+ *   - bytes are compared exactly, or after ASCII case folding for a KMPB_PAT_NOCASE pattern (kmpb_set_patterns_ex)
  *   - counts are 64-bit here (C int in the reference, serial.c:103).
  */
 #ifndef KMPB200_H
@@ -92,6 +93,20 @@ int kmpb_get_device(const kmpb_ctx *ctx);
  * the device, then expanded into the transition tables of both engines.  May be called again to
  * replace the set.  n_pat == 0 is valid (every count call then returns no counts). */
 int kmpb_set_patterns(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat);
+
+/* Per-pattern flags (kmpb_set_patterns_ex).  KMPB_PAT_NOCASE: the pattern matches at position k of a packet's text when
+ * fold(text[k+j]) == fold(p[j]) for every j, where fold maps A-Z (0x41-0x5A) to a-z and leaves every other byte as it
+ * is: no other pair of bytes that differ in bit 5 folds (@ `, [ {, \ |, ] }, ^ ~, _ DEL, and every byte >= 0x80: no
+ * locale, no Latin-1).  The text still ends at its first NUL, occurrences still overlap ("aA" nocase in "AaAa" = 3) and
+ * lie inside one packet.  Two patterns are the same distinct pattern iff they have the same flag and are equal, after
+ * folding when nocase, byte for byte when not: "Ack", "ACK" and "ack", all nocase, are one (each gets the full count,
+ * their find records carry the lowest file-order index of the three); "ack" case-sensitive and "ACK" nocase are two,
+ * and one text occurrence of "ack" yields a record for each.  kmpb_get_prefix of a nocase pattern returns the failure
+ * table of its folded form.  Every count and find form, the savefile pipeline and kmpb_stream_* honour the flags. */
+#define KMPB_PAT_NOCASE 1u
+/* kmpb_set_patterns with flags[n_pat], one byte per pattern; flags == NULL is exactly kmpb_set_patterns.  A bit other
+ * than KMPB_PAT_NOCASE is KMPB_EINVAL, naming the pattern. */
+int kmpb_set_patterns_ex(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, const uint8_t *flags);
 uint32_t kmpb_pattern_count(const kmpb_ctx *ctx);
 /* The device-built failure table of pattern i, copied back as the int[m] that kmp_prefix returns
  * (serial.c:217-238).  pi_out must hold m = pat_off[i+1]-pat_off[i] entries. */

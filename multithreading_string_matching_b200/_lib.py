@@ -12,6 +12,8 @@ c_u32p = ctypes.POINTER(ctypes.c_uint32)
 c_u64p = ctypes.POINTER(ctypes.c_uint64)
 c_i32p = ctypes.POINTER(ctypes.c_int32)
 
+KMPB_PAT_NOCASE = 1  # kmpb_set_patterns_ex: ASCII case-insensitive pattern
+
 
 class KmpbError(RuntimeError):
     def __init__(self, code, message):
@@ -46,6 +48,7 @@ SIGNATURES = {
     "kmpb_set_engine": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
     "kmpb_get_device": (ctypes.c_int, [ctypes.c_void_p]),
     "kmpb_set_patterns": (ctypes.c_int, [ctypes.c_void_p, c_u8p, c_u32p, ctypes.c_uint32]),
+    "kmpb_set_patterns_ex": (ctypes.c_int, [ctypes.c_void_p, c_u8p, c_u32p, ctypes.c_uint32, c_u8p]),
     "kmpb_pattern_count": (ctypes.c_uint32, [ctypes.c_void_p]),
     "kmpb_get_prefix": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint32, c_i32p, ctypes.c_uint32]),
     "kmpb_count_host": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, c_u64p]),

@@ -430,11 +430,16 @@ int kmpb_last_timing(const kmpb_ctx *ctx, double *ms_out, int n)
 
 int kmpb_set_patterns(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat)
 {
+    return kmpb_set_patterns_ex(ctx, blob, pat_off, n_pat, nullptr);
+}
+
+int kmpb_set_patterns_ex(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, const uint8_t *flags)
+{
     if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL context");
     int rc = use_device(ctx);
     if (rc) return rc;
     kmpb_tables fresh;
-    rc = kmpb_tables_build(&fresh, blob, pat_off, n_pat);
+    rc = kmpb_tables_build_flags(&fresh, blob, pat_off, n_pat, flags, 0);
     if (rc) return rc;
     KMPB_CUDA(cudaDeviceSynchronize());
     kmpb_release_tables(ctx);

@@ -24,6 +24,7 @@ struct kmpb_device_tables {
     uint8_t *uniq_blob = nullptr;   // [sum len]
     uint32_t *uniq_off = nullptr;   // [n_uniq+1]
     uint32_t *uniq_len = nullptr;   // [n_uniq]
+    uint8_t *uniq_flags = nullptr;  // [n_uniq] KMPB_PAT_NOCASE or 0
     uint32_t *pat_to_uniq = nullptr; // [n_pat]
     // per-pattern engine: failure tables and byte-indexed KMP DFAs, both built on the device
     int32_t *pi = nullptr;          // [sum len], pattern u at uniq_off[u]

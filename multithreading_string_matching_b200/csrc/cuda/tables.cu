@@ -32,18 +32,21 @@ __global__ void kmpb_build_prefix_kernel(const uint8_t *__restrict__ blob, const
 // One block per distinct pattern, one thread per byte value: column c of the pattern's DFA.
 // Entry = next state (0..m-1) | 0x80 when the transition completes the pattern; after a hit the
 // state drops to pi[m-1] exactly as kmp_matcher does (serial.c:203-206), so m states suffice.
+// A nocase pattern (flags[u], its bytes folded) reads the folded text: column c is column fold(c).
 __global__ void kmpb_expand_dfa_kernel(const uint8_t *__restrict__ blob, const uint32_t *__restrict__ off,
-                                       const int32_t *__restrict__ pi, uint8_t *__restrict__ dfa)
+                                       const uint8_t *__restrict__ flags, const int32_t *__restrict__ pi,
+                                       uint8_t *__restrict__ dfa)
 {
     uint32_t u = blockIdx.x;
     uint32_t c = threadIdx.x;
+    const uint32_t fc = (flags[u] & KMPB_PAT_NOCASE) && c >= 'A' && c <= 'Z' ? c + 32 : c;
     const uint8_t *p = blob + off[u];
     const int32_t *f = pi + off[u];
     uint8_t *rows = dfa + 256ull * off[u];
     int m = (int)(off[u + 1] - off[u]);
     for (int j = 0; j < m; j++) {
         uint8_t entry;
-        if (p[j] == c) entry = (j + 1 == m) ? (uint8_t)(f[m - 1] | 0x80) : (uint8_t)(j + 1);
+        if (p[j] == fc) entry = (j + 1 == m) ? (uint8_t)(f[m - 1] | 0x80) : (uint8_t)(j + 1);
         else entry = j == 0 ? 0 : rows[256 * f[j - 1] + c]; // mismatch: what the border state does on c
         rows[256 * j + c] = entry;
     }
@@ -60,7 +63,7 @@ static int upload(T **dst, const T *src, size_t n, cudaStream_t s)
 void kmpb_release_tables(kmpb_ctx *ctx)
 {
     kmpb_device_tables &d = ctx->dev;
-    cudaFree(d.uniq_blob); cudaFree(d.uniq_off); cudaFree(d.uniq_len); cudaFree(d.pat_to_uniq);
+    cudaFree(d.uniq_blob); cudaFree(d.uniq_off); cudaFree(d.uniq_len); cudaFree(d.uniq_flags); cudaFree(d.pat_to_uniq);
     cudaFree(d.pi); cudaFree(d.perpat_dfa); cudaFree(d.filter); cudaFree(d.vtab); cudaFree(d.gate); cudaFree(d.uniq_first);
     d = kmpb_device_tables();
     cudaFree(ctx->d_uniq_counts); ctx->d_uniq_counts = nullptr;
@@ -81,6 +84,7 @@ int kmpb_upload_tables(kmpb_ctx *ctx)
     if ((rc = upload(&d.uniq_blob, h.uniq_blob, blob_len, s))) return rc;
     if ((rc = upload(&d.uniq_off, h.uniq_off, (size_t)h.n_uniq + 1, s))) return rc;
     if ((rc = upload(&d.uniq_len, h.uniq_len, h.n_uniq, s))) return rc;
+    if ((rc = upload(&d.uniq_flags, h.uniq_flags, h.n_uniq, s))) return rc;
     if ((rc = upload(&d.pat_to_uniq, h.pat_to_uniq, h.n_pat, s))) return rc;
     if ((rc = upload(&d.vtab, h.vtab, (size_t)h.vtab_words, s))) return rc;
     if ((rc = upload(&d.filter, h.filter6, 256, s))) return rc;
@@ -101,7 +105,7 @@ int kmpb_upload_tables(kmpb_ctx *ctx)
     KMPB_CUDA(cudaMalloc((void **)&ctx->d_counts, (size_t)(h.n_pat ? h.n_pat : 1) * sizeof(uint64_t)));
     if (h.n_uniq) {
         kmpb_build_prefix_kernel<<<(h.n_uniq + 127) / 128, 128, 0, s>>>(d.uniq_blob, d.uniq_off, h.n_uniq, d.pi);
-        kmpb_expand_dfa_kernel<<<h.n_uniq, 256, 0, s>>>(d.uniq_blob, d.uniq_off, d.pi, d.perpat_dfa);
+        kmpb_expand_dfa_kernel<<<h.n_uniq, 256, 0, s>>>(d.uniq_blob, d.uniq_off, d.uniq_flags, d.pi, d.perpat_dfa);
         ctx->launches += 2;
         KMPB_CUDA(cudaGetLastError());
     }

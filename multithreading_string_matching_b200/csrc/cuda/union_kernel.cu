@@ -463,7 +463,10 @@ struct probe_consts {
 // table B (the longer ones); the slots' records carry the pattern's first 8 bytes and their masks, so a record costs one
 // 16-byte load and one masked compare, and only a record that agrees on those bytes is looked at further (patterns of
 // more than 8 bytes: word by word against the text in global memory -- L2, the row was read a moment ago).
-template <bool VS, bool EMIT>
+// NOCASE (the set has a nocase pattern, automaton.c): a nocase record's masks clear bit 5 at the pattern's letters, so
+// the masked compare is the case-insensitive one, and past byte 8 the record's tail masks (word 7, 0 = none) do the
+// same for the word-by-word compare; the nocase one-byte patterns have a second 256-word table after the first.
+template <bool VS, bool EMIT, bool NOCASE>
 __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_consts &pc, const uint32_t x0, const uint32_t x1,
                                             const uint32_t room, const uint64_t pos)
 {
@@ -479,6 +482,10 @@ __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_con
     if (vt_one) { // one-byte patterns: a direct table (room >= 1 always holds)
         const uint32_t u = vt(vt_one + (x0 & 0xffu));
         if (u != 0xffffffffu) hit<EMIT>(d, u, pos);
+        if (NOCASE) {
+            const uint32_t un = vt(vt_one + 256u + (x0 & 0xffu));
+            if (un != 0xffffffffu) hit<EMIT>(d, un, pos);
+        }
     }
     if (room < 2) return;
     uint2 ea = make_uint2(0, 0), eb = make_uint2(0, 0); // {first record, records}
@@ -499,10 +506,12 @@ __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_con
         bool same = true;
         if (m > 8) {
             const uint32_t pw0 = dc(DC_BLOB) + vt(r + 6);
+            const uint32_t tm = NOCASE ? vt(r + 7) : 0u;
             const uint8_t *g = dc_ptr(DC_TEXT_LO) + pos;
             for (uint32_t jj = 8; jj < m && same; jj += 4) { // pattern bytes jj..jj+3 against text bytes jj..
                 const uint32_t pw = vt(pw0 + (jj >> 2)), rem = m - jj;
-                const uint32_t diff = text_window(g + jj, rem) ^ pw;
+                uint32_t diff = text_window(g + jj, rem) ^ pw;
+                if (NOCASE && tm) diff &= vt(tm + (jj >> 2));
                 same = (rem >= 4 ? diff : diff & ((1u << (8 * rem)) - 1u)) == 0;
             }
         }
@@ -516,7 +525,7 @@ __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_con
 // free-running counters, slots handed out and slots verified.
 __device__ __forceinline__ uint32_t warp_c_sa() { return smem_sa() + UN_OFF_C + (threadIdx.x >> 5) * (UN_CCAP * UN_C_BYTES1); }
 // verify the n (<= 32) candidates from slot `head` on, one per lane
-template <bool EMIT>
+template <bool EMIT, bool NOCASE>
 __device__ __forceinline__ void verify_round(const drain_args &d, const uint32_t head, const uint32_t n)
 {
     const uint32_t lane = threadIdx.x & 31;
@@ -528,12 +537,12 @@ __device__ __forceinline__ void verify_round(const drain_args &d, const uint32_t
         pc.slots_a = c0.x; pc.shift_a = c0.y; pc.slots_b = c0.z; pc.shift_b = c0.w; pc.one = c1.x; pc.rec = c1.y;
         const uint4 e = lds128v(warp_c_sa() + ((head + lane) & (UN_CCAP - 1)) * UN_C_BYTES1);
         const uint64_t pos = ((uint64_t)(e.w >> 8) << 32) | e.z;
-        if (d.vtab_sa) verify_cand<true, EMIT>(d, pc, e.x, e.y, e.w & 0xffu, pos);
-        else verify_cand<false, EMIT>(d, pc, e.x, e.y, e.w & 0xffu, pos);
+        if (d.vtab_sa) verify_cand<true, EMIT, NOCASE>(d, pc, e.x, e.y, e.w & 0xffu, pos);
+        else verify_cand<false, EMIT, NOCASE>(d, pc, e.x, e.y, e.w & 0xffu, pos);
     }
 }
 // the candidates still waiting at the end of a batch
-template <bool EMIT>
+template <bool EMIT, bool NOCASE>
 __device__ __forceinline__ void flush_body()
 {
     drain_args d;
@@ -543,13 +552,15 @@ __device__ __forceinline__ void flush_body()
     d.counts_sa = dc(DC_COUNTS_SA);
     __syncwarp();
     const uint2 cs = lds64v(d.scratch_sa + SC_CAND); // {handed out, verified}: fewer than 32 apart between resolve steps
-    verify_round<EMIT>(d, cs.y, cs.x - cs.y);
+    verify_round<EMIT, NOCASE>(d, cs.y, cs.x - cs.y);
     __syncwarp();
     if ((threadIdx.x & 31) == 0) sts32v(d.scratch_sa + SC_CAND + 4, cs.x);
     __syncwarp();
 }
-__device__ __noinline__ void flush_candidates() { flush_body<false>(); }
-__device__ __noinline__ void flush_candidates_find() { flush_body<true>(); }
+__device__ __noinline__ void flush_candidates() { flush_body<false, false>(); }
+__device__ __noinline__ void flush_candidates_find() { flush_body<true, false>(); }
+__device__ __noinline__ void flush_candidates_nc() { flush_body<false, true>(); }
+__device__ __noinline__ void flush_candidates_find_nc() { flush_body<true, true>(); }
 
 // Phase 0 of a resolve step, on its own so that the row loop can issue it a row or two ahead: the n (<= 32) oldest
 // events' groups (32 B + 8 B lookahead), one per lane, from L2 (the rows were read a few microseconds ago) straight
@@ -589,7 +600,7 @@ __device__ __forceinline__ void drain_fetch(const uint32_t head, const uint32_t 
 // event carries its item's parity, and what the resolve step has to know about either item waits in the warp's
 // scratch words, where the warp put it when it took the item: no lane has to look anything up in global memory for
 // it, and the row loop does not keep it in registers.  Positions are relative to the item's row0 (32 bits).
-template <bool EMIT>
+template <bool EMIT, bool NOCASE>
 __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n)
 {
     drain_args d;
@@ -821,14 +832,14 @@ __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n
             ctail += __popc(any);
             __syncwarp();
             if (ctail - chead >= 32u) {
-                verify_round<EMIT>(d, chead, 32u);
+                verify_round<EMIT, NOCASE>(d, chead, 32u);
                 chead += 32u;
                 __syncwarp();
             }
         }
     }
     while (ctail - chead >= 32u) {
-        verify_round<EMIT>(d, chead, 32u);
+        verify_round<EMIT, NOCASE>(d, chead, 32u);
         chead += 32u;
     }
     __syncwarp();
@@ -841,12 +852,22 @@ __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n
 __device__ __noinline__ void drain_events(const uint32_t head, const uint32_t n)
 {
     drain_fetch(head, n);
-    drain_body<false>(head, n);
+    drain_body<false, false>(head, n);
 }
 __device__ __noinline__ void drain_events_find(const uint32_t head, const uint32_t n)
 {
     drain_fetch(head, n);
-    drain_body<true>(head, n);
+    drain_body<true, false>(head, n);
+}
+__device__ __noinline__ void drain_events_nc(const uint32_t head, const uint32_t n)
+{
+    drain_fetch(head, n);
+    drain_body<false, true>(head, n);
+}
+__device__ __noinline__ void drain_events_find_nc(const uint32_t head, const uint32_t n)
+{
+    drain_fetch(head, n);
+    drain_body<true, true>(head, n);
 }
 
 // NUL-dense row.  An event without candidates exists only to tell later candidates where the last NUL before them
@@ -867,9 +888,10 @@ __device__ __forceinline__ uint32_t uni(uint32_t v) { return __shfl_sync(FULL, v
 __device__ __forceinline__ uint64_t uni(uint64_t v) { return __shfl_sync(FULL, v, 0); }
 #undef DP_SEL
 #define DP_SEL(k) p.sel[k]
-// The kernel body, in two instantiations: the count kernel (EMIT = false) and the find kernel (EMIT = true), which
-// also writes a record per match; what it needs of the record buffer waits in the DC_* words, not in registers.
-template <bool EMIT>
+// The kernel body, in four instantiations: the count kernel (EMIT = false) and the find kernel (EMIT = true), which
+// also writes a record per match; what it needs of the record buffer waits in the DC_* words, not in registers.  Each
+// comes with NOCASE = true for pattern sets with a nocase pattern: only the verifier differs (verify_cand).
+template <bool EMIT, bool NOCASE>
 __device__ __forceinline__ void union_body(const union_params &__restrict__ p, const kmpb_find_out &__restrict__ fo)
 {
     uint32_t *lut = reinterpret_cast<uint32_t *>(smem);                      // L, then G
@@ -938,8 +960,13 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
     // resolve the oldest min(pending, 32) events (out of line: the rare places)
     auto resolve_oldest = [&]() {
         const uint32_t qn = pending(), n = qn < UN_QDRAIN ? qn : UN_QDRAIN;
-        if (EMIT) drain_events_find(oldest(), n);
-        else drain_events(oldest(), n);
+        if (NOCASE) {
+            if (EMIT) drain_events_find_nc(oldest(), n);
+            else drain_events_nc(oldest(), n);
+        } else {
+            if (EMIT) drain_events_find(oldest(), n);
+            else drain_events(oldest(), n);
+        }
         qs -= n;
     };
 
@@ -1102,7 +1129,7 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
             // loop, inlined (one copy of the code, and no call whose register needs the loop would have to respect).
             while ((qs & QS_FETCHED) || pending() >= 2 * UN_QDRAIN) {
                 if (!(qs & QS_FETCHED)) drain_fetch(oldest(), UN_QDRAIN);
-                drain_body<EMIT>(oldest(), UN_QDRAIN);
+                drain_body<EMIT, NOCASE>(oldest(), UN_QDRAIN);
                 qs = (qs & ~QS_FETCHED) - UN_QDRAIN;
                 if (lane == 0) { // that many fewer events of older items
                     const uint32_t older = lds32v(warp_scratch_sa() + SC_STATE + 4);
@@ -1141,8 +1168,13 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
     }
     // leftovers
     while (pending()) resolve_oldest();
-    if (EMIT) flush_candidates_find();
-    else flush_candidates();
+    if (NOCASE) {
+        if (EMIT) flush_candidates_find_nc();
+        else flush_candidates_nc();
+    } else {
+        if (EMIT) flush_candidates_find();
+        else flush_candidates();
+    }
 
     __syncthreads();
     if (p.counts_in_smem)
@@ -1171,13 +1203,24 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
 
 __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_kernel(const __grid_constant__ union_params p)
 {
-    union_body<false>(p, kmpb_find_out());
+    union_body<false, false>(p, kmpb_find_out());
 }
 
 __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_find_kernel(const __grid_constant__ union_params p,
                                                                         const __grid_constant__ kmpb_find_out fo)
 {
-    union_body<true>(p, fo);
+    union_body<true, false>(p, fo);
+}
+
+__global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_nocase_kernel(const __grid_constant__ union_params p)
+{
+    union_body<false, true>(p, kmpb_find_out());
+}
+
+__global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_find_nocase_kernel(const __grid_constant__ union_params p,
+                                                                               const __grid_constant__ kmpb_find_out fo)
+{
+    union_body<true, true>(p, fo);
 }
 
 // ---- host side ------------------------------------------------------------------------------------
@@ -1254,6 +1297,8 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     if (!ctx->attr_union_set) {
         KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
         KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_find_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
+        KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_nocase_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
+        KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_find_nocase_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
         ctx->attr_union_set = true;
     }
     kmpb_union_partition_kernel<<<(n_items + 1 + 255) / 256, 256, 0, stream>>>(b.d_offsets, (uint32_t)b.n_packets, n_items,
@@ -1291,8 +1336,15 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     int grid = (int)std::min<uint32_t>((uint32_t)ctx->sm_count, (warps_needed + UN_WARPS - 1) / UN_WARPS);
     if (grid < 1) grid = 1;
     if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[0], stream));
-    if (find) kmpb_union_find_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, *find);
-    else kmpb_union_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p);
+    // The kernel: count or find, and the nocase instantiation exactly when the set has a nocase pattern (its tables
+    // then have the layout the nocase verifier reads: the second one-byte table, tail masks).
+    if (h.n_nocase) {
+        if (find) kmpb_union_find_nocase_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, *find);
+        else kmpb_union_nocase_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p);
+    } else {
+        if (find) kmpb_union_find_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, *find);
+        else kmpb_union_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p);
+    }
     if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[1], stream));
     ctx->launches += 2;
     KMPB_CUDA(cudaGetLastError());

@@ -8,6 +8,11 @@
  * (build_verify_tables).  Counting every occurrence once at its start gives the numbers P independent
  * kmp_matcher calls give (overlapping occurrences are separate occurrences either way).
  *
+ * Case-insensitive patterns (KMPB_PAT_NOCASE, kmpb_tables_build_flags) are a matter of these tables alone: such a
+ * pattern is stored folded, admits both cases of its letters in the filter and the gate, is entered under every case
+ * variant of its probe key, and its records' masks clear bit 5 at its letters.  With every flag zero the tables are
+ * word for word those of kmpb_tables_build.
+ *
  * For the table tests only (kmpb_tables_build_ex with_dfa): the P KMP automata merged into one DFA over
  * the trie of all pattern prefixes -- state = longest suffix of the text read so far that is a prefix of
  * some pattern; for a single pattern exactly the automaton kmp_matcher steps through (j, with the drop
@@ -27,10 +32,17 @@
 /* ---- distinct patterns ------------------------------------------------------------------------ */
 
 typedef struct {
-    const uint8_t *p;
+    const uint8_t *p; /* folded when nc */
     uint32_t len, index;
+    uint32_t nc;      /* KMPB_PAT_NOCASE */
 } pat_ref;
 
+/* ASCII case folding (kmpb200.h): A-Z to a-z, every other byte as it is */
+static uint8_t fold(uint8_t c) { return c >= 'A' && c <= 'Z' ? (uint8_t)(c + 32) : c; }
+/* a byte of a folded nocase pattern that matches two text bytes: a lower-case letter (the other is c ^ 0x20) */
+static int folds(uint32_t nc, uint8_t c) { return nc && c >= 'a' && c <= 'z'; }
+
+/* distinct patterns are equal (bytes, flag); the order is content, then flag, then file order */
 static int cmp_content(const void *a, const void *b)
 {
     const pat_ref *x = a, *y = b;
@@ -38,6 +50,7 @@ static int cmp_content(const void *a, const void *b)
     int c = memcmp(x->p, y->p, n);
     if (c) return c;
     if (x->len != y->len) return x->len < y->len ? -1 : 1;
+    if (x->nc != y->nc) return x->nc < y->nc ? -1 : 1;
     return x->index < y->index ? -1 : (x->index > y->index);
 }
 
@@ -61,8 +74,10 @@ typedef struct {
 static void sets_add(bucket_sets *s, const pat_ref *r)
 {
     for (uint32_t d = 0; d < FILTER_DEPTH; d++) {
-        if (d < r->len) s->set[d][r->p[d] >> 6] |= 1ull << (r->p[d] & 63);
-        else s->open[d] = 1;
+        if (d < r->len) {
+            s->set[d][r->p[d] >> 6] |= 1ull << (r->p[d] & 63);
+            if (folds(r->nc, r->p[d])) s->set[d][(r->p[d] ^ 0x20) >> 6] |= 1ull << ((r->p[d] ^ 0x20) & 63);
+        } else s->open[d] = 1;
     }
 }
 
@@ -151,9 +166,11 @@ static void bag_change(bucket_bag *g, const pat_ref *r, int add)
 {
     for (uint32_t d = 0; d < FILTER_DEPTH; d++) {
         if (d >= r->len) { g->open[d] += add ? 1 : -1; continue; }
-        uint16_t *c = &g->count[d][r->p[d]];
-        if (add) { if ((*c)++ == 0) g->distinct[d]++; }
-        else if (--(*c) == 0) g->distinct[d]--;
+        for (int v = 0; v <= folds(r->nc, r->p[d]); v++) { /* a nocase letter: both cases */
+            uint16_t *c = &g->count[d][r->p[d] ^ (v ? 0x20 : 0)];
+            if (add) { if ((*c)++ == 0) g->distinct[d]++; }
+            else if (--(*c) == 0) g->distinct[d]--;
+        }
     }
     g->members += add ? 1 : -1;
 }
@@ -271,6 +288,7 @@ int kmpb_filter6_build(const kmpb_tables *t, uint32_t words[256], double *estima
         uniq[u].p = t->uniq_blob + t->uniq_off[u];
         uniq[u].len = t->uniq_len[u];
         uniq[u].index = u;
+        uniq[u].nc = t->uniq_flags ? t->uniq_flags[u] : 0u;
     }
     const double e = build_filter_words(t->n_uniq, uniq, N_BUCKET, 6, words);
     free(uniq);
@@ -284,24 +302,29 @@ int kmpb_filter6_build(const kmpb_tables *t, uint32_t words[256], double *estima
 
 /* ---- union automaton -------------------------------------------------------------------------- */
 
-static int build_dfa(kmpb_tables *t)
-{
-    /* byte classes */
-    int used[256] = {0};
-    for (uint32_t i = 0; i < t->uniq_off[t->n_uniq]; i++) used[t->uniq_blob[i]] = 1;
-    t->n_class = 1;
-    for (int c = 0; c < 256; c++) t->byte_class[c] = used[c] ? (uint8_t)t->n_class++ : 0;
-    if (t->n_class > 256) { /* all 256 byte values used: cannot happen (no NUL), but keep u8 safe */
-        return kmpb_fail(KMPB_ELIMIT, "pattern set uses every byte value");
-    }
-    const uint32_t nc = t->n_class;
-    uint64_t max_state = (uint64_t)t->uniq_off[t->n_uniq] + 1;
-    if (max_state * nc >= (1ull << 31))
-        return kmpb_fail(KMPB_ELIMIT, "pattern set too large: %llu trie states x %u byte classes exceeds 2^31 table entries",
-                         (unsigned long long)max_state, nc);
+/* The merged automaton of the distinct patterns with flag nc, over t's byte classes.  For nocase patterns (stored folded)
+ * the column of an upper-case letter is copied from its lower-case letter's: the automaton then reads fold(text). */
+typedef struct {
+    uint32_t n_state;
+    uint32_t *next, *trie, *term, *out_head, *out_id;
+} ac_automaton;
 
-    uint32_t *next = calloc((size_t)max_state * nc, sizeof *next); /* 0 = no child yet (root is never a child) */
-    uint32_t *term = malloc((size_t)max_state * sizeof *term);     /* uniq id ending at the state, or ~0 */
+static void ac_free(ac_automaton *a)
+{
+    free(a->next); free(a->trie); free(a->term); free(a->out_head); free(a->out_id);
+    memset(a, 0, sizeof *a);
+}
+
+static int ac_build(const kmpb_tables *t, uint32_t nc, ac_automaton *a)
+{
+    memset(a, 0, sizeof *a);
+    const uint32_t ncl = t->n_class;
+    uint64_t max_state = (uint64_t)t->uniq_off[t->n_uniq] + 1;
+    if (max_state * ncl >= (1ull << 31))
+        return kmpb_fail(KMPB_ELIMIT, "pattern set too large: %llu trie states x %u byte classes exceeds 2^31 table entries",
+                         (unsigned long long)max_state, ncl);
+    uint32_t *next = calloc((size_t)max_state * ncl, sizeof *next); /* 0 = no child yet (root is never a child) */
+    uint32_t *term = malloc((size_t)max_state * sizeof *term);      /* uniq id ending at the state, or ~0 */
     uint32_t *fail = calloc((size_t)max_state, sizeof *fail);
     uint32_t *queue = malloc((size_t)max_state * sizeof *queue);
     uint32_t *n_out = calloc((size_t)max_state, sizeof *n_out);
@@ -314,44 +337,55 @@ static int build_dfa(kmpb_tables *t)
     /* trie of all pattern prefixes */
     uint32_t n_state = 1;
     for (uint32_t u = 0; u < t->n_uniq; u++) {
+        if ((t->uniq_flags ? t->uniq_flags[u] : 0u) != nc) continue;
         uint32_t s = 0;
         for (uint32_t i = t->uniq_off[u]; i < t->uniq_off[u + 1]; i++) {
             uint32_t cls = t->byte_class[t->uniq_blob[i]];
-            if (next[(size_t)s * nc + cls] == 0) next[(size_t)s * nc + cls] = n_state++;
-            s = next[(size_t)s * nc + cls];
+            if (next[(size_t)s * ncl + cls] == 0) next[(size_t)s * ncl + cls] = n_state++;
+            s = next[(size_t)s * ncl + cls];
         }
         term[s] = u;
     }
+    /* nocase: an upper-case letter goes where its lower-case letter goes */
+    const uint8_t *bc = t->byte_class;
+#define AC_FOLD_COLUMNS(tab)                                                                                  \
+    if (nc)                                                                                                   \
+        for (uint32_t s_ = 0; s_ < n_state; s_++)                                                             \
+            for (int c_ = 'A'; c_ <= 'Z'; c_++)                                                               \
+                if (bc[c_] != bc[c_ + 32]) (tab)[(size_t)s_ * ncl + bc[c_]] = (tab)[(size_t)s_ * ncl + bc[c_ + 32]];
 
-    /* the bare trie (goto function only, 0 = no edge), kept for the device's start-anchored
-     * verification walk: bit 31 of an edge says a pattern ends at the child */
-    uint32_t *trie = malloc((size_t)n_state * nc * sizeof *trie);
+    /* the bare trie (goto function only, 0 = no edge), for the start-anchored walk of the table tests: bit 31 of an
+     * edge says a pattern ends at the child */
+    uint32_t *trie = malloc((size_t)n_state * ncl * sizeof *trie);
     if (!trie) {
         free(next); free(term); free(fail); free(queue); free(n_out);
         return kmpb_fail(KMPB_ENOMEM, "out of memory building the trie");
     }
-    for (size_t e = 0; e < (size_t)n_state * nc; e++)
+    for (size_t e = 0; e < (size_t)n_state * ncl; e++)
         trie[e] = next[e] ? (next[e] | (term[next[e]] != 0xffffffffu ? 0x80000000u : 0u)) : 0u;
+    AC_FOLD_COLUMNS(trie);
 
     /* breadth-first: failure link of a child = where the parent's failure state goes on the same
      * byte (the KMP "while j>0 && p[j]!=c: j=prefix[j-1]" loop, resolved once per (state, byte));
      * missing edges are filled with the failure state's edge, turning the trie into a full DFA */
     uint32_t head = 0, tail = 0;
-    for (uint32_t cls = 0; cls < nc; cls++)
+    for (uint32_t cls = 0; cls < ncl; cls++)
         if (next[cls]) queue[tail++] = next[cls]; /* depth-1 states fail to the root */
     while (head < tail) {
         uint32_t s = queue[head++];
         n_out[s] = (term[s] != 0xffffffffu) + n_out[fail[s]];
-        for (uint32_t cls = 0; cls < nc; cls++) {
-            uint32_t child = next[(size_t)s * nc + cls], via = next[(size_t)fail[s] * nc + cls];
+        for (uint32_t cls = 0; cls < ncl; cls++) {
+            uint32_t child = next[(size_t)s * ncl + cls], via = next[(size_t)fail[s] * ncl + cls];
             if (child) {
                 fail[child] = via;
                 queue[tail++] = child;
             } else {
-                next[(size_t)s * nc + cls] = via;
+                next[(size_t)s * ncl + cls] = via;
             }
         }
     }
+    AC_FOLD_COLUMNS(next);
+#undef AC_FOLD_COLUMNS
 
     /* outputs: own pattern first (the longest), then the failure chain's */
     uint32_t *out_head = malloc(((size_t)n_state + 1) * sizeof *out_head);
@@ -371,20 +405,111 @@ static int build_dfa(kmpb_tables *t)
     out_head[n_state] = at;
 
     /* "the target state reports something" flag in bit 31 */
-    for (size_t e = 0; e < (size_t)n_state * nc; e++) {
+    for (size_t e = 0; e < (size_t)n_state * ncl; e++) {
         uint32_t target = next[e];
         next[e] = target | (n_out[target] ? 0x80000000u : 0u);
     }
-    uint32_t *shrunk = realloc(next, (size_t)n_state * nc * sizeof *next);
-    t->next = shrunk ? shrunk : next;
-    t->n_state = n_state;
-    t->out_head = out_head;
-    t->out_id = out_id;
-    t->trie = trie;
+    uint32_t *shrunk = realloc(next, (size_t)n_state * ncl * sizeof *next);
+    a->next = shrunk ? shrunk : next;
+    a->n_state = n_state;
+    a->out_head = out_head;
+    a->out_id = out_id;
+    a->trie = trie;
     uint32_t *term_shrunk = realloc(term, (size_t)n_state * sizeof *term);
-    t->state_term = term_shrunk ? term_shrunk : term;
+    a->term = term_shrunk ? term_shrunk : term;
     free(fail); free(queue); free(n_out);
     return KMPB_OK;
+}
+
+/* A set of case-sensitive and nocase patterns: the product of the two automata (a state is the pair of their states,
+ * its outputs both lists).  Only the pairs reachable from the roots are kept.  There is no bare trie for such a set. */
+static int ac_product(const kmpb_tables *t, const ac_automaton *x, const ac_automaton *y, kmpb_tables *out)
+{
+    const uint32_t ncl = t->n_class;
+    const uint64_t pairs = (uint64_t)x->n_state * y->n_state;
+    if (pairs >= (1ull << 28)) return kmpb_fail(KMPB_ELIMIT, "mixed pattern set too large for the merged automaton");
+    uint32_t *id = calloc(pairs, sizeof *id); /* 1 + state of a pair, 0 = not reached yet */
+    uint32_t cap = 1024, n = 1;
+    uint32_t *px = malloc(cap * sizeof *px), *py = malloc(cap * sizeof *py);
+    uint32_t *next = malloc((size_t)cap * ncl * sizeof *next);
+    if (!id || !px || !py || !next) { free(id); free(px); free(py); free(next); return kmpb_fail(KMPB_ENOMEM, "out of memory"); }
+    px[0] = 0; py[0] = 0; id[0] = 1;
+    for (uint32_t s = 0; s < n; s++)
+        for (uint32_t cls = 0; cls < ncl; cls++) {
+            const uint32_t a = x->next[(size_t)px[s] * ncl + cls] & 0x7fffffffu, b = y->next[(size_t)py[s] * ncl + cls] & 0x7fffffffu;
+            uint32_t *slot = &id[(uint64_t)a * y->n_state + b];
+            if (*slot == 0) {
+                if (n == cap) {
+                    cap *= 2;
+                    uint32_t *nx = realloc(px, cap * sizeof *px), *ny = realloc(py, cap * sizeof *py);
+                    uint32_t *nn = realloc(next, (size_t)cap * ncl * sizeof *next);
+                    if (nx) px = nx;
+                    if (ny) py = ny;
+                    if (nn) next = nn;
+                    if (!nx || !ny || !nn) { free(id); free(px); free(py); free(next); return kmpb_fail(KMPB_ENOMEM, "out of memory"); }
+                }
+                px[n] = a; py[n] = b;
+                *slot = ++n;
+            }
+            next[(size_t)s * ncl + cls] = *slot - 1;
+        }
+    uint32_t *out_head = malloc(((size_t)n + 1) * sizeof *out_head);
+    uint64_t total = 0;
+    for (uint32_t s = 0; s < n; s++)
+        total += (x->out_head[px[s] + 1] - x->out_head[px[s]]) + (y->out_head[py[s] + 1] - y->out_head[py[s]]);
+    uint32_t *out_id = malloc((size_t)(total ? total : 1) * sizeof *out_id);
+    if (!out_head || !out_id) {
+        free(id); free(px); free(py); free(next); free(out_head); free(out_id);
+        return kmpb_fail(KMPB_ENOMEM, "out of memory");
+    }
+    uint32_t at = 0;
+    for (uint32_t s = 0; s < n; s++) {
+        out_head[s] = at;
+        for (uint32_t o = x->out_head[px[s]]; o < x->out_head[px[s] + 1]; o++) out_id[at++] = x->out_id[o];
+        for (uint32_t o = y->out_head[py[s]]; o < y->out_head[py[s] + 1]; o++) out_id[at++] = y->out_id[o];
+    }
+    out_head[n] = at;
+    for (size_t e = 0; e < (size_t)n * ncl; e++)
+        next[e] |= out_head[next[e] + 1] > out_head[next[e]] ? 0x80000000u : 0u;
+    free(id); free(px); free(py);
+    out->next = next;
+    out->n_state = n;
+    out->out_head = out_head;
+    out->out_id = out_id;
+    return KMPB_OK;
+}
+
+static int build_dfa(kmpb_tables *t)
+{
+    /* byte classes: every byte a pattern can match has its own (both cases of a nocase pattern's letters) */
+    int used[256] = {0};
+    uint32_t has[2] = {0, 0};
+    for (uint32_t u = 0; u < t->n_uniq; u++) {
+        const uint32_t nc = t->uniq_flags ? t->uniq_flags[u] : 0u;
+        has[nc] = 1;
+        for (uint32_t i = t->uniq_off[u]; i < t->uniq_off[u + 1]; i++) {
+            used[t->uniq_blob[i]] = 1;
+            if (folds(nc, t->uniq_blob[i])) used[t->uniq_blob[i] ^ 0x20] = 1;
+        }
+    }
+    t->n_class = 1;
+    for (int c = 0; c < 256; c++) t->byte_class[c] = used[c] ? (uint8_t)t->n_class++ : 0;
+    if (t->n_class > 256) { /* all 256 byte values used: cannot happen (no NUL), but keep u8 safe */
+        return kmpb_fail(KMPB_ELIMIT, "pattern set uses every byte value");
+    }
+    ac_automaton a[2];
+    int rc = ac_build(t, has[1] && !has[0] ? 1u : 0u, &a[0]);
+    if (rc) return rc;
+    if (!(has[0] && has[1])) { /* one kind of pattern: its automaton */
+        t->next = a[0].next; t->n_state = a[0].n_state; t->out_head = a[0].out_head; t->out_id = a[0].out_id;
+        t->trie = a[0].trie; t->state_term = a[0].term;
+        return KMPB_OK;
+    }
+    rc = ac_build(t, 1u, &a[1]);
+    if (rc == KMPB_OK) rc = ac_product(t, &a[0], &a[1], t);
+    ac_free(&a[0]);
+    ac_free(&a[1]);
+    return rc;
 }
 
 /* ---- start-anchored verification tables ---------------------------------------------------------- */
@@ -401,10 +526,10 @@ static uint32_t word_of(const uint8_t *p, uint32_t len, uint32_t from)
     for (uint32_t i = from; i < from + 4 && i < len; i++) k |= (uint32_t)p[i] << (8 * (i - from));
     return k;
 }
-static uint32_t mask_of(uint32_t len, uint32_t from)
+static uint32_t mask_of(const uint8_t *p, uint32_t len, uint32_t nc, uint32_t from)
 {
     uint32_t k = 0;
-    for (uint32_t i = from; i < from + 4 && i < len; i++) k |= 0xffu << (8 * (i - from));
+    for (uint32_t i = from; i < from + 4 && i < len; i++) k |= (folds(nc, p[i]) ? 0xdfu : 0xffu) << (8 * (i - from));
     return k;
 }
 
@@ -412,65 +537,116 @@ static uint32_t mask_of(uint32_t len, uint32_t from)
  * (the first three) */
 static uint32_t vt_key(const uint8_t *p, uint32_t len) { return word_of(p, len < 3 ? len : 3, 0); }
 
+/* The keys a text position that matches the pattern can have: the pattern's own, and for a nocase pattern every case
+ * variant of the letters among its key bytes (at most 8).  Returns how many; keys[0] is the pattern's own. */
+static uint32_t vt_keys(const uint8_t *p, uint32_t len, uint32_t nc, uint32_t keys[8])
+{
+    const uint32_t kl = len < 3 ? len : 3;
+    uint32_t n = 1;
+    keys[0] = vt_key(p, len);
+    for (uint32_t i = 0; i < kl; i++)
+        if (folds(nc, p[i]))
+            for (uint32_t j = 0, m = n; j < m; j++) keys[n++] = keys[j] ^ (0x20u << (8 * i));
+    return n;
+}
+
+/* The distinct probe-table slots of those keys (two case variants can hash to one slot: the pattern's record goes in
+ * once).  Returns how many. */
+static uint32_t vt_slots(const uint8_t *p, uint32_t len, uint32_t nc, uint32_t shift, uint32_t slots[8])
+{
+    uint32_t keys[8], n = 0;
+    const uint32_t nk = vt_keys(p, len, nc, keys);
+    for (uint32_t k = 0; k < nk; k++) {
+        const uint32_t s = kmpb_vtab_slot(keys[k], shift);
+        uint32_t j = 0;
+        while (j < n && slots[j] != s) j++;
+        if (j == n) slots[n++] = s;
+    }
+    return n;
+}
+
 static int build_verify_tables(kmpb_tables *t)
 {
-    /* Two probe tables, one slot per hash value of the key, at least four slots per pattern: most slots are empty and
+    /* Two probe tables, one slot per hash value of the key, at least four slots per key: most slots are empty and
      * most occupied slots hold the patterns of a single key.  Keying the longer patterns by three bytes instead of two
      * (round 1) cuts the longest chain of strings.txt from 6 records ("se..") to 3 ("htt", "por") -- a warp walks as
-     * many records as its longest chain. */
-    uint32_t n_a = 0, n_b = 0, n1 = 0, blob_words = 0;
+     * many records as its longest chain.  A nocase pattern is entered under every case variant of its key. */
+    uint32_t n_a = 0, n_b = 0, n1 = 0, blob_words = 0, mask_words = 0, keys[8];
     for (uint32_t u = 0; u < t->n_uniq; u++) {
-        if (t->uniq_len[u] >= 3) n_b++; else if (t->uniq_len[u] == 2) n_a++; else n1++;
-        blob_words += (t->uniq_len[u] + 3) / 4;
+        const uint8_t *p = t->uniq_blob + t->uniq_off[u];
+        const uint32_t len = t->uniq_len[u], nc = t->uniq_flags[u];
+        if (len >= 3) n_b += vt_keys(p, len, nc, keys); else if (len == 2) n_a += vt_keys(p, len, nc, keys); else n1++;
+        blob_words += (len + 3) / 4;
+        if (nc && len > 8) mask_words += (len + 3) / 4;
     }
     uint32_t log_a = 4, log_b = 6;
     while (log_a < 16 && (1u << log_a) < 4 * n_a) log_a++;
     while (log_b < 20 && (1u << log_b) < 4 * n_b) log_b++;
     const uint32_t slots_a = n_a ? 1u << log_a : 0, slots_b = n_b ? 1u << log_b : 0;
+    /* records: one per pattern and distinct slot */
+    uint32_t n_rec = 0, sl[8];
+    for (uint32_t u = 0; u < t->n_uniq; u++) {
+        const uint32_t len = t->uniq_len[u];
+        if (len >= 2) n_rec += vt_slots(t->uniq_blob + t->uniq_off[u], len, t->uniq_flags[u], len >= 3 ? 32 - log_b : 32 - log_a, sl);
+    }
     uint32_t at = VT_HEADER;
     const uint32_t slot_a_off = n_a ? at : 0;
     at += 2 * slots_a;
     const uint32_t slot_b_off = n_b ? at : 0;
     at += 2 * slots_b;
+    /* the one-byte table: 256 words of case-sensitive ids, then -- in a set with a nocase pattern -- 256 of nocase ids,
+     * so that `A` and nocase `a` can both claim byte `A` */
     const uint32_t one_off = n1 ? at : 0;
-    if (n1) at += 256;
+    if (n1) at += t->n_nocase ? 512 : 256;
     at = (at + 3u) & ~3u; /* records are read 16 bytes at a time */
     const uint32_t rec_off = at;
-    at += 8 * (n_a + n_b);
+    at += 8 * n_rec;
     const uint32_t blob_off = at;
     at += blob_words;
+    const uint32_t mask_off = at; /* the masks of the nocase patterns of more than 8 bytes, laid out like their words */
+    at += mask_words;
     uint32_t *v = calloc(at ? at : 1, sizeof *v);
     uint32_t *fill = calloc((size_t)slots_a + slots_b + 1, sizeof *fill);
     if (!v || !fill) { free(v); free(fill); return kmpb_fail(KMPB_ENOMEM, "out of memory building the verification tables"); }
     v[0] = at; v[1] = slot_a_off; v[2] = 32 - log_a; v[3] = slot_b_off; v[4] = 32 - log_b; v[5] = one_off;
     v[6] = rec_off; v[7] = blob_off;
-    for (uint32_t i = 0; n1 && i < 256; i++) v[one_off + i] = 0xffffffffu;
+    for (uint32_t i = 0; n1 && i < (t->n_nocase ? 512u : 256u); i++) v[one_off + i] = 0xffffffffu;
     /* chain lengths, then chain starts (records of one slot are contiguous; table A's records come first) */
     for (uint32_t u = 0; u < t->n_uniq; u++) {
         const uint8_t *p = t->uniq_blob + t->uniq_off[u];
         const uint32_t len = t->uniq_len[u];
-        if (len >= 3) v[slot_b_off + 2 * kmpb_vtab_slot(vt_key(p, len), 32 - log_b) + 1]++;
-        else if (len == 2) v[slot_a_off + 2 * kmpb_vtab_slot(vt_key(p, len), 32 - log_a) + 1]++;
+        if (len < 2) continue;
+        const uint32_t ns = vt_slots(p, len, t->uniq_flags[u], len >= 3 ? 32 - log_b : 32 - log_a, sl);
+        for (uint32_t k = 0; k < ns; k++) v[(len >= 3 ? slot_b_off : slot_a_off) + 2 * sl[k] + 1]++;
     }
     uint32_t first = 0;
     for (uint32_t s = 0; s < slots_a; s++) { v[slot_a_off + 2 * s] = first; first += v[slot_a_off + 2 * s + 1]; }
     for (uint32_t s = 0; s < slots_b; s++) { v[slot_b_off + 2 * s] = first; first += v[slot_b_off + 2 * s + 1]; }
-    uint32_t bw = 0;
+    uint32_t bw = 0, mw = 0;
     for (uint32_t u = 0; u < t->n_uniq; u++) {
         const uint8_t *p = t->uniq_blob + t->uniq_off[u];
-        const uint32_t len = t->uniq_len[u];
+        const uint32_t len = t->uniq_len[u], nc = t->uniq_flags[u];
         memcpy((uint8_t *)(v + blob_off + bw), p, len); /* rest of the last word stays zero */
+        /* a nocase pattern's masks clear bit 5 at its letters: the masked compare then accepts exactly the case
+         * variants (the only byte that differs from a letter in bit 5 alone is the same letter in the other case) */
+        const uint32_t tail = nc && len > 8 ? mask_off + mw : 0;
+        for (uint32_t w = 0; tail && w < (len + 3) / 4; w++) v[tail + w] = mask_of(p, len, nc, 4 * w);
         if (len >= 2) {
-            const uint32_t s = len >= 3 ? kmpb_vtab_slot(vt_key(p, len), 32 - log_b) : kmpb_vtab_slot(vt_key(p, len), 32 - log_a);
-            const uint32_t so = len >= 3 ? slot_b_off : slot_a_off, fi = len >= 3 ? slots_a + s : s;
-            uint32_t *rec = v + rec_off + 8 * (v[so + 2 * s] + fill[fi]++);
-            rec[0] = word_of(p, len, 0); rec[1] = mask_of(len, 0);
-            rec[2] = word_of(p, len, 4); rec[3] = mask_of(len, 4);
-            rec[4] = len; rec[5] = u; rec[6] = bw; rec[7] = 0;
+            const uint32_t so = len >= 3 ? slot_b_off : slot_a_off, fo = len >= 3 ? slots_a : 0;
+            const uint32_t ns = vt_slots(p, len, nc, len >= 3 ? 32 - log_b : 32 - log_a, sl);
+            for (uint32_t k = 0; k < ns; k++) {
+                uint32_t *rec = v + rec_off + 8 * (v[so + 2 * sl[k]] + fill[fo + sl[k]]++);
+                rec[0] = word_of(p, len, 0); rec[1] = mask_of(p, len, nc, 0);
+                rec[2] = word_of(p, len, 4); rec[3] = mask_of(p, len, nc, 4);
+                rec[4] = len; rec[5] = u; rec[6] = bw; rec[7] = tail;
+            }
+        } else if (folds(nc, p[0])) {
+            v[one_off + 256 + p[0]] = v[one_off + 256 + (p[0] ^ 0x20)] = u;
         } else {
-            v[one_off + p[0]] = u;
+            v[one_off + (nc ? 256 : 0) + p[0]] = u;
         }
         bw += (len + 3) / 4;
+        if (tail) mw += (len + 3) / 4;
     }
     free(fill);
     t->vtab = v;
@@ -496,7 +672,9 @@ static int build_gate(kmpb_tables *t)
     uint32_t keys = 0, last = 0xffffffffu; /* distinct patterns are in content order: equal first two bytes are adjacent */
     for (uint32_t u = 0; u < t->n_uniq; u++) {
         const uint8_t *p = t->uniq_blob + t->uniq_off[u];
-        if (t->uniq_len[u] == 1) { keys += 256; continue; }
+        const uint32_t nc = t->uniq_flags[u];
+        if (t->uniq_len[u] == 1) { keys += 256u << folds(nc, p[0]); continue; }
+        if (nc) { keys += 1u << (folds(nc, p[0]) + folds(nc, p[1])); continue; } /* its case variants */
         const uint32_t k = p[0] | (uint32_t)p[1] << 8;
         keys += k != last;
         last = k;
@@ -508,11 +686,18 @@ static int build_gate(kmpb_tables *t)
     if (!g) return kmpb_fail(KMPB_ENOMEM, "out of memory building the prefix gate");
     for (uint32_t u = 0; u < t->n_uniq; u++) {
         const uint8_t *p = t->uniq_blob + t->uniq_off[u];
-        const uint32_t len = t->uniq_len[u];
-        if (len == 1)
-            for (uint32_t c = 0; c < 256; c++) g[kmpb_gate_slot(p[0] | c << 8, shift)] = 0xffffffffu;
-        else
-            g[kmpb_gate_slot(p[0] | (uint32_t)p[1] << 8, shift)] |= len == 2 ? 0xffffffffu : 0x80000000u >> (p[2] & 31);
+        const uint32_t len = t->uniq_len[u], nc = t->uniq_flags[u];
+        /* a nocase pattern sets the bits of every case variant of its first two bytes; the bit, third byte & 31, is the
+         * same for both cases of a letter */
+        for (uint32_t v0 = 0; v0 <= (uint32_t)folds(nc, p[0]); v0++) {
+            const uint32_t b0 = p[0] ^ (v0 << 5);
+            if (len == 1) {
+                for (uint32_t c = 0; c < 256; c++) g[kmpb_gate_slot(b0 | c << 8, shift)] = 0xffffffffu;
+                continue;
+            }
+            for (uint32_t v1 = 0; v1 <= (uint32_t)folds(nc, p[1]); v1++)
+                g[kmpb_gate_slot(b0 | (uint32_t)(p[1] ^ (v1 << 5)) << 8, shift)] |= len == 2 ? 0xffffffffu : 0x80000000u >> (p[2] & 31);
+        }
     }
     uint64_t set = 0;
     for (uint32_t i = 0; i < words; i++) set += (uint64_t)__builtin_popcount(g[i]);
@@ -530,12 +715,19 @@ static int build_gate(kmpb_tables *t)
 
 int kmpb_tables_build(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat)
 {
-    return kmpb_tables_build_ex(t, blob, pat_off, n_pat, 0);
+    return kmpb_tables_build_flags(t, blob, pat_off, n_pat, NULL, 0);
+}
+
+int kmpb_tables_build_ex(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, int with_dfa)
+{
+    return kmpb_tables_build_flags(t, blob, pat_off, n_pat, NULL, with_dfa);
 }
 
 /* with_dfa != 0 also builds the merged automaton of all patterns (next / trie / out_*): the reference the table tests
- * check the filter and the verification tables against.  The device never sees it, so the library does not build it. */
-int kmpb_tables_build_ex(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, int with_dfa)
+ * check the filter and the verification tables against.  The device never sees it, so the library does not build it.
+ * flags[n_pat] (NULL: all zero) holds each pattern's KMPB_PAT_* bits. */
+int kmpb_tables_build_flags(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat,
+                            const uint8_t *flags, int with_dfa)
 {
     memset(t, 0, sizeof *t);
     if (n_pat && (blob == NULL || pat_off == NULL)) return kmpb_fail(KMPB_EINVAL, "kmpb_set_patterns: NULL pattern data");
@@ -555,32 +747,49 @@ int kmpb_tables_build_ex(kmpb_tables *t, const uint8_t *blob, const uint32_t *pa
             free(refs); kmpb_tables_free(t);
             return kmpb_fail(KMPB_EINVAL, "pattern %u contains a NUL byte", i);
         }
+        if (flags && (flags[i] & ~KMPB_PAT_NOCASE)) {
+            free(refs); kmpb_tables_free(t);
+            return kmpb_fail(KMPB_EINVAL, "pattern %u has unknown flag bits 0x%02x", i, flags[i] & ~KMPB_PAT_NOCASE);
+        }
         refs[i].p = blob + pat_off[i];
         refs[i].len = len;
         refs[i].index = i;
+        refs[i].nc = flags ? flags[i] & KMPB_PAT_NOCASE : 0u;
         blob_len += len;
+    }
+    /* nocase patterns are matched in their folded form */
+    uint8_t *folded = malloc(blob_len ? blob_len : 1);
+    if (!folded) { free(refs); kmpb_tables_free(t); return kmpb_fail(KMPB_ENOMEM, "out of memory"); }
+    for (uint64_t i = 0, at = 0; i < n_pat; at += refs[i].len, i++) {
+        for (uint32_t k = 0; k < refs[i].len; k++) folded[at + k] = refs[i].nc ? fold(refs[i].p[k]) : refs[i].p[k];
+        refs[i].p = folded + at;
     }
     /* distinct patterns, numbered in content order */
     qsort(refs, n_pat, sizeof *refs, cmp_content);
     t->uniq_off = malloc(((size_t)n_pat + 1) * sizeof *t->uniq_off);
     t->uniq_len = malloc(((size_t)n_pat + 1) * sizeof *t->uniq_len);
+    t->uniq_flags = calloc((size_t)n_pat + 1, 1);
     t->uniq_blob = malloc(blob_len ? blob_len : 1);
     pat_ref *uniq = malloc(((size_t)n_pat + 1) * sizeof *uniq);
-    if (!t->uniq_off || !t->uniq_len || !t->uniq_blob || !uniq) {
-        free(refs); free(uniq); kmpb_tables_free(t);
+    if (!t->uniq_off || !t->uniq_len || !t->uniq_flags || !t->uniq_blob || !uniq) {
+        free(refs); free(uniq); free(folded); kmpb_tables_free(t);
         return kmpb_fail(KMPB_ENOMEM, "out of memory");
     }
     uint32_t nu = 0, at = 0;
     t->min_len = n_pat ? KMPB_MAX_PATTERN_LEN : 0;
     for (uint32_t i = 0; i < n_pat; i++) {
-        int same = i > 0 && refs[i].len == refs[i - 1].len && memcmp(refs[i].p, refs[i - 1].p, refs[i].len) == 0;
+        int same = i > 0 && refs[i].len == refs[i - 1].len && refs[i].nc == refs[i - 1].nc &&
+                   memcmp(refs[i].p, refs[i - 1].p, refs[i].len) == 0;
         if (!same) {
             t->uniq_off[nu] = at;
             t->uniq_len[nu] = refs[i].len;
+            t->uniq_flags[nu] = (uint8_t)refs[i].nc;
+            t->n_nocase += refs[i].nc;
             memcpy(t->uniq_blob + at, refs[i].p, refs[i].len);
             uniq[nu].p = t->uniq_blob + at;
             uniq[nu].len = refs[i].len;
             uniq[nu].index = nu;
+            uniq[nu].nc = refs[i].nc;
             at += refs[i].len;
             nu++;
             if (refs[i].len > t->max_len) t->max_len = refs[i].len;
@@ -591,6 +800,7 @@ int kmpb_tables_build_ex(kmpb_tables *t, const uint8_t *blob, const uint32_t *pa
     t->uniq_off[nu] = at;
     t->n_uniq = nu;
     free(refs);
+    free(folded);
 
     int rc = with_dfa ? build_dfa(t) : KMPB_OK;
     if (rc == KMPB_OK) rc = build_verify_tables(t);
@@ -607,6 +817,7 @@ void kmpb_tables_free(kmpb_tables *t)
     free(t->uniq_len);
     free(t->uniq_off);
     free(t->uniq_blob);
+    free(t->uniq_flags);
     free(t->next);
     free(t->trie);
     free(t->state_term);

@@ -1,6 +1,7 @@
 /* find_main.c -- kmp_find: where the patterns of a strings file occur in a savefile, one line per match.
  *
  *   kmp_find <file.pcap> <string.txt> [udp|tcp]
+ *   kmp_find -i <file.pcap> <string.txt> [udp|tcp]     every token case-insensitive (ASCII letters, KMPB_PAT_NOCASE)
  *
  * stdout: "<frame> <offset> <pattern>\n" per match, ordered by (frame, offset, pattern index): frame is the 1-based
  * capture record number (the numbering Wireshark shows), offset the position of the match's first byte inside the
@@ -25,6 +26,11 @@ int main(int argc, char **argv)
 {
     const char *prog = "./kmp_find";
     int proto = KMPB_PROTO_UDP;
+    const int nocase = argc > 1 && strcmp(argv[1], "-i") == 0; /* then the arguments follow as without it */
+    if (nocase) {
+        argv++;
+        argc--;
+    }
     if (argc < 3 || argc > 4) {
         printf("USAGE: %s <file.pcap> <string.txt> [tcp/udp]\n", prog);
         return 1;
@@ -59,7 +65,11 @@ int main(int argc, char **argv)
     }
     kmpb_ctx *ctx = NULL;
     if (kmpb_create(&ctx, kmpb_device_ordinal(0)) != 0) return fail("GPU");
-    if (kmpb_set_patterns(ctx, pats.blob, pats.pat_off, pats.n_pat) != 0) return fail("patterns");
+    uint8_t *flags = nocase ? malloc(pats.n_pat ? pats.n_pat : 1) : NULL;
+    if (flags) memset(flags, KMPB_PAT_NOCASE, pats.n_pat);
+    rc = kmpb_set_patterns_ex(ctx, pats.blob, pats.pat_off, pats.n_pat, flags);
+    free(flags);
+    if (rc != 0) return fail("patterns");
 
     /* a guess first (C3-like traffic has one match per ~400 payload bytes), then the exact size if it was short */
     const uint64_t n_packets = kmpb_pcap_packets(pc);

@@ -25,7 +25,9 @@ typedef struct kmpb_tables {
     uint32_t *pat_to_uniq;   /* [n_pat] */
     uint32_t *uniq_len;      /* [n_uniq] */
     uint32_t *uniq_off;      /* [n_uniq+1] into uniq_blob */
-    uint8_t *uniq_blob;
+    uint8_t *uniq_blob;      /* a nocase pattern's bytes are folded (A-Z to a-z) */
+    uint8_t *uniq_flags;     /* [n_uniq] KMPB_PAT_NOCASE or 0: part of a distinct pattern's identity */
+    uint32_t n_nocase;       /* distinct nocase patterns (non-zero: the union engine runs its nocase kernels) */
     uint32_t max_len, min_len;
 
     /* byte classes: bytes that occur in no pattern share class 0 */
@@ -33,7 +35,8 @@ typedef struct kmpb_tables {
     uint8_t byte_class[256];
 
     /* union DFA: next[state * n_class + class] = target state, bit 31 set when the target state
-     * reports at least one pattern */
+     * reports at least one pattern.  It reads the text as it is; a nocase pattern's upper-case letters go where its
+     * lower-case ones go.  A set of both kinds gets the product of the two kinds' automata, and no bare trie. */
     uint32_t n_state;
     uint32_t *next;          /* [n_state * n_class] */
     /* the same states as a bare trie: trie[state * n_class + class] = child (0 = none), bit 31 set when
@@ -58,18 +61,23 @@ typedef struct kmpb_tables {
      *   [0] total words
      *   [1] word offset of the slots of A (0 = no two-byte patterns)   [2] hash shift of A (slots = 1 << (32 - shift))
      *   [3] word offset of the slots of B (0 = none)                   [4] hash shift of B
-     *   [5] word offset of the one-byte patterns' table (256 words: distinct id or 0xffffffff), 0 = there are none
+     *   [5] word offset of the one-byte patterns' table (256 words: distinct id or 0xffffffff, by text byte), 0 = there
+     *       are none; in a set with a nocase pattern 512 words, the second 256 for the nocase one-byte patterns
      *   [6] word offset of the records   [7] word offset of the pattern words
      *   records (8 words, 16-byte aligned): {pattern bytes 0..3, mask of those that exist, bytes 4..7, their mask,
-     *            length, distinct id, word offset of the pattern's bytes inside the pattern words, 0}
-     *   pattern words: every pattern zero-padded to a multiple of 4 bytes */
+     *            length, distinct id, word offset of the pattern's bytes inside the pattern words, tail masks}
+     *   pattern words: every pattern zero-padded to a multiple of 4 bytes
+     *   tail masks: for a nocase pattern of more than 8 bytes, one mask word per pattern word (0xdf at its letters, 0xff
+     *            at its other bytes, 0 past its end); the record's last word is their vtab word offset, else 0.
+     * A nocase pattern is stored folded, its masks clear bit 5 at its letters, and it has a record in the slot of every
+     * case variant of its key (up to 4 in A, 8 in B; once per distinct slot). */
     uint32_t *vtab;
     uint32_t vtab_words;
 
     /* prefix gate (automaton.c build_gate): a hashed bitmap that every position at which some pattern starts passes.
      * Word kmpb_gate_slot(first two bytes, gate_shift) of a position; in it, a pattern of three and more bytes sets bit
      * 31 - (third byte & 31), a two-byte pattern every bit, a one-byte pattern every bit of the words of all 256 second
-     * bytes.  gate_words = 0: no gate (too full to be worth its lookups: the resolve step re-runs the filter instead). */
+     * bytes; a nocase pattern does so for every case variant of its first two bytes.  gate_words = 0: no gate (too full to be worth its lookups: the resolve step re-runs the filter instead). */
     uint32_t *gate;
     uint32_t gate_words, gate_shift;
 } kmpb_tables;
@@ -93,6 +101,9 @@ uint32_t kmpb_gate_slot(uint32_t x, uint32_t shift);
 int kmpb_tables_build(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat);
 /* ... and, with_dfa != 0, the merged automaton of all patterns the table tests compare against (never uploaded) */
 int kmpb_tables_build_ex(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, int with_dfa);
+/* ... with per-pattern KMPB_PAT_* flags[n_pat] (NULL = all zero, which builds word for word what kmpb_tables_build does) */
+int kmpb_tables_build_flags(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat,
+                            const uint8_t *flags, int with_dfa);
 /* the prefilter words (5 pattern buckets + NUL in 6-bit fields, depth 4 + a lingering field): automaton.c */
 int kmpb_filter6_build(const kmpb_tables *t, uint32_t words[256], double *estimate);
 void kmpb_tables_free(kmpb_tables *t);

@@ -3,6 +3,9 @@
  *   kmp_match <file.pcap> <string.txt> [udp|tcp]            serial.c:3,33-51
  *   kmp_match <file.pcap> <string.txt> <n> [tcp|udp]        openmp_data.c:2,35-54; <n> = number of
  *                                                           GPUs (the reference's thread count)
+ *   kmp_match -i <file.pcap> <string.txt> [n] [udp|tcp]     every token case-insensitive (ASCII letters,
+ *                                                           KMPB_PAT_NOCASE); the report lists each token as
+ *                                                           the strings file spells it
  *
  * stdout is the reference's, byte for byte (serial.c:163-169): header line, one "pattern: N times!"
  * line per pattern with a non-zero count in file order, then "Elapsed time = %f seconds" -- the
@@ -43,6 +46,7 @@ typedef struct {
     int device; /* CUDA ordinal */
     int rank;   /* which share of the packets */
     const kmpb_patterns *pats;
+    const uint8_t *flags; /* per-pattern KMPB_PAT_* flags, NULL = none */
     ingest_gate *gate;
     uint64_t *counts;
     double start;
@@ -58,7 +62,7 @@ static void *run_shard(void *arg)
     shard_job *job = arg;
     kmpb_ctx *ctx = NULL;
     job->rc = kmpb_create(&ctx, job->device);
-    if (job->rc == 0) job->rc = kmpb_set_patterns(ctx, job->pats->blob, job->pats->pat_off, job->pats->n_pat);
+    if (job->rc == 0) job->rc = kmpb_set_patterns_ex(ctx, job->pats->blob, job->pats->pat_off, job->pats->n_pat, job->flags);
     if (job->rc == 0) job->rc = kmpb_reserve_staging(ctx, 0, 0); /* pinned staging, while the main thread frames the savefile */
     if (job->rc != 0) snprintf(job->err, sizeof job->err, "%s", kmpb_last_error());
     if (getenv("KMPB_STATS")) fprintf(stderr, "kmp_match: GPU %d context, pattern tables and staging buffers ready %.3f s after start\n", job->device, now_seconds() - job->start);
@@ -80,6 +84,11 @@ int main(int argc, char **argv)
 {
     int proto = KMPB_PROTO_UDP, n_gpus = 1, openmp_form = 0;
     const char *prog = "./kmp_match";
+    const int nocase = argc > 1 && strcmp(argv[1], "-i") == 0; /* then the arguments follow as without it */
+    if (nocase) {
+        argv++;
+        argc--;
+    }
     if (argc >= 4 && strcmp(argv[3], "udp") != 0 && strcmp(argv[3], "tcp") != 0 && atoi(argv[3]) > 0) openmp_form = 1;
     const char *usage_colon = openmp_form ? "USAGE: %s <file.pcap> <string.txt> gpu_number [tcp/udp]\n"
                                           : "USAGE: %s <file.pcap> <string.txt> [tcp/udp]\n";
@@ -117,6 +126,8 @@ int main(int argc, char **argv)
         return 1;
     }
     if (n_gpus > available) n_gpus = available;
+    uint8_t *flags = nocase ? malloc(pats.n_pat ? pats.n_pat : 1) : NULL;
+    if (flags) memset(flags, KMPB_PAT_NOCASE, pats.n_pat);
 
     double start = now_seconds();
     ingest_gate gate;
@@ -132,6 +143,7 @@ int main(int argc, char **argv)
         jobs[g].device = kmpb_device_ordinal(g); /* the g-th usable GPU, whatever else the box holds */
         jobs[g].rank = g;
         jobs[g].pats = &pats;
+        jobs[g].flags = flags;
         jobs[g].gate = &gate;
         jobs[g].start = start;
         jobs[g].counts = calloc(pats.n_pat ? pats.n_pat : 1, sizeof(uint64_t));
@@ -179,6 +191,7 @@ int main(int argc, char **argv)
     free(jobs);
     free(threads);
     free(counts);
+    free(flags);
     kmpb_pcap_close(pc);
     kmpb_free_patterns(&pats);
     return 0;

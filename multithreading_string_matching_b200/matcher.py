@@ -13,7 +13,7 @@ import tempfile
 import numpy as np
 
 from . import _lib
-from ._lib import CCsr, CPatterns, CSynth, KmpbError, c_i32p, c_u8p, c_u32p, c_u64p, check, lib
+from ._lib import KMPB_PAT_NOCASE, CCsr, CPatterns, CSynth, KmpbError, c_i32p, c_u8p, c_u32p, c_u64p, check, lib
 
 ENGINE_AUTO, ENGINE_PERPAT, ENGINE_UNION = 0, 1, 2
 PROTO_UDP, PROTO_TCP = 0, 1
@@ -121,6 +121,7 @@ class Matcher:
         check(lib().kmpb_create(ctypes.byref(self._ctx), device))
         self.device = device
         self.patterns = []
+        self.nocase = []
         self.set_engine(engine)
 
     def close(self):
@@ -147,12 +148,22 @@ class Matcher:
     def set_engine(self, engine):
         check(lib().kmpb_set_engine(self._ctx, _ENGINE[engine]))
 
-    def set_patterns(self, patterns):
-        """serial.c:148-152: builds the failure tables (on the device) for the whole set."""
+    def set_patterns(self, patterns, nocase=False):
+        """serial.c:148-152: builds the failure tables (on the device) for the whole set.  nocase: True makes every
+        pattern case-insensitive (ASCII letters only, KMPB_PAT_NOCASE), a sequence of len(patterns) bools each one."""
         patterns = [bytes(p) for p in patterns]
+        if isinstance(nocase, (bool, np.bool_)):
+            nocase = [bool(nocase)] * len(patterns)
+        else:
+            nocase = [bool(x) for x in nocase]
+            if len(nocase) != len(patterns):
+                raise ValueError("nocase has %d entries for %d patterns" % (len(nocase), len(patterns)))
         blob, off = pack_patterns(patterns)
-        check(lib().kmpb_set_patterns(self._ctx, blob.ctypes.data_as(c_u8p), off.ctypes.data_as(c_u32p), len(patterns)))
+        flags = np.array([KMPB_PAT_NOCASE if x else 0 for x in nocase] or [0], dtype=np.uint8)
+        check(lib().kmpb_set_patterns_ex(self._ctx, blob.ctypes.data_as(c_u8p), off.ctypes.data_as(c_u32p), len(patterns),
+                                         flags.ctypes.data_as(c_u8p) if any(nocase) else None))
         self.patterns = patterns
+        self.nocase = nocase
 
     def prefix(self, index):
         """The device-built failure table of pattern `index`, as kmp_prefix returns it (serial.c:217-238)."""

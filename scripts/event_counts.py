@@ -3,7 +3,8 @@
 verification rounds, per KB of payload and per resolve step.  Builds the library with the diagnostic counters
 (EXTRA_NVFLAGS=-DKMPB_UN_STATS, absent from the production build) into a temporary directory, so the tree is left as
 it is.  scripts/filter_model.py gate models the same numbers on the CPU.
-Usage: scripts/event_counts.py [--packets N] [--flags "-DKMPB_UN_GATE_AND"]"""
+With --nocase every token of strings.txt is case-insensitive (KMPB_PAT_NOCASE).
+Usage: scripts/event_counts.py [--packets N] [--flags "-DKMPB_UN_GATE_AND"] [--nocase]"""
 import argparse, ctypes, json, os, shutil, subprocess, sys, tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,6 +15,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--packets", type=int, default=2_000_000, help="C3 packets of 1400 bytes")
     ap.add_argument("--flags", default="", help="more nvcc flags for the diagnostic build")
+    ap.add_argument("--nocase", action="store_true", help="every pattern case-insensitive")
     args = ap.parse_args()
     tmp = tempfile.mkdtemp(prefix="kmpb_stats_")
     try:
@@ -31,7 +33,7 @@ def main():
         L.kmpb_union_stats.argtypes = [ctypes.POINTER(ctypes.c_uint64), ctypes.c_int]
         pats = kmp.load_patterns(os.path.join(ROOT, "tests", "golden", "data", "strings.txt"))
         m = kmp.Matcher(0, engine="union")
-        m.set_patterns(pats)
+        m.set_patterns(pats, nocase=args.nocase)
         synth = kmp.Synth(seed=0xB200, payload_len=1400, plants=2, plant_patterns=pats)
         n = args.packets
         nb = synth.nbytes(0, n)
@@ -48,7 +50,7 @@ def main():
         L.kmpb_union_stats(st, 1)
         ev, steps, cand, rounds = (int(x) for x in st)
         kb = nb / 1024.0
-        print(json.dumps({"packets": n, "bytes": nb, "flags": args.flags, "matches": int(d_counts.sum().item()),
+        print(json.dumps({"packets": n, "bytes": nb, "flags": args.flags, "nocase": args.nocase, "matches": int(d_counts.sum().item()),
                           "events": ev, "resolve_steps": steps, "candidates": cand, "verify_rounds": rounds,
                           "events_per_kb": round(ev / kb, 4), "candidates_per_kb": round(cand / kb, 4),
                           "candidates_per_event": round(cand / max(ev, 1), 4),

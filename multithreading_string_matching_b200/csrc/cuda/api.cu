@@ -9,20 +9,7 @@
 
 #include "kmpb_device.cuh"
 
-// a CUDA call inside a chunk loop: on failure nothing of the call stays in flight
-#define KMPB_CUDA_Q(ctx, call)                                                                   \
-    do {                                                                                         \
-        cudaError_t e_ = (call);                                                                 \
-        if (e_ != cudaSuccess) {                                                                 \
-            quiesce(ctx);                                                                        \
-            return kmpb_fail(KMPB_ECUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), \
-                             __FILE__, __LINE__);                                                \
-        }                                                                                        \
-    } while (0)
-
 namespace {
-
-void quiesce(kmpb_ctx *ctx);
 
 int use_device(const kmpb_ctx *ctx)
 {
@@ -107,6 +94,36 @@ int ensure_host_staging(kmpb_ctx *ctx, uint64_t max_bytes, uint64_t max_pkts)
     return KMPB_OK;
 }
 
+// everything a chunked form needs for chunks of up to max_bytes / max_pkts: the device slots, their pinned twins when
+// the chunks are packed on the host first, the union engine's scratch
+int reserve(kmpb_ctx *ctx, uint64_t max_bytes, uint64_t max_pkts, bool pinned)
+{
+    int rc;
+    if ((rc = ensure_staging(ctx, max_bytes, max_pkts)) || (pinned && (rc = ensure_host_staging(ctx, max_bytes, max_pkts))))
+        return rc;
+    return kmpb_union_scratch(ctx, max_bytes);
+}
+
+// The host may write a slot's pinned buffers again once their last copy to the device has left them.  (An event never
+// recorded, or recorded by an earlier call that has finished, is complete: the wait returns at once.)
+int wait_pinned(kmpb_ctx *ctx, int slot)
+{
+    KMPB_CUDA(cudaEventSynchronize(ctx->ev_h2d[slot]));
+    return KMPB_OK;
+}
+
+// the n packets (nbytes of payload) packed into the slot's pinned buffers to its device twin, on the slot's stream
+int submit_pinned(kmpb_ctx *ctx, int slot, uint64_t n, uint64_t nbytes, kmpb_batch &b)
+{
+    cudaStream_t s = ctx->copy_stream[slot];
+    memset(ctx->h_stage_bytes[slot] + nbytes, 0, 64);
+    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_bytes[slot], ctx->h_stage_bytes[slot], nbytes + 64, cudaMemcpyHostToDevice, s));
+    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_off[slot], ctx->h_stage_off[slot], (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    KMPB_CUDA(cudaEventRecord(ctx->ev_h2d[slot], s));
+    b = kmpb_batch{ctx->d_stage_bytes[slot], 0, ctx->d_stage_off[slot], n, 0, nbytes};
+    return KMPB_OK;
+}
+
 // sums the per-slot accumulators into file order, copies them out and reports device-side error flags
 int finish_chunked(kmpb_ctx *ctx, int n_slots, uint64_t *counts_out)
 {
@@ -169,26 +186,76 @@ int check_pcap_lengths(const kmpb_pcap *pc, uint64_t first, uint64_t count)
                      (unsigned long long)k, KMPB_PACKET_LIMIT);
 }
 
-// chunk plan of a host batch: whole packets, ~chunk_bytes each; the largest chunk's bytes (from its 512-byte aligned
-// base) and packets
-struct host_chunk { uint64_t k0, k1; };
-std::vector<host_chunk> plan_host_chunks(const uint64_t *offsets, uint64_t n_packets, uint64_t chunk_bytes, uint64_t &max_bytes,
-                                         uint64_t &max_pkts)
+// Chunk plan of the chunked forms: packets [k0, k1) of every chunk, whole packets of ~chunk_bytes each (a packet larger
+// than a chunk still travels whole), and the largest chunk's bytes and packets, which the staging slots must hold.
+// Chunk c goes to stream slot c % KMPB_COPY_STREAMS; k0 is also the packet index the find records of the chunk start at.
+struct chunk { uint64_t k0, k1; };
+struct chunk_plan {
+    std::vector<chunk> chunks;
+    uint64_t max_bytes = 0, max_pkts = 0;
+    void add(uint64_t k0, uint64_t k1, uint64_t bytes)
+    {
+        chunks.push_back({k0, k1});
+        max_bytes = std::max(max_bytes, bytes);
+        max_pkts = std::max(max_pkts, k1 - k0);
+    }
+    int slots() const { return (int)std::min<size_t>(KMPB_COPY_STREAMS, chunks.size()); }
+};
+
+// a host batch; a chunk's bytes count from its 512-byte aligned base
+chunk_plan plan_host(const uint64_t *offsets, uint64_t n_packets, uint64_t chunk_bytes)
 {
-    std::vector<host_chunk> plan;
-    max_bytes = max_pkts = 0;
+    chunk_plan plan;
     for (uint64_t k0 = 0; k0 < n_packets;) {
         const uint64_t want = offsets[k0] + chunk_bytes;
         uint64_t k1 = (uint64_t)(std::lower_bound(offsets + k0 + 1, offsets + n_packets, want) - offsets);
         if (k1 > n_packets) k1 = n_packets;
         k1 = std::min<uint64_t>(k1, k0 + ((1ull << 31) - 2));
-        plan.push_back({k0, k1});
-        const uint64_t base = offsets[k0] & ~511ull;
-        max_bytes = std::max(max_bytes, offsets[k1] - base);
-        max_pkts = std::max(max_pkts, k1 - k0);
+        plan.add(k0, k1, offsets[k1] - (offsets[k0] & ~511ull));
         k0 = k1;
     }
     return plan;
+}
+
+// accepted packets [first, last) of a savefile, at most 2^22 packets a chunk
+chunk_plan plan_pcap(const kmpb_pcap *pc, uint64_t first, uint64_t last, uint64_t chunk_bytes)
+{
+    chunk_plan plan;
+    for (uint64_t k0 = first; k0 < last;) {
+        uint64_t bytes = 0;
+        const uint64_t k1 = kmpb_pcap_chunk_end(pc, k0, last, chunk_bytes, 1ull << 22, &bytes);
+        plan.add(k0, k1, bytes);
+        k0 = k1;
+    }
+    return plan;
+}
+
+// A chunk into its slot's device buffers, copies on the slot's stream.  Host batch: copied from the caller's memory.
+int stage_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, const chunk &ch, int slot, kmpb_batch &b)
+{
+    cudaStream_t s = ctx->copy_stream[slot];
+    const uint64_t k0 = ch.k0, k1 = ch.k1, base = offsets[k0] & ~511ull;
+    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_bytes[slot], bytes + base, offsets[k1] - base, cudaMemcpyHostToDevice, s));
+    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_off[slot], offsets + k0, (k1 - k0 + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    b = kmpb_batch{ctx->d_stage_bytes[slot], base, ctx->d_stage_off[slot], k1 - k0, offsets[k0], offsets[k1]};
+    return KMPB_OK;
+}
+
+double now_s() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; }
+
+// Savefile: packed into the slot's pinned buffers (all host threads), then copied over.  t[0] and t[1] add up the
+// seconds spent waiting for the slot and packing.
+int stage_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, const chunk &ch, int slot, kmpb_batch &b, double t[2])
+{
+    const uint64_t n = ch.k1 - ch.k0;
+    const double t0 = now_s();
+    const int rc = wait_pinned(ctx, slot);
+    if (rc) return rc;
+    const double t1 = now_s();
+    kmpb_pcap_pack(pc, ch.k0, n, ctx->h_stage_bytes[slot], ctx->h_stage_off[slot]);
+    t[0] += t1 - t0;
+    t[1] += now_s() - t1;
+    return submit_pinned(ctx, slot, n, ctx->h_stage_off[slot][n], b);
 }
 
 int init_context(kmpb_ctx *ctx)
@@ -230,62 +297,80 @@ int ensure_find_rec(kmpb_ctx *ctx, int slot, uint64_t records)
     return KMPB_OK;
 }
 
-// The chunk pipeline of the host find forms.  stage(c, slot, batch, packet_base) puts chunk c on the device in the
-// slot's staging buffers (copies on the slot's stream) -- kmpb_count_host's or kmpb_count_pcap's way; the find kernel
-// follows on the same stream.  Chunk c is finished (its match count read, its records sorted and copied out) just
-// before its slot takes chunk c + KMPB_COPY_STREAMS, so the copies and kernels of the chunks in between keep the device
-// busy meanwhile.  A chunk whose records overflowed the slot's buffer is matched again, from the copy still on the
-// device, into a buffer of the exact size; once `capacity` records are out, later chunks are only counted.
+// The two chunk pipelines: stage(chunk, slot, batch) puts a chunk of the plan on the device in its slot's staging
+// buffers (stage_host or stage_pcap), and its kernels follow on the slot's stream, so the copies of chunk c+1.. overlap
+// the kernels of chunk c.  Both leave nothing of the call in flight when they return an error.
+//
+// Counting: the count engine adds every chunk into its slot's accumulators; the caller then calls finish_chunked.
 template <class Stage>
-int find_chunks(kmpb_ctx *ctx, uint64_t n_chunks, uint64_t guess, Stage &&stage, kmpb_match *out, uint64_t capacity,
-                uint64_t *n_found)
+int count_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage)
 {
+    KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
+    KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * ctx->host.n_uniq * sizeof(uint64_t), ctx->stream));
+    KMPB_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
+    for (int s = 0; s < plan.slots(); s++) KMPB_CUDA(cudaStreamWaitEvent(ctx->copy_stream[s], ctx->ev[2], 0));
+    for (size_t c = 0; c < plan.chunks.size(); c++) {
+        const int slot = (int)(c % KMPB_COPY_STREAMS);
+        kmpb_batch b;
+        int rc;
+        if ((rc = stage(plan.chunks[c], slot, b)) || (rc = run_engine(ctx, b, slot, ctx->copy_stream[slot]))) {
+            quiesce(ctx);
+            return rc;
+        }
+    }
+    return KMPB_OK;
+}
+
+// Finding: the find kernel writes a chunk's records into its slot's buffer.  Chunk c is finished (its match count read,
+// its records sorted and copied out) just before its slot takes chunk c + KMPB_COPY_STREAMS, so the copies and kernels of
+// the chunks in between keep the device busy meanwhile.  A chunk whose records overflowed the slot's buffer is matched
+// again, from the copy still on the device, into a buffer of the exact size; once `capacity` records are out, later
+// chunks are only counted.
+template <class Stage>
+int find_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage, kmpb_match *out, uint64_t capacity, uint64_t *n_found)
+{
+    const uint64_t n_chunks = plan.chunks.size();
     kmpb_batch batch[KMPB_COPY_STREAMS] = {};
-    uint64_t base[KMPB_COPY_STREAMS] = {};
     uint64_t total = 0, written = 0;
-    int rc;
     auto finish = [&](uint64_t c) -> int {
         const int slot = (int)(c % KMPB_COPY_STREAMS);
         cudaStream_t s = ctx->copy_stream[slot];
         unsigned long long n = 0;
-        KMPB_CUDA_Q(ctx, cudaMemcpyAsync(&n, ctx->d_find_found + slot, sizeof n, cudaMemcpyDeviceToHost, s));
-        KMPB_CUDA_Q(ctx, cudaStreamSynchronize(s));
+        KMPB_CUDA(cudaMemcpyAsync(&n, ctx->d_find_found + slot, sizeof n, cudaMemcpyDeviceToHost, s));
+        KMPB_CUDA(cudaStreamSynchronize(s));
         const uint64_t take = std::min<uint64_t>(n, capacity - written);
         if (take) {
-            int rc2;
-            if (n > ctx->find_rec_cap[slot]) {
-                if ((rc2 = ensure_find_rec(ctx, slot, n)) || (rc2 = kmpb_find_match(ctx, batch[slot], slot, ctx->d_find_rec[slot], n,
-                                                                                     ctx->d_find_found + slot, s))) {
-                    quiesce(ctx);
-                    return rc2;
-                }
-            }
-            if ((rc2 = kmpb_find_finish(ctx, batch[slot], base[slot], ctx->d_find_rec[slot], n, ctx->d_find_found + slot, true, s))) {
-                quiesce(ctx);
-                return rc2;
-            }
-            KMPB_CUDA_Q(ctx, cudaMemcpyAsync(out + written, ctx->d_find_rec[slot], take * sizeof(kmpb_match), cudaMemcpyDeviceToHost, s));
-            KMPB_CUDA_Q(ctx, cudaStreamSynchronize(s));
+            int rc;
+            if (n > ctx->find_rec_cap[slot] &&
+                ((rc = ensure_find_rec(ctx, slot, n)) ||
+                 (rc = kmpb_find_match(ctx, batch[slot], slot, ctx->d_find_rec[slot], n, ctx->d_find_found + slot, s))))
+                return rc;
+            if ((rc = kmpb_find_finish(ctx, batch[slot], plan.chunks[c].k0, ctx->d_find_rec[slot], n, ctx->d_find_found + slot, true, s)))
+                return rc;
+            KMPB_CUDA(cudaMemcpyAsync(out + written, ctx->d_find_rec[slot], take * sizeof(kmpb_match), cudaMemcpyDeviceToHost, s));
+            KMPB_CUDA(cudaStreamSynchronize(s));
         }
         total += n;
         written += take;
         return KMPB_OK;
     };
-    for (uint64_t c = 0; c < n_chunks; c++) {
+    int rc = KMPB_OK;
+    for (uint64_t c = 0; c < n_chunks && !rc; c++) {
         const int slot = (int)(c % KMPB_COPY_STREAMS);
-        if (c >= (uint64_t)KMPB_COPY_STREAMS && (rc = finish(c - KMPB_COPY_STREAMS))) return rc;
-        if ((rc = ensure_find_rec(ctx, slot, guess))) { quiesce(ctx); return rc; }
-        if ((rc = stage(c, slot, batch[slot], base[slot])) ||
-            (rc = kmpb_find_match(ctx, batch[slot], slot, ctx->d_find_rec[slot], ctx->find_rec_cap[slot], ctx->d_find_found + slot,
-                                  ctx->copy_stream[slot]))) {
-            quiesce(ctx);
-            return rc;
-        }
+        if ((c >= (uint64_t)KMPB_COPY_STREAMS && (rc = finish(c - KMPB_COPY_STREAMS))) ||
+            (rc = ensure_find_rec(ctx, slot, plan.max_bytes / 256)) || (rc = stage(plan.chunks[c], slot, batch[slot])))
+            break;
+        rc = kmpb_find_match(ctx, batch[slot], slot, ctx->d_find_rec[slot], ctx->find_rec_cap[slot], ctx->d_find_found + slot,
+                             ctx->copy_stream[slot]);
     }
-    for (uint64_t c = n_chunks > (uint64_t)KMPB_COPY_STREAMS ? n_chunks - KMPB_COPY_STREAMS : 0; c < n_chunks; c++)
-        if ((rc = finish(c))) return rc;
+    for (uint64_t c = n_chunks > (uint64_t)KMPB_COPY_STREAMS ? n_chunks - KMPB_COPY_STREAMS : 0; c < n_chunks && !rc; c++)
+        rc = finish(c);
+    if (rc) {
+        quiesce(ctx);
+        return rc;
+    }
     *n_found = total;
-    return KMPB_OK; // (as in finish_chunked: the stage's caller checked every packet's size first)
+    return KMPB_OK; // (as in finish_chunked: the caller checked every packet's size first)
 }
 
 // the argument checks every find form starts with
@@ -543,7 +628,7 @@ int kmpb_count_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets
 {
     if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL context");
     if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "count before kmpb_set_patterns");
-    const uint32_t n_pat = ctx->host.n_pat, nu = ctx->host.n_uniq;
+    const uint32_t n_pat = ctx->host.n_pat;
     if (n_pat == 0) return KMPB_OK;
     if (counts_out == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL counts_out");
     memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
@@ -552,28 +637,10 @@ int kmpb_count_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets
     int rc = check_offsets(offsets, n_packets);
     if (rc) return rc;
     if ((rc = use_device(ctx))) return rc;
-
-    uint64_t max_bytes = 0, max_pkts = 0;
-    const std::vector<host_chunk> plan = plan_host_chunks(offsets, n_packets, chunk_bytes_setting(), max_bytes, max_pkts);
-    const int n_slots = (int)std::min<size_t>(KMPB_COPY_STREAMS, plan.size());
-    if ((rc = ensure_staging(ctx, max_bytes, max_pkts))) return rc;
-    if ((rc = kmpb_union_scratch(ctx, max_bytes))) return rc;
-
-    KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
-    KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * nu * sizeof(uint64_t), ctx->stream));
-    KMPB_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
-    for (int s = 0; s < n_slots; s++) KMPB_CUDA(cudaStreamWaitEvent(ctx->copy_stream[s], ctx->ev[2], 0));
-    for (size_t c = 0; c < plan.size(); c++) {
-        const int slot = (int)(c % KMPB_COPY_STREAMS);
-        cudaStream_t s = ctx->copy_stream[slot];
-        const uint64_t k0 = plan[c].k0, k1 = plan[c].k1;
-        const uint64_t base = offsets[k0] & ~511ull;
-        KMPB_CUDA_Q(ctx, cudaMemcpyAsync(ctx->d_stage_bytes[slot], bytes + base, offsets[k1] - base, cudaMemcpyHostToDevice, s));
-        KMPB_CUDA_Q(ctx, cudaMemcpyAsync(ctx->d_stage_off[slot], offsets + k0, (k1 - k0 + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-        kmpb_batch b{ctx->d_stage_bytes[slot], base, ctx->d_stage_off[slot], k1 - k0, offsets[k0], offsets[k1]};
-        if ((rc = run_engine(ctx, b, slot, s))) { quiesce(ctx); return rc; }
-    }
-    return finish_chunked(ctx, n_slots, counts_out);
+    const chunk_plan plan = plan_host(offsets, n_packets, chunk_bytes_setting());
+    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_host(ctx, bytes, offsets, ch, slot, b); };
+    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, false)) || (rc = count_chunks(ctx, plan, stage))) return rc;
+    return finish_chunked(ctx, plan.slots(), counts_out);
 }
 
 // Streamed savefile path: pack a chunk of payloads into a pinned staging slot (all host threads), copy
@@ -586,16 +653,14 @@ int kmpb_reserve_staging(kmpb_ctx *ctx, uint64_t max_batch_bytes, uint64_t max_p
     if (max_packets == 0) max_packets = 1ull << 20;
     int rc = use_device(ctx);
     if (rc) return rc;
-    if ((rc = ensure_staging(ctx, max_batch_bytes, max_packets))) return rc;
-    if ((rc = ensure_host_staging(ctx, max_batch_bytes, max_packets))) return rc;
-    return kmpb_union_scratch(ctx, max_batch_bytes);
+    return reserve(ctx, max_batch_bytes, max_packets, true);
 }
 
 int kmpb_count_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count, uint64_t *counts_out)
 {
     if (ctx == nullptr || pc == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
     if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "count before kmpb_set_patterns");
-    const uint32_t n_pat = ctx->host.n_pat, nu = ctx->host.n_uniq;
+    const uint32_t n_pat = ctx->host.n_pat;
     if (n_pat == 0) return KMPB_OK;
     if (counts_out == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL counts_out");
     memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
@@ -605,56 +670,16 @@ int kmpb_count_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t
     int rc = check_pcap_lengths(pc, first, count);
     if (rc) return rc;
     if ((rc = use_device(ctx))) return rc;
-    if (rc) return rc;
-    const uint64_t chunk_bytes = chunk_bytes_setting();
-    const uint64_t max_pkts = 1ull << 22, last = first + count;
-    // a packet larger than a chunk still travels whole: size the slots for the largest chunk of the plan
-    uint64_t max_bytes = 0, max_n = 0, n_chunks = 0;
-    for (uint64_t k0 = first; k0 < last; n_chunks++) {
-        uint64_t b = 0;
-        const uint64_t k1 = kmpb_pcap_chunk_end(pc, k0, last, chunk_bytes, max_pkts, &b);
-        max_bytes = std::max(max_bytes, b);
-        max_n = std::max(max_n, k1 - k0);
-        k0 = k1;
-    }
-    if ((rc = ensure_staging(ctx, max_bytes, max_n))) return rc;
-    if ((rc = ensure_host_staging(ctx, max_bytes, max_n))) return rc;
-    if ((rc = kmpb_union_scratch(ctx, max_bytes))) return rc;
-    const int n_slots = (int)std::min<uint64_t>(KMPB_COPY_STREAMS, n_chunks);
-
-    KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
-    KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * nu * sizeof(uint64_t), ctx->stream));
-    KMPB_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
-    for (int s = 0; s < n_slots; s++) KMPB_CUDA(cudaStreamWaitEvent(ctx->copy_stream[s], ctx->ev[2], 0));
-    uint64_t c = 0;
-    double t_wait = 0, t_pack = 0, t_issue = 0;
-    const bool stats = getenv("KMPB_STATS") != nullptr;
-    auto now = []() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; };
-    for (uint64_t k0 = first; k0 < last; c++) {
-        const int slot = (int)(c % KMPB_COPY_STREAMS);
-        cudaStream_t s = ctx->copy_stream[slot];
-        uint64_t nbytes = 0;
-        const uint64_t k1 = kmpb_pcap_chunk_end(pc, k0, last, chunk_bytes, max_pkts, &nbytes);
-        const double t0 = now();
-        if (c >= KMPB_COPY_STREAMS) KMPB_CUDA_Q(ctx, cudaEventSynchronize(ctx->ev_h2d[slot])); // the slot's last copy has left it
-        const double t1 = now();
-        kmpb_pcap_pack(pc, k0, k1 - k0, ctx->h_stage_bytes[slot], ctx->h_stage_off[slot]);
-        memset(ctx->h_stage_bytes[slot] + nbytes, 0, 64);
-        const double t2 = now();
-        KMPB_CUDA_Q(ctx, cudaMemcpyAsync(ctx->d_stage_bytes[slot], ctx->h_stage_bytes[slot], nbytes + 64, cudaMemcpyHostToDevice, s));
-        KMPB_CUDA_Q(ctx, cudaMemcpyAsync(ctx->d_stage_off[slot], ctx->h_stage_off[slot], (k1 - k0 + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-        KMPB_CUDA_Q(ctx, cudaEventRecord(ctx->ev_h2d[slot], s));
-        kmpb_batch b{ctx->d_stage_bytes[slot], 0, ctx->d_stage_off[slot], k1 - k0, 0, nbytes};
-        if ((rc = run_engine(ctx, b, slot, s))) { quiesce(ctx); return rc; }
-        k0 = k1;
-        t_wait += t1 - t0;
-        t_pack += t2 - t1;
-        t_issue += now() - t2;
-    }
-    if (stats)
+    const chunk_plan plan = plan_pcap(pc, first, first + count, chunk_bytes_setting());
+    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, true))) return rc;
+    double t[2] = {0, 0}; // waiting for a free slot, packing
+    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_pcap(ctx, pc, ch, slot, b, t); };
+    const double t0 = now_s();
+    if ((rc = count_chunks(ctx, plan, stage))) return rc;
+    if (getenv("KMPB_STATS"))
         fprintf(stderr, "kmpb_count_pcap: %llu chunks; waiting for a free slot %.3f s, packing %.3f s, issuing copies and kernels %.3f s\n",
-                (unsigned long long)c, t_wait, t_pack, t_issue);
-    return finish_chunked(ctx, n_slots, counts_out);
+                (unsigned long long)plan.chunks.size(), t[0], t[1], now_s() - t0 - t[0] - t[1]);
+    return finish_chunked(ctx, plan.slots(), counts_out);
 }
 
 // ---- find: where the patterns occur (include/kmpb200.h; kernels in union_kernel.cu and find.cu) ----------------
@@ -686,21 +711,10 @@ int kmpb_find_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets,
     if (bytes == nullptr || offsets == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL batch pointer");
     if ((rc = check_offsets(offsets, n_packets))) return rc;
     if ((rc = use_device(ctx))) return rc;
-    uint64_t max_bytes = 0, max_pkts = 0;
-    const std::vector<host_chunk> plan = plan_host_chunks(offsets, n_packets, chunk_bytes_setting(), max_bytes, max_pkts);
-    if ((rc = ensure_staging(ctx, max_bytes, max_pkts))) return rc;
-    if ((rc = kmpb_union_scratch(ctx, max_bytes))) return rc;
-    auto stage = [&](uint64_t c, int slot, kmpb_batch &b, uint64_t &base) -> int {
-        cudaStream_t s = ctx->copy_stream[slot];
-        const uint64_t k0 = plan[c].k0, k1 = plan[c].k1;
-        const uint64_t abs_base = offsets[k0] & ~511ull;
-        KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_bytes[slot], bytes + abs_base, offsets[k1] - abs_base, cudaMemcpyHostToDevice, s));
-        KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_off[slot], offsets + k0, (k1 - k0 + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-        b = kmpb_batch{ctx->d_stage_bytes[slot], abs_base, ctx->d_stage_off[slot], k1 - k0, offsets[k0], offsets[k1]};
-        base = k0;
-        return KMPB_OK;
-    };
-    return find_chunks(ctx, plan.size(), max_bytes / 256, stage, out, capacity, n_found);
+    const chunk_plan plan = plan_host(offsets, n_packets, chunk_bytes_setting());
+    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, false))) return rc;
+    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_host(ctx, bytes, offsets, ch, slot, b); };
+    return find_chunks(ctx, plan, stage, out, capacity, n_found);
 }
 
 int kmpb_find_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count, kmpb_match *out, uint64_t capacity,
@@ -716,36 +730,11 @@ int kmpb_find_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t 
     if (count == 0) return KMPB_OK;
     if ((rc = check_pcap_lengths(pc, first, count))) return rc;
     if ((rc = use_device(ctx))) return rc;
-    const uint64_t chunk_bytes = chunk_bytes_setting();
-    const uint64_t max_pkts = 1ull << 22, last = first + count;
-    std::vector<uint64_t> starts; // first packet of every chunk, then `last`
-    uint64_t max_bytes = 0, max_n = 0;
-    for (uint64_t k0 = first; k0 < last;) {
-        uint64_t nb = 0;
-        const uint64_t k1 = kmpb_pcap_chunk_end(pc, k0, last, chunk_bytes, max_pkts, &nb);
-        starts.push_back(k0);
-        max_bytes = std::max(max_bytes, nb);
-        max_n = std::max(max_n, k1 - k0);
-        k0 = k1;
-    }
-    starts.push_back(last);
-    if ((rc = ensure_staging(ctx, max_bytes, max_n))) return rc;
-    if ((rc = ensure_host_staging(ctx, max_bytes, max_n))) return rc;
-    if ((rc = kmpb_union_scratch(ctx, max_bytes))) return rc;
-    // (a slot's pinned buffers are free again: its previous chunk has been finished, which waited for its stream)
-    auto stage = [&](uint64_t c, int slot, kmpb_batch &b, uint64_t &base) -> int {
-        cudaStream_t s = ctx->copy_stream[slot];
-        const uint64_t k0 = starts[c], k1 = starts[c + 1];
-        kmpb_pcap_pack(pc, k0, k1 - k0, ctx->h_stage_bytes[slot], ctx->h_stage_off[slot]);
-        const uint64_t nbytes = ctx->h_stage_off[slot][k1 - k0];
-        memset(ctx->h_stage_bytes[slot] + nbytes, 0, 64);
-        KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_bytes[slot], ctx->h_stage_bytes[slot], nbytes + 64, cudaMemcpyHostToDevice, s));
-        KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_off[slot], ctx->h_stage_off[slot], (k1 - k0 + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-        b = kmpb_batch{ctx->d_stage_bytes[slot], 0, ctx->d_stage_off[slot], k1 - k0, 0, nbytes};
-        base = k0;
-        return KMPB_OK;
-    };
-    return find_chunks(ctx, starts.size() - 1, max_bytes / 256, stage, out, capacity, n_found);
+    const chunk_plan plan = plan_pcap(pc, first, first + count, chunk_bytes_setting());
+    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, true))) return rc;
+    double t[2] = {0, 0};
+    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_pcap(ctx, pc, ch, slot, b, t); };
+    return find_chunks(ctx, plan, stage, out, capacity, n_found);
 }
 
 // ---- frames pushed one at a time (the live-capture shape) ----------------------------------------
@@ -763,20 +752,16 @@ static int stream_submit(kmpb_stream *st)
     kmpb_ctx *ctx = st->ctx;
     if (st->n == 0) return KMPB_OK;
     const int slot = st->slot;
-    cudaStream_t s = ctx->copy_stream[slot];
     ctx->h_stage_off[slot][st->n] = st->bytes;
-    memset(ctx->h_stage_bytes[slot] + st->bytes, 0, 64);
-    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_bytes[slot], ctx->h_stage_bytes[slot], st->bytes + 64, cudaMemcpyHostToDevice, s));
-    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_off[slot], ctx->h_stage_off[slot], (st->n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    KMPB_CUDA(cudaEventRecord(ctx->ev_h2d[slot], s));
-    kmpb_batch b{ctx->d_stage_bytes[slot], 0, ctx->d_stage_off[slot], st->n, 0, st->bytes};
-    int rc = run_engine(ctx, b, slot, s); // accumulates into the slot's distinct-pattern counters
-    if (rc) return rc;
+    kmpb_batch b;
+    int rc;
+    if ((rc = submit_pinned(ctx, slot, st->n, st->bytes, b)) ||
+        (rc = run_engine(ctx, b, slot, ctx->copy_stream[slot]))) // accumulates into the slot's distinct-pattern counters
+        return rc;
     st->batches++;
     st->slot = (slot + 1) % KMPB_COPY_STREAMS;
     st->n = st->bytes = 0;
-    if (st->batches >= (uint64_t)KMPB_COPY_STREAMS) KMPB_CUDA(cudaEventSynchronize(ctx->ev_h2d[st->slot])); // its last copy has left it
-    return KMPB_OK;
+    return wait_pinned(ctx, st->slot); // kmpb_stream_push fills it next
 }
 
 int kmpb_stream_open(kmpb_ctx *ctx, int proto, uint64_t batch_bytes, kmpb_stream **out)
@@ -790,9 +775,7 @@ int kmpb_stream_open(kmpb_ctx *ctx, int proto, uint64_t batch_bytes, kmpb_stream
     if (batch_bytes == 0) batch_bytes = 8ull << 20;
     if (batch_bytes < 65536) batch_bytes = 65536; // a frame's payload is at most 65535 - headers bytes long... jumbo included
     const uint64_t max_pkts = 1ull << 20;
-    if ((rc = ensure_staging(ctx, batch_bytes, max_pkts))) return rc;
-    if ((rc = ensure_host_staging(ctx, batch_bytes, max_pkts))) return rc;
-    if ((rc = kmpb_union_scratch(ctx, batch_bytes))) return rc;
+    if ((rc = reserve(ctx, batch_bytes, max_pkts, true))) return rc;
     const uint32_t nu = ctx->host.n_uniq;
     KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
     KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * (nu ? nu : 1) * sizeof(uint64_t), ctx->stream));

@@ -375,7 +375,7 @@ def test_device_form_capacity(matcher, strings, finder):
 
 
 @pytest.mark.gpu
-def test_many_chunks_and_slices(matcher, oracle, strings, monkeypatch, finder):
+def test_many_chunks_and_slices(matcher, oracle, strings, monkeypatch, finder, tmp_path):
     monkeypatch.setenv("KMPB_CHUNK_MB", "1")
     synth = kmp.Synth(seed=7, len_mode=1, plants=2, plant_patterns=strings)
     data, offsets = synth.fill_host(0, 12000)  # ~20 MB of mixed sizes: ~20 chunks, every slot reused
@@ -391,6 +391,37 @@ def test_many_chunks_and_slices(matcher, oracle, strings, monkeypatch, finder):
         got = matcher.find_pcap(path, first=first, count=count)
         sel = pwant[(pwant["packet"] >= first) & (pwant["packet"] < first + count)]
         assert np.array_equal(got[["packet", "offset", "pattern"]].astype(kmp.MATCH_DTYPE), sel), (first, count)
+    # Plans of exactly 1, KMPB_COPY_STREAMS (4) and KMPB_COPY_STREAMS + 1 chunks (a 1 MiB chunk is 256 packets of 4096
+    # bytes), and a packet of over 3 MiB, larger than a chunk: the four host and savefile forms against the oracle and
+    # the reference finder
+    sdata, soff = kmp.Synth(seed=11, payload_len=4096, plants=2, plant_patterns=strings).fill_host(0, 5 * 256)
+    pkts = [bytes(sdata[int(a):int(b)]) for a, b in zip(soff[:-1], soff[1:])]
+    assert {len(p) for p in pkts} == {4096}
+    rng = np.random.default_rng(11)
+    giant = bytearray(rng.choice(np.frombuffer(b"acdeikoprstu ", np.uint8), (3 << 20) + 123).tobytes())
+    for at in rng.integers(0, len(giant) - 16, 500).tolist():
+        p = strings[at % len(strings)]
+        giant[at:at + len(p)] = p
+    for label, case in (("1 chunk", pkts[:256]), ("4 chunks", pkts[:1024]), ("5 chunks", pkts),
+                        ("a packet larger than a chunk", pkts[:300] + [bytes(giant)] + pkts[300:600])):
+        data, offsets = csr(case)
+        path = str(tmp_path / "chunks.pcap")
+        with open(path, "wb") as f:  # UDP frames; a payload is its frame's captured length less the headers
+            f.write(struct.pack("<IHHiIII", 0xA1B2C3D4, 2, 4, 0, 0, 262144, 1))
+            for p in case:
+                frame = bytes(12) + b"\x08\x00" + bytes([0x45, 0, 0, 0, 0, 0, 0, 0, 64, 17]) + bytes(18) + p
+                f.write(struct.pack("<IIII", 0, 0, len(frame), len(frame)) + frame)
+        counts = oracle.count_csr(data, offsets, strings)
+        want = finder.find_csr(data, offsets, strings)
+        assert len(want) > 1000, label
+        assert matcher.count_host(data, offsets) == counts, label
+        assert matcher.count_pcap_streamed(path) == counts, label
+        got = matcher.find_host(data, offsets)
+        assert np.array_equal(got, want), label
+        assert_invariant(counts, got, strings)
+        got = matcher.find_pcap(path)[["packet", "offset", "pattern"]].astype(kmp.MATCH_DTYPE)
+        assert np.array_equal(got, want), label
+        assert_invariant(counts, got, strings)
 
 
 @pytest.mark.gpu

@@ -132,7 +132,10 @@ int kmpb_count_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets
  * are device memory on the context's GPU; d_counts[n_pat] (device, uint64) is ACCUMULATED into, so
  * a caller can sum several batches and all-reduce once (mpi_dumping.c:202).  Asynchronous on
  * `stream` (a cudaStream_t passed as void*; NULL = CUDA's default stream, as in the runtime API).
- * One device-form call may be in flight per context at a time (they share scratch buffers). */
+ * Device-form calls (kmpb_count_device*, kmpb_find_device_span) on one context share scratch buffers, so they run on the
+ * device in call order, whatever streams they are issued on: each call's work waits, on the device, for the work of the
+ * one issued before it.  The host forms and kmpb_stream_open run after every device-form call issued before them.  Work
+ * of the caller's own on other streams is not ordered by this: order it with events as usual. */
 int kmpb_count_device(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets,
                       uint64_t n_packets, uint64_t *d_counts, void *stream);
 /* Same, for a caller that already knows first_byte = offsets[0] and end_byte = offsets[n_packets]:
@@ -197,8 +200,8 @@ typedef struct kmpb_match {
  * total number of matches, which may exceed capacity.  With KMPB_FIND_SORTED and no overflow the records are sorted;
  * the sort costs time in proportion to `capacity`, so size the buffer close to the total (the sum of the kmpb_count_*
  * counts of the batch is exact).  On overflow the records written are an unspecified subset of the matches, in no
- * particular order: run again with a larger buffer.  Unsorted, the records come in an unspecified order.  One call in
- * flight per context; it shares scratch buffers with the count forms. */
+ * particular order: run again with a larger buffer.  Unsorted, the records come in an unspecified order.  It shares
+ * scratch buffers with the count forms and is ordered with them like every device-form call (kmpb_count_device). */
 int kmpb_find_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets, uint64_t n_packets,
                           uint64_t first_byte, uint64_t end_byte, kmpb_match *d_out, uint64_t capacity,
                           uint64_t *d_n_found, uint32_t flags, void *stream);
@@ -283,7 +286,13 @@ int kmpb_pcap_frame_index(const kmpb_pcap *pc, uint64_t first, uint64_t count, u
  * appends the accepted payload to the current batch in pinned memory; a full batch (batch_bytes, 0 =
  * 8 MiB) is copied to the device and matched asynchronously while the caller keeps pushing.
  * kmpb_stream_flush submits the partial batch, waits, and returns the counts accumulated since
- * kmpb_stream_open in counts_out[n_pat]; pushing may continue afterwards.  One producer thread. */
+ * kmpb_stream_open in counts_out[n_pat]; pushing may continue afterwards.  One producer thread.
+ * An open stream owns its context until kmpb_stream_close: its counts and its partly filled batch live in the context's
+ * per-slot counters and pinned staging buffers, which every other matching call reuses.  So while a stream is open,
+ * kmpb_set_patterns(_ex), every count and find form, kmpb_reserve_staging and a second kmpb_stream_open return
+ * KMPB_ESTATE without touching it; kmpb_set_engine, the getters, kmpb_get_prefix, kmpb_check_device_errors and
+ * kmpb_synth_fill_device still work.  Other work during a capture takes a second context.  Close every stream of a
+ * context before kmpb_destroy. */
 typedef struct kmpb_stream kmpb_stream;
 int kmpb_stream_open(kmpb_ctx *ctx, int proto, uint64_t batch_bytes, kmpb_stream **out);
 int kmpb_stream_push(kmpb_stream *st, const uint8_t *frame, uint32_t captured_len);

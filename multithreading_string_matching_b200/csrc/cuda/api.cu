@@ -271,6 +271,39 @@ int init_context(kmpb_ctx *ctx)
     for (auto &s : ctx->copy_stream) KMPB_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
     for (auto &ev : ctx->ev) KMPB_CUDA(cudaEventCreate(&ev));
     for (auto &ev : ctx->ev_kernel) KMPB_CUDA(cudaEventCreate(&ev));
+    KMPB_CUDA(cudaEventCreateWithFlags(&ctx->ev_dev, cudaEventDisableTiming));
+    return KMPB_OK;
+}
+
+// An open frame stream owns the context until kmpb_stream_close: its batches accumulate in the per-slot counters and
+// its partly filled batch sits in a pinned staging slot, both of which every count and find form, kmpb_set_patterns
+// and kmpb_reserve_staging reuse.  Those calls refuse while a stream is open (they call this first).
+int no_open_stream(const kmpb_ctx *ctx, const char *call)
+{
+    if (ctx->open_streams == 0) return KMPB_OK;
+    return kmpb_fail(KMPB_ESTATE, "%s while a frame stream (kmpb_stream_open) is open on this context: close the stream "
+                     "first, or use a second context", call);
+}
+
+// Device-form calls of one context run in call order, whatever streams they are issued on: each makes its stream wait
+// for ev_dev, which the previous one recorded after its last enqueued work, and records ev_dev after its own.  The host
+// forms and kmpb_stream_open make the streams they start on wait for it as well, so they run after every device-form
+// call issued before them.  Nothing here waits on the host.  (An event never recorded is complete.)
+int after_device_calls(kmpb_ctx *ctx, cudaStream_t stream)
+{
+    KMPB_CUDA(cudaStreamWaitEvent(stream, ctx->ev_dev, 0));
+    return KMPB_OK;
+}
+
+template <class Enqueue>
+int device_ordered(kmpb_ctx *ctx, cudaStream_t stream, Enqueue &&enqueue)
+{
+    int rc = after_device_calls(ctx, stream);
+    if (rc) return rc;
+    rc = enqueue();
+    const cudaError_t e = cudaEventRecord(ctx->ev_dev, stream); // also after a failure: whatever was enqueued is covered
+    if (rc) return rc;
+    KMPB_CUDA(e);
     return KMPB_OK;
 }
 
@@ -305,6 +338,8 @@ int ensure_find_rec(kmpb_ctx *ctx, int slot, uint64_t records)
 template <class Stage>
 int count_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage)
 {
+    int rc = after_device_calls(ctx, ctx->stream); // (the copy streams wait for ev[2], recorded behind it)
+    if (rc) return rc;
     KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
     KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * ctx->host.n_uniq * sizeof(uint64_t), ctx->stream));
     KMPB_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
@@ -312,7 +347,6 @@ int count_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage)
     for (size_t c = 0; c < plan.chunks.size(); c++) {
         const int slot = (int)(c % KMPB_COPY_STREAMS);
         kmpb_batch b;
-        int rc;
         if ((rc = stage(plan.chunks[c], slot, b)) || (rc = run_engine(ctx, b, slot, ctx->copy_stream[slot]))) {
             quiesce(ctx);
             return rc;
@@ -357,7 +391,8 @@ int find_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage, kmpb_match
     int rc = KMPB_OK;
     for (uint64_t c = 0; c < n_chunks && !rc; c++) {
         const int slot = (int)(c % KMPB_COPY_STREAMS);
-        if ((c >= (uint64_t)KMPB_COPY_STREAMS && (rc = finish(c - KMPB_COPY_STREAMS))) ||
+        if ((c < (uint64_t)KMPB_COPY_STREAMS && (rc = after_device_calls(ctx, ctx->copy_stream[slot]))) || // first chunk
+            (c >= (uint64_t)KMPB_COPY_STREAMS && (rc = finish(c - KMPB_COPY_STREAMS))) ||
             (rc = ensure_find_rec(ctx, slot, plan.max_bytes / 256)) || (rc = stage(plan.chunks[c], slot, batch[slot])))
             break;
         rc = kmpb_find_match(ctx, batch[slot], slot, ctx->d_find_rec[slot], ctx->find_rec_cap[slot], ctx->d_find_found + slot,
@@ -374,9 +409,10 @@ int find_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage, kmpb_match
 }
 
 // the argument checks every find form starts with
-int find_args(kmpb_ctx *ctx, const void *out, uint64_t capacity, const void *n_found)
+int find_args(kmpb_ctx *ctx, const void *out, uint64_t capacity, const void *n_found, const char *call)
 {
     if (ctx == nullptr || n_found == nullptr || (out == nullptr && capacity)) return kmpb_fail(KMPB_EINVAL, "NULL argument");
+    if (int rc = no_open_stream(ctx, call)) return rc;
     if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "find before kmpb_set_patterns");
     return KMPB_OK;
 }
@@ -469,6 +505,7 @@ void kmpb_destroy(kmpb_ctx *ctx)
     }
     for (auto &ev : ctx->ev) if (ev) cudaEventDestroy(ev);
     for (auto &ev : ctx->ev_kernel) if (ev) cudaEventDestroy(ev);
+    if (ctx->ev_dev) cudaEventDestroy(ctx->ev_dev);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
 }
@@ -521,8 +558,8 @@ int kmpb_set_patterns(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_of
 int kmpb_set_patterns_ex(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, const uint8_t *flags)
 {
     if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL context");
-    int rc = use_device(ctx);
-    if (rc) return rc;
+    int rc = no_open_stream(ctx, "kmpb_set_patterns");
+    if (rc || (rc = use_device(ctx))) return rc;
     kmpb_tables fresh;
     rc = kmpb_tables_build_flags(&fresh, blob, pat_off, n_pat, flags, 0);
     if (rc) return rc;
@@ -554,9 +591,10 @@ int kmpb_get_prefix(kmpb_ctx *ctx, uint32_t pattern_index, int32_t *pi_out, uint
 // last block does that itself, so a pass is two launches (work partition, match) and no collective.
 static int count_device_span_into(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets, uint64_t n_packets,
                                   uint64_t first_byte, uint64_t end_byte, uint64_t *const *d_counts, uint32_t n_vectors,
-                                  void *stream_v)
+                                  void *stream_v, const char *call)
 {
     if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL context");
+    if (int rc = no_open_stream(ctx, call)) return rc;
     if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "count before kmpb_set_patterns");
     if (ctx->host.n_pat == 0) return KMPB_OK;
     if (d_counts == nullptr || n_vectors == 0 || n_vectors > (uint32_t)KMPB_MAX_OUT)
@@ -570,44 +608,52 @@ static int count_device_span_into(kmpb_ctx *ctx, const uint8_t *d_bytes, const u
     cudaStream_t stream = (cudaStream_t)stream_v; // NULL is CUDA's default stream, as in the runtime API
     if ((rc = kmpb_union_scratch(ctx, end_byte - first_byte))) return rc;
     const uint32_t nu = ctx->host.n_uniq;
-    KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)nu * sizeof(uint64_t), stream));
     kmpb_batch b{d_bytes, 0, d_offsets, n_packets, first_byte, end_byte};
     const bool fused = ctx->engine != KMPB_ENGINE_PERPAT && n_packets > 0 && end_byte > first_byte && nu > 0;
-    if (fused) {
-        kmpb_fused_out out;
-        out.n = n_vectors;
-        for (uint32_t r = 0; r < n_vectors; r++) out.vec[r] = (unsigned long long *)d_counts[r];
-        return kmpb_launch_union(ctx, b, 0, ctx->d_uniq_counts, stream, out);
-    }
-    if ((rc = run_engine(ctx, b, 0, stream))) return rc;
-    for (uint32_t r = 0; r < n_vectors; r++) {
-        kmpb_expand_counts_kernel<<<(ctx->host.n_pat + 255) / 256, 256, 0, stream>>>(
-            (const unsigned long long *)ctx->d_uniq_counts, nu, 1, ctx->dev.pat_to_uniq, ctx->host.n_pat,
-            (unsigned long long *)d_counts[r], n_vectors > 1 ? 2 : 1);
-        ctx->launches++;
-    }
-    KMPB_CUDA(cudaGetLastError());
-    return KMPB_OK;
+    return device_ordered(ctx, stream, [&]() -> int {
+        KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)nu * sizeof(uint64_t), stream));
+        if (fused) {
+            kmpb_fused_out out;
+            out.n = n_vectors;
+            for (uint32_t r = 0; r < n_vectors; r++) out.vec[r] = (unsigned long long *)d_counts[r];
+            return kmpb_launch_union(ctx, b, 0, ctx->d_uniq_counts, stream, out);
+        }
+        int rc2 = run_engine(ctx, b, 0, stream);
+        if (rc2) return rc2;
+        for (uint32_t r = 0; r < n_vectors; r++) {
+            kmpb_expand_counts_kernel<<<(ctx->host.n_pat + 255) / 256, 256, 0, stream>>>(
+                (const unsigned long long *)ctx->d_uniq_counts, nu, 1, ctx->dev.pat_to_uniq, ctx->host.n_pat,
+                (unsigned long long *)d_counts[r], n_vectors > 1 ? 2 : 1);
+            ctx->launches++;
+        }
+        KMPB_CUDA(cudaGetLastError());
+        return KMPB_OK;
+    });
 }
 
 int kmpb_count_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets, uint64_t n_packets,
                            uint64_t first_byte, uint64_t end_byte, uint64_t *d_counts, void *stream_v)
 {
     uint64_t *one[1] = {d_counts};
-    return count_device_span_into(ctx, d_bytes, d_offsets, n_packets, first_byte, end_byte, one, 1, stream_v);
+    return count_device_span_into(ctx, d_bytes, d_offsets, n_packets, first_byte, end_byte, one, 1, stream_v,
+                                  "kmpb_count_device_span");
 }
 
 int kmpb_count_device_span_peers(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets, uint64_t n_packets,
                                  uint64_t first_byte, uint64_t end_byte, uint64_t *const *d_counts_all,
                                  uint32_t n_vectors, void *stream_v)
 {
-    return count_device_span_into(ctx, d_bytes, d_offsets, n_packets, first_byte, end_byte, d_counts_all, n_vectors, stream_v);
+    return count_device_span_into(ctx, d_bytes, d_offsets, n_packets, first_byte, end_byte, d_counts_all, n_vectors, stream_v,
+                                  "kmpb_count_device_span_peers");
 }
 
+// (the span read touches only the caller's offsets: the ordering after earlier device-form calls starts in
+// kmpb_count_device_span, so the host waits for this call's stream alone, as before)
 int kmpb_count_device(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets, uint64_t n_packets,
                       uint64_t *d_counts, void *stream_v)
 {
     if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL context");
+    if (int rc = no_open_stream(ctx, "kmpb_count_device")) return rc;
     if (n_packets == 0) return KMPB_OK;
     if (d_offsets == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL device pointer");
     int rc = use_device(ctx);
@@ -627,6 +673,7 @@ int kmpb_count_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets
                     uint64_t *counts_out)
 {
     if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL context");
+    if (int rc = no_open_stream(ctx, "kmpb_count_host")) return rc;
     if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "count before kmpb_set_patterns");
     const uint32_t n_pat = ctx->host.n_pat;
     if (n_pat == 0) return KMPB_OK;
@@ -649,16 +696,18 @@ int kmpb_count_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets
 int kmpb_reserve_staging(kmpb_ctx *ctx, uint64_t max_batch_bytes, uint64_t max_packets)
 {
     if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
+    int rc = no_open_stream(ctx, "kmpb_reserve_staging");
+    if (rc) return rc;
     if (max_batch_bytes == 0) max_batch_bytes = (64ull << 20) + 65536; // a ~64 MiB batch of whole packets
     if (max_packets == 0) max_packets = 1ull << 20;
-    int rc = use_device(ctx);
-    if (rc) return rc;
+    if ((rc = use_device(ctx))) return rc;
     return reserve(ctx, max_batch_bytes, max_packets, true);
 }
 
 int kmpb_count_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count, uint64_t *counts_out)
 {
     if (ctx == nullptr || pc == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
+    if (int rc = no_open_stream(ctx, "kmpb_count_pcap")) return rc;
     if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "count before kmpb_set_patterns");
     const uint32_t n_pat = ctx->host.n_pat;
     if (n_pat == 0) return KMPB_OK;
@@ -687,7 +736,7 @@ int kmpb_find_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t 
                           uint64_t first_byte, uint64_t end_byte, kmpb_match *d_out, uint64_t capacity,
                           uint64_t *d_n_found, uint32_t flags, void *stream_v)
 {
-    int rc = find_args(ctx, d_out, capacity, d_n_found);
+    int rc = find_args(ctx, d_out, capacity, d_n_found, "kmpb_find_device_span");
     if (rc) return rc;
     if (flags & ~KMPB_FIND_SORTED) return kmpb_fail(KMPB_EINVAL, "unknown find flags 0x%x", flags);
     if (n_packets && (d_bytes == nullptr || d_offsets == nullptr)) return kmpb_fail(KMPB_EINVAL, "NULL device pointer");
@@ -697,14 +746,16 @@ int kmpb_find_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t 
     if ((rc = kmpb_union_scratch(ctx, end_byte - first_byte))) return rc;
     const kmpb_batch b{d_bytes, 0, d_offsets, n_packets, first_byte, end_byte};
     unsigned long long *found = reinterpret_cast<unsigned long long *>(d_n_found);
-    if ((rc = kmpb_find_match(ctx, b, 0, d_out, capacity, found, stream))) return rc;
-    return kmpb_find_finish(ctx, b, 0, d_out, capacity, found, (flags & KMPB_FIND_SORTED) != 0, stream);
+    return device_ordered(ctx, stream, [&]() -> int {
+        const int rc2 = kmpb_find_match(ctx, b, 0, d_out, capacity, found, stream);
+        return rc2 ? rc2 : kmpb_find_finish(ctx, b, 0, d_out, capacity, found, (flags & KMPB_FIND_SORTED) != 0, stream);
+    });
 }
 
 int kmpb_find_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, uint64_t n_packets,
                    kmpb_match *out, uint64_t capacity, uint64_t *n_found)
 {
-    int rc = find_args(ctx, out, capacity, n_found);
+    int rc = find_args(ctx, out, capacity, n_found, "kmpb_find_host");
     if (rc) return rc;
     *n_found = 0;
     if (ctx->host.n_pat == 0 || n_packets == 0) return KMPB_OK;
@@ -721,7 +772,7 @@ int kmpb_find_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t 
                    uint64_t *n_found)
 {
     if (pc == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
-    int rc = find_args(ctx, out, capacity, n_found);
+    int rc = find_args(ctx, out, capacity, n_found, "kmpb_find_pcap");
     if (rc) return rc;
     *n_found = 0;
     if (ctx->host.n_pat == 0) return KMPB_OK;
@@ -768,15 +819,17 @@ int kmpb_stream_open(kmpb_ctx *ctx, int proto, uint64_t batch_bytes, kmpb_stream
 {
     if (ctx == nullptr || out == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
     *out = nullptr;
+    int rc = no_open_stream(ctx, "kmpb_stream_open");
+    if (rc) return rc;
     if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "stream before kmpb_set_patterns");
     if (proto != KMPB_PROTO_UDP && proto != KMPB_PROTO_TCP) return kmpb_fail(KMPB_EINVAL, "unknown protocol %d", proto);
-    int rc = use_device(ctx);
-    if (rc) return rc;
+    if ((rc = use_device(ctx))) return rc;
     if (batch_bytes == 0) batch_bytes = 8ull << 20;
     if (batch_bytes < 65536) batch_bytes = 65536; // a frame's payload is at most 65535 - headers bytes long... jumbo included
     const uint64_t max_pkts = 1ull << 20;
     if ((rc = reserve(ctx, batch_bytes, max_pkts, true))) return rc;
     const uint32_t nu = ctx->host.n_uniq;
+    if ((rc = after_device_calls(ctx, ctx->stream))) return rc;
     KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
     KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * (nu ? nu : 1) * sizeof(uint64_t), ctx->stream));
     KMPB_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -788,6 +841,7 @@ int kmpb_stream_open(kmpb_ctx *ctx, int proto, uint64_t batch_bytes, kmpb_stream
     st->max_pkts = max_pkts;
     st->slot = 0;
     st->n = st->bytes = st->batches = st->frames = st->packets = 0;
+    ctx->open_streams++;
     *out = st;
     return KMPB_OK;
 }
@@ -833,6 +887,7 @@ void kmpb_stream_close(kmpb_stream *st)
     if (st == nullptr) return;
     cudaSetDevice(st->ctx->device);
     cudaDeviceSynchronize();
+    st->ctx->open_streams--;
     delete st;
 }
 

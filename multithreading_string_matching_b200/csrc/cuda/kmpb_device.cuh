@@ -45,6 +45,8 @@ struct kmpb_ctx {
     cudaStream_t copy_stream[KMPB_COPY_STREAMS] = {};   // H2D + kernel pipeline of kmpb_count_host
     cudaEvent_t ev[4] = {};
     cudaEvent_t ev_kernel[2] = {};                      // around the dominant kernel when profile is on
+    cudaEvent_t ev_dev = nullptr;                       // after the last device-form call's work, on its stream
+    int open_streams = 0;                               // kmpb_stream_open without kmpb_stream_close yet
     bool profile = false;
     kmpb_tables host = {};
     bool have_tables = false;

@@ -435,7 +435,7 @@ def test_count_before_and_after_find(matcher, oracle, strings):
     d_bytes[: len(data)] = torch.from_numpy(np.array(data))
     d_off = torch.from_numpy(offsets.astype(np.int64)).to("cuda:0")
 
-    def counts():  # (the device form shares scratch with the host form: it has to be finished first)
+    def counts():  # (the device form's counts are read once it has finished; tests/test_call_order.py overlaps calls)
         d_counts = torch.zeros(len(strings), dtype=torch.int64, device="cuda:0")
         matcher.count_device(d_bytes.data_ptr(), d_off.data_ptr(), len(offsets) - 1, d_counts.data_ptr(), span=(0, len(data)))
         torch.cuda.synchronize()

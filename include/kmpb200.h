@@ -132,7 +132,7 @@ int kmpb_count_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets
  * are device memory on the context's GPU; d_counts[n_pat] (device, uint64) is ACCUMULATED into, so
  * a caller can sum several batches and all-reduce once (mpi_dumping.c:202).  Asynchronous on
  * `stream` (a cudaStream_t passed as void*; NULL = CUDA's default stream, as in the runtime API).
- * Device-form calls (kmpb_count_device*, kmpb_find_device_span) on one context share scratch buffers, so they run on the
+ * Device-form calls (kmpb_count_device*, kmpb_find_device_span, kmpb_select_device_span) on one context share scratch buffers, so they run on the
  * device in call order, whatever streams they are issued on: each call's work waits, on the device, for the work of the
  * one issued before it.  The host forms and kmpb_stream_open run after every device-form call issued before them.  Work
  * of the caller's own on other streams is not ordered by this: order it with events as usual. */
@@ -281,6 +281,50 @@ int kmpb_find_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t 
  * Savefiles of 2^32 records or more are outside the documented limits. */
 int kmpb_pcap_frame_index(const kmpb_pcap *pc, uint64_t first, uint64_t count, uint64_t *frames_out);
 
+/* ---- selecting: which packets match -------------------------------------------------------- */
+/* A packet is SELECTED iff it holds at least one match that the count forms count, under each pattern's case flag:
+ * exactly the packets that kmpb_find_* on the same batch yields a record for.  Selecting always runs the union engine,
+ * like finding; one pass gives the per-packet verdicts and, when asked for, the counts.  Its match kernel sets one bit
+ * per match in a start-position bitmap of the batch (one bit per payload byte: span / 8 bytes of device memory, 1.75 GB
+ * for a 14 GB batch, 8 GiB at the 64 GiB limit), which a verdict pass turns into one flag per packet and leaves zero
+ * again.  The device form uses the bitmap of the context's first stream slot; the host and savefile forms one per stream
+ * slot their chunk plan uses, as long as the largest chunk (a chunk can be a single packet of close to 2 GiB: 256 MiB).  All of it is owned
+ * by the context and grows on demand.  Errors: KMPB_ESTATE before kmpb_set_patterns or while a frame stream is open,
+ * KMPB_EINVAL for a NULL pointer or an unknown flag, KMPB_ENODEVICE without a B200. */
+#define KMPB_SELECT_INVERT 1u /* kmpb_select_device_span: d_index lists the packets that are NOT selected */
+/* Device form: asynchronous on `stream`, with the preconditions, limits and call-order rules of kmpb_count_device_span
+ * (a packet of KMPB_PACKET_LIMIT bytes or more is reported by kmpb_check_device_errors).  d_flags[n_packets] (uint8,
+ * device) is OVERWRITTEN: 1 = the packet is selected, 0 = not.  d_index (uint64[n_packets], device, may be NULL)
+ * receives the ascending indices of the selected packets (KMPB_SELECT_INVERT: of the others), and *d_n_selected
+ * (uint64, device) is overwritten with their number; d_n_selected may be NULL when d_index is (the verdicts alone).
+ * d_counts may be NULL; when given, it is ACCUMULATED into exactly as kmpb_count_device_span does. */
+int kmpb_select_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets, uint64_t n_packets,
+                            uint64_t first_byte, uint64_t end_byte, uint8_t *d_flags, uint64_t *d_index,
+                            uint64_t *d_n_selected, uint64_t *d_counts, uint32_t flags, void *stream);
+/* Host form: synchronous, chunked and overlapped like kmpb_count_host (KMPB_CHUNK_MB sets the chunk size; a packet of
+ * KMPB_PACKET_LIMIT bytes or more is KMPB_ELIMIT before anything runs).  flags_out[n_packets] (host) is overwritten
+ * with the verdicts, *n_selected (may be NULL) with the number of selected packets; counts_out[n_pat] may be NULL, and
+ * when given is overwritten with the batch's counts, as kmpb_count_host does. */
+int kmpb_select_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, uint64_t n_packets,
+                     uint8_t *flags_out, uint64_t *n_selected, uint64_t *counts_out);
+/* The same for accepted packets [first, first+count) of a savefile, through kmpb_count_pcap's packing pipeline:
+ * flags_out[j] is the verdict of accepted packet first + j. */
+int kmpb_select_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count,
+                     uint8_t *flags_out, uint64_t *n_selected, uint64_t *counts_out);
+/* Plain C, no GPU: writes the capture records of the accepted packets [first, first+count) of `pc` for which
+ * (flags[j] != 0) != (invert != 0) to out_path, as a savefile of the input's format, byte for byte as they are in the
+ * input, in file order.  A classic savefile keeps its 24-byte header (byte order, usec / nsec magic, snaplen, link
+ * type) and every chosen record (header and captured bytes, a record cut short by its snaplen as it is).  A pcapng file
+ * keeps every block that holds no packet (section headers, interface descriptions, name resolution, statistics, ...) in
+ * file order and the chosen packet blocks (enhanced, simple, obsolete packet blocks), so every section and its
+ * interface numbering stay valid; a section header's Section Length is written as -1 (not specified), since the
+ * section is shorter than the input's.  Frames whose payload the extractor refused are in neither output, inverted or not;
+ * nor is whatever the ingest walk stops at (a truncated record, a malformed block) or follows it.  *n_written (may be
+ * NULL) receives the number of records written.  KMPB_EINVAL when out_path names the input file itself (it is mapped
+ * while it is read), KMPB_EIO when the file cannot be written; on failure no partial output is left behind. */
+int kmpb_pcap_write_selected(const kmpb_pcap *pc, uint64_t first, uint64_t count, const uint8_t *flags, int invert,
+                             const char *out_path, uint64_t *n_written);
+
 /* Frames arriving one at a time (live_openmp_task.c:160-217: pcap_next in a loop, batches handed to
  * tasks while the capture goes on).  kmpb_stream_push runs the extractor on one captured frame and
  * appends the accepted payload to the current batch in pinned memory; a full batch (batch_bytes, 0 =
@@ -289,7 +333,7 @@ int kmpb_pcap_frame_index(const kmpb_pcap *pc, uint64_t first, uint64_t count, u
  * kmpb_stream_open in counts_out[n_pat]; pushing may continue afterwards.  One producer thread.
  * An open stream owns its context until kmpb_stream_close: its counts and its partly filled batch live in the context's
  * per-slot counters and pinned staging buffers, which every other matching call reuses.  So while a stream is open,
- * kmpb_set_patterns(_ex), every count and find form, kmpb_reserve_staging and a second kmpb_stream_open return
+ * kmpb_set_patterns(_ex), every count, find and select form, kmpb_reserve_staging and a second kmpb_stream_open return
  * KMPB_ESTATE without touching it; kmpb_set_engine, the getters, kmpb_get_prefix, kmpb_check_device_errors and
  * kmpb_synth_fill_device still work.  Other work during a capture takes a second context.  Close every stream of a
  * context before kmpb_destroy. */

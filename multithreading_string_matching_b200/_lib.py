@@ -87,6 +87,15 @@ SIGNATURES = {
                                       ctypes.c_void_p, ctypes.c_uint64, c_u64p]),
     "kmpb_find_pcap": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64,
                                       ctypes.c_void_p, ctypes.c_uint64, c_u64p]),
+    "kmpb_select_device_span": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64,
+                                               ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p,
+                                               ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.c_void_p]),
+    "kmpb_select_host": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64,
+                                        ctypes.c_void_p, c_u64p, ctypes.c_void_p]),
+    "kmpb_select_pcap": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64,
+                                        ctypes.c_void_p, c_u64p, ctypes.c_void_p]),
+    "kmpb_pcap_write_selected": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p,
+                                                ctypes.c_int, ctypes.c_char_p, c_u64p]),
     "kmpb_pcap_frame_index": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p]),
     "kmpb_stream_open": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.POINTER(ctypes.c_void_p)]),
     "kmpb_stream_push": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_uint32]),

@@ -408,6 +408,81 @@ int find_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage, kmpb_match
     return KMPB_OK; // (as in finish_chunked: the caller checked every packet's size first)
 }
 
+// Selecting: every chunk's mark kernel and verdict pass run on its slot's stream into the slot's bitmap and verdicts,
+// which are copied to the slot's pinned twin; chunk c's verdicts are copied out (and their packets counted) just before
+// its slot takes chunk c + KMPB_COPY_STREAMS, as find_chunks does with records.  The counts go to the slots'
+// accumulators as in count_chunks; the caller then calls finish_chunked if it wants them.  flags_out[k - k_base] is
+// packet k's verdict.
+template <class Stage>
+int select_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage, uint64_t k_base, uint8_t *flags_out, uint64_t *n_selected)
+{
+    int rc = after_device_calls(ctx, ctx->stream);
+    if (rc) return rc;
+    KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
+    KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * ctx->host.n_uniq * sizeof(uint64_t), ctx->stream));
+    KMPB_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
+    for (int s = 0; s < plan.slots(); s++) KMPB_CUDA(cudaStreamWaitEvent(ctx->copy_stream[s], ctx->ev[2], 0));
+    const uint64_t n_chunks = plan.chunks.size();
+    uint64_t selected = 0;
+    auto finish = [&](uint64_t c) -> int {
+        const int slot = (int)(c % KMPB_COPY_STREAMS);
+        KMPB_CUDA(cudaStreamSynchronize(ctx->copy_stream[slot]));
+        const chunk &ch = plan.chunks[c];
+        const uint8_t *f = ctx->h_sel_flags[slot];
+        uint64_t n = 0;
+        for (uint64_t j = 0; j < ch.k1 - ch.k0; j++) n += f[j];
+        memcpy(flags_out + (ch.k0 - k_base), f, ch.k1 - ch.k0);
+        selected += n;
+        return KMPB_OK;
+    };
+    for (uint64_t c = 0; c < n_chunks && !rc; c++) {
+        const int slot = (int)(c % KMPB_COPY_STREAMS);
+        cudaStream_t s = ctx->copy_stream[slot];
+        kmpb_batch b;
+        if ((c >= (uint64_t)KMPB_COPY_STREAMS && (rc = finish(c - KMPB_COPY_STREAMS))) || (rc = stage(plan.chunks[c], slot, b)) ||
+            (rc = kmpb_select_match(ctx, b, slot, ctx->d_sel_flags[slot], s)))
+            break;
+        const cudaError_t e = cudaMemcpyAsync(ctx->h_sel_flags[slot], ctx->d_sel_flags[slot], b.n_packets, cudaMemcpyDeviceToHost, s);
+        if (e != cudaSuccess) rc = kmpb_fail(KMPB_ECUDA, "verdict copy failed: %s", cudaGetErrorString(e));
+    }
+    for (uint64_t c = n_chunks > (uint64_t)KMPB_COPY_STREAMS ? n_chunks - KMPB_COPY_STREAMS : 0; c < n_chunks && !rc; c++)
+        rc = finish(c);
+    if (rc) {
+        quiesce(ctx);
+        return rc;
+    }
+    if (n_selected) *n_selected = selected;
+    return KMPB_OK;
+}
+
+// the bitmaps and verdict buffers of the chunked select forms: those of the slots the plan uses, for chunks of up to
+// max_bytes / max_pkts (a single chunk of one packet close to 2 GiB takes one 256 MiB bitmap, not four)
+int reserve_select(kmpb_ctx *ctx, const chunk_plan &plan)
+{
+    for (int s = 0; s < plan.slots(); s++) {
+        if (int rc = kmpb_ensure_mark(ctx, s, plan.max_bytes / 32 + 8, ctx->copy_stream[s])) return rc;
+        if (plan.max_pkts <= ctx->sel_flags_cap[s] && ctx->d_sel_flags[s]) continue;
+        KMPB_CUDA(cudaDeviceSynchronize());
+        cudaFree(ctx->d_sel_flags[s]); ctx->d_sel_flags[s] = nullptr;
+        cudaFreeHost(ctx->h_sel_flags[s]); ctx->h_sel_flags[s] = nullptr;
+        ctx->sel_flags_cap[s] = 0;
+        const uint64_t cap = plan.max_pkts ? plan.max_pkts : 1;
+        KMPB_CUDA(cudaMalloc((void **)&ctx->d_sel_flags[s], cap));
+        KMPB_CUDA(cudaHostAlloc((void **)&ctx->h_sel_flags[s], cap, cudaHostAllocDefault));
+        ctx->sel_flags_cap[s] = cap;
+    }
+    return KMPB_OK;
+}
+
+// the argument checks every select form starts with
+int select_args(kmpb_ctx *ctx, const void *flags_out, uint64_t n_packets, const char *call)
+{
+    if (ctx == nullptr || (flags_out == nullptr && n_packets)) return kmpb_fail(KMPB_EINVAL, "NULL argument");
+    if (int rc = no_open_stream(ctx, call)) return rc;
+    if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "select before kmpb_set_patterns");
+    return KMPB_OK;
+}
+
 // the argument checks every find form starts with
 int find_args(kmpb_ctx *ctx, const void *out, uint64_t capacity, const void *n_found, const char *call)
 {
@@ -494,7 +569,11 @@ void kmpb_destroy(kmpb_ctx *ctx)
     cudaFree(ctx->d_sort_keys[0]);
     cudaFree(ctx->d_sort_keys[1]);
     cudaFree(ctx->d_sort_temp);
+    cudaFree(ctx->d_select_temp);
     for (int i = 0; i < KMPB_COPY_STREAMS; i++) {
+        cudaFree(ctx->d_mark[i]);
+        cudaFree(ctx->d_sel_flags[i]);
+        cudaFreeHost(ctx->h_sel_flags[i]);
         cudaFree(ctx->d_find_rec[i]);
         cudaFree(ctx->d_stage_bytes[i]);
         cudaFree(ctx->d_stage_off[i]);
@@ -786,6 +865,75 @@ int kmpb_find_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t 
     double t[2] = {0, 0};
     auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_pcap(ctx, pc, ch, slot, b, t); };
     return find_chunks(ctx, plan, stage, out, capacity, n_found);
+}
+
+// ---- select: which packets match (include/kmpb200.h; kernels in union_kernel.cu and select.cu) ------------------
+int kmpb_select_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_offsets, uint64_t n_packets,
+                            uint64_t first_byte, uint64_t end_byte, uint8_t *d_flags, uint64_t *d_index,
+                            uint64_t *d_n_selected, uint64_t *d_counts, uint32_t flags, void *stream_v)
+{
+    int rc = select_args(ctx, d_flags, n_packets, "kmpb_select_device_span");
+    if (rc) return rc;
+    if (flags & ~KMPB_SELECT_INVERT) return kmpb_fail(KMPB_EINVAL, "unknown select flags 0x%x", flags);
+    if (d_index && !d_n_selected) return kmpb_fail(KMPB_EINVAL, "d_index without d_n_selected");
+    if (n_packets && (d_bytes == nullptr || d_offsets == nullptr)) return kmpb_fail(KMPB_EINVAL, "NULL device pointer");
+    if (end_byte < first_byte) return kmpb_fail(KMPB_EINVAL, "offsets decrease");
+    if ((rc = use_device(ctx))) return rc;
+    cudaStream_t stream = (cudaStream_t)stream_v;
+    if ((rc = kmpb_union_scratch(ctx, end_byte - first_byte))) return rc;
+    const kmpb_batch b{d_bytes, 0, d_offsets, n_packets, first_byte, end_byte};
+    kmpb_fused_out out;
+    out.n = d_counts ? 1 : 0;
+    out.vec[0] = reinterpret_cast<unsigned long long *>(d_counts);
+    return device_ordered(ctx, stream, [&]() -> int {
+        if (ctx->host.n_uniq) KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)ctx->host.n_uniq * sizeof(uint64_t), stream));
+        int rc2 = kmpb_select_match(ctx, b, 0, d_flags, stream, out);
+        if (rc2 || !d_n_selected) return rc2;
+        return kmpb_select_compact(ctx, d_flags, n_packets, (flags & KMPB_SELECT_INVERT) != 0, d_index, d_n_selected, stream);
+    });
+}
+
+int kmpb_select_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, uint64_t n_packets, uint8_t *flags_out,
+                     uint64_t *n_selected, uint64_t *counts_out)
+{
+    int rc = select_args(ctx, flags_out, n_packets, "kmpb_select_host");
+    if (rc) return rc;
+    const uint32_t n_pat = ctx->host.n_pat;
+    if (n_selected) *n_selected = 0;
+    if (counts_out) memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
+    if (n_packets) memset(flags_out, 0, n_packets);
+    if (n_pat == 0 || n_packets == 0) return KMPB_OK;
+    if (bytes == nullptr || offsets == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL batch pointer");
+    if ((rc = check_offsets(offsets, n_packets)) || (rc = use_device(ctx))) return rc;
+    const chunk_plan plan = plan_host(offsets, n_packets, chunk_bytes_setting());
+    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, false)) || (rc = reserve_select(ctx, plan)))
+        return rc;
+    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_host(ctx, bytes, offsets, ch, slot, b); };
+    if ((rc = select_chunks(ctx, plan, stage, 0, flags_out, n_selected))) return rc;
+    return counts_out ? finish_chunked(ctx, plan.slots(), counts_out) : KMPB_OK;
+}
+
+int kmpb_select_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count, uint8_t *flags_out,
+                     uint64_t *n_selected, uint64_t *counts_out)
+{
+    if (pc == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
+    int rc = select_args(ctx, flags_out, count, "kmpb_select_pcap");
+    if (rc) return rc;
+    const uint64_t total = kmpb_pcap_packets(pc);
+    if (first > total || count > total - first) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
+    const uint32_t n_pat = ctx->host.n_pat;
+    if (n_selected) *n_selected = 0;
+    if (counts_out) memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
+    if (count) memset(flags_out, 0, count);
+    if (n_pat == 0 || count == 0) return KMPB_OK;
+    if ((rc = check_pcap_lengths(pc, first, count)) || (rc = use_device(ctx))) return rc;
+    const chunk_plan plan = plan_pcap(pc, first, first + count, chunk_bytes_setting());
+    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, true)) || (rc = reserve_select(ctx, plan)))
+        return rc;
+    double t[2] = {0, 0};
+    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_pcap(ctx, pc, ch, slot, b, t); };
+    if ((rc = select_chunks(ctx, plan, stage, first, flags_out, n_selected))) return rc;
+    return counts_out ? finish_chunked(ctx, plan.slots(), counts_out) : KMPB_OK;
 }
 
 // ---- frames pushed one at a time (the live-capture shape) ----------------------------------------

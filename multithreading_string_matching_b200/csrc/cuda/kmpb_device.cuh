@@ -73,6 +73,16 @@ struct kmpb_ctx {
     uint64_t sort_cap = 0;
     void *d_sort_temp = nullptr;
     size_t sort_temp_bytes = 0;
+    // select: the start-position bitmaps (per stream slot: one bit per payload byte, all zero between calls), the
+    // verdicts of the chunked forms (per slot, device and pinned host), the compaction's CUB scratch
+    uint32_t *d_mark[KMPB_COPY_STREAMS] = {};
+    uint64_t mark_words_cap[KMPB_COPY_STREAMS] = {};
+    bool mark_dirty[KMPB_COPY_STREAMS] = {};   // a call failed after its mark kernel: the bitmap may hold bits
+    uint8_t *d_sel_flags[KMPB_COPY_STREAMS] = {};
+    uint8_t *h_sel_flags[KMPB_COPY_STREAMS] = {};
+    uint64_t sel_flags_cap[KMPB_COPY_STREAMS] = {};
+    void *d_select_temp = nullptr;
+    size_t select_temp_bytes = 0;
     bool attr_union_set = false, attr_perpat_set = false; // per-device function attributes
     uint64_t launches = 0;
     double last_ms[2] = {0, 0};
@@ -110,8 +120,10 @@ void kmpb_release_tables(kmpb_ctx *ctx);
 // perpat_kernel.cu
 int kmpb_launch_perpat(kmpb_ctx *ctx, const kmpb_batch &b, uint64_t *d_uniq_counts, cudaStream_t stream);
 // union_kernel.cu
+// mark (select.cu): the start-position bitmap of the batch, word 0 holding byte first_byte (find must be null)
 int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_uniq_counts, cudaStream_t stream,
-                      const kmpb_fused_out &out = kmpb_fused_out(), const kmpb_find_out *find = nullptr);
+                      const kmpb_fused_out &out = kmpb_fused_out(), const kmpb_find_out *find = nullptr,
+                      uint32_t *mark = nullptr);
 int kmpb_union_scratch(kmpb_ctx *ctx, uint64_t max_batch_bytes);
 // find.cu: the find kernel into d_rec[capacity] (*d_found = every match of the batch), then the records turned into
 // kmpb_match (packet index + packet_base), sorted or not
@@ -119,5 +131,15 @@ int kmpb_find_match(kmpb_ctx *ctx, const kmpb_batch &b, int slot, kmpb_match *d_
                     cudaStream_t stream);
 int kmpb_find_finish(kmpb_ctx *ctx, const kmpb_batch &b, uint64_t packet_base, kmpb_match *d_rec, uint64_t capacity,
                      const unsigned long long *d_found, bool sorted, cudaStream_t stream);
+// select.cu: the words of a batch's start-position bitmap; the bitmap of a stream slot at least that long (zeroed when
+// allocated and when a failed call left it dirty, on `stream`); mark kernel + verdict into d_flags[n_packets] (zeroed
+// first), the counts added to the slot's distinct-pattern counters (and to out when out.n > 0); the ascending indices
+// of the packets whose flag is (invert ? 0 : 1) into d_index (may be null) and their number into *d_n_selected
+uint64_t kmpb_mark_words(const kmpb_batch &b);
+int kmpb_ensure_mark(kmpb_ctx *ctx, int slot, uint64_t words, cudaStream_t stream);
+int kmpb_select_match(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint8_t *d_flags, cudaStream_t stream,
+                      const kmpb_fused_out &out = kmpb_fused_out());
+int kmpb_select_compact(kmpb_ctx *ctx, const uint8_t *d_flags, uint64_t n_packets, bool invert, uint64_t *d_index,
+                        uint64_t *d_n_selected, cudaStream_t stream);
 // api.cu
 int kmpb_launch_expand(kmpb_ctx *ctx, const uint64_t *d_uniq_counts, uint64_t *d_counts, cudaStream_t stream);

@@ -360,6 +360,7 @@ enum { DC_TEXT_LO = 0, DC_TEXT_HI,   // p.bytes - p.abs_base: absolute byte 0
        DC_CAP_LO, DC_CAP_HI,     // ... its capacity in records
        DC_FOUND_LO, DC_FOUND_HI, // ... the uint64 counter of every match found (also those past the capacity)
        DC_GATE_SA, DC_GATE_SHIFT, // shared address of the prefix gate (0 = none: phase 1 re-runs the filter), its hash shift
+       DC_MARK_LO, DC_MARK_HI,   // mark kernel: the start-position bitmap, biased (mark_hit)
        DC_LAST = 31 };           // "I am the last block" flag
 
 // The scratch words of a warp (128 bytes): two sets of 32 bytes, one per item parity --
@@ -435,11 +436,22 @@ __device__ __forceinline__ void emit_hit(const uint64_t pos, const uint32_t u)
         __stcs(rec, make_uint4((uint32_t)pos, (uint32_t)(pos >> 32), 0u, u));
     }
 }
-template <bool EMIT>
+// The mark kernel's hit (after count_hit): bit pos & 31 of word pos >> 5 of the start-position bitmap (select.cu).  The
+// DC_MARK_* words hold the bitmap's base less the word index of the batch's first byte, so the bitmap's word 0 is the
+// one that holds first_byte.  No slot to reserve, no record: a verified hit costs one reduction.
+__device__ __forceinline__ void mark_hit(const uint64_t pos)
+{
+    uint32_t *w = reinterpret_cast<uint32_t *>(const_cast<uint8_t *>(dc_ptr(DC_MARK_LO))) + (pos >> 5);
+    asm volatile("red.global.or.b32 [%0], %1;" ::"l"(w), "r"(1u << (uint32_t)(pos & 31u)) : "memory");
+}
+// what a kernel does with a verified hit besides counting it: nothing (count), a record (find), a bitmap bit (mark)
+enum : int { UN_COUNT = 0, UN_FIND = 1, UN_MARK = 2 };
+template <int OUT>
 __device__ __forceinline__ void hit(const drain_args &d, const uint32_t u, const uint64_t pos)
 {
     count_hit(d, u);
-    if (EMIT) emit_hit(pos, u);
+    if (OUT == UN_FIND) emit_hit(pos, u);
+    if (OUT == UN_MARK) mark_hit(pos);
 }
 
 // 4 text bytes starting at g, of which the first `need` (>= 1) matter: never read past the word that holds the last
@@ -466,7 +478,7 @@ struct probe_consts {
 // NOCASE (the set has a nocase pattern, automaton.c): a nocase record's masks clear bit 5 at the pattern's letters, so
 // the masked compare is the case-insensitive one, and past byte 8 the record's tail masks (word 7, 0 = none) do the
 // same for the word-by-word compare; the nocase one-byte patterns have a second 256-word table after the first.
-template <bool VS, bool EMIT, bool NOCASE>
+template <bool VS, int OUT, bool NOCASE>
 __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_consts &pc, const uint32_t x0, const uint32_t x1,
                                             const uint32_t room, const uint64_t pos)
 {
@@ -481,10 +493,10 @@ __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_con
     const uint32_t vt_one = pc.one, vt_slots_a = pc.slots_a, vt_slots_b = pc.slots_b;
     if (vt_one) { // one-byte patterns: a direct table (room >= 1 always holds)
         const uint32_t u = vt(vt_one + (x0 & 0xffu));
-        if (u != 0xffffffffu) hit<EMIT>(d, u, pos);
+        if (u != 0xffffffffu) hit<OUT>(d, u, pos);
         if (NOCASE) {
             const uint32_t un = vt(vt_one + 256u + (x0 & 0xffu));
-            if (un != 0xffffffffu) hit<EMIT>(d, un, pos);
+            if (un != 0xffffffffu) hit<OUT>(d, un, pos);
         }
     }
     if (room < 2) return;
@@ -515,7 +527,7 @@ __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_con
                 same = (rem >= 4 ? diff : diff & ((1u << (8 * rem)) - 1u)) == 0;
             }
         }
-        if (same) hit<EMIT>(d, b.y, pos);
+        if (same) hit<OUT>(d, b.y, pos);
     }
 }
 
@@ -525,7 +537,7 @@ __device__ __forceinline__ void verify_cand(const drain_args &d, const probe_con
 // free-running counters, slots handed out and slots verified.
 __device__ __forceinline__ uint32_t warp_c_sa() { return smem_sa() + UN_OFF_C + (threadIdx.x >> 5) * (UN_CCAP * UN_C_BYTES1); }
 // verify the n (<= 32) candidates from slot `head` on, one per lane
-template <bool EMIT, bool NOCASE>
+template <int OUT, bool NOCASE>
 __device__ __forceinline__ void verify_round(const drain_args &d, const uint32_t head, const uint32_t n)
 {
     const uint32_t lane = threadIdx.x & 31;
@@ -537,12 +549,12 @@ __device__ __forceinline__ void verify_round(const drain_args &d, const uint32_t
         pc.slots_a = c0.x; pc.shift_a = c0.y; pc.slots_b = c0.z; pc.shift_b = c0.w; pc.one = c1.x; pc.rec = c1.y;
         const uint4 e = lds128v(warp_c_sa() + ((head + lane) & (UN_CCAP - 1)) * UN_C_BYTES1);
         const uint64_t pos = ((uint64_t)(e.w >> 8) << 32) | e.z;
-        if (d.vtab_sa) verify_cand<true, EMIT, NOCASE>(d, pc, e.x, e.y, e.w & 0xffu, pos);
-        else verify_cand<false, EMIT, NOCASE>(d, pc, e.x, e.y, e.w & 0xffu, pos);
+        if (d.vtab_sa) verify_cand<true, OUT, NOCASE>(d, pc, e.x, e.y, e.w & 0xffu, pos);
+        else verify_cand<false, OUT, NOCASE>(d, pc, e.x, e.y, e.w & 0xffu, pos);
     }
 }
 // the candidates still waiting at the end of a batch
-template <bool EMIT, bool NOCASE>
+template <int OUT, bool NOCASE>
 __device__ __forceinline__ void flush_body()
 {
     drain_args d;
@@ -552,15 +564,17 @@ __device__ __forceinline__ void flush_body()
     d.counts_sa = dc(DC_COUNTS_SA);
     __syncwarp();
     const uint2 cs = lds64v(d.scratch_sa + SC_CAND); // {handed out, verified}: fewer than 32 apart between resolve steps
-    verify_round<EMIT, NOCASE>(d, cs.y, cs.x - cs.y);
+    verify_round<OUT, NOCASE>(d, cs.y, cs.x - cs.y);
     __syncwarp();
     if ((threadIdx.x & 31) == 0) sts32v(d.scratch_sa + SC_CAND + 4, cs.x);
     __syncwarp();
 }
-__device__ __noinline__ void flush_candidates() { flush_body<false, false>(); }
-__device__ __noinline__ void flush_candidates_find() { flush_body<true, false>(); }
-__device__ __noinline__ void flush_candidates_nc() { flush_body<false, true>(); }
-__device__ __noinline__ void flush_candidates_find_nc() { flush_body<true, true>(); }
+__device__ __noinline__ void flush_candidates() { flush_body<UN_COUNT, false>(); }
+__device__ __noinline__ void flush_candidates_find() { flush_body<UN_FIND, false>(); }
+__device__ __noinline__ void flush_candidates_nc() { flush_body<UN_COUNT, true>(); }
+__device__ __noinline__ void flush_candidates_find_nc() { flush_body<UN_FIND, true>(); }
+__device__ __noinline__ void flush_candidates_mark() { flush_body<UN_MARK, false>(); }
+__device__ __noinline__ void flush_candidates_mark_nc() { flush_body<UN_MARK, true>(); }
 
 // Phase 0 of a resolve step, on its own so that the row loop can issue it a row or two ahead: the n (<= 32) oldest
 // events' groups (32 B + 8 B lookahead), one per lane, from L2 (the rows were read a few microseconds ago) straight
@@ -600,7 +614,7 @@ __device__ __forceinline__ void drain_fetch(const uint32_t head, const uint32_t 
 // event carries its item's parity, and what the resolve step has to know about either item waits in the warp's
 // scratch words, where the warp put it when it took the item: no lane has to look anything up in global memory for
 // it, and the row loop does not keep it in registers.  Positions are relative to the item's row0 (32 bits).
-template <bool EMIT, bool NOCASE>
+template <int OUT, bool NOCASE>
 __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n)
 {
     drain_args d;
@@ -832,14 +846,14 @@ __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n
             ctail += __popc(any);
             __syncwarp();
             if (ctail - chead >= 32u) {
-                verify_round<EMIT, NOCASE>(d, chead, 32u);
+                verify_round<OUT, NOCASE>(d, chead, 32u);
                 chead += 32u;
                 __syncwarp();
             }
         }
     }
     while (ctail - chead >= 32u) {
-        verify_round<EMIT, NOCASE>(d, chead, 32u);
+        verify_round<OUT, NOCASE>(d, chead, 32u);
         chead += 32u;
     }
     __syncwarp();
@@ -852,22 +866,32 @@ __device__ __forceinline__ void drain_body(const uint32_t head, const uint32_t n
 __device__ __noinline__ void drain_events(const uint32_t head, const uint32_t n)
 {
     drain_fetch(head, n);
-    drain_body<false, false>(head, n);
+    drain_body<UN_COUNT, false>(head, n);
 }
 __device__ __noinline__ void drain_events_find(const uint32_t head, const uint32_t n)
 {
     drain_fetch(head, n);
-    drain_body<true, false>(head, n);
+    drain_body<UN_FIND, false>(head, n);
 }
 __device__ __noinline__ void drain_events_nc(const uint32_t head, const uint32_t n)
 {
     drain_fetch(head, n);
-    drain_body<false, true>(head, n);
+    drain_body<UN_COUNT, true>(head, n);
 }
 __device__ __noinline__ void drain_events_find_nc(const uint32_t head, const uint32_t n)
 {
     drain_fetch(head, n);
-    drain_body<true, true>(head, n);
+    drain_body<UN_FIND, true>(head, n);
+}
+__device__ __noinline__ void drain_events_mark(const uint32_t head, const uint32_t n)
+{
+    drain_fetch(head, n);
+    drain_body<UN_MARK, false>(head, n);
+}
+__device__ __noinline__ void drain_events_mark_nc(const uint32_t head, const uint32_t n)
+{
+    drain_fetch(head, n);
+    drain_body<UN_MARK, true>(head, n);
 }
 
 // NUL-dense row.  An event without candidates exists only to tell later candidates where the last NUL before them
@@ -888,11 +912,13 @@ __device__ __forceinline__ uint32_t uni(uint32_t v) { return __shfl_sync(FULL, v
 __device__ __forceinline__ uint64_t uni(uint64_t v) { return __shfl_sync(FULL, v, 0); }
 #undef DP_SEL
 #define DP_SEL(k) p.sel[k]
-// The kernel body, in four instantiations: the count kernel (EMIT = false) and the find kernel (EMIT = true), which
-// also writes a record per match; what it needs of the record buffer waits in the DC_* words, not in registers.  Each
-// comes with NOCASE = true for pattern sets with a nocase pattern: only the verifier differs (verify_cand).
-template <bool EMIT, bool NOCASE>
-__device__ __forceinline__ void union_body(const union_params &__restrict__ p, const kmpb_find_out &__restrict__ fo)
+// The kernel body, in six instantiations: the count kernel (OUT = UN_COUNT), the find kernel (UN_FIND), which also
+// writes a record per match, and the mark kernel (UN_MARK), which also sets the match's bit in a start-position bitmap;
+// what they need of the record buffer or the bitmap waits in the DC_* words, not in registers.  Each comes with
+// NOCASE = true for pattern sets with a nocase pattern: only the verifier differs (verify_cand).
+template <int OUT, bool NOCASE>
+__device__ __forceinline__ void union_body(const union_params &__restrict__ p, const kmpb_find_out &__restrict__ fo,
+                                           uint32_t *mark = nullptr)
 {
     uint32_t *lut = reinterpret_cast<uint32_t *>(smem);                      // L, then G
     uint32_t *s_misc = reinterpret_cast<uint32_t *>(smem + UN_OFF_MISC);
@@ -930,11 +956,15 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
         s_misc[DC_COUNTS_SA] = p.counts_in_smem ? saddr_of(s_counts) : 0u;
         s_misc[DC_GATE_SA] = p.gate_in_smem ? saddr_of(s_gate) : 0u;
         s_misc[DC_GATE_SHIFT] = p.gate_shift;
-        if (EMIT) {
+        if (OUT == UN_FIND) {
             const uint64_t rec = reinterpret_cast<uint64_t>(fo.rec), found = reinterpret_cast<uint64_t>(fo.found);
             s_misc[DC_REC_LO] = (uint32_t)rec; s_misc[DC_REC_HI] = (uint32_t)(rec >> 32);
             s_misc[DC_CAP_LO] = (uint32_t)fo.capacity; s_misc[DC_CAP_HI] = (uint32_t)(fo.capacity >> 32);
             s_misc[DC_FOUND_LO] = (uint32_t)found; s_misc[DC_FOUND_HI] = (uint32_t)(found >> 32);
+        }
+        if (OUT == UN_MARK) {
+            const uint64_t mk = reinterpret_cast<uint64_t>(mark);
+            s_misc[DC_MARK_LO] = (uint32_t)mk; s_misc[DC_MARK_HI] = (uint32_t)(mk >> 32);
         }
     }
     const uint32_t lane = threadIdx.x & 31;
@@ -961,10 +991,12 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
     auto resolve_oldest = [&]() {
         const uint32_t qn = pending(), n = qn < UN_QDRAIN ? qn : UN_QDRAIN;
         if (NOCASE) {
-            if (EMIT) drain_events_find_nc(oldest(), n);
+            if (OUT == UN_FIND) drain_events_find_nc(oldest(), n);
+            else if (OUT == UN_MARK) drain_events_mark_nc(oldest(), n);
             else drain_events_nc(oldest(), n);
         } else {
-            if (EMIT) drain_events_find(oldest(), n);
+            if (OUT == UN_FIND) drain_events_find(oldest(), n);
+            else if (OUT == UN_MARK) drain_events_mark(oldest(), n);
             else drain_events(oldest(), n);
         }
         qs -= n;
@@ -1129,7 +1161,7 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
             // loop, inlined (one copy of the code, and no call whose register needs the loop would have to respect).
             while ((qs & QS_FETCHED) || pending() >= 2 * UN_QDRAIN) {
                 if (!(qs & QS_FETCHED)) drain_fetch(oldest(), UN_QDRAIN);
-                drain_body<EMIT, NOCASE>(oldest(), UN_QDRAIN);
+                drain_body<OUT, NOCASE>(oldest(), UN_QDRAIN);
                 qs = (qs & ~QS_FETCHED) - UN_QDRAIN;
                 if (lane == 0) { // that many fewer events of older items
                     const uint32_t older = lds32v(warp_scratch_sa() + SC_STATE + 4);
@@ -1169,10 +1201,12 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
     // leftovers
     while (pending()) resolve_oldest();
     if (NOCASE) {
-        if (EMIT) flush_candidates_find_nc();
+        if (OUT == UN_FIND) flush_candidates_find_nc();
+        else if (OUT == UN_MARK) flush_candidates_mark_nc();
         else flush_candidates_nc();
     } else {
-        if (EMIT) flush_candidates_find();
+        if (OUT == UN_FIND) flush_candidates_find();
+        else if (OUT == UN_MARK) flush_candidates_mark();
         else flush_candidates();
     }
 
@@ -1203,24 +1237,37 @@ __device__ __forceinline__ void union_body(const union_params &__restrict__ p, c
 
 __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_kernel(const __grid_constant__ union_params p)
 {
-    union_body<false, false>(p, kmpb_find_out());
+    union_body<UN_COUNT, false>(p, kmpb_find_out());
 }
 
 __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_find_kernel(const __grid_constant__ union_params p,
                                                                         const __grid_constant__ kmpb_find_out fo)
 {
-    union_body<true, false>(p, fo);
+    union_body<UN_FIND, false>(p, fo);
 }
 
 __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_nocase_kernel(const __grid_constant__ union_params p)
 {
-    union_body<false, true>(p, kmpb_find_out());
+    union_body<UN_COUNT, true>(p, kmpb_find_out());
 }
 
 __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_find_nocase_kernel(const __grid_constant__ union_params p,
                                                                                const __grid_constant__ kmpb_find_out fo)
 {
-    union_body<true, true>(p, fo);
+    union_body<UN_FIND, true>(p, fo);
+}
+
+// mark: the bitmap pointer is biased (mark_hit); the kernel writes no record
+__global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_mark_kernel(const __grid_constant__ union_params p,
+                                                                        uint32_t *const mark)
+{
+    union_body<UN_MARK, false>(p, kmpb_find_out(), mark);
+}
+
+__global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_mark_nocase_kernel(const __grid_constant__ union_params p,
+                                                                               uint32_t *const mark)
+{
+    union_body<UN_MARK, true>(p, kmpb_find_out(), mark);
 }
 
 // ---- host side ------------------------------------------------------------------------------------
@@ -1257,7 +1304,7 @@ extern "C" int kmpb_union_stats(uint64_t out[4], int reset)
 #endif
 
 int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_uniq_counts, cudaStream_t stream,
-                      const kmpb_fused_out &out, const kmpb_find_out *find)
+                      const kmpb_fused_out &out, const kmpb_find_out *find, uint32_t *mark)
 {
     const kmpb_tables &h = ctx->host;
     if (h.n_uniq == 0 || b.n_packets == 0 || b.end_byte == b.first_byte) return KMPB_OK;
@@ -1299,6 +1346,8 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
         KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_find_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
         KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_nocase_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
         KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_find_nocase_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
+        KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_mark_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
+        KMPB_CUDA(cudaFuncSetAttribute(kmpb_union_mark_nocase_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UN_SMEM_MAX));
         ctx->attr_union_set = true;
     }
     kmpb_union_partition_kernel<<<(n_items + 1 + 255) / 256, 256, 0, stream>>>(b.d_offsets, (uint32_t)b.n_packets, n_items,
@@ -1336,13 +1385,18 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     int grid = (int)std::min<uint32_t>((uint32_t)ctx->sm_count, (warps_needed + UN_WARPS - 1) / UN_WARPS);
     if (grid < 1) grid = 1;
     if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[0], stream));
-    // The kernel: count or find, and the nocase instantiation exactly when the set has a nocase pattern (its tables
-    // then have the layout the nocase verifier reads: the second one-byte table, tail masks).
+    // The kernel: count, find or mark, and the nocase instantiation exactly when the set has a nocase pattern (its
+    // tables then have the layout the nocase verifier reads: the second one-byte table, tail masks).  The bitmap's word 0
+    // holds byte first_byte: mark_hit adds pos >> 5 to a base biased by first_byte >> 5 words.
+    uint32_t *const mark_biased =
+        mark ? reinterpret_cast<uint32_t *>(reinterpret_cast<uintptr_t>(mark) - 4u * (uintptr_t)(b.first_byte >> 5)) : nullptr;
     if (h.n_nocase) {
         if (find) kmpb_union_find_nocase_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, *find);
+        else if (mark) kmpb_union_mark_nocase_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, mark_biased);
         else kmpb_union_nocase_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p);
     } else {
         if (find) kmpb_union_find_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, *find);
+        else if (mark) kmpb_union_mark_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, mark_biased);
         else kmpb_union_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p);
     }
     if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[1], stream));

@@ -199,6 +199,8 @@ struct kmpb_pcap {
     size_t size;
     payload_ref *refs;
     uint64_t n_packets, n_frames, total_bytes;
+    dev_t dev; /* the mapped file, which kmpb_pcap_write_selected must not overwrite */
+    ino_t ino;
 };
 
 int kmpb_pcap_open(const char *path, int proto, kmpb_pcap **out)
@@ -264,6 +266,8 @@ int kmpb_pcap_open(const char *path, int proto, kmpb_pcap **out)
     pc->total_bytes = list.bytes;
     pc->file = file;
     pc->size = size;
+    pc->dev = st.st_dev;
+    pc->ino = st.st_ino;
     *out = pc;
     if (stats)
         fprintf(stderr, "kmpb_pcap_open: %zu bytes mapped and faulted in %.3f s, %llu records framed in %.3f s\n", size,
@@ -348,4 +352,150 @@ void kmpb_free_csr(kmpb_csr *csr)
     if (csr->pinned) { kmpb_host_free(csr->bytes); kmpb_host_free(csr->offsets); }
     else { free(csr->bytes); free(csr->offsets); }
     memset(csr, 0, sizeof *csr);
+}
+
+/* ---- kmpb_pcap_write_selected: the chosen records, verbatim ------------------------------------------------------ */
+/* The writer walks the framing once more (the ingest walk keeps no record bounds; it should not slow down for a writer
+ * few callers use) with the same rules as index_classic / index_pcapng, so its n-th packet record is frame n.  Runs
+ * of consecutive records to keep are written with one fwrite each. */
+typedef struct {
+    FILE *f;
+    const uint8_t *file;
+    size_t run_at, run_len; /* the pending run of bytes to write */
+    int err;
+    /* the chosen frames, in ascending order: frame of accepted packet first + j for the j whose verdict is chosen */
+    const payload_ref *refs;
+    const uint8_t *flags;
+    uint64_t count, j;
+    int invert;
+    uint64_t next; /* the next chosen frame, UINT64_MAX when there is none */
+    uint64_t frame, written;
+} sel_writer;
+
+static void next_chosen(sel_writer *w)
+{
+    while (w->j < w->count && (w->flags[w->j] != 0) == (w->invert != 0)) w->j++;
+    w->next = w->j < w->count ? w->refs[w->j].frame : UINT64_MAX;
+    w->j++;
+}
+
+static void keep(sel_writer *w, size_t at, size_t len)
+{
+    if (w->run_len && w->run_at + w->run_len == at) {
+        w->run_len += len;
+        return;
+    }
+    if (w->run_len && fwrite(w->file + w->run_at, 1, w->run_len, w->f) != w->run_len) w->err = 1;
+    w->run_at = at;
+    w->run_len = len;
+}
+
+/* bytes that are not in the input as they are: after the pending run */
+static void emit(sel_writer *w, const void *bytes, size_t len)
+{
+    keep(w, 0, 0); /* writes the pending run, leaves none */
+    if (fwrite(bytes, 1, len, w->f) != len) w->err = 1;
+}
+
+/* a Section Header Block at [at, at + total), total >= 24: copied with its Section Length set to -1 ("not specified";
+ * all ones in either byte order), since the written section holds fewer blocks than the input's did */
+static void section_header(sel_writer *w, size_t at, size_t total)
+{
+    static const uint8_t unspecified[8] = {0xff, 0xff, 0xff, 0xff, 0xff, 0xff, 0xff, 0xff};
+    keep(w, at, 16);
+    emit(w, unspecified, sizeof unspecified);
+    keep(w, at + 24, total - 24);
+}
+
+/* a packet record at [at, at + len): the next frame */
+static void packet_record(sel_writer *w, size_t at, size_t len)
+{
+    if (w->frame++ != w->next) return;
+    keep(w, at, len);
+    w->written++;
+    next_chosen(w);
+}
+
+static void write_classic(sel_writer *w, size_t size, int swapped)
+{
+    const uint8_t *file = w->file;
+    keep(w, 0, PCAP_GLOBAL_HDR);
+    size_t at = PCAP_GLOBAL_HDR;
+    while (size - at >= PCAP_RECORD_HDR && w->next != UINT64_MAX) {
+        const uint32_t caplen = load32(file + at + 8, swapped);
+        if (caplen > size - at - PCAP_RECORD_HDR) break;
+        packet_record(w, at, PCAP_RECORD_HDR + (size_t)caplen);
+        at += PCAP_RECORD_HDR + (size_t)caplen;
+    }
+}
+
+static void write_pcapng(sel_writer *w, size_t size)
+{
+    const uint8_t *file = w->file;
+    size_t at = 0;
+    int swapped = 0;
+    while (size - at >= 12) {
+        uint32_t type_raw;
+        memcpy(&type_raw, file + at, 4);
+        if (type_raw == NG_SHB) {
+            if (size - at < 28) break;
+            uint32_t bom;
+            memcpy(&bom, file + at + 8, 4);
+            if (bom == NG_BYTE_ORDER) swapped = 0;
+            else if (__builtin_bswap32(bom) == NG_BYTE_ORDER) swapped = 1;
+            else break;
+        }
+        const uint32_t type = type_raw == NG_SHB ? NG_SHB : load32(file + at, swapped);
+        const uint32_t total = load32(file + at + 4, swapped);
+        if (total < 12 || (total & 3u) || total > size - at) break;
+        const size_t body = at + 8, body_len = total - 12;
+        if (type == 6u || type == 2u) { /* enhanced / obsolete packet block: the walk stops where index_pcapng does */
+            if (body_len < 20 || load32(file + body + 12, swapped) > body_len - 20) break;
+            packet_record(w, at, total);
+        } else if (type == 3u) {
+            if (body_len < 4) break;
+            packet_record(w, at, total);
+        } else if (type == NG_SHB && total >= 24) {
+            section_header(w, at, total);
+        } else {
+            keep(w, at, total);
+        }
+        at += total;
+    }
+}
+
+int kmpb_pcap_write_selected(const kmpb_pcap *pc, uint64_t first, uint64_t count, const uint8_t *flags, int invert,
+                             const char *out_path, uint64_t *n_written)
+{
+    if (pc == NULL || out_path == NULL || (flags == NULL && count)) return kmpb_fail(KMPB_EINVAL, "kmpb_pcap_write_selected: NULL argument");
+    if (first > pc->n_packets || count > pc->n_packets - first) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
+    if (n_written) *n_written = 0;
+    struct stat st;
+    if (stat(out_path, &st) == 0 && st.st_dev == pc->dev && st.st_ino == pc->ino)
+        return kmpb_fail(KMPB_EINVAL, "%s is the input savefile itself", out_path);
+    FILE *f = fopen(out_path, "wb");
+    if (f == NULL) {
+        const int e = errno;
+        kmpb_fail(KMPB_EIO, "%s: %s", out_path, strerror(e));
+        errno = e;
+        return KMPB_EIO;
+    }
+    setvbuf(f, NULL, _IOFBF, 1 << 20);
+    sel_writer w = {f, pc->file, 0, 0, 0, pc->refs + first, flags, count, 0, invert, 0, 0, 0};
+    next_chosen(&w);
+    uint32_t magic;
+    memcpy(&magic, pc->file, 4);
+    if (magic == NG_SHB) write_pcapng(&w, pc->size);
+    else write_classic(&w, pc->size, magic == 0xd4c3b2a1u || magic == 0x4d3cb2a1u);
+    keep(&w, 0, 0); /* the last run */
+    const int e = w.err ? errno : 0;
+    if (fclose(f) != 0 || w.err) {
+        const int e2 = e ? e : errno;
+        unlink(out_path);
+        kmpb_fail(KMPB_EIO, "%s: %s", out_path, strerror(e2));
+        errno = e2;
+        return KMPB_EIO;
+    }
+    if (n_written) *n_written = w.written;
+    return KMPB_OK;
 }

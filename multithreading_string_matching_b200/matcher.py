@@ -19,6 +19,7 @@ ENGINE_AUTO, ENGINE_PERPAT, ENGINE_UNION = 0, 1, 2
 PROTO_UDP, PROTO_TCP = 0, 1
 _PROTO = {"udp": PROTO_UDP, "tcp": PROTO_TCP, PROTO_UDP: PROTO_UDP, PROTO_TCP: PROTO_TCP}
 FIND_SORTED = 1
+SELECT_INVERT = 1
 # one kmpb_match record (include/kmpb200.h): where a pattern occurs
 MATCH_DTYPE = np.dtype([("packet", "<u8"), ("offset", "<u4"), ("pattern", "<u4")])
 _ENGINE = {"auto": ENGINE_AUTO, "perpat": ENGINE_PERPAT, "union": ENGINE_UNION,
@@ -70,6 +71,36 @@ def load_patterns(path):
         return [data[offs[i]:offs[i + 1]] for i in range(cp.n_pat)]
     finally:
         lib().kmpb_free_patterns(ctypes.byref(cp))
+
+
+class _Savefile:
+    """kmpb_pcap_open / kmpb_pcap_close around a with-block; `first`, `count` checked against its accepted packets"""
+
+    def __init__(self, path, proto):
+        self.pc = ctypes.c_void_p()
+        check(lib().kmpb_pcap_open(os.fsencode(path), _PROTO[proto], ctypes.byref(self.pc)))
+        self.packets = lib().kmpb_pcap_packets(self.pc)
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        lib().kmpb_pcap_close(self.pc)
+
+    def write_selected(self, flags, out, first, invert):
+        flags = np.ascontiguousarray(flags, dtype=np.uint8)
+        written = ctypes.c_uint64(0)
+        check(lib().kmpb_pcap_write_selected(self.pc, first, len(flags), flags.ctypes.data if flags.size else None,
+                                             1 if invert else 0, os.fsencode(out), ctypes.byref(written)))
+        return written.value
+
+
+def write_selected(path, proto, flags, out, first=0, invert=False):
+    """Write the capture records of accepted packets [first, first + len(flags)) of the savefile at `path` whose flag is
+    true (invert: false) to `out`, verbatim, as a savefile of the input's format (kmpb_pcap_write_selected; no GPU).
+    Returns the number of records written."""
+    with _Savefile(path, proto) as f:
+        return f.write_selected(flags, out, first, invert)
 
 
 class PayloadBatch:
@@ -276,6 +307,37 @@ class Matcher:
         the total) are device pointers."""
         check(lib().kmpb_find_device_span(self._ctx, d_bytes, d_offsets, n_packets, span[0], span[1], d_out, capacity,
                                           d_n_found, FIND_SORTED if sorted else 0, stream))
+
+    def select_host(self, data, offsets):
+        """Which packets of a host CSR batch hold a match (kmpb_select_host): (bool array of n_packets, per-pattern counts)."""
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        data = _as_u8(data)
+        n = len(offsets) - 1
+        flags = np.zeros(max(n, 1), dtype=np.uint8)
+        counts = np.zeros(max(len(self.patterns), 1), dtype=np.uint64)
+        check(lib().kmpb_select_host(self._ctx, data.ctypes.data, offsets.ctypes.data, n, flags.ctypes.data, None,
+                                     counts.ctypes.data))
+        return flags[:n].astype(bool), counts[: len(self.patterns)].tolist()
+
+    def select_pcap(self, path, proto="udp", first=0, count=None, out=None, invert=False):
+        """Which accepted packets [first, first+count) of a savefile hold a match (kmpb_select_pcap): a bool array; with
+        `out`, the records of the selected packets (invert: of the others) are also written there as a savefile."""
+        with _Savefile(path, proto) as f:
+            count = f.packets - first if count is None else count
+            flags = np.zeros(max(count, 1), dtype=np.uint8)
+            check(lib().kmpb_select_pcap(self._ctx, f.pc, first, count, flags.ctypes.data, None, None))
+            flags = flags[:count]
+            if out is not None:
+                f.write_selected(flags, out, first, invert)
+        return flags.astype(bool)
+
+    def select_device(self, d_bytes, d_offsets, n_packets, d_flags, span, d_index=None, d_n_selected=None, d_counts=None,
+                      invert=False, stream=None):
+        """kmpb_select_device_span: asynchronous; d_flags (uint8[n_packets]) is overwritten with the verdicts, d_index
+        (uint64[n_packets], optional) with the ascending indices of the selected packets (invert: of the others) and
+        d_n_selected (uint64) with their number; d_counts (uint64[n_pat], optional) is accumulated into."""
+        check(lib().kmpb_select_device_span(self._ctx, d_bytes, d_offsets, n_packets, span[0], span[1], d_flags, d_index,
+                                            d_n_selected, d_counts, SELECT_INVERT if invert else 0, stream))
 
     def stream(self, proto="udp", batch_bytes=0):
         """Frames one at a time (the live_openmp_task.c shape): returns a FrameStream."""

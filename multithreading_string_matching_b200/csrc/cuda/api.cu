@@ -50,57 +50,16 @@ int run_engine(kmpb_ctx *ctx, const kmpb_batch &b, int slot, cudaStream_t stream
     return kmpb_launch_union(ctx, b, slot, acc, stream);
 }
 
-// device staging slots for chunked host input (grown on demand, kept for the next call)
-int ensure_staging(kmpb_ctx *ctx, uint64_t max_bytes, uint64_t max_pkts)
-{
-    if (max_bytes + 1024 <= ctx->stage_bytes_cap && max_pkts + 1 <= ctx->stage_off_cap) return KMPB_OK;
-    KMPB_CUDA(cudaDeviceSynchronize());
-    const size_t bcap = std::max<size_t>(ctx->stage_bytes_cap, (size_t)max_bytes + 1024);
-    const size_t ocap = std::max<size_t>(ctx->stage_off_cap, (size_t)max_pkts + 1);
-    for (int i = 0; i < KMPB_COPY_STREAMS; i++) {
-        cudaFree(ctx->d_stage_bytes[i]); ctx->d_stage_bytes[i] = nullptr;
-        cudaFree(ctx->d_stage_off[i]); ctx->d_stage_off[i] = nullptr;
-    }
-    ctx->stage_bytes_cap = ctx->stage_off_cap = 0;
-    for (int i = 0; i < KMPB_COPY_STREAMS; i++) {
-        KMPB_CUDA(cudaMalloc((void **)&ctx->d_stage_bytes[i], bcap));
-        KMPB_CUDA(cudaMemset(ctx->d_stage_bytes[i], 0, bcap));
-        KMPB_CUDA(cudaMalloc((void **)&ctx->d_stage_off[i], ocap * sizeof(uint64_t)));
-    }
-    ctx->stage_bytes_cap = bcap;
-    ctx->stage_off_cap = ocap;
-    return KMPB_OK;
-}
-
-// ... and their pinned twins on the host
-int ensure_host_staging(kmpb_ctx *ctx, uint64_t max_bytes, uint64_t max_pkts)
-{
-    if (max_bytes + 1024 <= ctx->h_stage_bytes_cap && max_pkts + 1 <= ctx->h_stage_off_cap) return KMPB_OK;
-    KMPB_CUDA(cudaDeviceSynchronize());
-    const size_t bcap = std::max<size_t>(ctx->h_stage_bytes_cap, (size_t)max_bytes + 1024);
-    const size_t ocap = std::max<size_t>(ctx->h_stage_off_cap, (size_t)max_pkts + 1);
-    for (int i = 0; i < KMPB_COPY_STREAMS; i++) {
-        cudaFreeHost(ctx->h_stage_bytes[i]); ctx->h_stage_bytes[i] = nullptr;
-        cudaFreeHost(ctx->h_stage_off[i]); ctx->h_stage_off[i] = nullptr;
-    }
-    ctx->h_stage_bytes_cap = ctx->h_stage_off_cap = 0;
-    for (int i = 0; i < KMPB_COPY_STREAMS; i++) {
-        KMPB_CUDA(cudaHostAlloc((void **)&ctx->h_stage_bytes[i], bcap, cudaHostAllocDefault));
-        KMPB_CUDA(cudaHostAlloc((void **)&ctx->h_stage_off[i], ocap * sizeof(uint64_t), cudaHostAllocDefault));
-        if (!ctx->ev_h2d[i]) KMPB_CUDA(cudaEventCreateWithFlags(&ctx->ev_h2d[i], cudaEventDisableTiming));
-    }
-    ctx->h_stage_bytes_cap = bcap;
-    ctx->h_stage_off_cap = ocap;
-    return KMPB_OK;
-}
-
-// everything a chunked form needs for chunks of up to max_bytes / max_pkts: the device slots, their pinned twins when
-// the chunks are packed on the host first, the union engine's scratch
+// everything a chunked form needs for chunks of up to max_bytes / max_pkts: the device staging slots (zero-filled when
+// new), their pinned twins when the chunks are packed on the host first, the union engine's scratch
 int reserve(kmpb_ctx *ctx, uint64_t max_bytes, uint64_t max_pkts, bool pinned)
 {
-    int rc;
-    if ((rc = ensure_staging(ctx, max_bytes, max_pkts)) || (pinned && (rc = ensure_host_staging(ctx, max_bytes, max_pkts))))
-        return rc;
+    for (int i = 0; i < KMPB_COPY_STREAMS; i++) {
+        int rc;
+        if ((rc = ctx->d_stage_bytes[i].reserve(max_bytes + 1024, true)) || (rc = ctx->d_stage_off[i].reserve(max_pkts + 1)) ||
+            (pinned && ((rc = ctx->h_stage_bytes[i].reserve(max_bytes + 1024)) || (rc = ctx->h_stage_off[i].reserve(max_pkts + 1)))))
+            return rc;
+    }
     return kmpb_union_scratch(ctx, max_bytes);
 }
 
@@ -116,11 +75,13 @@ int wait_pinned(kmpb_ctx *ctx, int slot)
 int submit_pinned(kmpb_ctx *ctx, int slot, uint64_t n, uint64_t nbytes, kmpb_batch &b)
 {
     cudaStream_t s = ctx->copy_stream[slot];
-    memset(ctx->h_stage_bytes[slot] + nbytes, 0, 64);
-    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_bytes[slot], ctx->h_stage_bytes[slot], nbytes + 64, cudaMemcpyHostToDevice, s));
-    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_off[slot], ctx->h_stage_off[slot], (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    uint8_t *h_bytes = ctx->h_stage_bytes[slot].p, *d_bytes = ctx->d_stage_bytes[slot].p;
+    uint64_t *d_off = ctx->d_stage_off[slot].p;
+    memset(h_bytes + nbytes, 0, 64);
+    KMPB_CUDA(cudaMemcpyAsync(d_bytes, h_bytes, nbytes + 64, cudaMemcpyHostToDevice, s));
+    KMPB_CUDA(cudaMemcpyAsync(d_off, ctx->h_stage_off[slot].p, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
     KMPB_CUDA(cudaEventRecord(ctx->ev_h2d[slot], s));
-    b = kmpb_batch{ctx->d_stage_bytes[slot], 0, ctx->d_stage_off[slot], n, 0, nbytes};
+    b = kmpb_batch{d_bytes, 0, d_off, n, 0, nbytes};
     return KMPB_OK;
 }
 
@@ -230,33 +191,7 @@ chunk_plan plan_pcap(const kmpb_pcap *pc, uint64_t first, uint64_t last, uint64_
     return plan;
 }
 
-// A chunk into its slot's device buffers, copies on the slot's stream.  Host batch: copied from the caller's memory.
-int stage_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, const chunk &ch, int slot, kmpb_batch &b)
-{
-    cudaStream_t s = ctx->copy_stream[slot];
-    const uint64_t k0 = ch.k0, k1 = ch.k1, base = offsets[k0] & ~511ull;
-    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_bytes[slot], bytes + base, offsets[k1] - base, cudaMemcpyHostToDevice, s));
-    KMPB_CUDA(cudaMemcpyAsync(ctx->d_stage_off[slot], offsets + k0, (k1 - k0 + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    b = kmpb_batch{ctx->d_stage_bytes[slot], base, ctx->d_stage_off[slot], k1 - k0, offsets[k0], offsets[k1]};
-    return KMPB_OK;
-}
-
 double now_s() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; }
-
-// Savefile: packed into the slot's pinned buffers (all host threads), then copied over.  t[0] and t[1] add up the
-// seconds spent waiting for the slot and packing.
-int stage_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, const chunk &ch, int slot, kmpb_batch &b, double t[2])
-{
-    const uint64_t n = ch.k1 - ch.k0;
-    const double t0 = now_s();
-    const int rc = wait_pinned(ctx, slot);
-    if (rc) return rc;
-    const double t1 = now_s();
-    kmpb_pcap_pack(pc, ch.k0, n, ctx->h_stage_bytes[slot], ctx->h_stage_off[slot]);
-    t[0] += t1 - t0;
-    t[1] += now_s() - t1;
-    return submit_pinned(ctx, slot, n, ctx->h_stage_off[slot][n], b);
-}
 
 int init_context(kmpb_ctx *ctx)
 {
@@ -271,6 +206,7 @@ int init_context(kmpb_ctx *ctx)
     for (auto &s : ctx->copy_stream) KMPB_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
     for (auto &ev : ctx->ev) KMPB_CUDA(cudaEventCreate(&ev));
     for (auto &ev : ctx->ev_kernel) KMPB_CUDA(cudaEventCreate(&ev));
+    for (auto &ev : ctx->ev_h2d) KMPB_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
     KMPB_CUDA(cudaEventCreateWithFlags(&ctx->ev_dev, cudaEventDisableTiming));
     return KMPB_OK;
 }
@@ -316,143 +252,208 @@ void quiesce(kmpb_ctx *ctx)
     cudaGetLastError();
 }
 
-// the record buffer of a stream slot of the chunked find forms, at least `records` long (grown by an eighth more)
-int ensure_find_rec(kmpb_ctx *ctx, int slot, uint64_t records)
-{
-    if (!ctx->d_find_found) KMPB_CUDA(cudaMalloc((void **)&ctx->d_find_found, KMPB_COPY_STREAMS * sizeof(unsigned long long)));
-    if (records <= ctx->find_rec_cap[slot] && ctx->d_find_rec[slot]) return KMPB_OK;
-    const uint64_t cap = records + records / 8 + 1024;
-    cudaFree(ctx->d_find_rec[slot]);
-    ctx->d_find_rec[slot] = nullptr;
-    ctx->find_rec_cap[slot] = 0;
-    KMPB_CUDA(cudaMalloc((void **)&ctx->d_find_rec[slot], cap * sizeof(kmpb_match)));
-    ctx->find_rec_cap[slot] = cap;
-    return KMPB_OK;
-}
-
-// The two chunk pipelines: stage(chunk, slot, batch) puts a chunk of the plan on the device in its slot's staging
-// buffers (stage_host or stage_pcap), and its kernels follow on the slot's stream, so the copies of chunk c+1.. overlap
-// the kernels of chunk c.  Both leave nothing of the call in flight when they return an error.
-//
-// Counting: the count engine adds every chunk into its slot's accumulators; the caller then calls finish_chunked.
-template <class Stage>
-int count_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage)
-{
-    int rc = after_device_calls(ctx, ctx->stream); // (the copy streams wait for ev[2], recorded behind it)
-    if (rc) return rc;
-    KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
-    KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * ctx->host.n_uniq * sizeof(uint64_t), ctx->stream));
-    KMPB_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
-    for (int s = 0; s < plan.slots(); s++) KMPB_CUDA(cudaStreamWaitEvent(ctx->copy_stream[s], ctx->ev[2], 0));
-    for (size_t c = 0; c < plan.chunks.size(); c++) {
-        const int slot = (int)(c % KMPB_COPY_STREAMS);
-        kmpb_batch b;
-        if ((rc = stage(plan.chunks[c], slot, b)) || (rc = run_engine(ctx, b, slot, ctx->copy_stream[slot]))) {
-            quiesce(ctx);
-            return rc;
-        }
-    }
-    return KMPB_OK;
-}
-
-// Finding: the find kernel writes a chunk's records into its slot's buffer.  Chunk c is finished (its match count read,
-// its records sorted and copied out) just before its slot takes chunk c + KMPB_COPY_STREAMS, so the copies and kernels of
-// the chunks in between keep the device busy meanwhile.  A chunk whose records overflowed the slot's buffer is matched
-// again, from the copy still on the device, into a buffer of the exact size; once `capacity` records are out, later
-// chunks are only counted.
-template <class Stage>
-int find_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage, kmpb_match *out, uint64_t capacity, uint64_t *n_found)
-{
-    const uint64_t n_chunks = plan.chunks.size();
-    kmpb_batch batch[KMPB_COPY_STREAMS] = {};
-    uint64_t total = 0, written = 0;
-    auto finish = [&](uint64_t c) -> int {
-        const int slot = (int)(c % KMPB_COPY_STREAMS);
-        cudaStream_t s = ctx->copy_stream[slot];
-        unsigned long long n = 0;
-        KMPB_CUDA(cudaMemcpyAsync(&n, ctx->d_find_found + slot, sizeof n, cudaMemcpyDeviceToHost, s));
-        KMPB_CUDA(cudaStreamSynchronize(s));
-        const uint64_t take = std::min<uint64_t>(n, capacity - written);
-        if (take) {
-            int rc;
-            if (n > ctx->find_rec_cap[slot] &&
-                ((rc = ensure_find_rec(ctx, slot, n)) ||
-                 (rc = kmpb_find_match(ctx, batch[slot], slot, ctx->d_find_rec[slot], n, ctx->d_find_found + slot, s))))
-                return rc;
-            if ((rc = kmpb_find_finish(ctx, batch[slot], plan.chunks[c].k0, ctx->d_find_rec[slot], n, ctx->d_find_found + slot, true, s)))
-                return rc;
-            KMPB_CUDA(cudaMemcpyAsync(out + written, ctx->d_find_rec[slot], take * sizeof(kmpb_match), cudaMemcpyDeviceToHost, s));
-            KMPB_CUDA(cudaStreamSynchronize(s));
-        }
-        total += n;
-        written += take;
-        return KMPB_OK;
-    };
-    int rc = KMPB_OK;
-    for (uint64_t c = 0; c < n_chunks && !rc; c++) {
-        const int slot = (int)(c % KMPB_COPY_STREAMS);
-        if ((c < (uint64_t)KMPB_COPY_STREAMS && (rc = after_device_calls(ctx, ctx->copy_stream[slot]))) || // first chunk
-            (c >= (uint64_t)KMPB_COPY_STREAMS && (rc = finish(c - KMPB_COPY_STREAMS))) ||
-            (rc = ensure_find_rec(ctx, slot, plan.max_bytes / 256)) || (rc = stage(plan.chunks[c], slot, batch[slot])))
-            break;
-        rc = kmpb_find_match(ctx, batch[slot], slot, ctx->d_find_rec[slot], ctx->find_rec_cap[slot], ctx->d_find_found + slot,
-                             ctx->copy_stream[slot]);
-    }
-    for (uint64_t c = n_chunks > (uint64_t)KMPB_COPY_STREAMS ? n_chunks - KMPB_COPY_STREAMS : 0; c < n_chunks && !rc; c++)
-        rc = finish(c);
-    if (rc) {
-        quiesce(ctx);
-        return rc;
-    }
-    *n_found = total;
-    return KMPB_OK; // (as in finish_chunked: the caller checked every packet's size first)
-}
-
-// Selecting: every chunk's mark kernel and verdict pass run on its slot's stream into the slot's bitmap and verdicts,
-// which are copied to the slot's pinned twin; chunk c's verdicts are copied out (and their packets counted) just before
-// its slot takes chunk c + KMPB_COPY_STREAMS, as find_chunks does with records.  The counts go to the slots'
-// accumulators as in count_chunks; the caller then calls finish_chunked if it wants them.  flags_out[k - k_base] is
-// packet k's verdict.
-template <class Stage>
-int select_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage, uint64_t k_base, uint8_t *flags_out, uint64_t *n_selected)
+// The start of a chunked call or a frame stream: after every device-form call issued before it, ev[0] recorded (where
+// the interval of kmpb_last_timing begins), the slots' distinct-pattern counters zeroed, and the copy streams of the
+// first n_slots slots behind all of that.
+int start_chunks(kmpb_ctx *ctx, int n_slots)
 {
     int rc = after_device_calls(ctx, ctx->stream);
     if (rc) return rc;
     KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
     KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * ctx->host.n_uniq * sizeof(uint64_t), ctx->stream));
     KMPB_CUDA(cudaEventRecord(ctx->ev[2], ctx->stream));
-    for (int s = 0; s < plan.slots(); s++) KMPB_CUDA(cudaStreamWaitEvent(ctx->copy_stream[s], ctx->ev[2], 0));
-    const uint64_t n_chunks = plan.chunks.size();
-    uint64_t selected = 0;
-    auto finish = [&](uint64_t c) -> int {
+    for (int s = 0; s < n_slots; s++) KMPB_CUDA(cudaStreamWaitEvent(ctx->copy_stream[s], ctx->ev[2], 0));
+    return KMPB_OK;
+}
+
+// The chunk pipeline of every host and savefile form.  Chunk c goes to stream slot c % KMPB_COPY_STREAMS: once the
+// slot's previous chunk, c - KMPB_COPY_STREAMS, is retired, the input stages chunk c into the slot's staging buffers
+// and enqueue(batch, slot) puts the operation's work on the slot's stream.  So the copies and kernels of the chunks in
+// between keep the device busy while the host retires a chunk.  The last iterations retire the last chunks.  An
+// operation supplies enqueue and retire(chunk, slot, batch); nothing of the call is left in flight when it returns an
+// error.
+template <class Input, class Enqueue, class Retire>
+int run_chunks(kmpb_ctx *ctx, Input &in, Enqueue &&enqueue, Retire &&retire)
+{
+    const std::vector<chunk> &chunks = in.plan.chunks;
+    kmpb_batch batch[KMPB_COPY_STREAMS] = {};
+    int rc = start_chunks(ctx, in.plan.slots());
+    for (size_t c = 0; c < chunks.size() + KMPB_COPY_STREAMS && !rc; c++) {
         const int slot = (int)(c % KMPB_COPY_STREAMS);
-        KMPB_CUDA(cudaStreamSynchronize(ctx->copy_stream[slot]));
-        const chunk &ch = plan.chunks[c];
-        const uint8_t *f = ctx->h_sel_flags[slot];
-        uint64_t n = 0;
-        for (uint64_t j = 0; j < ch.k1 - ch.k0; j++) n += f[j];
-        memcpy(flags_out + (ch.k0 - k_base), f, ch.k1 - ch.k0);
-        selected += n;
-        return KMPB_OK;
-    };
-    for (uint64_t c = 0; c < n_chunks && !rc; c++) {
-        const int slot = (int)(c % KMPB_COPY_STREAMS);
-        cudaStream_t s = ctx->copy_stream[slot];
-        kmpb_batch b;
-        if ((c >= (uint64_t)KMPB_COPY_STREAMS && (rc = finish(c - KMPB_COPY_STREAMS))) || (rc = stage(plan.chunks[c], slot, b)) ||
-            (rc = kmpb_select_match(ctx, b, slot, ctx->d_sel_flags[slot], s)))
-            break;
-        const cudaError_t e = cudaMemcpyAsync(ctx->h_sel_flags[slot], ctx->d_sel_flags[slot], b.n_packets, cudaMemcpyDeviceToHost, s);
-        if (e != cudaSuccess) rc = kmpb_fail(KMPB_ECUDA, "verdict copy failed: %s", cudaGetErrorString(e));
+        if (c >= (size_t)KMPB_COPY_STREAMS && (rc = retire(chunks[c - KMPB_COPY_STREAMS], slot, batch[slot]))) break;
+        if (c < chunks.size() && !(rc = in.stage(ctx, chunks[c], slot, batch[slot]))) rc = enqueue(batch[slot], slot);
     }
-    for (uint64_t c = n_chunks > (uint64_t)KMPB_COPY_STREAMS ? n_chunks - KMPB_COPY_STREAMS : 0; c < n_chunks && !rc; c++)
-        rc = finish(c);
-    if (rc) {
-        quiesce(ctx);
+    if (rc) quiesce(ctx);
+    return rc;
+}
+
+// The two inputs of the chunked forms.  in_range() checks the packet range; prepare() checks the input, selects the
+// device, plans the chunks (none for an empty input: the call has nothing more to do) and reserves the staging slots;
+// stage() puts a chunk into its slot's device buffers, copies on the slot's stream.  k_base is the packet index of the
+// input's first packet.
+//
+// A host CSR batch: a chunk is copied from the caller's memory, from its 512-byte aligned base (the MPI variant's
+// Scatterv, done by the copy engines instead of the network: mpi_dumping.c:161).
+struct host_input {
+    const uint8_t *bytes;
+    const uint64_t *offsets;
+    uint64_t n; // packets
+    uint64_t k_base = 0;
+    chunk_plan plan;
+
+    int in_range() const { return KMPB_OK; }
+
+    int prepare(kmpb_ctx *ctx)
+    {
+        if (n == 0) return KMPB_OK;
+        if (bytes == nullptr || offsets == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL batch pointer");
+        int rc = check_offsets(offsets, n);
+        if (rc || (rc = use_device(ctx))) return rc;
+        plan = plan_host(offsets, n, chunk_bytes_setting());
+        return reserve(ctx, plan.max_bytes, plan.max_pkts, false);
+    }
+
+    int stage(kmpb_ctx *ctx, const chunk &ch, int slot, kmpb_batch &b)
+    {
+        cudaStream_t s = ctx->copy_stream[slot];
+        const uint64_t k0 = ch.k0, k1 = ch.k1, base = offsets[k0] & ~511ull;
+        uint8_t *d_bytes = ctx->d_stage_bytes[slot].p;
+        uint64_t *d_off = ctx->d_stage_off[slot].p;
+        KMPB_CUDA(cudaMemcpyAsync(d_bytes, bytes + base, offsets[k1] - base, cudaMemcpyHostToDevice, s));
+        KMPB_CUDA(cudaMemcpyAsync(d_off, offsets + k0, (k1 - k0 + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+        b = kmpb_batch{d_bytes, base, d_off, k1 - k0, offsets[k0], offsets[k1]};
+        return KMPB_OK;
+    }
+
+    void report(const char *) const {} // (no waiting or packing to report)
+};
+
+// Accepted packets [k_base, k_base + n) of a savefile: a chunk is packed into the slot's pinned buffers (all host
+// threads), then copied over while the next chunk is packed -- the producer/consumer shape of openmp_task.c:113-178
+// with the GPU as the consumer.  t[0] and t[1] add up the seconds spent waiting for the slot and packing since t0.
+struct pcap_input {
+    const kmpb_pcap *pc;
+    uint64_t k_base, n;
+    chunk_plan plan;
+    double t0 = 0, t[2] = {0, 0};
+
+    int in_range() const
+    {
+        const uint64_t total = kmpb_pcap_packets(pc);
+        if (k_base > total || n > total - k_base) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
+        return KMPB_OK;
+    }
+
+    int prepare(kmpb_ctx *ctx)
+    {
+        int rc = in_range();
+        if (rc || n == 0) return rc;
+        if ((rc = check_pcap_lengths(pc, k_base, n)) || (rc = use_device(ctx))) return rc;
+        plan = plan_pcap(pc, k_base, k_base + n, chunk_bytes_setting());
+        rc = reserve(ctx, plan.max_bytes, plan.max_pkts, true);
+        t0 = now_s();
         return rc;
     }
-    if (n_selected) *n_selected = selected;
+
+    int stage(kmpb_ctx *ctx, const chunk &ch, int slot, kmpb_batch &b)
+    {
+        const uint64_t k = ch.k1 - ch.k0;
+        const double s0 = now_s();
+        const int rc = wait_pinned(ctx, slot);
+        if (rc) return rc;
+        const double s1 = now_s();
+        kmpb_pcap_pack(pc, ch.k0, k, ctx->h_stage_bytes[slot].p, ctx->h_stage_off[slot].p);
+        t[0] += s1 - s0;
+        t[1] += now_s() - s1;
+        return submit_pinned(ctx, slot, k, ctx->h_stage_off[slot].p[k], b);
+    }
+
+    void report(const char *call) const
+    {
+        fprintf(stderr, "%s: %llu chunks; waiting for a free slot %.3f s, packing %.3f s, issuing copies and kernels %.3f s\n",
+                call, (unsigned long long)plan.chunks.size(), t[0], t[1], now_s() - t0 - t[0] - t[1]);
+    }
+};
+
+// Counting: the count engine adds every chunk into its slot's accumulators, finish_chunked sums them.
+template <class Input>
+int count_chunked(kmpb_ctx *ctx, Input &in, uint64_t *counts_out, const char *call)
+{
+    if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL context");
+    if (int rc = no_open_stream(ctx, call)) return rc;
+    if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "count before kmpb_set_patterns");
+    const uint32_t n_pat = ctx->host.n_pat;
+    if (n_pat == 0) return KMPB_OK;
+    if (counts_out == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL counts_out");
+    memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
+    int rc = in.prepare(ctx);
+    if (rc || in.plan.chunks.empty()) return rc;
+    auto enqueue = [&](const kmpb_batch &b, int slot) { return run_engine(ctx, b, slot, ctx->copy_stream[slot]); };
+    auto retire = [](const chunk &, int, const kmpb_batch &) { return KMPB_OK; };
+    if ((rc = run_chunks(ctx, in, enqueue, retire))) return rc;
+    if (getenv("KMPB_STATS")) in.report(call);
+    return finish_chunked(ctx, in.plan.slots(), counts_out);
+}
+
+// the record buffer of a stream slot of the chunked find forms, at least `records` long (grown by an eighth more)
+int ensure_find_rec(kmpb_ctx *ctx, int slot, uint64_t records)
+{
+    kmpb_scratch<kmpb_match> &rec = ctx->d_find_rec[slot];
+    if (rec.p && records <= rec.cap) return KMPB_OK;
+    return rec.reserve(records + records / 8 + 1024);
+}
+
+// the argument checks every find form starts with
+int find_args(kmpb_ctx *ctx, const void *out, uint64_t capacity, const void *n_found, const char *call)
+{
+    if (ctx == nullptr || n_found == nullptr || (out == nullptr && capacity)) return kmpb_fail(KMPB_EINVAL, "NULL argument");
+    if (int rc = no_open_stream(ctx, call)) return rc;
+    if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "find before kmpb_set_patterns");
     return KMPB_OK;
+}
+
+// Finding: the find kernel writes a chunk's records into its slot's buffer, sized for one record per 256 bytes of the
+// largest chunk.  Retiring a chunk reads its match count, then sorts its records and copies them out behind the
+// previous chunk's.  A chunk whose records overflowed the slot's buffer is matched again, from the copy still on the
+// device, into a buffer of the exact size; once `capacity` records are out, later chunks are only counted.
+template <class Input>
+int find_chunked(kmpb_ctx *ctx, Input &in, kmpb_match *out, uint64_t capacity, uint64_t *n_found, const char *call)
+{
+    int rc = find_args(ctx, out, capacity, n_found, call);
+    if (rc) return rc;
+    *n_found = 0;
+    if (ctx->host.n_pat == 0) return KMPB_OK;
+    if ((rc = in.prepare(ctx)) || in.plan.chunks.empty() || (rc = ctx->d_find_found.reserve(KMPB_COPY_STREAMS))) return rc;
+    for (int s = 0; s < in.plan.slots(); s++)
+        if ((rc = ensure_find_rec(ctx, s, in.plan.max_bytes / 256))) return rc;
+    uint64_t total = 0, written = 0;
+    auto enqueue = [&](const kmpb_batch &b, int slot) {
+        return kmpb_find_match(ctx, b, slot, ctx->d_find_rec[slot].p, ctx->d_find_rec[slot].cap, ctx->d_find_found.p + slot,
+                               ctx->copy_stream[slot]);
+    };
+    auto retire = [&](const chunk &ch, int slot, const kmpb_batch &b) -> int {
+        cudaStream_t s = ctx->copy_stream[slot];
+        unsigned long long *found = ctx->d_find_found.p + slot;
+        unsigned long long n = 0;
+        KMPB_CUDA(cudaMemcpyAsync(&n, found, sizeof n, cudaMemcpyDeviceToHost, s));
+        KMPB_CUDA(cudaStreamSynchronize(s));
+        const uint64_t take = std::min<uint64_t>(n, capacity - written);
+        if (take) {
+            int rc2;
+            if (n > ctx->d_find_rec[slot].cap &&
+                ((rc2 = ensure_find_rec(ctx, slot, n)) || (rc2 = kmpb_find_match(ctx, b, slot, ctx->d_find_rec[slot].p, n, found, s))))
+                return rc2;
+            if ((rc2 = kmpb_find_finish(ctx, b, ch.k0, ctx->d_find_rec[slot].p, n, found, true, s))) return rc2;
+            KMPB_CUDA(cudaMemcpyAsync(out + written, ctx->d_find_rec[slot].p, take * sizeof(kmpb_match), cudaMemcpyDeviceToHost, s));
+            KMPB_CUDA(cudaStreamSynchronize(s));
+        }
+        total += n;
+        written += take;
+        return KMPB_OK;
+    };
+    if ((rc = run_chunks(ctx, in, enqueue, retire))) return rc;
+    *n_found = total;
+    return KMPB_OK; // (as in finish_chunked: the input's checks covered every packet's size)
 }
 
 // the bitmaps and verdict buffers of the chunked select forms: those of the slots the plan uses, for chunks of up to
@@ -460,16 +461,10 @@ int select_chunks(kmpb_ctx *ctx, const chunk_plan &plan, Stage &&stage, uint64_t
 int reserve_select(kmpb_ctx *ctx, const chunk_plan &plan)
 {
     for (int s = 0; s < plan.slots(); s++) {
-        if (int rc = kmpb_ensure_mark(ctx, s, plan.max_bytes / 32 + 8, ctx->copy_stream[s])) return rc;
-        if (plan.max_pkts <= ctx->sel_flags_cap[s] && ctx->d_sel_flags[s]) continue;
-        KMPB_CUDA(cudaDeviceSynchronize());
-        cudaFree(ctx->d_sel_flags[s]); ctx->d_sel_flags[s] = nullptr;
-        cudaFreeHost(ctx->h_sel_flags[s]); ctx->h_sel_flags[s] = nullptr;
-        ctx->sel_flags_cap[s] = 0;
-        const uint64_t cap = plan.max_pkts ? plan.max_pkts : 1;
-        KMPB_CUDA(cudaMalloc((void **)&ctx->d_sel_flags[s], cap));
-        KMPB_CUDA(cudaHostAlloc((void **)&ctx->h_sel_flags[s], cap, cudaHostAllocDefault));
-        ctx->sel_flags_cap[s] = cap;
+        int rc;
+        if ((rc = kmpb_ensure_mark(ctx, s, plan.max_bytes / 32 + 8, ctx->copy_stream[s])) ||
+            (rc = ctx->d_sel_flags[s].reserve(plan.max_pkts)) || (rc = ctx->h_sel_flags[s].reserve(plan.max_pkts)))
+            return rc;
     }
     return KMPB_OK;
 }
@@ -483,13 +478,38 @@ int select_args(kmpb_ctx *ctx, const void *flags_out, uint64_t n_packets, const 
     return KMPB_OK;
 }
 
-// the argument checks every find form starts with
-int find_args(kmpb_ctx *ctx, const void *out, uint64_t capacity, const void *n_found, const char *call)
+// Selecting: every chunk's mark kernel and verdict pass run into the slot's bitmap and verdicts, which are copied to the
+// slot's pinned twin; retiring a chunk copies its verdicts out (flags_out[k - k_base] is packet k's) and counts its
+// selected packets.  The counts go to the slots' accumulators as in counting, summed only when counts_out is given.
+// The packet range is checked before any output is written.
+template <class Input>
+int select_chunked(kmpb_ctx *ctx, Input &in, uint8_t *flags_out, uint64_t *n_selected, uint64_t *counts_out, const char *call)
 {
-    if (ctx == nullptr || n_found == nullptr || (out == nullptr && capacity)) return kmpb_fail(KMPB_EINVAL, "NULL argument");
-    if (int rc = no_open_stream(ctx, call)) return rc;
-    if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "find before kmpb_set_patterns");
-    return KMPB_OK;
+    int rc = select_args(ctx, flags_out, in.n, call);
+    if (rc || (rc = in.in_range())) return rc;
+    const uint32_t n_pat = ctx->host.n_pat;
+    if (n_selected) *n_selected = 0;
+    if (counts_out) memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
+    if (in.n) memset(flags_out, 0, in.n);
+    if (n_pat == 0) return KMPB_OK;
+    if ((rc = in.prepare(ctx)) || in.plan.chunks.empty() || (rc = reserve_select(ctx, in.plan))) return rc;
+    uint64_t selected = 0;
+    auto enqueue = [&](const kmpb_batch &b, int slot) -> int {
+        cudaStream_t s = ctx->copy_stream[slot];
+        if (int rc2 = kmpb_select_match(ctx, b, slot, ctx->d_sel_flags[slot].p, s)) return rc2;
+        const cudaError_t e = cudaMemcpyAsync(ctx->h_sel_flags[slot].p, ctx->d_sel_flags[slot].p, b.n_packets, cudaMemcpyDeviceToHost, s);
+        return e == cudaSuccess ? KMPB_OK : kmpb_fail(KMPB_ECUDA, "verdict copy failed: %s", cudaGetErrorString(e));
+    };
+    auto retire = [&](const chunk &ch, int slot, const kmpb_batch &) -> int {
+        KMPB_CUDA(cudaStreamSynchronize(ctx->copy_stream[slot]));
+        const uint8_t *f = ctx->h_sel_flags[slot].p;
+        for (uint64_t j = 0; j < ch.k1 - ch.k0; j++) selected += f[j];
+        memcpy(flags_out + (ch.k0 - in.k_base), f, ch.k1 - ch.k0);
+        return KMPB_OK;
+    };
+    if ((rc = run_chunks(ctx, in, enqueue, retire))) return rc;
+    if (n_selected) *n_selected = selected;
+    return counts_out ? finish_chunked(ctx, in.plan.slots(), counts_out) : KMPB_OK;
 }
 
 } // namespace
@@ -519,14 +539,14 @@ int kmpb_check_device_errors(kmpb_ctx *ctx)
     int rc = use_device(ctx);
     if (rc) return rc;
     KMPB_CUDA(cudaDeviceSynchronize());
-    if (ctx->d_work == nullptr) return KMPB_OK;
+    if (ctx->d_work.p == nullptr) return KMPB_OK;
     // the union engine's error flags, word 1 of every slot's work counters: set by its kernels, cleared only here
     uint32_t work[KMPB_COPY_STREAMS * 4];
-    KMPB_CUDA(cudaMemcpy(work, ctx->d_work, sizeof work, cudaMemcpyDeviceToHost));
+    KMPB_CUDA(cudaMemcpy(work, ctx->d_work.p, sizeof work, cudaMemcpyDeviceToHost));
     bool flagged = false;
     for (int s = 0; s < KMPB_COPY_STREAMS; s++) flagged |= work[s * 4 + 1] != 0;
     if (!flagged) return KMPB_OK;
-    KMPB_CUDA(cudaMemset(ctx->d_work, 0, sizeof work));
+    KMPB_CUDA(cudaMemset(ctx->d_work.p, 0, sizeof work));
     return kmpb_fail(KMPB_ELIMIT, "a device-form batch held a packet of %llu bytes (2 GiB - 1 MiB) or more: its results are "
                      "unspecified", KMPB_PACKET_LIMIT);
 }
@@ -563,22 +583,22 @@ void kmpb_destroy(kmpb_ctx *ctx)
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
     kmpb_release_tables(ctx);
-    cudaFree(ctx->d_work);
-    cudaFree(ctx->d_items);
-    cudaFree(ctx->d_find_found);
-    cudaFree(ctx->d_sort_keys[0]);
-    cudaFree(ctx->d_sort_keys[1]);
-    cudaFree(ctx->d_sort_temp);
-    cudaFree(ctx->d_select_temp);
+    ctx->d_work.release();
+    ctx->d_items.release();
+    ctx->d_find_found.release();
+    ctx->d_sort_keys[0].release();
+    ctx->d_sort_keys[1].release();
+    ctx->d_sort_temp.release();
+    ctx->d_select_temp.release();
     for (int i = 0; i < KMPB_COPY_STREAMS; i++) {
-        cudaFree(ctx->d_mark[i]);
-        cudaFree(ctx->d_sel_flags[i]);
-        cudaFreeHost(ctx->h_sel_flags[i]);
-        cudaFree(ctx->d_find_rec[i]);
-        cudaFree(ctx->d_stage_bytes[i]);
-        cudaFree(ctx->d_stage_off[i]);
-        cudaFreeHost(ctx->h_stage_bytes[i]);
-        cudaFreeHost(ctx->h_stage_off[i]);
+        ctx->d_mark[i].release();
+        ctx->d_sel_flags[i].release();
+        ctx->h_sel_flags[i].release();
+        ctx->d_find_rec[i].release();
+        ctx->d_stage_bytes[i].release();
+        ctx->d_stage_off[i].release();
+        ctx->h_stage_bytes[i].release();
+        ctx->h_stage_off[i].release();
         if (ctx->ev_h2d[i]) cudaEventDestroy(ctx->ev_h2d[i]);
         if (ctx->copy_stream[i]) cudaStreamDestroy(ctx->copy_stream[i]);
     }
@@ -745,33 +765,13 @@ int kmpb_count_device(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t *d_o
     return kmpb_count_device_span(ctx, d_bytes, d_offsets, n_packets, span[0], span[1], d_counts, stream_v);
 }
 
-// Host batch: chunks of whole packets are copied to per-stream staging buffers and matched there, so
-// the H2D copy of chunk c+1.. overlaps the kernels of chunk c (the MPI variant's Scatterv, done by
-// the copy engines instead of the network: mpi_dumping.c:161).
 int kmpb_count_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, uint64_t n_packets,
                     uint64_t *counts_out)
 {
-    if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL context");
-    if (int rc = no_open_stream(ctx, "kmpb_count_host")) return rc;
-    if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "count before kmpb_set_patterns");
-    const uint32_t n_pat = ctx->host.n_pat;
-    if (n_pat == 0) return KMPB_OK;
-    if (counts_out == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL counts_out");
-    memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
-    if (n_packets == 0) return KMPB_OK;
-    if (bytes == nullptr || offsets == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL batch pointer");
-    int rc = check_offsets(offsets, n_packets);
-    if (rc) return rc;
-    if ((rc = use_device(ctx))) return rc;
-    const chunk_plan plan = plan_host(offsets, n_packets, chunk_bytes_setting());
-    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_host(ctx, bytes, offsets, ch, slot, b); };
-    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, false)) || (rc = count_chunks(ctx, plan, stage))) return rc;
-    return finish_chunked(ctx, plan.slots(), counts_out);
+    host_input in{bytes, offsets, n_packets};
+    return count_chunked(ctx, in, counts_out, "kmpb_count_host");
 }
 
-// Streamed savefile path: pack a chunk of payloads into a pinned staging slot (all host threads), copy
-// it to the slot's device twin and match it on the slot's stream while the next chunk is packed -- the
-// producer/consumer shape of openmp_task.c:113-178 with the GPU as the consumer.
 int kmpb_reserve_staging(kmpb_ctx *ctx, uint64_t max_batch_bytes, uint64_t max_packets)
 {
     if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
@@ -786,28 +786,8 @@ int kmpb_reserve_staging(kmpb_ctx *ctx, uint64_t max_batch_bytes, uint64_t max_p
 int kmpb_count_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count, uint64_t *counts_out)
 {
     if (ctx == nullptr || pc == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
-    if (int rc = no_open_stream(ctx, "kmpb_count_pcap")) return rc;
-    if (!ctx->have_tables) return kmpb_fail(KMPB_ESTATE, "count before kmpb_set_patterns");
-    const uint32_t n_pat = ctx->host.n_pat;
-    if (n_pat == 0) return KMPB_OK;
-    if (counts_out == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL counts_out");
-    memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
-    const uint64_t total = kmpb_pcap_packets(pc);
-    if (first > total || count > total - first) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
-    if (count == 0) return KMPB_OK;
-    int rc = check_pcap_lengths(pc, first, count);
-    if (rc) return rc;
-    if ((rc = use_device(ctx))) return rc;
-    const chunk_plan plan = plan_pcap(pc, first, first + count, chunk_bytes_setting());
-    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, true))) return rc;
-    double t[2] = {0, 0}; // waiting for a free slot, packing
-    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_pcap(ctx, pc, ch, slot, b, t); };
-    const double t0 = now_s();
-    if ((rc = count_chunks(ctx, plan, stage))) return rc;
-    if (getenv("KMPB_STATS"))
-        fprintf(stderr, "kmpb_count_pcap: %llu chunks; waiting for a free slot %.3f s, packing %.3f s, issuing copies and kernels %.3f s\n",
-                (unsigned long long)plan.chunks.size(), t[0], t[1], now_s() - t0 - t[0] - t[1]);
-    return finish_chunked(ctx, plan.slots(), counts_out);
+    pcap_input in{pc, first, count};
+    return count_chunked(ctx, in, counts_out, "kmpb_count_pcap");
 }
 
 // ---- find: where the patterns occur (include/kmpb200.h; kernels in union_kernel.cu and find.cu) ----------------
@@ -834,37 +814,16 @@ int kmpb_find_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_t 
 int kmpb_find_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, uint64_t n_packets,
                    kmpb_match *out, uint64_t capacity, uint64_t *n_found)
 {
-    int rc = find_args(ctx, out, capacity, n_found, "kmpb_find_host");
-    if (rc) return rc;
-    *n_found = 0;
-    if (ctx->host.n_pat == 0 || n_packets == 0) return KMPB_OK;
-    if (bytes == nullptr || offsets == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL batch pointer");
-    if ((rc = check_offsets(offsets, n_packets))) return rc;
-    if ((rc = use_device(ctx))) return rc;
-    const chunk_plan plan = plan_host(offsets, n_packets, chunk_bytes_setting());
-    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, false))) return rc;
-    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_host(ctx, bytes, offsets, ch, slot, b); };
-    return find_chunks(ctx, plan, stage, out, capacity, n_found);
+    host_input in{bytes, offsets, n_packets};
+    return find_chunked(ctx, in, out, capacity, n_found, "kmpb_find_host");
 }
 
 int kmpb_find_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count, kmpb_match *out, uint64_t capacity,
                    uint64_t *n_found)
 {
     if (pc == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
-    int rc = find_args(ctx, out, capacity, n_found, "kmpb_find_pcap");
-    if (rc) return rc;
-    *n_found = 0;
-    if (ctx->host.n_pat == 0) return KMPB_OK;
-    const uint64_t total = kmpb_pcap_packets(pc);
-    if (first > total || count > total - first) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
-    if (count == 0) return KMPB_OK;
-    if ((rc = check_pcap_lengths(pc, first, count))) return rc;
-    if ((rc = use_device(ctx))) return rc;
-    const chunk_plan plan = plan_pcap(pc, first, first + count, chunk_bytes_setting());
-    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, true))) return rc;
-    double t[2] = {0, 0};
-    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_pcap(ctx, pc, ch, slot, b, t); };
-    return find_chunks(ctx, plan, stage, out, capacity, n_found);
+    pcap_input in{pc, first, count};
+    return find_chunked(ctx, in, out, capacity, n_found, "kmpb_find_pcap");
 }
 
 // ---- select: which packets match (include/kmpb200.h; kernels in union_kernel.cu and select.cu) ------------------
@@ -896,44 +855,16 @@ int kmpb_select_device_span(kmpb_ctx *ctx, const uint8_t *d_bytes, const uint64_
 int kmpb_select_host(kmpb_ctx *ctx, const uint8_t *bytes, const uint64_t *offsets, uint64_t n_packets, uint8_t *flags_out,
                      uint64_t *n_selected, uint64_t *counts_out)
 {
-    int rc = select_args(ctx, flags_out, n_packets, "kmpb_select_host");
-    if (rc) return rc;
-    const uint32_t n_pat = ctx->host.n_pat;
-    if (n_selected) *n_selected = 0;
-    if (counts_out) memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
-    if (n_packets) memset(flags_out, 0, n_packets);
-    if (n_pat == 0 || n_packets == 0) return KMPB_OK;
-    if (bytes == nullptr || offsets == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL batch pointer");
-    if ((rc = check_offsets(offsets, n_packets)) || (rc = use_device(ctx))) return rc;
-    const chunk_plan plan = plan_host(offsets, n_packets, chunk_bytes_setting());
-    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, false)) || (rc = reserve_select(ctx, plan)))
-        return rc;
-    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_host(ctx, bytes, offsets, ch, slot, b); };
-    if ((rc = select_chunks(ctx, plan, stage, 0, flags_out, n_selected))) return rc;
-    return counts_out ? finish_chunked(ctx, plan.slots(), counts_out) : KMPB_OK;
+    host_input in{bytes, offsets, n_packets};
+    return select_chunked(ctx, in, flags_out, n_selected, counts_out, "kmpb_select_host");
 }
 
 int kmpb_select_pcap(kmpb_ctx *ctx, const kmpb_pcap *pc, uint64_t first, uint64_t count, uint8_t *flags_out,
                      uint64_t *n_selected, uint64_t *counts_out)
 {
     if (pc == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL argument");
-    int rc = select_args(ctx, flags_out, count, "kmpb_select_pcap");
-    if (rc) return rc;
-    const uint64_t total = kmpb_pcap_packets(pc);
-    if (first > total || count > total - first) return kmpb_fail(KMPB_EINVAL, "packet range outside the file");
-    const uint32_t n_pat = ctx->host.n_pat;
-    if (n_selected) *n_selected = 0;
-    if (counts_out) memset(counts_out, 0, (size_t)n_pat * sizeof(uint64_t));
-    if (count) memset(flags_out, 0, count);
-    if (n_pat == 0 || count == 0) return KMPB_OK;
-    if ((rc = check_pcap_lengths(pc, first, count)) || (rc = use_device(ctx))) return rc;
-    const chunk_plan plan = plan_pcap(pc, first, first + count, chunk_bytes_setting());
-    if ((rc = reserve(ctx, plan.max_bytes, plan.max_pkts, true)) || (rc = reserve_select(ctx, plan)))
-        return rc;
-    double t[2] = {0, 0};
-    auto stage = [&](const chunk &ch, int slot, kmpb_batch &b) { return stage_pcap(ctx, pc, ch, slot, b, t); };
-    if ((rc = select_chunks(ctx, plan, stage, first, flags_out, n_selected))) return rc;
-    return counts_out ? finish_chunked(ctx, plan.slots(), counts_out) : KMPB_OK;
+    pcap_input in{pc, first, count};
+    return select_chunked(ctx, in, flags_out, n_selected, counts_out, "kmpb_select_pcap");
 }
 
 // ---- frames pushed one at a time (the live-capture shape) ----------------------------------------
@@ -951,7 +882,7 @@ static int stream_submit(kmpb_stream *st)
     kmpb_ctx *ctx = st->ctx;
     if (st->n == 0) return KMPB_OK;
     const int slot = st->slot;
-    ctx->h_stage_off[slot][st->n] = st->bytes;
+    ctx->h_stage_off[slot].p[st->n] = st->bytes;
     kmpb_batch b;
     int rc;
     if ((rc = submit_pinned(ctx, slot, st->n, st->bytes, b)) ||
@@ -975,11 +906,7 @@ int kmpb_stream_open(kmpb_ctx *ctx, int proto, uint64_t batch_bytes, kmpb_stream
     if (batch_bytes == 0) batch_bytes = 8ull << 20;
     if (batch_bytes < 65536) batch_bytes = 65536; // a frame's payload is at most 65535 - headers bytes long... jumbo included
     const uint64_t max_pkts = 1ull << 20;
-    if ((rc = reserve(ctx, batch_bytes, max_pkts, true))) return rc;
-    const uint32_t nu = ctx->host.n_uniq;
-    if ((rc = after_device_calls(ctx, ctx->stream))) return rc;
-    KMPB_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
-    KMPB_CUDA(cudaMemsetAsync(ctx->d_uniq_counts, 0, (size_t)KMPB_COPY_STREAMS * (nu ? nu : 1) * sizeof(uint64_t), ctx->stream));
+    if ((rc = reserve(ctx, batch_bytes, max_pkts, true)) || (rc = start_chunks(ctx, KMPB_COPY_STREAMS))) return rc;
     KMPB_CUDA(cudaStreamSynchronize(ctx->stream));
     kmpb_stream *st = new (std::nothrow) kmpb_stream();
     if (st == nullptr) return kmpb_fail(KMPB_ENOMEM, "out of memory");
@@ -1009,8 +936,8 @@ int kmpb_stream_push(kmpb_stream *st, const uint8_t *frame, uint32_t captured_le
     if (st->bytes + len > st->batch_bytes || st->n == st->max_pkts)
         if ((rc = stream_submit(st))) return rc;
     kmpb_ctx *ctx = st->ctx;
-    ctx->h_stage_off[st->slot][st->n] = st->bytes;
-    memcpy(ctx->h_stage_bytes[st->slot] + st->bytes, frame + off, len);
+    ctx->h_stage_off[st->slot].p[st->n] = st->bytes;
+    memcpy(ctx->h_stage_bytes[st->slot].p + st->bytes, frame + off, len);
     st->n++;
     st->bytes += len;
     st->packets++;

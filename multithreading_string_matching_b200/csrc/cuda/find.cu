@@ -87,25 +87,12 @@ int grid_for(const kmpb_ctx *ctx, uint64_t n)
 // the sort's key buffers (two of `items` keys) and CUB's temporary storage, grown on demand
 int ensure_sort_scratch(kmpb_ctx *ctx, uint64_t items, uint32_t end_bit, cudaStream_t stream)
 {
-    if (items > ctx->sort_cap) {
-        cudaFree(ctx->d_sort_keys[0]); cudaFree(ctx->d_sort_keys[1]);
-        ctx->d_sort_keys[0] = ctx->d_sort_keys[1] = nullptr;
-        ctx->sort_cap = 0;
-        KMPB_CUDA(cudaMalloc((void **)&ctx->d_sort_keys[0], items * sizeof(uint64_t)));
-        KMPB_CUDA(cudaMalloc((void **)&ctx->d_sort_keys[1], items * sizeof(uint64_t)));
-        ctx->sort_cap = items;
-    }
-    cub::DoubleBuffer<uint64_t> db(ctx->d_sort_keys[0], ctx->d_sort_keys[1]);
+    int rc;
+    if ((rc = ctx->d_sort_keys[0].reserve(items)) || (rc = ctx->d_sort_keys[1].reserve(items))) return rc;
+    cub::DoubleBuffer<uint64_t> db(ctx->d_sort_keys[0].p, ctx->d_sort_keys[1].p);
     size_t need = 0;
     KMPB_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, need, db, (int)items, 0, (int)end_bit, stream));
-    if (need > ctx->sort_temp_bytes) {
-        cudaFree(ctx->d_sort_temp);
-        ctx->d_sort_temp = nullptr;
-        ctx->sort_temp_bytes = 0;
-        KMPB_CUDA(cudaMalloc(&ctx->d_sort_temp, need));
-        ctx->sort_temp_bytes = need;
-    }
-    return KMPB_OK;
+    return ctx->d_sort_temp.reserve(need);
 }
 
 } // namespace
@@ -142,11 +129,11 @@ int kmpb_find_finish(kmpb_ctx *ctx, const kmpb_batch &b, uint64_t packet_base, k
     int rc = ensure_sort_scratch(ctx, capacity, (uint32_t)bits, stream);
     if (rc) return rc;
     kmpb_find_keys_kernel<<<grid_for(ctx, capacity), FIND_THREADS, 0, stream>>>(d_rec, capacity, d_found, b.first_byte, pbits,
-                                                                                ctx->dev.uniq_first, ctx->d_sort_keys[0]);
+                                                                                ctx->dev.uniq_first, ctx->d_sort_keys[0].p);
     KMPB_CUDA(cudaGetLastError());
-    cub::DoubleBuffer<uint64_t> db(ctx->d_sort_keys[0], ctx->d_sort_keys[1]);
-    size_t temp = ctx->sort_temp_bytes;
-    KMPB_CUDA(cub::DeviceRadixSort::SortKeys(ctx->d_sort_temp, temp, db, (int)capacity, 0, bits, stream));
+    cub::DoubleBuffer<uint64_t> db(ctx->d_sort_keys[0].p, ctx->d_sort_keys[1].p);
+    size_t temp = ctx->d_sort_temp.cap;
+    KMPB_CUDA(cub::DeviceRadixSort::SortKeys(ctx->d_sort_temp.p, temp, db, (int)capacity, 0, bits, stream));
     kmpb_locate_keys_kernel<<<grid_for(ctx, capacity), FIND_THREADS, 0, stream>>>(db.Current(), capacity, d_found, b.first_byte, pbits,
                                                                                   b.d_offsets, b.n_packets, packet_base, d_rec);
     ctx->launches += 3;

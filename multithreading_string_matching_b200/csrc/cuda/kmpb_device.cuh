@@ -14,8 +14,50 @@
                              __FILE__, __LINE__);                                                \
     } while (0)
 
-constexpr int KMPB_COPY_STREAMS = 4;          // H2D chunk pipeline depth of kmpb_count_host
+constexpr int KMPB_COPY_STREAMS = 4;          // stream slots of the chunk pipeline of the host and savefile forms
 constexpr uint32_t KMPB_SMEM_COUNTS_MAX = 4096; // distinct patterns counted in shared memory; above: global atomics
+
+// Per-context scratch that grows on demand: p holds cap elements of T, in device memory (pinned host memory when
+// PINNED); cap is 0 exactly when p is null.  reserve(n) keeps a buffer that holds n elements already.  Otherwise it
+// synchronises the device (a call in flight may still use the old buffer), frees the old buffer and allocates n
+// elements, whose contents are undefined.  With `zero` (device buffers) they are zero before it returns: the zeros go
+// out on the legacy default stream, which the context's non-blocking streams do not wait for, so it waits for them
+// itself.  A failure leaves the buffer null with capacity 0.
+template <class T, bool PINNED = false>
+struct kmpb_scratch {
+    T *p = nullptr;
+    uint64_t cap = 0;
+
+    int reserve(uint64_t n, bool zero = false)
+    {
+        if (p && n <= cap) return KMPB_OK;
+        if (p) {
+            KMPB_CUDA(cudaDeviceSynchronize());
+            release();
+        }
+        const size_t bytes = n * sizeof(T);
+        void *q = nullptr;
+        cudaError_t e = PINNED ? cudaHostAlloc(&q, bytes, cudaHostAllocDefault) : cudaMalloc(&q, bytes);
+        if (e != cudaSuccess)
+            return kmpb_fail(KMPB_ECUDA, "allocating %zu bytes of %s scratch failed: %s", bytes, PINNED ? "pinned" : "device",
+                             cudaGetErrorString(e));
+        p = static_cast<T *>(q);
+        cap = n;
+        if (zero && ((e = cudaMemsetAsync(p, 0, bytes, 0)) != cudaSuccess || (e = cudaStreamSynchronize(0)) != cudaSuccess)) {
+            release();
+            return kmpb_fail(KMPB_ECUDA, "zeroing %zu bytes of scratch failed: %s", bytes, cudaGetErrorString(e));
+        }
+        return KMPB_OK;
+    }
+
+    void release()
+    {
+        if (PINNED) cudaFreeHost(p);
+        else cudaFree(p);
+        p = nullptr;
+        cap = 0;
+    }
+};
 
 // Device-resident tables of one pattern set (device pointers).
 struct kmpb_device_tables {
@@ -42,7 +84,7 @@ struct kmpb_ctx {
     int engine = KMPB_ENGINE_AUTO;
     size_t smem_optin = 0;
     cudaStream_t stream = nullptr;                      // default stream of the context
-    cudaStream_t copy_stream[KMPB_COPY_STREAMS] = {};   // H2D + kernel pipeline of kmpb_count_host
+    cudaStream_t copy_stream[KMPB_COPY_STREAMS] = {};   // copies + kernels of one stream slot (chunk pipeline, frame stream)
     cudaEvent_t ev[4] = {};
     cudaEvent_t ev_kernel[2] = {};                      // around the dominant kernel when profile is on
     cudaEvent_t ev_dev = nullptr;                       // after the last device-form call's work, on its stream
@@ -51,38 +93,30 @@ struct kmpb_ctx {
     kmpb_tables host = {};
     bool have_tables = false;
     kmpb_device_tables dev;
+    uint64_t *d_uniq_counts = nullptr;   // [n_uniq] per-launch accumulators (per stream slot), with the tables
+    uint64_t *d_counts = nullptr;        // [n_pat] counts of the last finished chunked call (kmpb_device_counts)
     // scratch, grown on demand
-    uint64_t *d_uniq_counts = nullptr;   // [n_uniq] per-launch accumulators (per stream slot)
-    uint32_t *d_work = nullptr;          // work counters (per stream slot)
-    uint32_t *d_items = nullptr;         // item -> first packet table (per stream slot)
-    size_t items_cap = 0;                // entries per slot
-    uint8_t *d_stage_bytes[KMPB_COPY_STREAMS] = {};
-    uint64_t *d_stage_off[KMPB_COPY_STREAMS] = {};
-    size_t stage_bytes_cap = 0, stage_off_cap = 0;
-    // pinned twins of the staging slots for the streamed savefile path (kmpb_count_pcap)
-    uint8_t *h_stage_bytes[KMPB_COPY_STREAMS] = {};
-    uint64_t *h_stage_off[KMPB_COPY_STREAMS] = {};
-    size_t h_stage_bytes_cap = 0, h_stage_off_cap = 0;
+    kmpb_scratch<uint32_t> d_work;       // work counters, 4 words per stream slot (word 1: error flags)
+    kmpb_scratch<uint32_t> d_items;      // item -> first packet table, cap / KMPB_COPY_STREAMS entries per stream slot
+    // the staging slots of the host and savefile forms and the frame stream, and their pinned twins, into which
+    // savefile chunks and pushed frames are packed first
+    kmpb_scratch<uint8_t> d_stage_bytes[KMPB_COPY_STREAMS];
+    kmpb_scratch<uint64_t> d_stage_off[KMPB_COPY_STREAMS];
+    kmpb_scratch<uint8_t, true> h_stage_bytes[KMPB_COPY_STREAMS];
+    kmpb_scratch<uint64_t, true> h_stage_off[KMPB_COPY_STREAMS];
     cudaEvent_t ev_h2d[KMPB_COPY_STREAMS] = {};
-    uint64_t *d_counts = nullptr;        // [n_pat] result of kmpb_count_host
     // find: record buffers and found counters of the chunked forms (per stream slot), the sort's keys and CUB scratch
-    kmpb_match *d_find_rec[KMPB_COPY_STREAMS] = {};
-    uint64_t find_rec_cap[KMPB_COPY_STREAMS] = {};
-    unsigned long long *d_find_found = nullptr; // [KMPB_COPY_STREAMS]
-    uint64_t *d_sort_keys[2] = {};
-    uint64_t sort_cap = 0;
-    void *d_sort_temp = nullptr;
-    size_t sort_temp_bytes = 0;
+    kmpb_scratch<kmpb_match> d_find_rec[KMPB_COPY_STREAMS];
+    kmpb_scratch<unsigned long long> d_find_found; // [KMPB_COPY_STREAMS]
+    kmpb_scratch<uint64_t> d_sort_keys[2];
+    kmpb_scratch<uint8_t> d_sort_temp;
     // select: the start-position bitmaps (per stream slot: one bit per payload byte, all zero between calls), the
     // verdicts of the chunked forms (per slot, device and pinned host), the compaction's CUB scratch
-    uint32_t *d_mark[KMPB_COPY_STREAMS] = {};
-    uint64_t mark_words_cap[KMPB_COPY_STREAMS] = {};
+    kmpb_scratch<uint32_t> d_mark[KMPB_COPY_STREAMS];
     bool mark_dirty[KMPB_COPY_STREAMS] = {};   // a call failed after its mark kernel: the bitmap may hold bits
-    uint8_t *d_sel_flags[KMPB_COPY_STREAMS] = {};
-    uint8_t *h_sel_flags[KMPB_COPY_STREAMS] = {};
-    uint64_t sel_flags_cap[KMPB_COPY_STREAMS] = {};
-    void *d_select_temp = nullptr;
-    size_t select_temp_bytes = 0;
+    kmpb_scratch<uint8_t> d_sel_flags[KMPB_COPY_STREAMS];
+    kmpb_scratch<uint8_t, true> h_sel_flags[KMPB_COPY_STREAMS];
+    kmpb_scratch<uint8_t> d_select_temp;
     bool attr_union_set = false, attr_perpat_set = false; // per-device function attributes
     uint64_t launches = 0;
     double last_ms[2] = {0, 0};

@@ -115,14 +115,9 @@ uint64_t kmpb_mark_words(const kmpb_batch &b)
 int kmpb_ensure_mark(kmpb_ctx *ctx, int slot, uint64_t words, cudaStream_t stream)
 {
     words = (words + 3) & ~3ull;
-    if (words > ctx->mark_words_cap[slot] || !ctx->d_mark[slot]) {
-        KMPB_CUDA(cudaDeviceSynchronize()); // a call in flight may still be reading the old one
-        cudaFree(ctx->d_mark[slot]);
-        ctx->d_mark[slot] = nullptr;
-        ctx->mark_words_cap[slot] = 0;
-        const uint64_t cap = words > 4 ? words : 4;
-        KMPB_CUDA(cudaMalloc((void **)&ctx->d_mark[slot], cap * sizeof(uint32_t)));
-        ctx->mark_words_cap[slot] = cap;
+    kmpb_scratch<uint32_t> &mark = ctx->d_mark[slot];
+    if (words > mark.cap || !mark.p) {
+        if (int rc = mark.reserve(words > 4 ? words : 4)) return rc;
         ctx->mark_dirty[slot] = true; // zeroed below on `stream`, ahead of the mark kernel that runs there
     }
     // (cudaMemset would run on the legacy default stream, which the context's non-blocking streams do not wait for: the
@@ -130,7 +125,7 @@ int kmpb_ensure_mark(kmpb_ctx *ctx, int slot, uint64_t words, cudaStream_t strea
     // theirs as well.
     if (ctx->mark_dirty[slot]) {
         KMPB_CUDA(cudaStreamWaitEvent(stream, ctx->ev_dev, 0));
-        KMPB_CUDA(cudaMemsetAsync(ctx->d_mark[slot], 0, ctx->mark_words_cap[slot] * sizeof(uint32_t), stream));
+        KMPB_CUDA(cudaMemsetAsync(mark.p, 0, mark.cap * sizeof(uint32_t), stream));
         ctx->mark_dirty[slot] = false;
     }
     return KMPB_OK;
@@ -146,10 +141,10 @@ int kmpb_select_match(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint8_t *d_f
     int rc = kmpb_ensure_mark(ctx, slot, words, stream);
     if (rc) return rc;
     ctx->mark_dirty[slot] = true; // until the verdict pass is on its way
-    if ((rc = kmpb_launch_union(ctx, b, slot, ctx->d_uniq_counts + (size_t)slot * h.n_uniq, stream, out, nullptr, ctx->d_mark[slot])))
+    if ((rc = kmpb_launch_union(ctx, b, slot, ctx->d_uniq_counts + (size_t)slot * h.n_uniq, stream, out, nullptr, ctx->d_mark[slot].p)))
         return rc;
     const uint64_t blocks = (words + VERDICT_TILE - 1) / VERDICT_TILE;
-    kmpb_verdict_kernel<<<(unsigned)blocks, VERDICT_THREADS, 0, stream>>>(ctx->d_mark[slot], words, b.first_byte & ~31ull,
+    kmpb_verdict_kernel<<<(unsigned)blocks, VERDICT_THREADS, 0, stream>>>(ctx->d_mark[slot].p, words, b.first_byte & ~31ull,
                                                                          b.d_offsets, b.n_packets, d_flags);
     ctx->launches++;
     KMPB_CUDA(cudaGetLastError());
@@ -171,17 +166,10 @@ int kmpb_select_compact(kmpb_ctx *ctx, const uint8_t *d_flags, uint64_t n_packet
     size_t need = 0;
     if (d_index) KMPB_CUDA(cub::DeviceSelect::If(nullptr, need, in, d_index, d_n_selected, n, pred, stream));
     else KMPB_CUDA(cub::DeviceSelect::If(nullptr, need, in, thrust::discard_iterator<>(), d_n_selected, n, pred, stream));
-    if (need > ctx->select_temp_bytes) {
-        KMPB_CUDA(cudaDeviceSynchronize()); // a call in flight may still be using the old one
-        cudaFree(ctx->d_select_temp);
-        ctx->d_select_temp = nullptr;
-        ctx->select_temp_bytes = 0;
-        KMPB_CUDA(cudaMalloc(&ctx->d_select_temp, need));
-        ctx->select_temp_bytes = need;
-    }
-    size_t temp = ctx->select_temp_bytes;
-    if (d_index) KMPB_CUDA(cub::DeviceSelect::If(ctx->d_select_temp, temp, in, d_index, d_n_selected, n, pred, stream));
-    else KMPB_CUDA(cub::DeviceSelect::If(ctx->d_select_temp, temp, in, thrust::discard_iterator<>(), d_n_selected, n, pred, stream));
+    if (int rc = ctx->d_select_temp.reserve(need)) return rc;
+    size_t temp = ctx->d_select_temp.cap;
+    if (d_index) KMPB_CUDA(cub::DeviceSelect::If(ctx->d_select_temp.p, temp, in, d_index, d_n_selected, n, pred, stream));
+    else KMPB_CUDA(cub::DeviceSelect::If(ctx->d_select_temp.p, temp, in, thrust::discard_iterator<>(), d_n_selected, n, pred, stream));
     ctx->launches += 2;
     return KMPB_OK;
 }

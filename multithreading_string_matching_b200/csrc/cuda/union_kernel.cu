@@ -1275,18 +1275,9 @@ __global__ void __launch_bounds__(UN_THREADS, 1) kmpb_union_mark_nocase_kernel(c
 // scratch for batches of up to max_batch_bytes: work counters and the item table, one set per slot
 int kmpb_union_scratch(kmpb_ctx *ctx, uint64_t max_batch_bytes)
 {
-    size_t need = (size_t)(max_batch_bytes / UN_ITEM_BYTES) + UN_TAIL_ITEMS + 8;
-    if (need <= ctx->items_cap && ctx->d_items && ctx->d_work) return KMPB_OK;
-    cudaFree(ctx->d_items);
-    ctx->d_items = nullptr;
-    ctx->items_cap = 0;
-    if (!ctx->d_work) {
-        KMPB_CUDA(cudaMalloc((void **)&ctx->d_work, KMPB_COPY_STREAMS * 4 * sizeof(uint32_t)));
-        KMPB_CUDA(cudaMemset(ctx->d_work, 0, KMPB_COPY_STREAMS * 4 * sizeof(uint32_t))); // no error flags yet
-    }
-    KMPB_CUDA(cudaMalloc((void **)&ctx->d_items, (size_t)KMPB_COPY_STREAMS * need * sizeof(uint32_t)));
-    ctx->items_cap = need;
-    return KMPB_OK;
+    const size_t need = (size_t)(max_batch_bytes / UN_ITEM_BYTES) + UN_TAIL_ITEMS + 8;
+    const int rc = ctx->d_work.reserve(KMPB_COPY_STREAMS * 4, true); // no error flags yet
+    return rc ? rc : ctx->d_items.reserve((uint64_t)KMPB_COPY_STREAMS * need);
 }
 
 #ifdef KMPB_UN_STATS
@@ -1329,9 +1320,10 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     const uint32_t n_big = (uint32_t)(whole - tail_items);
     const uint64_t small_span = span - (uint64_t)n_big * item_bytes;
     const uint32_t n_items = n_big + (uint32_t)((small_span + small_bytes - 1) / small_bytes);
-    if ((size_t)n_items + 1 > ctx->items_cap) return kmpb_fail(KMPB_ESTATE, "union scratch too small");
-    uint32_t *d_items = ctx->d_items + (size_t)slot * ctx->items_cap;
-    uint32_t *d_work = ctx->d_work + slot * 4;
+    const uint64_t items_per_slot = ctx->d_items.cap / KMPB_COPY_STREAMS;
+    if ((uint64_t)n_items + 1 > items_per_slot) return kmpb_fail(KMPB_ESTATE, "union scratch too small");
+    uint32_t *d_items = ctx->d_items.p + slot * items_per_slot;
+    uint32_t *d_work = ctx->d_work.p + slot * 4;
 
     // the counters and the probe tables go into shared memory if the block's 227 KB allow it
     const bool counts_in_smem = UN_SMEM_FIXED + 4ull * h.n_uniq + 16 <= UN_SMEM_MAX - 8192;

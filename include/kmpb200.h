@@ -26,6 +26,7 @@
  *   - occurrences are counted with overlaps ("aa" in "aaaa" = 3)               serial.c:203-206
  *   - patterns are counted independently; duplicated patterns each get the count
  *   - bytes are compared exactly, or after ASCII case folding for a KMPB_PAT_NOCASE pattern (kmpb_set_patterns_ex)
+ *   - a pattern may be restricted to start offsets [lo, hi] of each payload (kmpb_set_patterns_win)
  *   - counts are 64-bit here (C int in the reference, serial.c:103).
  */
 #ifndef KMPB200_H
@@ -107,6 +108,27 @@ int kmpb_set_patterns(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_of
 /* kmpb_set_patterns with flags[n_pat], one byte per pattern; flags == NULL is exactly kmpb_set_patterns.  A bit other
  * than KMPB_PAT_NOCASE is KMPB_EINVAL, naming the pattern. */
 int kmpb_set_patterns_ex(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, const uint8_t *flags);
+/* Position windows (kmpb_set_patterns_win).  A pattern with window [lo, hi] matches at offset o of a packet iff it
+ * matches there under the rules above (the text ends at the first NUL, occurrences overlap and lie inside one packet,
+ * case folding when nocase) and lo <= o <= hi: its count is the number of its unwindowed matches whose first byte lies
+ * at a payload offset in [lo, hi], its find records exactly those matches, and a packet is selected iff it holds a
+ * counted match of any pattern, windowed or not.  {0, KMPB_WINDOW_ANY} is no window: the pattern behaves as in
+ * kmpb_set_patterns_ex.  Otherwise 0 <= lo <= hi <= KMPB_WINDOW_MAX; anything else (lo > hi, hi above KMPB_WINDOW_MAX, a
+ * window open at the top: lo > 0 with hi = KMPB_WINDOW_ANY) is KMPB_EINVAL, naming the pattern.  Two patterns are the
+ * same distinct pattern iff they have the same bytes (folded when nocase), the same flag and the same window: "GET"
+ * unwindowed and "GET" in [0, 0] are two, and an occurrence at offset 0 yields a record for each.  kmpb_get_prefix does
+ * not depend on the window.  The union engine matches the windowed patterns in a pass of their own that reads only each
+ * packet's first max(hi + pattern length) bytes; every count, find and select form and kmpb_stream_* honour the
+ * windows. */
+typedef struct kmpb_window {
+    uint32_t lo, hi;
+} kmpb_window;
+#define KMPB_WINDOW_ANY 0xffffffffu
+#define KMPB_WINDOW_MAX 65535u
+/* kmpb_set_patterns_ex with win[n_pat], one window per pattern; win == NULL is exactly kmpb_set_patterns_ex.  Refused
+ * with KMPB_ESTATE while a frame stream is open, like the other pattern calls. */
+int kmpb_set_patterns_win(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, const uint8_t *flags,
+                          const kmpb_window *win);
 uint32_t kmpb_pattern_count(const kmpb_ctx *ctx);
 /* The device-built failure table of pattern i, copied back as the int[m] that kmp_prefix returns
  * (serial.c:217-238).  pi_out must hold m = pat_off[i+1]-pat_off[i] entries. */
@@ -161,8 +183,8 @@ int kmpb_check_device_errors(kmpb_ctx *ctx);
  * context's GPU), for callers that combine several GPUs with a collective (mpi_dumping.c:202). */
 uint64_t *kmpb_device_counts(kmpb_ctx *ctx);
 
-/* Profiling hooks for bench.py: with profile on, the dominant match kernel of each count call is
- * bracketed by CUDA events on the stream it is launched on; kmpb_last_kernel_ms waits for and returns
+/* Profiling hooks for bench.py: with profile on, the dominant match kernel of each count call (with windowed patterns:
+ * the window kernel and the union kernel together) is bracketed by CUDA events on the stream it is launched on; kmpb_last_kernel_ms waits for and returns
  * the duration of the most recent one (device-form calls only). */
 int kmpb_set_profile(kmpb_ctx *ctx, int on);
 int kmpb_last_kernel_ms(kmpb_ctx *ctx, double *ms_out);

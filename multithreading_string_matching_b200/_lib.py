@@ -13,6 +13,8 @@ c_u64p = ctypes.POINTER(ctypes.c_uint64)
 c_i32p = ctypes.POINTER(ctypes.c_int32)
 
 KMPB_PAT_NOCASE = 1  # kmpb_set_patterns_ex: ASCII case-insensitive pattern
+KMPB_WINDOW_ANY = 0xFFFFFFFF  # kmpb_set_patterns_win: {0, KMPB_WINDOW_ANY} is no window
+KMPB_WINDOW_MAX = 65535  # the largest hi of a window
 
 
 class KmpbError(RuntimeError):
@@ -28,6 +30,10 @@ class CPatterns(ctypes.Structure):
 class CCsr(ctypes.Structure):
     _fields_ = [("bytes", c_u8p), ("offsets", c_u64p), ("n_packets", ctypes.c_uint64),
                 ("n_frames", ctypes.c_uint64), ("total_bytes", ctypes.c_uint64), ("pinned", ctypes.c_int)]
+
+
+class CWindow(ctypes.Structure):
+    _fields_ = [("lo", ctypes.c_uint32), ("hi", ctypes.c_uint32)]
 
 
 class CSynth(ctypes.Structure):
@@ -49,6 +55,8 @@ SIGNATURES = {
     "kmpb_get_device": (ctypes.c_int, [ctypes.c_void_p]),
     "kmpb_set_patterns": (ctypes.c_int, [ctypes.c_void_p, c_u8p, c_u32p, ctypes.c_uint32]),
     "kmpb_set_patterns_ex": (ctypes.c_int, [ctypes.c_void_p, c_u8p, c_u32p, ctypes.c_uint32, c_u8p]),
+    "kmpb_set_patterns_win": (ctypes.c_int, [ctypes.c_void_p, c_u8p, c_u32p, ctypes.c_uint32, c_u8p,
+                                             ctypes.POINTER(CWindow)]),
     "kmpb_pattern_count": (ctypes.c_uint32, [ctypes.c_void_p]),
     "kmpb_get_prefix": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint32, c_i32p, ctypes.c_uint32]),
     "kmpb_count_host": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, c_u64p]),

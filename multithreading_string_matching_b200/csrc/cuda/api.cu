@@ -656,11 +656,17 @@ int kmpb_set_patterns(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_of
 
 int kmpb_set_patterns_ex(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, const uint8_t *flags)
 {
+    return kmpb_set_patterns_win(ctx, blob, pat_off, n_pat, flags, nullptr);
+}
+
+int kmpb_set_patterns_win(kmpb_ctx *ctx, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat, const uint8_t *flags,
+                          const kmpb_window *win)
+{
     if (ctx == nullptr) return kmpb_fail(KMPB_EINVAL, "NULL context");
     int rc = no_open_stream(ctx, "kmpb_set_patterns");
     if (rc || (rc = use_device(ctx))) return rc;
     kmpb_tables fresh;
-    rc = kmpb_tables_build_flags(&fresh, blob, pat_off, n_pat, flags, 0);
+    rc = kmpb_tables_build_win(&fresh, blob, pat_off, n_pat, flags, win, 0);
     if (rc) return rc;
     KMPB_CUDA(cudaDeviceSynchronize());
     kmpb_release_tables(ctx);

@@ -76,6 +76,9 @@ struct kmpb_device_tables {
     uint32_t *filter = nullptr;     // [256]
     uint32_t *gate = nullptr;       // [host.gate_words] prefix gate (automaton.c build_gate), null when there is none
     uint32_t *uniq_first = nullptr; // [n_uniq] lowest file-order index of each distinct pattern (the find records' pattern)
+    // window kernel: the windowed patterns' probe tables and windows (automaton.c), null when the set has none
+    uint32_t *wvtab = nullptr;      // [host.wvtab_words]
+    uint32_t *uniq_lo = nullptr, *uniq_hi = nullptr; // [n_uniq - host.n_union]
 };
 
 struct kmpb_ctx {
@@ -159,6 +162,11 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
                       const kmpb_fused_out &out = kmpb_fused_out(), const kmpb_find_out *find = nullptr,
                       uint32_t *mark = nullptr);
 int kmpb_union_scratch(kmpb_ctx *ctx, uint64_t max_batch_bytes);
+// window.cu: the windowed patterns of a batch (launched by kmpb_launch_union alone, before its own kernels): counts into
+// d_uniq_counts, records into *find or bits into the biased bitmap mark_biased (as the union kernel's), and the
+// file-order counts added to out when out.n > 0 (the caller passes that only when the union kernel does not run)
+int kmpb_launch_window(kmpb_ctx *ctx, const kmpb_batch &b, uint32_t *d_work, uint64_t *d_uniq_counts, cudaStream_t stream,
+                       const kmpb_fused_out &out, const kmpb_find_out *find, uint32_t *mark_biased);
 // find.cu: the find kernel into d_rec[capacity] (*d_found = every match of the batch), then the records turned into
 // kmpb_match (packet index + packet_base), sorted or not
 int kmpb_find_match(kmpb_ctx *ctx, const kmpb_batch &b, int slot, kmpb_match *d_rec, uint64_t capacity, unsigned long long *d_found,

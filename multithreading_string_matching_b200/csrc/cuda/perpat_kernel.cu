@@ -163,6 +163,49 @@ kmpb_perpat_kernel(const uint8_t *__restrict__ bytes, uint64_t abs_base, const u
         if (s_counts[t]) atomicAdd(&uniq_counts[u0 + t], (unsigned long long)s_counts[t]);
 }
 
+// The windowed patterns (distinct ids [u0, u0 + n_win), kmpb_set_patterns_win): each by its own DFA walk over the bytes
+// [lo, hi + m) of every packet's text, from the start state at lo, so that a hit is a match that starts in [lo, hi].  One
+// warp per packet: the text's end (its first NUL) among the first `reach` bytes, then per pattern the 32 lanes walk a
+// chunk each of that range, with the run-in of walk_chunk clipped at lo.  It shares nothing with the window kernel
+// (window.cu) or its tables, so it stays an independent cross-check of it.
+constexpr int PPW_THREADS = 256;
+__global__ void __launch_bounds__(PPW_THREADS)
+kmpb_perpat_window_kernel(const uint8_t *__restrict__ bytes, uint64_t abs_base, const uint64_t *__restrict__ offsets,
+                          uint64_t n_packets, const uint8_t *__restrict__ dfa_all, const uint32_t *__restrict__ uniq_off,
+                          const uint32_t *__restrict__ win_lo, const uint32_t *__restrict__ win_hi, uint32_t u0, uint32_t n_win,
+                          uint32_t reach, unsigned long long *__restrict__ uniq_counts)
+{
+    const uint32_t lane = threadIdx.x & 31;
+    const uint64_t n_warps = (uint64_t)gridDim.x * (PPW_THREADS / 32);
+    for (uint64_t k = (uint64_t)blockIdx.x * (PPW_THREADS / 32) + (threadIdx.x >> 5); k < n_packets; k += n_warps) {
+        const uint64_t beg = offsets[k];
+        const uint32_t head = (uint32_t)min(offsets[k + 1] - beg, (uint64_t)reach);
+        const uint8_t *text = bytes + (beg - abs_base);
+        uint32_t z = head;
+        for (uint32_t i = lane; i < head; i += 32)
+            if (text[i] == 0) { z = i; break; }
+        const uint32_t n = __reduce_min_sync(0xffffffffu, z);
+        for (uint32_t w = 0; w < n_win; w++) {
+            const uint32_t u = u0 + w, m = uniq_off[u + 1] - uniq_off[u], lo = win_lo[w];
+            const uint32_t e = min(win_hi[w] + m, n);
+            if (lo + m > e) continue; // (warp-uniform)
+            const uint32_t chunk = (e - lo + 31) / 32, a = lo + lane * chunk, stop = min(a + chunk, e);
+            const uint8_t *rows = dfa_all + 256ull * uniq_off[u];
+            uint32_t hits = 0;
+            if (a < e) {
+                uint32_t state = 0;
+                for (uint32_t i = a >= lo + (m - 1) ? a - (m - 1) : lo; i < stop; i++) {
+                    const uint32_t entry = __ldg(rows + 256u * state + text[i]);
+                    if (i >= a) hits += entry >> 7;
+                    state = entry & 0x7fu;
+                }
+            }
+            const uint32_t total = __reduce_add_sync(0xffffffffu, hits);
+            if (lane == 0 && total) atomicAdd(&uniq_counts[u], (unsigned long long)total);
+        }
+    }
+}
+
 int kmpb_launch_perpat(kmpb_ctx *ctx, const kmpb_batch &b, uint64_t *d_uniq_counts, cudaStream_t stream)
 {
     const kmpb_tables &h = ctx->host;
@@ -173,12 +216,21 @@ int kmpb_launch_perpat(kmpb_ctx *ctx, const kmpb_batch &b, uint64_t *d_uniq_coun
         KMPB_CUDA(cudaFuncSetAttribute(kmpb_perpat_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget));
         ctx->attr_perpat_set = true;
     }
+    if (h.n_union < h.n_uniq) { // the windowed patterns
+        if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[0], stream));
+        const int grid = (int)std::min<uint64_t>((uint64_t)ctx->sm_count * 8, (b.n_packets + PPW_THREADS / 32 - 1) / (PPW_THREADS / 32));
+        kmpb_perpat_window_kernel<<<grid, PPW_THREADS, 0, stream>>>(
+            b.d_bytes, b.abs_base, b.d_offsets, b.n_packets, ctx->dev.perpat_dfa, ctx->dev.uniq_off, ctx->dev.uniq_lo,
+            ctx->dev.uniq_hi, h.n_union, h.n_uniq - h.n_union, h.win_reach, (unsigned long long *)d_uniq_counts);
+        ctx->launches++;
+        KMPB_CUDA(cudaGetLastError());
+    }
     uint32_t u0 = 0;
-    while (u0 < h.n_uniq) {
+    while (u0 < h.n_union) {
         // largest tile [u0, u1) whose counters + offsets + DFA rows fit
         uint32_t u1 = u0;
         size_t need = 0;
-        while (u1 < h.n_uniq) {
+        while (u1 < h.n_union) {
             uint32_t nt = u1 + 1 - u0;
             size_t want = ((8u * nt + 4u + 15u) & ~15u) + 256ull * (h.uniq_off[u1 + 1] - h.uniq_off[u0]);
             if (want > budget) break;
@@ -188,7 +240,7 @@ int kmpb_launch_perpat(kmpb_ctx *ctx, const kmpb_batch &b, uint64_t *d_uniq_coun
         if (u1 == u0) return kmpb_fail(KMPB_ELIMIT, "pattern %u does not fit in shared memory", u0);
         uint64_t warps_wanted = b.n_packets;
         int grid = (int)std::min<uint64_t>((uint64_t)ctx->sm_count, (warps_wanted + PP_THREADS / 32 - 1) / (PP_THREADS / 32));
-        if (ctx->profile && u0 == 0) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[0], stream));
+        if (ctx->profile && u0 == 0 && h.n_union == h.n_uniq) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[0], stream));
         kmpb_perpat_kernel<<<grid, PP_THREADS, need, stream>>>(b.d_bytes, b.abs_base, b.d_offsets, b.n_packets,
                                                                ctx->dev.perpat_dfa, ctx->dev.uniq_off, u0, u1,
                                                                (unsigned long long *)d_uniq_counts);

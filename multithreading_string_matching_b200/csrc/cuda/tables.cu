@@ -65,6 +65,7 @@ void kmpb_release_tables(kmpb_ctx *ctx)
     kmpb_device_tables &d = ctx->dev;
     cudaFree(d.uniq_blob); cudaFree(d.uniq_off); cudaFree(d.uniq_len); cudaFree(d.uniq_flags); cudaFree(d.pat_to_uniq);
     cudaFree(d.pi); cudaFree(d.perpat_dfa); cudaFree(d.filter); cudaFree(d.vtab); cudaFree(d.gate); cudaFree(d.uniq_first);
+    cudaFree(d.wvtab); cudaFree(d.uniq_lo); cudaFree(d.uniq_hi);
     d = kmpb_device_tables();
     cudaFree(ctx->d_uniq_counts); ctx->d_uniq_counts = nullptr;
     cudaFree(ctx->d_counts); ctx->d_counts = nullptr;
@@ -89,6 +90,10 @@ int kmpb_upload_tables(kmpb_ctx *ctx)
     if ((rc = upload(&d.vtab, h.vtab, (size_t)h.vtab_words, s))) return rc;
     if ((rc = upload(&d.filter, h.filter6, 256, s))) return rc;
     if (h.gate_words && (rc = upload(&d.gate, h.gate, h.gate_words, s))) return rc;
+    if (h.n_union < h.n_uniq &&
+        ((rc = upload(&d.wvtab, h.wvtab, (size_t)h.wvtab_words, s)) || (rc = upload(&d.uniq_lo, h.uniq_lo, h.n_uniq - h.n_union, s)) ||
+         (rc = upload(&d.uniq_hi, h.uniq_hi, h.n_uniq - h.n_union, s))))
+        return rc;
     {
         uint32_t *first = (uint32_t *)malloc((h.n_uniq ? h.n_uniq : 1) * sizeof(uint32_t));
         if (first == nullptr) return kmpb_fail(KMPB_ENOMEM, "out of memory");

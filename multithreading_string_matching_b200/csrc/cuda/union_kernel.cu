@@ -1306,6 +1306,21 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
         return kmpb_fail(KMPB_ELIMIT, "absolute stream offsets of 2^56 and more");
     if (b.end_byte - b.abs_base >= (1ull << 36))
         return kmpb_fail(KMPB_ELIMIT, "more than 64 GiB of payload in one batch");
+    uint32_t *d_work = ctx->d_work.p + slot * 4;
+    // The bitmap's word 0 holds byte first_byte: mark_hit adds pos >> 5 to a base biased by first_byte >> 5 words.
+    uint32_t *const mark_biased =
+        mark ? reinterpret_cast<uint32_t *>(reinterpret_cast<uintptr_t>(mark) - 4u * (uintptr_t)(b.first_byte >> 5)) : nullptr;
+    // The windowed patterns (ids n_union and up) first, by the window kernel (window.cu) on the same stream; when there
+    // is no other pattern it also delivers the fused expansion, and the union kernel does not run.
+    if (h.n_union < h.n_uniq) {
+        if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[0], stream));
+        const int rc = kmpb_launch_window(ctx, b, d_work, d_uniq_counts, stream, h.n_union ? kmpb_fused_out() : out, find, mark_biased);
+        if (rc) return rc;
+        if (h.n_union == 0) {
+            if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[1], stream));
+            return KMPB_OK;
+        }
+    }
     const uint64_t span = b.end_byte - b.first_byte;
     // Taking an item costs a warp three dependent trips to L2 (ticket, item table, offsets); large batches
     // afford larger items (C3, 14 GB: 64 KB items 2.96 TB/s, 256 KB items 3.00 TB/s).
@@ -1323,11 +1338,10 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     const uint64_t items_per_slot = ctx->d_items.cap / KMPB_COPY_STREAMS;
     if ((uint64_t)n_items + 1 > items_per_slot) return kmpb_fail(KMPB_ESTATE, "union scratch too small");
     uint32_t *d_items = ctx->d_items.p + slot * items_per_slot;
-    uint32_t *d_work = ctx->d_work.p + slot * 4;
 
     // the counters and the probe tables go into shared memory if the block's 227 KB allow it
-    const bool counts_in_smem = UN_SMEM_FIXED + 4ull * h.n_uniq + 16 <= UN_SMEM_MAX - 8192;
-    const size_t counts_bytes = counts_in_smem ? ((4ull * h.n_uniq + 15) & ~15ull) : 0;
+    const bool counts_in_smem = UN_SMEM_FIXED + 4ull * h.n_union + 16 <= UN_SMEM_MAX - 8192;
+    const size_t counts_bytes = counts_in_smem ? ((4ull * h.n_union + 15) & ~15ull) : 0;
     const bool vtab_in_smem = UN_SMEM_FIXED + counts_bytes + 4ull * h.vtab_words <= UN_SMEM_MAX;
     const size_t vtab_bytes = vtab_in_smem ? 4ull * h.vtab_words : 0;
     // the prefix gate after them, if there is one and it fits; without it the resolve step re-runs the filter
@@ -1353,7 +1367,7 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     p.n_items = n_items;
     p.work = d_work;
     p.filter = ctx->dev.filter;
-    p.n_uniq = h.n_uniq;
+    p.n_uniq = h.n_union;
     p.counts_in_smem = counts_in_smem ? 1u : 0u;
     p.vtab_in_smem = vtab_in_smem ? 1u : 0u;
     p.vtab = ctx->dev.vtab;
@@ -1376,12 +1390,9 @@ int kmpb_launch_union(kmpb_ctx *ctx, const kmpb_batch &b, int slot, uint64_t *d_
     const uint32_t warps_needed = n_items;
     int grid = (int)std::min<uint32_t>((uint32_t)ctx->sm_count, (warps_needed + UN_WARPS - 1) / UN_WARPS);
     if (grid < 1) grid = 1;
-    if (ctx->profile) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[0], stream));
-    // The kernel: count, find or mark, and the nocase instantiation exactly when the set has a nocase pattern (its
-    // tables then have the layout the nocase verifier reads: the second one-byte table, tail masks).  The bitmap's word 0
-    // holds byte first_byte: mark_hit adds pos >> 5 to a base biased by first_byte >> 5 words.
-    uint32_t *const mark_biased =
-        mark ? reinterpret_cast<uint32_t *>(reinterpret_cast<uintptr_t>(mark) - 4u * (uintptr_t)(b.first_byte >> 5)) : nullptr;
+    if (ctx->profile && h.n_union == h.n_uniq) KMPB_CUDA(cudaEventRecord(ctx->ev_kernel[0], stream));
+    // The kernel: count, find or mark, and the nocase instantiation exactly when the set has a nocase pattern without a
+    // window (its tables then have the layout the nocase verifier reads: the second one-byte table, tail masks).
     if (h.n_nocase) {
         if (find) kmpb_union_find_nocase_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, *find);
         else if (mark) kmpb_union_mark_nocase_kernel<<<grid, UN_THREADS, smem_bytes, stream>>>(p, mark_biased);

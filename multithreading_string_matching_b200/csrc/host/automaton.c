@@ -35,22 +35,48 @@ typedef struct {
     const uint8_t *p; /* folded when nc */
     uint32_t len, index;
     uint32_t nc;      /* KMPB_PAT_NOCASE */
+    uint32_t lo, hi;  /* window; {0, KMPB_WINDOW_ANY} = none */
 } pat_ref;
+
+static int windowed(const pat_ref *r) { return r->hi != KMPB_WINDOW_ANY; }
 
 /* ASCII case folding (kmpb200.h): A-Z to a-z, every other byte as it is */
 static uint8_t fold(uint8_t c) { return c >= 'A' && c <= 'Z' ? (uint8_t)(c + 32) : c; }
 /* a byte of a folded nocase pattern that matches two text bytes: a lower-case letter (the other is c ^ 0x20) */
 static int folds(uint32_t nc, uint8_t c) { return nc && c >= 'a' && c <= 'z'; }
 
-/* distinct patterns are equal (bytes, flag); the order is content, then flag, then file order */
-static int cmp_content(const void *a, const void *b)
+/* content, then flag */
+static int cmp_bytes_flag(const pat_ref *x, const pat_ref *y)
 {
-    const pat_ref *x = a, *y = b;
     uint32_t n = x->len < y->len ? x->len : y->len;
     int c = memcmp(x->p, y->p, n);
     if (c) return c;
     if (x->len != y->len) return x->len < y->len ? -1 : 1;
     if (x->nc != y->nc) return x->nc < y->nc ? -1 : 1;
+    return 0;
+}
+
+/* distinct patterns are equal (bytes, flag); the order is content, then flag, then file order */
+static int cmp_content(const void *a, const void *b)
+{
+    const pat_ref *x = a, *y = b;
+    const int c = cmp_bytes_flag(x, y);
+    if (c) return c;
+    return x->index < y->index ? -1 : (x->index > y->index);
+}
+
+/* the order of the distinct ids: the patterns without a window first, in content order (so they are numbered as in a
+ * set without windows), then the windowed ones by content, flag and window -- so the windowed patterns of one byte
+ * and flag have consecutive ids, and the one-byte table of their probe tables, which holds the last of them, leads
+ * the window kernel to all of them */
+static int cmp_distinct(const void *a, const void *b)
+{
+    const pat_ref *x = a, *y = b;
+    if (windowed(x) != windowed(y)) return windowed(x) - windowed(y);
+    const int c = cmp_bytes_flag(x, y);
+    if (c) return c;
+    if (x->lo != y->lo) return x->lo < y->lo ? -1 : 1;
+    if (x->hi != y->hi) return x->hi < y->hi ? -1 : 1;
     return x->index < y->index ? -1 : (x->index > y->index);
 }
 
@@ -282,15 +308,15 @@ static double build_filter_words(uint32_t n_uniq, pat_ref *uniq, uint32_t n_buck
  * refined by hill climbing (moves and swaps) on the estimated candidate probability. */
 int kmpb_filter6_build(const kmpb_tables *t, uint32_t words[256], double *estimate)
 {
-    pat_ref *uniq = malloc((t->n_uniq ? t->n_uniq : 1) * sizeof *uniq);
+    pat_ref *uniq = malloc((t->n_union ? t->n_union : 1) * sizeof *uniq);
     if (!uniq) return kmpb_fail(KMPB_ENOMEM, "out of memory building the prefilter");
-    for (uint32_t u = 0; u < t->n_uniq; u++) {
+    for (uint32_t u = 0; u < t->n_union; u++) {
         uniq[u].p = t->uniq_blob + t->uniq_off[u];
         uniq[u].len = t->uniq_len[u];
         uniq[u].index = u;
         uniq[u].nc = t->uniq_flags ? t->uniq_flags[u] : 0u;
     }
-    const double e = build_filter_words(t->n_uniq, uniq, N_BUCKET, 6, words);
+    const double e = build_filter_words(t->n_union, uniq, N_BUCKET, 6, words);
     free(uniq);
     /* the NUL detector: depth 0 passes on NUL only, depths 1..3 always -- it reports three bytes after the NUL, when a
      * pattern starting at the NUL would report, so that a report's "candidate" and "NUL" bits speak of the same byte */
@@ -319,7 +345,7 @@ static int ac_build(const kmpb_tables *t, uint32_t nc, ac_automaton *a)
 {
     memset(a, 0, sizeof *a);
     const uint32_t ncl = t->n_class;
-    uint64_t max_state = (uint64_t)t->uniq_off[t->n_uniq] + 1;
+    uint64_t max_state = (uint64_t)t->uniq_off[t->n_union] + 1;
     if (max_state * ncl >= (1ull << 31))
         return kmpb_fail(KMPB_ELIMIT, "pattern set too large: %llu trie states x %u byte classes exceeds 2^31 table entries",
                          (unsigned long long)max_state, ncl);
@@ -336,7 +362,7 @@ static int ac_build(const kmpb_tables *t, uint32_t nc, ac_automaton *a)
 
     /* trie of all pattern prefixes */
     uint32_t n_state = 1;
-    for (uint32_t u = 0; u < t->n_uniq; u++) {
+    for (uint32_t u = 0; u < t->n_union; u++) {
         if ((t->uniq_flags ? t->uniq_flags[u] : 0u) != nc) continue;
         uint32_t s = 0;
         for (uint32_t i = t->uniq_off[u]; i < t->uniq_off[u + 1]; i++) {
@@ -484,7 +510,7 @@ static int build_dfa(kmpb_tables *t)
     /* byte classes: every byte a pattern can match has its own (both cases of a nocase pattern's letters) */
     int used[256] = {0};
     uint32_t has[2] = {0, 0};
-    for (uint32_t u = 0; u < t->n_uniq; u++) {
+    for (uint32_t u = 0; u < t->n_union; u++) {
         const uint32_t nc = t->uniq_flags ? t->uniq_flags[u] : 0u;
         has[nc] = 1;
         for (uint32_t i = t->uniq_off[u]; i < t->uniq_off[u + 1]; i++) {
@@ -565,14 +591,17 @@ static uint32_t vt_slots(const uint8_t *p, uint32_t len, uint32_t nc, uint32_t s
     return n;
 }
 
-static int build_verify_tables(kmpb_tables *t)
+/* The probe tables of distinct ids [u0, u0 + n), n_nocase of them nocase, into *out (*out_words words): vtab for
+ * the patterns without a window, wvtab for the windowed ones. */
+static int build_verify_tables(const kmpb_tables *t, uint32_t u0, uint32_t n, uint32_t n_nocase, uint32_t **out,
+                               uint32_t *out_words)
 {
     /* Two probe tables, one slot per hash value of the key, at least four slots per key: most slots are empty and
      * most occupied slots hold the patterns of a single key.  Keying the longer patterns by three bytes instead of two
      * (round 1) cuts the longest chain of strings.txt from 6 records ("se..") to 3 ("htt", "por") -- a warp walks as
      * many records as its longest chain.  A nocase pattern is entered under every case variant of its key. */
     uint32_t n_a = 0, n_b = 0, n1 = 0, blob_words = 0, mask_words = 0, keys[8];
-    for (uint32_t u = 0; u < t->n_uniq; u++) {
+    for (uint32_t u = u0; u < u0 + n; u++) {
         const uint8_t *p = t->uniq_blob + t->uniq_off[u];
         const uint32_t len = t->uniq_len[u], nc = t->uniq_flags[u];
         if (len >= 3) n_b += vt_keys(p, len, nc, keys); else if (len == 2) n_a += vt_keys(p, len, nc, keys); else n1++;
@@ -585,7 +614,7 @@ static int build_verify_tables(kmpb_tables *t)
     const uint32_t slots_a = n_a ? 1u << log_a : 0, slots_b = n_b ? 1u << log_b : 0;
     /* records: one per pattern and distinct slot */
     uint32_t n_rec = 0, sl[8];
-    for (uint32_t u = 0; u < t->n_uniq; u++) {
+    for (uint32_t u = u0; u < u0 + n; u++) {
         const uint32_t len = t->uniq_len[u];
         if (len >= 2) n_rec += vt_slots(t->uniq_blob + t->uniq_off[u], len, t->uniq_flags[u], len >= 3 ? 32 - log_b : 32 - log_a, sl);
     }
@@ -597,7 +626,7 @@ static int build_verify_tables(kmpb_tables *t)
     /* the one-byte table: 256 words of case-sensitive ids, then -- in a set with a nocase pattern -- 256 of nocase ids,
      * so that `A` and nocase `a` can both claim byte `A` */
     const uint32_t one_off = n1 ? at : 0;
-    if (n1) at += t->n_nocase ? 512 : 256;
+    if (n1) at += n_nocase ? 512 : 256;
     at = (at + 3u) & ~3u; /* records are read 16 bytes at a time */
     const uint32_t rec_off = at;
     at += 8 * n_rec;
@@ -610,9 +639,9 @@ static int build_verify_tables(kmpb_tables *t)
     if (!v || !fill) { free(v); free(fill); return kmpb_fail(KMPB_ENOMEM, "out of memory building the verification tables"); }
     v[0] = at; v[1] = slot_a_off; v[2] = 32 - log_a; v[3] = slot_b_off; v[4] = 32 - log_b; v[5] = one_off;
     v[6] = rec_off; v[7] = blob_off;
-    for (uint32_t i = 0; n1 && i < (t->n_nocase ? 512u : 256u); i++) v[one_off + i] = 0xffffffffu;
+    for (uint32_t i = 0; n1 && i < (n_nocase ? 512u : 256u); i++) v[one_off + i] = 0xffffffffu;
     /* chain lengths, then chain starts (records of one slot are contiguous; table A's records come first) */
-    for (uint32_t u = 0; u < t->n_uniq; u++) {
+    for (uint32_t u = u0; u < u0 + n; u++) {
         const uint8_t *p = t->uniq_blob + t->uniq_off[u];
         const uint32_t len = t->uniq_len[u];
         if (len < 2) continue;
@@ -623,7 +652,7 @@ static int build_verify_tables(kmpb_tables *t)
     for (uint32_t s = 0; s < slots_a; s++) { v[slot_a_off + 2 * s] = first; first += v[slot_a_off + 2 * s + 1]; }
     for (uint32_t s = 0; s < slots_b; s++) { v[slot_b_off + 2 * s] = first; first += v[slot_b_off + 2 * s + 1]; }
     uint32_t bw = 0, mw = 0;
-    for (uint32_t u = 0; u < t->n_uniq; u++) {
+    for (uint32_t u = u0; u < u0 + n; u++) {
         const uint8_t *p = t->uniq_blob + t->uniq_off[u];
         const uint32_t len = t->uniq_len[u], nc = t->uniq_flags[u];
         memcpy((uint8_t *)(v + blob_off + bw), p, len); /* rest of the last word stays zero */
@@ -649,9 +678,29 @@ static int build_verify_tables(kmpb_tables *t)
         if (tail) mw += (len + 3) / 4;
     }
     free(fill);
-    t->vtab = v;
-    t->vtab_words = at;
+    *out = v;
+    *out_words = at;
     return KMPB_OK;
+}
+
+/* The window kernel's tables: the windowed patterns' probe tables, their windows' extremes and reach, and the bytes
+ * they can start with (both cases of a nocase pattern's letter). */
+static int build_window_tables(kmpb_tables *t)
+{
+    const uint32_t nw = t->n_uniq - t->n_union;
+    if (nw == 0) return KMPB_OK;
+    t->win_lo_min = KMPB_WINDOW_MAX;
+    for (uint32_t w = 0; w < nw; w++) {
+        const uint32_t u = t->n_union + w, len = t->uniq_len[u];
+        const uint8_t c = t->uniq_blob[t->uniq_off[u]];
+        if (t->uniq_lo[w] < t->win_lo_min) t->win_lo_min = t->uniq_lo[w];
+        if (t->uniq_hi[w] > t->win_hi_max) t->win_hi_max = t->uniq_hi[w];
+        if (t->uniq_hi[w] + len > t->win_reach) t->win_reach = t->uniq_hi[w] + len;
+        t->win_nocase += t->uniq_flags[u];
+        t->win_first[c >> 5] |= 1u << (c & 31);
+        if (folds(t->uniq_flags[u], c)) t->win_first[(c ^ 0x20) >> 5] |= 1u << ((c ^ 0x20) & 31);
+    }
+    return build_verify_tables(t, t->n_union, nw, t->win_nocase, &t->wvtab, &t->wvtab_words);
 }
 
 /* ---- prefix gate ------------------------------------------------------------------------------ */
@@ -670,7 +719,7 @@ uint32_t kmpb_gate_slot(uint32_t x, uint32_t shift) { return (x * KMPB_GATE_MUL)
 static int build_gate(kmpb_tables *t)
 {
     uint32_t keys = 0, last = 0xffffffffu; /* distinct patterns are in content order: equal first two bytes are adjacent */
-    for (uint32_t u = 0; u < t->n_uniq; u++) {
+    for (uint32_t u = 0; u < t->n_union; u++) {
         const uint8_t *p = t->uniq_blob + t->uniq_off[u];
         const uint32_t nc = t->uniq_flags[u];
         if (t->uniq_len[u] == 1) { keys += 256u << folds(nc, p[0]); continue; }
@@ -684,7 +733,7 @@ static int build_gate(kmpb_tables *t)
     const uint32_t words = 1u << log_w, shift = 32 - log_w;
     uint32_t *g = calloc(words, sizeof *g);
     if (!g) return kmpb_fail(KMPB_ENOMEM, "out of memory building the prefix gate");
-    for (uint32_t u = 0; u < t->n_uniq; u++) {
+    for (uint32_t u = 0; u < t->n_union; u++) {
         const uint8_t *p = t->uniq_blob + t->uniq_off[u];
         const uint32_t len = t->uniq_len[u], nc = t->uniq_flags[u];
         /* a nocase pattern sets the bits of every case variant of its first two bytes; the bit, third byte & 31, is the
@@ -701,7 +750,7 @@ static int build_gate(kmpb_tables *t)
     }
     uint64_t set = 0;
     for (uint32_t i = 0; i < words; i++) set += (uint64_t)__builtin_popcount(g[i]);
-    if (t->n_uniq == 0 || 8 * set > 32ull * words) {
+    if (t->n_union == 0 || 8 * set > 32ull * words) {
         free(g);
         return KMPB_OK;
     }
@@ -723,11 +772,18 @@ int kmpb_tables_build_ex(kmpb_tables *t, const uint8_t *blob, const uint32_t *pa
     return kmpb_tables_build_flags(t, blob, pat_off, n_pat, NULL, with_dfa);
 }
 
-/* with_dfa != 0 also builds the merged automaton of all patterns (next / trie / out_*): the reference the table tests
- * check the filter and the verification tables against.  The device never sees it, so the library does not build it.
- * flags[n_pat] (NULL: all zero) holds each pattern's KMPB_PAT_* bits. */
 int kmpb_tables_build_flags(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat,
                             const uint8_t *flags, int with_dfa)
+{
+    return kmpb_tables_build_win(t, blob, pat_off, n_pat, flags, NULL, with_dfa);
+}
+
+/* with_dfa != 0 also builds the merged automaton of all patterns without a window (next / trie / out_*): the reference
+ * the table tests check the filter and the verification tables against.  The device never sees it, so the library does
+ * not build it.  flags[n_pat] (NULL: all zero) holds each pattern's KMPB_PAT_* bits, win[n_pat] (NULL: none) its
+ * window. */
+int kmpb_tables_build_win(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat,
+                          const uint8_t *flags, const kmpb_window *win, int with_dfa)
 {
     memset(t, 0, sizeof *t);
     if (n_pat && (blob == NULL || pat_off == NULL)) return kmpb_fail(KMPB_EINVAL, "kmpb_set_patterns: NULL pattern data");
@@ -755,6 +811,17 @@ int kmpb_tables_build_flags(kmpb_tables *t, const uint8_t *blob, const uint32_t 
         refs[i].len = len;
         refs[i].index = i;
         refs[i].nc = flags ? flags[i] & KMPB_PAT_NOCASE : 0u;
+        refs[i].lo = win ? win[i].lo : 0u;
+        refs[i].hi = win ? win[i].hi : KMPB_WINDOW_ANY;
+        if (refs[i].lo == 0 && refs[i].hi == KMPB_WINDOW_ANY) { /* no window */
+        } else if (refs[i].hi == KMPB_WINDOW_ANY) {
+            free(refs); kmpb_tables_free(t);
+            return kmpb_fail(KMPB_EINVAL, "pattern %u has window [%u, any]: a window open at the top is not supported", i, win[i].lo);
+        } else if (refs[i].lo > refs[i].hi || refs[i].hi > KMPB_WINDOW_MAX) {
+            free(refs); kmpb_tables_free(t);
+            return kmpb_fail(KMPB_EINVAL, "pattern %u has window [%u, %u]; 0 <= lo <= hi <= %u required", i, win[i].lo,
+                             win[i].hi, KMPB_WINDOW_MAX);
+        }
         blob_len += len;
     }
     /* nocase patterns are matched in their folded form */
@@ -764,14 +831,16 @@ int kmpb_tables_build_flags(kmpb_tables *t, const uint8_t *blob, const uint32_t 
         for (uint32_t k = 0; k < refs[i].len; k++) folded[at + k] = refs[i].nc ? fold(refs[i].p[k]) : refs[i].p[k];
         refs[i].p = folded + at;
     }
-    /* distinct patterns, numbered in content order */
-    qsort(refs, n_pat, sizeof *refs, cmp_content);
+    /* distinct patterns: those without a window numbered in content order, then the windowed ones */
+    qsort(refs, n_pat, sizeof *refs, cmp_distinct);
     t->uniq_off = malloc(((size_t)n_pat + 1) * sizeof *t->uniq_off);
     t->uniq_len = malloc(((size_t)n_pat + 1) * sizeof *t->uniq_len);
     t->uniq_flags = calloc((size_t)n_pat + 1, 1);
     t->uniq_blob = malloc(blob_len ? blob_len : 1);
     pat_ref *uniq = malloc(((size_t)n_pat + 1) * sizeof *uniq);
-    if (!t->uniq_off || !t->uniq_len || !t->uniq_flags || !t->uniq_blob || !uniq) {
+    t->uniq_lo = malloc(((size_t)n_pat + 1) * sizeof *t->uniq_lo);
+    t->uniq_hi = malloc(((size_t)n_pat + 1) * sizeof *t->uniq_hi);
+    if (!t->uniq_off || !t->uniq_len || !t->uniq_flags || !t->uniq_blob || !uniq || !t->uniq_lo || !t->uniq_hi) {
         free(refs); free(uniq); free(folded); kmpb_tables_free(t);
         return kmpb_fail(KMPB_ENOMEM, "out of memory");
     }
@@ -779,12 +848,19 @@ int kmpb_tables_build_flags(kmpb_tables *t, const uint8_t *blob, const uint32_t 
     t->min_len = n_pat ? KMPB_MAX_PATTERN_LEN : 0;
     for (uint32_t i = 0; i < n_pat; i++) {
         int same = i > 0 && refs[i].len == refs[i - 1].len && refs[i].nc == refs[i - 1].nc &&
+                   refs[i].lo == refs[i - 1].lo && refs[i].hi == refs[i - 1].hi &&
                    memcmp(refs[i].p, refs[i - 1].p, refs[i].len) == 0;
         if (!same) {
             t->uniq_off[nu] = at;
             t->uniq_len[nu] = refs[i].len;
             t->uniq_flags[nu] = (uint8_t)refs[i].nc;
-            t->n_nocase += refs[i].nc;
+            if (windowed(&refs[i])) {
+                t->uniq_lo[nu - t->n_union] = refs[i].lo;
+                t->uniq_hi[nu - t->n_union] = refs[i].hi;
+            } else {
+                t->n_nocase += refs[i].nc;
+                t->n_union = nu + 1;
+            }
             memcpy(t->uniq_blob + at, refs[i].p, refs[i].len);
             uniq[nu].p = t->uniq_blob + at;
             uniq[nu].len = refs[i].len;
@@ -803,7 +879,8 @@ int kmpb_tables_build_flags(kmpb_tables *t, const uint8_t *blob, const uint32_t 
     free(folded);
 
     int rc = with_dfa ? build_dfa(t) : KMPB_OK;
-    if (rc == KMPB_OK) rc = build_verify_tables(t);
+    if (rc == KMPB_OK) rc = build_verify_tables(t, 0, t->n_union, t->n_nocase, &t->vtab, &t->vtab_words);
+    if (rc == KMPB_OK) rc = build_window_tables(t);
     if (rc == KMPB_OK) rc = build_gate(t);
     if (rc == KMPB_OK) rc = kmpb_filter6_build(t, t->filter6, &t->filter6_fp_estimate);
     free(uniq);
@@ -825,5 +902,8 @@ void kmpb_tables_free(kmpb_tables *t)
     free(t->out_id);
     free(t->vtab);
     free(t->gate);
+    free(t->uniq_lo);
+    free(t->uniq_hi);
+    free(t->wvtab);
     memset(t, 0, sizeof *t);
 }

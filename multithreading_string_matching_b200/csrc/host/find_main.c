@@ -2,6 +2,8 @@
  *
  *   kmp_find <file.pcap> <string.txt> [udp|tcp]
  *   kmp_find -i <file.pcap> <string.txt> [udp|tcp]     every token case-insensitive (ASCII letters, KMPB_PAT_NOCASE)
+ *   kmp_find -w LO:HI <file.pcap> <string.txt> ...     only the matches that start at a payload offset in [LO, HI]
+ *                                                      (cli_window.h); -i and -w combine, in either order
  *
  * stdout: "<frame> <offset> <pattern>\n" per match, ordered by (frame, offset, pattern index): frame is the 1-based
  * capture record number (the numbering Wireshark shows), offset the position of the match's first byte inside the
@@ -14,6 +16,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include "cli_window.h"
 #include "kmpb200.h"
 
 static int fail(const char *what)
@@ -26,8 +29,17 @@ int main(int argc, char **argv)
 {
     const char *prog = "./kmp_find";
     int proto = KMPB_PROTO_UDP;
-    const int nocase = argc > 1 && strcmp(argv[1], "-i") == 0; /* then the arguments follow as without it */
-    if (nocase) {
+    /* -i and -w LO:HI, each at most once, in either order; then the arguments follow as without them */
+    int nocase = 0, windowed = 0;
+    kmpb_window window;
+    for (int k = 0; k < 2 && argc > 1; k++) {
+        if (!nocase && strcmp(argv[1], "-i") == 0) nocase = 1;
+        else if (!windowed && strcmp(argv[1], "-w") == 0) {
+            if (!parse_window_arg(argc > 2 ? argv[2] : NULL, &window)) return bad_window(argc > 2 ? argv[2] : NULL);
+            windowed = 1;
+            argv++;
+            argc--;
+        } else break;
         argv++;
         argc--;
     }
@@ -67,8 +79,11 @@ int main(int argc, char **argv)
     if (kmpb_create(&ctx, kmpb_device_ordinal(0)) != 0) return fail("GPU");
     uint8_t *flags = nocase ? malloc(pats.n_pat ? pats.n_pat : 1) : NULL;
     if (flags) memset(flags, KMPB_PAT_NOCASE, pats.n_pat);
-    rc = kmpb_set_patterns_ex(ctx, pats.blob, pats.pat_off, pats.n_pat, flags);
+    kmpb_window *win = window_array(windowed ? &window : NULL, pats.n_pat);
+    if (windowed && win == NULL) return fail("out of memory");
+    rc = kmpb_set_patterns_win(ctx, pats.blob, pats.pat_off, pats.n_pat, flags, win);
     free(flags);
+    free(win);
     if (rc != 0) return fail("patterns");
 
     /* a guess first (C3-like traffic has one match per ~400 payload bytes), then the exact size if it was short */

@@ -27,8 +27,18 @@ typedef struct kmpb_tables {
     uint32_t *uniq_off;      /* [n_uniq+1] into uniq_blob */
     uint8_t *uniq_blob;      /* a nocase pattern's bytes are folded (A-Z to a-z) */
     uint8_t *uniq_flags;     /* [n_uniq] KMPB_PAT_NOCASE or 0: part of a distinct pattern's identity */
-    uint32_t n_nocase;       /* distinct nocase patterns (non-zero: the union engine runs its nocase kernels) */
+    uint32_t n_nocase;       /* distinct nocase patterns without a window (non-zero: the union engine runs its nocase kernels) */
     uint32_t max_len, min_len;
+    /* Distinct ids [0, n_union) are the patterns without a window, in the order a set without windows gives them; the
+     * filter, the probe tables (vtab), the gate and the automaton below hold these alone.  Ids [n_union, n_uniq) are
+     * the windowed ones (kmpb_tables_build_win), matched by the window kernel through wvtab. */
+    uint32_t n_union;
+    uint32_t *uniq_lo, *uniq_hi; /* [n_uniq - n_union] window of distinct id n_union + w */
+    uint32_t win_lo_min, win_hi_max, win_reach; /* min lo, max hi, max(hi + len) over the windowed patterns */
+    uint32_t win_nocase;     /* windowed distinct nocase patterns (wvtab then has the nocase layout) */
+    uint32_t win_first[8];   /* bit c: some windowed pattern can start with byte c */
+    uint32_t *wvtab;         /* the windowed patterns' probe tables, in vtab's layout (distinct ids as above) */
+    uint32_t wvtab_words;
 
     /* byte classes: bytes that occur in no pattern share class 0 */
     uint32_t n_class;
@@ -104,6 +114,9 @@ int kmpb_tables_build_ex(kmpb_tables *t, const uint8_t *blob, const uint32_t *pa
 /* ... with per-pattern KMPB_PAT_* flags[n_pat] (NULL = all zero, which builds word for word what kmpb_tables_build does) */
 int kmpb_tables_build_flags(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat,
                             const uint8_t *flags, int with_dfa);
+/* ... with per-pattern windows win[n_pat] (NULL = none, which builds word for word what kmpb_tables_build_flags does) */
+int kmpb_tables_build_win(kmpb_tables *t, const uint8_t *blob, const uint32_t *pat_off, uint32_t n_pat,
+                          const uint8_t *flags, const kmpb_window *win, int with_dfa);
 /* the prefilter words (5 pattern buckets + NUL in 6-bit fields, depth 4 + a lingering field): automaton.c */
 int kmpb_filter6_build(const kmpb_tables *t, uint32_t words[256], double *estimate);
 void kmpb_tables_free(kmpb_tables *t);

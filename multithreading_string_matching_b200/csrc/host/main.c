@@ -6,6 +6,9 @@
  *   kmp_match -i <file.pcap> <string.txt> [n] [udp|tcp]     every token case-insensitive (ASCII letters,
  *                                                           KMPB_PAT_NOCASE); the report lists each token as
  *                                                           the strings file spells it
+ *   kmp_match -w LO:HI <file.pcap> <string.txt> ...         every token counted only where it starts at a
+ *                                                           payload offset in [LO, HI] (kmpb_set_patterns_win,
+ *                                                           cli_window.h); -i and -w combine, in either order
  *
  * stdout is the reference's, byte for byte (serial.c:163-169): header line, one "pattern: N times!"
  * line per pattern with a non-zero count in file order, then "Elapsed time = %f seconds" -- the
@@ -25,6 +28,7 @@
 #include <string.h>
 #include <sys/time.h>
 
+#include "cli_window.h"
 #include "kmpb200.h"
 
 static double now_seconds(void)
@@ -47,6 +51,7 @@ typedef struct {
     int rank;   /* which share of the packets */
     const kmpb_patterns *pats;
     const uint8_t *flags; /* per-pattern KMPB_PAT_* flags, NULL = none */
+    const kmpb_window *win; /* per-pattern windows, NULL = none */
     ingest_gate *gate;
     uint64_t *counts;
     double start;
@@ -62,7 +67,7 @@ static void *run_shard(void *arg)
     shard_job *job = arg;
     kmpb_ctx *ctx = NULL;
     job->rc = kmpb_create(&ctx, job->device);
-    if (job->rc == 0) job->rc = kmpb_set_patterns_ex(ctx, job->pats->blob, job->pats->pat_off, job->pats->n_pat, job->flags);
+    if (job->rc == 0) job->rc = kmpb_set_patterns_win(ctx, job->pats->blob, job->pats->pat_off, job->pats->n_pat, job->flags, job->win);
     if (job->rc == 0) job->rc = kmpb_reserve_staging(ctx, 0, 0); /* pinned staging, while the main thread frames the savefile */
     if (job->rc != 0) snprintf(job->err, sizeof job->err, "%s", kmpb_last_error());
     if (getenv("KMPB_STATS")) fprintf(stderr, "kmp_match: GPU %d context, pattern tables and staging buffers ready %.3f s after start\n", job->device, now_seconds() - job->start);
@@ -84,8 +89,17 @@ int main(int argc, char **argv)
 {
     int proto = KMPB_PROTO_UDP, n_gpus = 1, openmp_form = 0;
     const char *prog = "./kmp_match";
-    const int nocase = argc > 1 && strcmp(argv[1], "-i") == 0; /* then the arguments follow as without it */
-    if (nocase) {
+    /* -i and -w LO:HI, each at most once, in either order; then the arguments follow as without them */
+    int nocase = 0, windowed = 0;
+    kmpb_window window;
+    for (int k = 0; k < 2 && argc > 1; k++) {
+        if (!nocase && strcmp(argv[1], "-i") == 0) nocase = 1;
+        else if (!windowed && strcmp(argv[1], "-w") == 0) {
+            if (!parse_window_arg(argc > 2 ? argv[2] : NULL, &window)) return bad_window(argc > 2 ? argv[2] : NULL);
+            windowed = 1;
+            argv++;
+            argc--;
+        } else break;
         argv++;
         argc--;
     }
@@ -128,6 +142,11 @@ int main(int argc, char **argv)
     if (n_gpus > available) n_gpus = available;
     uint8_t *flags = nocase ? malloc(pats.n_pat ? pats.n_pat : 1) : NULL;
     if (flags) memset(flags, KMPB_PAT_NOCASE, pats.n_pat);
+    kmpb_window *win = window_array(windowed ? &window : NULL, pats.n_pat);
+    if (windowed && win == NULL) {
+        fprintf(stderr, "error: out of memory\n");
+        return 1;
+    }
 
     double start = now_seconds();
     ingest_gate gate;
@@ -144,6 +163,7 @@ int main(int argc, char **argv)
         jobs[g].rank = g;
         jobs[g].pats = &pats;
         jobs[g].flags = flags;
+        jobs[g].win = win;
         jobs[g].gate = &gate;
         jobs[g].start = start;
         jobs[g].counts = calloc(pats.n_pat ? pats.n_pat : 1, sizeof(uint64_t));
@@ -192,6 +212,7 @@ int main(int argc, char **argv)
     free(threads);
     free(counts);
     free(flags);
+    free(win);
     kmpb_pcap_close(pc);
     kmpb_free_patterns(&pats);
     return 0;

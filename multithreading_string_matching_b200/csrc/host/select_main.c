@@ -3,7 +3,8 @@
  *   kmp_select [-i] [-v] <file.pcap> <string.txt> <out.pcap> [udp|tcp]
  *
  * -i makes every token case-insensitive (ASCII letters, KMPB_PAT_NOCASE), as for kmp_find; -v writes the frames that
- * hold NO match instead (dropping known noise).  A frame is selected when its UDP or TCP payload holds at least one
+ * hold NO match instead (dropping known noise); -w LO:HI counts a token only where it starts at a payload offset in
+ * [LO, HI] (cli_window.h).  The options come in any order before the file names.  A frame is selected when its UDP or TCP payload holds at least one
  * match that kmp_match counts, i.e. when kmp_find prints a line for it.  The output has the input's format (classic
  * or pcapng, byte order, timestamp resolution, link type) and holds the chosen records byte for byte; frames whose
  * payload the extractor refused are in neither output.  stdout is one line, "<selected> of <accepted> packets written
@@ -14,6 +15,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include "cli_window.h"
 #include "kmpb200.h"
 
 static int fail(const char *what)
@@ -25,11 +27,17 @@ static int fail(const char *what)
 int main(int argc, char **argv)
 {
     const char *prog = "./kmp_select";
-    int proto = KMPB_PROTO_UDP, nocase = 0, invert = 0;
+    int proto = KMPB_PROTO_UDP, nocase = 0, invert = 0, windowed = 0;
+    kmpb_window window;
     for (; argc > 1 && argv[1][0] == '-' && argv[1][1] && !argv[1][2]; argv++, argc--) {
         if (argv[1][1] == 'i') nocase = 1;
         else if (argv[1][1] == 'v') invert = 1;
-        else break;
+        else if (argv[1][1] == 'w') {
+            if (!parse_window_arg(argc > 2 ? argv[2] : NULL, &window)) return bad_window(argc > 2 ? argv[2] : NULL);
+            windowed = 1;
+            argv++;
+            argc--;
+        } else break;
     }
     if (argc < 4 || argc > 5) {
         printf("USAGE: %s [-i] [-v] <file.pcap> <string.txt> <out.pcap> [tcp/udp]\n", prog);
@@ -67,8 +75,11 @@ int main(int argc, char **argv)
     if (kmpb_create(&ctx, kmpb_device_ordinal(0)) != 0) return fail("GPU");
     uint8_t *pflags = nocase ? malloc(pats.n_pat ? pats.n_pat : 1) : NULL;
     if (pflags) memset(pflags, KMPB_PAT_NOCASE, pats.n_pat);
-    rc = kmpb_set_patterns_ex(ctx, pats.blob, pats.pat_off, pats.n_pat, pflags);
+    kmpb_window *win = window_array(windowed ? &window : NULL, pats.n_pat);
+    if (windowed && win == NULL) return fail("out of memory");
+    rc = kmpb_set_patterns_win(ctx, pats.blob, pats.pat_off, pats.n_pat, pflags, win);
     free(pflags);
+    free(win);
     if (rc != 0) return fail("patterns");
 
     const uint64_t n_packets = kmpb_pcap_packets(pc);

@@ -13,7 +13,8 @@ import tempfile
 import numpy as np
 
 from . import _lib
-from ._lib import KMPB_PAT_NOCASE, CCsr, CPatterns, CSynth, KmpbError, c_i32p, c_u8p, c_u32p, c_u64p, check, lib
+from ._lib import (KMPB_PAT_NOCASE, KMPB_WINDOW_ANY, KMPB_WINDOW_MAX, CCsr, CPatterns, CSynth, CWindow, KmpbError, c_i32p, c_u8p, c_u32p,
+                   c_u64p, check, lib)
 
 ENGINE_AUTO, ENGINE_PERPAT, ENGINE_UNION = 0, 1, 2
 PROTO_UDP, PROTO_TCP = 0, 1
@@ -144,6 +145,11 @@ def format_report(patterns, counts):
         return open(tmp.name, "rb").read()
 
 
+def _is_pair(window):
+    """(lo, hi): one window for every pattern, as opposed to a sequence of per-pattern windows"""
+    return len(window) == 2 and all(isinstance(x, (int, np.integer)) for x in window)
+
+
 class Matcher:
     """One GPU context (kmpb_ctx).  Raises KmpbError(KMPB_ENODEVICE) when there is no B200: no fallback."""
 
@@ -153,6 +159,7 @@ class Matcher:
         self.device = device
         self.patterns = []
         self.nocase = []
+        self.window = []
         self.set_engine(engine)
 
     def close(self):
@@ -179,9 +186,11 @@ class Matcher:
     def set_engine(self, engine):
         check(lib().kmpb_set_engine(self._ctx, _ENGINE[engine]))
 
-    def set_patterns(self, patterns, nocase=False):
+    def set_patterns(self, patterns, nocase=False, window=None):
         """serial.c:148-152: builds the failure tables (on the device) for the whole set.  nocase: True makes every
-        pattern case-insensitive (ASCII letters only, KMPB_PAT_NOCASE), a sequence of len(patterns) bools each one."""
+        pattern case-insensitive (ASCII letters only, KMPB_PAT_NOCASE), a sequence of len(patterns) bools each one.
+        window: None, one (lo, hi) pair for every pattern, or a sequence of len(patterns) pairs or Nones: a windowed
+        pattern matches only at payload offsets lo..hi (0 <= lo <= hi <= 65535, kmpb_set_patterns_win)."""
         patterns = [bytes(p) for p in patterns]
         if isinstance(nocase, (bool, np.bool_)):
             nocase = [bool(nocase)] * len(patterns)
@@ -189,12 +198,26 @@ class Matcher:
             nocase = [bool(x) for x in nocase]
             if len(nocase) != len(patterns):
                 raise ValueError("nocase has %d entries for %d patterns" % (len(nocase), len(patterns)))
+        if window is None or _is_pair(window):
+            window = [None if window is None else (int(window[0]), int(window[1]))] * len(patterns)
+        else:
+            window = [None if w is None else (int(w[0]), int(w[1])) for w in window]
+            if len(window) != len(patterns):
+                raise ValueError("window has %d entries for %d patterns" % (len(window), len(patterns)))
+        for w in window:
+            if w is not None and not (0 <= w[0] <= KMPB_WINDOW_MAX and 0 <= w[1] <= KMPB_WINDOW_MAX):
+                raise ValueError("window %r: lo and hi must lie in 0..%d" % (w, KMPB_WINDOW_MAX))
         blob, off = pack_patterns(patterns)
         flags = np.array([KMPB_PAT_NOCASE if x else 0 for x in nocase] or [0], dtype=np.uint8)
-        check(lib().kmpb_set_patterns_ex(self._ctx, blob.ctypes.data_as(c_u8p), off.ctypes.data_as(c_u32p), len(patterns),
-                                         flags.ctypes.data_as(c_u8p) if any(nocase) else None))
+        win = (CWindow * max(1, len(patterns)))()
+        for i, w in enumerate(window):
+            win[i].lo, win[i].hi = w if w is not None else (0, KMPB_WINDOW_ANY)
+        check(lib().kmpb_set_patterns_win(self._ctx, blob.ctypes.data_as(c_u8p), off.ctypes.data_as(c_u32p), len(patterns),
+                                          flags.ctypes.data_as(c_u8p) if any(nocase) else None,
+                                          win if any(w is not None for w in window) else None))
         self.patterns = patterns
         self.nocase = nocase
+        self.window = window
 
     def prefix(self, index):
         """The device-built failure table of pattern `index`, as kmp_prefix returns it (serial.c:217-238)."""

@@ -95,11 +95,12 @@ def device_counts(m, data, offsets, n_vectors=1):
     return [[c - 3 for c in v[: len(m.patterns)].cpu().tolist()] for v in vecs]
 
 
-def check(engines, finder, patterns, nocase, window, packets, label="", forms=True):
-    """both engines' counts and, with forms, every in-memory count, find and select form against the expected answers"""
+def check(engines, finder, patterns, nocase, window, packets, label="", forms=True, answers=None):
+    """both engines' counts and, with forms, every in-memory count, find and select form against the expected answers
+    (`answers`: (counts, sorted records, verdicts) computed by the caller, in place of `expected`'s)"""
     union, perpat = engines
     data, offsets = csr(packets)
-    want_counts, want, verdicts = expected(finder, patterns, nocase, window, data, offsets)
+    want_counts, want, verdicts = answers if answers is not None else expected(finder, patterns, nocase, window, data, offsets)
     for m in (union, perpat):
         m.set_patterns(patterns, nocase, window)
         assert m.count_host(data, offsets) == want_counts, (label, m is union)

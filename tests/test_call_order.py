@@ -23,7 +23,8 @@ import pytest
 
 import bench
 import multithreading_string_matching_b200 as kmp
-from test_find import RefFinder, assert_invariant
+from kmpb_harness import DeviceBatch, udp_frame
+from kmpb_reference import ORDER, assert_invariant, expected, keys
 
 pytestmark = pytest.mark.gpu
 
@@ -32,33 +33,6 @@ FORMS = ["count_device_span", "count_device", "count_device_span_peers", "find_s
 C_NAME = {"count_device_span": "kmpb_count_device_span", "count_device": "kmpb_count_device",
           "count_device_span_peers": "kmpb_count_device_span_peers", "find_sorted": "kmpb_find_device_span",
           "find_unsorted": "kmpb_find_device_span"}
-
-
-def keys(rec):
-    """records -> one uint64 each, in the order of (packet, offset, pattern)"""
-    assert len(rec) == 0 or (int(rec["packet"].max()) < 1 << 24 and int(rec["pattern"].max()) < 256)
-    return (rec["packet"].astype(np.uint64) << np.uint64(40)) | (rec["offset"].astype(np.uint64) << np.uint64(8)) | \
-        rec["pattern"].astype(np.uint64)
-
-
-def fold(data):
-    """ASCII case folding (A-Z to a-z, nothing else) of a uint8 array"""
-    out = np.array(data, dtype=np.uint8)
-    out[(out >= 0x41) & (out <= 0x5A)] += 0x20
-    return out
-
-
-def udp_frame(payload, proto=17, ihl=5):
-    """Ethernet + IPv4 (ihl words) + UDP header + payload"""
-    return b"\x02" * 12 + b"\x08\x00" + bytes([0x40 | ihl, 0, 0, 0, 0, 0, 0, 0, 64, proto]) + bytes(10 + 8) + bytes(payload)
-
-
-def device_copy(data, offsets):
-    import torch
-
-    d_bytes = torch.zeros(len(data) + 64, dtype=torch.uint8, device="cuda:0")
-    d_bytes[: len(data)] = torch.from_numpy(np.ascontiguousarray(data))
-    return d_bytes, torch.from_numpy(offsets.astype(np.int64)).to("cuda:0")
 
 
 class Call:
@@ -118,44 +92,36 @@ def strings(strings_txt):
 
 
 @pytest.fixture(scope="module")
-def finder(tmp_path_factory):
-    return RefFinder(str(tmp_path_factory.mktemp("kmp_find_ref")))
-
-
-@pytest.fixture(scope="module")
 def m(strings):
     with kmp.Matcher(0) as m:
         m.set_patterns(strings)
         yield m
 
 
-def expected(b, oracle, finder, patterns):
-    b.counts = oracle.count_csr(b.data, b.offsets, patterns)
-    rec = finder.find_csr(b.data, b.offsets, patterns)
-    assert_invariant(b.counts, rec, patterns)
-    b.keys = keys(rec)
+def batch(data, offsets, oracle, patterns):
+    """the batch on the host and the device, with its expected counts and record keys"""
+    counts, rec, _ = expected(patterns, data, offsets, oracle=oracle)
+    d = DeviceBatch(data, offsets)
+    b = SimpleNamespace(data=data, offsets=offsets, n=len(offsets) - 1, span=(0, int(offsets[-1])), counts=counts,
+                        keys=keys(rec), d_bytes=d.d_bytes, d_off=d.d_off)
     assert len(b.keys) > 1000
     return b
 
 
 @pytest.fixture(scope="module")
-def A(oracle, finder, strings):
+def A(oracle, strings):
     data, offsets = kmp.Synth(seed=0xA, payload_len=1400, plants=2, plant_patterns=strings).fill_host(0, 20_000)
-    a = expected(SimpleNamespace(data=data, offsets=offsets, n=len(offsets) - 1, span=(0, int(offsets[-1]))),
-                 oracle, finder, strings)
-    a.d_bytes, a.d_off = device_copy(data, offsets)
+    a = batch(data, offsets, oracle, strings)
     a.other = strings[::5] + [b"zz", b"~~", b"Ab"]  # a second pattern set, and its counts on A
     a.other_counts = oracle.count_csr(data, offsets, a.other)
     return a
 
 
 @pytest.fixture(scope="module")
-def B(oracle, finder, strings, tmp_path_factory):
+def B(oracle, strings, tmp_path_factory):
     data, offsets = kmp.Synth(seed=0xB, len_mode=1, plants=2, plant_patterns=strings).fill_host(0, 12_000)
-    b = expected(SimpleNamespace(data=data, offsets=offsets, n=len(offsets) - 1, span=(0, int(offsets[-1]))),
-                 oracle, finder, strings)
+    b = batch(data, offsets, oracle, strings)
     assert len(set(np.diff(offsets.astype(np.int64)).tolist())) == 4  # 64, 576, 1400 and 9000 bytes
-    b.d_bytes, b.d_off = device_copy(data, offsets)
     b.path = str(tmp_path_factory.mktemp("call_order") / "b.pcap")
     bench.write_pcap(b.path, data, offsets)
     b.frames = [udp_frame(data[int(x):int(y)]) for x, y in zip(offsets[:-1], offsets[1:])]
@@ -263,7 +229,7 @@ def test_host_work_behind_a_device_call(m, strings, A, B, L, work):
             elif work == "count_pcap":
                 ok = m.count_pcap_streamed(B.path) == B.counts
             elif work == "find_pcap":
-                rec = m.find_pcap(B.path)[["packet", "offset", "pattern"]].astype(kmp.MATCH_DTYPE)
+                rec = m.find_pcap(B.path)[ORDER].astype(kmp.MATCH_DTYPE)
                 ok = np.array_equal(keys(rec), B.keys)
             elif work == "stream":
                 with m.stream("udp") as st:
@@ -343,7 +309,7 @@ def test_open_stream_refuses_other_work(m, oracle, strings, A, B):
         torch.cuda.synchronize()
         assert c.mismatch() is None, form
     assert m.count_pcap_streamed(B.path) == B.counts
-    assert np.array_equal(keys(m.find_pcap(B.path)[["packet", "offset", "pattern"]].astype(kmp.MATCH_DTYPE)), B.keys)
+    assert np.array_equal(keys(m.find_pcap(B.path)[ORDER].astype(kmp.MATCH_DTYPE)), B.keys)
     kmp.matcher.check(kmp.lib().kmpb_reserve_staging(m.handle, 0, 0))
     with m.stream("udp") as st:
         for f in B.frames:
@@ -397,15 +363,14 @@ def test_stream_batch_edges():
 
 # ---- 5. two contexts, two host threads ------------------------------------------------------------------------------
 
-def test_two_contexts_two_threads(oracle, finder, strings, A, B):
+def test_two_contexts_two_threads(oracle, strings, A, B):
     """Each context has its own pattern set (one of them all nocase) and its own batch; their calls overlap."""
     import torch
 
     nc = [p.upper() if i % 2 else p.swapcase() for i, p in enumerate(strings)] + [b"HtTp", b"UDP"]
-    folded = fold(B.data)
+    nc_counts, nc_rec, _ = expected(nc, B.data, B.offsets, nocase=True, oracle=oracle)
     jobs = [SimpleNamespace(patterns=strings, nocase=False, b=A, counts=A.counts, keys=A.keys),
-            SimpleNamespace(patterns=nc, nocase=True, b=B, counts=oracle.count_csr(folded, B.offsets, [p.lower() for p in nc]),
-                            keys=keys(finder.find_csr(folded, B.offsets, [p.lower() for p in nc])))]
+            SimpleNamespace(patterns=nc, nocase=True, b=B, counts=nc_counts, keys=keys(nc_rec))]
     assert jobs[1].counts != oracle.count_csr(B.data, B.offsets, nc)
     errors = []
     start = threading.Barrier(len(jobs))

@@ -5,8 +5,8 @@ overflows it many times over."""
 import numpy as np
 import pytest
 
-from test_find import RefFinder, assert_invariant, csr
-from test_host import _udp_frame, _write_pcap
+from kmpb_harness import udp_frame, write_pcap
+from kmpb_reference import assert_invariant, csr, finder
 
 import multithreading_string_matching_b200 as kmp
 
@@ -18,10 +18,10 @@ def test_find_records_past_the_slot_buffer(monkeypatch, tmp_path):
     packets = [sparse] * 256 + [b"a" * 4096] * 1024  # 4096 records a packet: every later chunk overflows it
     data, offsets = csr(packets)
     patterns = [b"a"]
-    want = RefFinder(str(tmp_path)).find_csr(data, offsets, patterns)
+    want = finder().find_csr(data, offsets, patterns)
     assert len(want) == 256 * 8 + 1024 * 4096
     path = str(tmp_path / "dense.pcap")
-    _write_pcap(path, [_udp_frame(p) for p in packets])
+    write_pcap(path, [udp_frame(p) for p in packets])
     with kmp.Matcher(0) as m:
         m.set_patterns(patterns)
         counts = m.count_host(data, offsets)

@@ -9,6 +9,8 @@ import numpy as np
 import pytest
 
 from conftest import DATA, GOLDEN, ROOT, golden_runs
+from kmpb_harness import MATCH, build_integration_snippet, pcap_frames
+from kmpb_reference import csr
 
 import multithreading_string_matching_b200 as kmp
 
@@ -27,13 +29,6 @@ def matchers():
 @pytest.fixture(scope="module")
 def strings(strings_txt):
     return kmp.load_patterns(strings_txt)
-
-
-def csr(packets):
-    offsets = np.zeros(len(packets) + 1, dtype=np.uint64)
-    if packets:
-        np.cumsum([len(p) for p in packets], out=offsets[1:])
-    return np.frombuffer(b"".join(packets) + b"\0" * 16, dtype=np.uint8)[: int(offsets[-1])], offsets
 
 
 def check_all(matchers, oracle, patterns, packets, engines=ENGINES, label=""):
@@ -96,28 +91,13 @@ def test_streamed_path_chunks_and_slices(matchers, oracle, strings, tmp_path):
     assert m.count_pcap_streamed(path) == want
 
 
-def _classic_frames(path):
-    import struct
-    raw = open(path, "rb").read()
-    e = "<" if raw[:4] in (b"\xd4\xc3\xb2\xa1", b"\x4d\x3c\xb2\xa1") else ">"
-    at, out = 24, []
-    while at + 16 <= len(raw):
-        caplen = struct.unpack_from(e + "I", raw, at + 8)[0]
-        at += 16
-        if at + caplen > len(raw):
-            break
-        out.append(raw[at:at + caplen])
-        at += caplen
-    return out
-
-
 @pytest.mark.parametrize("pcap,proto,expected", golden_runs(), ids=lambda v: v if isinstance(v, str) else "")
 def test_frames_pushed_one_at_a_time(matchers, strings, pcap, proto, expected):
     """kmpb_stream_*: the live-capture shape (live_openmp_task.c:160-217) fed with the frames of a savefile;
     64 KB batches so that the staging slots are reused many times, a flush in the middle."""
     m = matchers["union"]
     m.set_patterns(strings)
-    frames = _classic_frames(os.path.join(DATA, pcap + ".pcap"))
+    frames = pcap_frames(os.path.join(DATA, pcap + ".pcap"))
     with m.stream(proto, batch_bytes=65536) as st:
         for f in frames[: len(frames) // 2]:
             st.push(f)
@@ -129,10 +109,9 @@ def test_frames_pushed_one_at_a_time(matchers, strings, pcap, proto, expected):
 
 
 def test_cli_output_is_the_reference_output(strings):
-    exe = os.path.join(ROOT, "multithreading_string_matching_b200", "bin", "kmp_match")
     for pcap, proto, expected in golden_runs():
         for argv in [[proto], ["1", proto]] + ([[]] if proto == "udp" else []):
-            r = subprocess.run([exe, os.path.join(DATA, pcap + ".pcap"), os.path.join(DATA, "strings.txt"), *argv],
+            r = subprocess.run([MATCH, os.path.join(DATA, pcap + ".pcap"), os.path.join(DATA, "strings.txt"), *argv],
                                capture_output=True)
             assert r.returncode == 0, r.stderr
             lines = r.stdout.splitlines(keepends=True)
@@ -160,7 +139,6 @@ def test_bench_dump_outputs_are_the_stream_counts(oracle, strings, tmp_path):
 def test_integration_snippet_counts(tmp_path):
     """INTEGRATION.md section 1 as a C program (tests/c/integration_snippet.c): overlapping "aa" in "aaaa" = 3, the
     text of a payload ends at its NUL."""
-    from test_host import build_integration_snippet
     r = subprocess.run([build_integration_snippet(tmp_path)], capture_output=True, text=True)
     assert r.returncode == 0 and r.stdout == "aa: 3 times!\nhttp: 3 times!\n", (r.stdout, r.stderr)
 

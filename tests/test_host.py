@@ -10,7 +10,8 @@ import subprocess
 import numpy as np
 import pytest
 
-from conftest import DATA, GOLDEN, ROOT, golden_runs
+from conftest import DATA, GOLDEN, ROOT
+from kmpb_harness import MATCH, PCAPS, build_integration_snippet, pcapng, udp_frame, write_pcap
 
 import multithreading_string_matching_b200 as kmp
 
@@ -82,7 +83,7 @@ def test_extractors_match_reference_vectors(oracle):
         assert got == oracle.extract(frame, v["proto"])
 
 
-@pytest.mark.parametrize("pcap", ["udp", "udp_1000", "big_udp", "very_big_udp", "tcp"])
+@pytest.mark.parametrize("pcap", PCAPS)
 @pytest.mark.parametrize("proto", ["udp", "tcp"])
 def test_packer_matches_oracle_csr(oracle, pcap, proto):
     path = os.path.join(DATA, pcap + ".pcap")
@@ -93,28 +94,13 @@ def test_packer_matches_oracle_csr(oracle, pcap, proto):
     assert np.array_equal(batch.data, data)
 
 
-def _write_pcap(path, frames, magic=0xA1B2C3D4, swapped=False, caplens=None):
-    e = ">" if swapped else "<"
-    with open(path, "wb") as f:
-        f.write(struct.pack(e + "IHHiIII", magic, 2, 4, 0, 0, 262144, 1))
-        for i, fr in enumerate(frames):
-            cap = len(fr) if caplens is None else caplens[i]
-            f.write(struct.pack(e + "IIII", 1, 2, cap, len(fr)))
-            f.write(fr[:cap])
-
-
-def _udp_frame(payload, ihl=5):
-    ip = bytes([0x40 | ihl, 0, 0, 0, 0, 0, 0, 0, 64, 17]) + b"\0" * (ihl * 4 - 10)
-    return b"\x02" * 12 + b"\x08\x00" + ip + b"\0" * 8 + payload
-
-
 def test_packer_savefile_variants(oracle, tmp_path):
-    frames = [_udp_frame(b"hello world"), b"short", _udp_frame(b"", ihl=6), _udp_frame(b"x" * 1400), _udp_frame(b"a\0b")]
+    frames = [udp_frame(b"hello world"), b"short", udp_frame(b"", ihl=6), udp_frame(b"x" * 1400), udp_frame(b"a\0b")]
     want = None
     for name, kw in {"le_usec": {}, "le_nsec": {"magic": 0xA1B23C4D}, "be_usec": {"swapped": True},
                      "be_nsec": {"magic": 0xA1B23C4D, "swapped": True}}.items():
         p = str(tmp_path / (name + ".pcap"))
-        _write_pcap(p, frames, **kw)
+        write_pcap(p, frames, **kw)
         b = kmp.PayloadBatch(p, "udp")
         got = (b.n_frames, b.offsets.tolist(), b.data.tobytes())
         assert got[0] == 5 and got[1] == [0, 11, 11, 1411, 1414]
@@ -124,7 +110,7 @@ def test_packer_savefile_variants(oracle, tmp_path):
         assert (fr, o.tolist(), d.tobytes()) == got
     # a truncated trailing record ends the walk silently, like the reference's `>= 0` loop
     p = str(tmp_path / "trunc.pcap")
-    _write_pcap(p, frames)
+    write_pcap(p, frames)
     size = os.path.getsize(p)
     with open(p, "r+b") as f:
         f.truncate(size - 3)
@@ -134,7 +120,7 @@ def test_packer_savefile_variants(oracle, tmp_path):
     assert (fr, len(o) - 1) == (4, 3)
     # caplen < len: the captured bytes are what is parsed (openmp_data.c:114-116)
     p = str(tmp_path / "snap.pcap")
-    _write_pcap(p, [_udp_frame(b"abcdefgh")], caplens=[46])
+    write_pcap(p, [udp_frame(b"abcdefgh")], caplens=[46])
     b = kmp.PayloadBatch(p, "udp")
     assert b.data.tobytes() == b"abcd"
     # not a pcap
@@ -151,8 +137,8 @@ def test_savefile_payload_length_scan(tmp_path):
     """kmpb_pcap_first_long: the scan the savefile forms run over the accepted packets before anything else, to refuse
     a payload of KMPB_PACKET_LIMIT bytes or more (a payload is the captured length less the headers: any size)."""
     p = str(tmp_path / "lens.pcap")
-    _write_pcap(p, [_udp_frame(b"x" * 10), b"not udp", _udp_frame(b"y" * 300), _udp_frame(b""), _udp_frame(b"z" * 5000),
-                    _udp_frame(b"w" * 7)])
+    write_pcap(p, [udp_frame(b"x" * 10), b"not udp", udp_frame(b"y" * 300), udp_frame(b""), udp_frame(b"z" * 5000),
+                    udp_frame(b"w" * 7)])
     lib = kmp.lib()
     fn = lib.kmpb_pcap_first_long
     fn.restype = ctypes.c_uint64
@@ -173,52 +159,23 @@ def test_savefile_payload_length_scan(tmp_path):
         lib.kmpb_pcap_close(pc)
 
 
-def _pcapng(frames, big_endian=False, simple_from=None, second_section_at=None):
-    """A pcapng file by hand: SHB, IDB, one packet block per frame (Enhanced; Simple from index `simple_from`
-    on), a name-resolution block in the middle, optionally a second section in the other byte order."""
-    import struct
-
-    def blocks(frames, e, first_index):
-        def block(btype, body):
-            body += b"\0" * (-len(body) % 4)
-            total = len(body) + 12
-            return struct.pack(e + "II", btype, total) + body + struct.pack(e + "I", total)
-
-        out = block(0x0A0D0D0A, struct.pack(e + "IHHq", 0x1A2B3C4D, 1, 0, -1) + struct.pack(e + "HH", 2, 5) + b"shark\0\0\0" + struct.pack(e + "HH", 0, 0))
-        out += block(1, struct.pack(e + "HHI", 1, 0, 262144))
-        for k, f in enumerate(frames):
-            if k == 1:
-                out += block(4, b"\0" * 8)  # a Name Resolution Block: skipped
-            if simple_from is not None and first_index + k >= simple_from:
-                out += block(3, struct.pack(e + "I", len(f)) + f)
-            else:
-                out += block(6, struct.pack(e + "IIIII", 0, 0, k, len(f), len(f)) + f + b"\0" * (-len(f) % 4) + struct.pack(e + "HHI", 1, 4, 0x64636261) + struct.pack(e + "HH", 0, 0))
-        return out
-
-    e = ">" if big_endian else "<"
-    if second_section_at is None:
-        return blocks(frames, e, 0)
-    other = "<" if big_endian else ">"
-    return blocks(frames[:second_section_at], e, 0) + blocks(frames[second_section_at:], other, second_section_at)
-
-
 def test_packer_reads_pcapng(tmp_path):
     """SURVEY 8f-3: libpcap also hands the reference pcapng files; same frames, same batch."""
-    frames = [_udp_frame(b"hello world"), b"short", _udp_frame(b"", ihl=6), _udp_frame(b"x" * 1401), _udp_frame(b"a\0b")]
+    frames = [udp_frame(b"hello world"), b"short", udp_frame(b"", ihl=6), udp_frame(b"x" * 1401), udp_frame(b"a\0b")]
     classic = str(tmp_path / "classic.pcap")
-    _write_pcap(classic, frames)
+    write_pcap(classic, frames)
     b = kmp.PayloadBatch(classic, "udp")
     want = (b.n_frames, b.offsets.tolist(), b.data.tobytes())
     for name, kw in {"le": {}, "be": {"big_endian": True}, "simple": {"simple_from": 2},
                      "two_sections": {"second_section_at": 3}, "two_sections_be": {"big_endian": True, "second_section_at": 2}}.items():
         p = str(tmp_path / (name + ".pcapng"))
         with open(p, "wb") as f:
-            f.write(_pcapng(frames, **kw))
+            f.write(pcapng(frames, **kw))
         b = kmp.PayloadBatch(p, "udp")
         assert (b.n_frames, b.offsets.tolist(), b.data.tobytes()) == want, name
     # a block cut short ends the walk silently
     p = str(tmp_path / "cut.pcapng")
-    data = _pcapng(frames)
+    data = pcapng(frames)
     with open(p, "wb") as f:
         f.write(data[:-30])
     b = kmp.PayloadBatch(p, "udp")
@@ -279,14 +236,13 @@ def test_host_tables_selfcheck(tmp_path):
 
 def test_cli_usage_and_errors(tmp_path):
     """serial.c:43,49,60-63: usage on stdout + exit 1; unreadable strings file -> perror + exit 1."""
-    exe = os.path.join(ROOT, "multithreading_string_matching_b200", "bin", "kmp_match")
-    r = subprocess.run([exe], capture_output=True, text=True)
+    r = subprocess.run([MATCH], capture_output=True, text=True)
     assert r.returncode == 1 and r.stdout.startswith("USAGE: ") and "<file.pcap> <string.txt> [tcp/udp]" in r.stdout
-    r = subprocess.run([exe, "a", "b", "icmp"], capture_output=True, text=True)
+    r = subprocess.run([MATCH, "a", "b", "icmp"], capture_output=True, text=True)
     assert r.returncode == 1 and r.stdout.startswith("USAGE ")
-    r = subprocess.run([exe, "a", "b", "2", "icmp"], capture_output=True, text=True)
+    r = subprocess.run([MATCH, "a", "b", "2", "icmp"], capture_output=True, text=True)
     assert r.returncode == 1 and "gpu_number" in r.stdout
-    r = subprocess.run([exe, os.path.join(DATA, "udp.pcap"), str(tmp_path / "missing.txt")], capture_output=True, text=True)
+    r = subprocess.run([MATCH, os.path.join(DATA, "udp.pcap"), str(tmp_path / "missing.txt")], capture_output=True, text=True)
     assert r.returncode == 1 and r.stderr.startswith("error opening file: ")
 
 
@@ -354,9 +310,9 @@ def test_host_side_is_sanitizer_clean(tmp_path):
     damaged += [str(tmp_path / "noise.pcap"), str(tmp_path / "lying.pcap")]
     damaged += [str(tmp_path / "noise.pcap"), str(tmp_path / "lying.pcap")]
     # pcapng: both byte orders and several sections, whole and cut at every eighth byte, and with corrupted block lengths
-    frames = [_udp_frame(b"hello world"), b"short", _udp_frame(b"", ihl=6), _udp_frame(b"x" * 1401), _udp_frame(b"a\0b")]
+    frames = [udp_frame(b"hello world"), b"short", udp_frame(b"", ihl=6), udp_frame(b"x" * 1401), udp_frame(b"a\0b")]
     for name, kw in {"le": {}, "be": {"big_endian": True}, "simple": {"simple_from": 2}, "two": {"second_section_at": 3}}.items():
-        ng = _pcapng(frames, **kw)
+        ng = pcapng(frames, **kw)
         for cut in list(range(0, min(len(ng), 400), 8)) + [len(ng) - 1, len(ng)]:
             p = tmp_path / ("%s_%d.pcapng" % (name, cut))
             p.write_bytes(ng[:cut])
@@ -374,17 +330,6 @@ def test_host_side_is_sanitizer_clean(tmp_path):
                  "big_udp.pcap udp packets=3358 bytes=599424 nulfree=1038", "very_big_udp.pcap udp packets=13768 bytes=1321746 nulfree=0",
                  "tcp.pcap tcp packets=13 ", "udp_1000.pcap tcp packets=20 "):
         assert want in r.stdout, (want, r.stdout)
-
-
-def build_integration_snippet(tmp_path):
-    """tests/c/integration_snippet.c (the call sequence of INTEGRATION.md section 1) against include/kmpb200.h and
-    libkmpb200.so only."""
-    exe = str(tmp_path / "integration_snippet")
-    pkg = os.path.join(ROOT, "multithreading_string_matching_b200")
-    subprocess.run(["/usr/bin/gcc" if os.path.exists("/usr/bin/gcc") else "gcc", "-O1", "-g", "-Wall", "-Wextra", "-Werror",
-                    "-I" + os.path.join(ROOT, "include"), os.path.join(ROOT, "tests", "c", "integration_snippet.c"),
-                    "-L" + pkg, "-lkmpb200", "-Wl,-rpath," + pkg, "-o", exe], check=True)
-    return exe
 
 
 def test_integration_snippet_links_and_refuses_without_a_device(tmp_path):

@@ -23,7 +23,8 @@ from types import SimpleNamespace
 import numpy as np
 import pytest
 
-from test_find import RefFinder, first_index
+from kmpb_harness import DeviceBatch, udp_frame
+from kmpb_reference import finder, firsts, keys
 
 import multithreading_string_matching_b200 as kmp
 
@@ -60,21 +61,9 @@ def pattern_set(strings):
     return pats
 
 
-def keys_of(packet, offset, pattern):
-    """one sortable uint64 per record: (packet, offset, pattern) order is key order"""
-    packet, offset, pattern = (np.asarray(a, dtype=np.uint64) for a in (packet, offset, pattern))
-    if packet.size:
-        assert int(packet.max()) < 1 << 23 and int(offset.max()) < 1 << 31 and int(pattern.max()) < 1 << 10
-    return (packet << np.uint64(41)) | (offset << np.uint64(10)) | pattern
-
-
-def rec_keys(rec):
-    return keys_of(rec["packet"], rec["offset"], rec["pattern"])
-
-
-def key_counts(keys, patterns):
-    hist = np.bincount((keys & np.uint64(1023)).astype(np.int64), minlength=len(patterns))
-    return [int(hist[f]) for f in first_index(patterns)]
+def key_counts(k, patterns):
+    hist = np.bincount((k & np.uint64(1023)).astype(np.int64), minlength=len(patterns))
+    return [int(hist[f]) for f in firsts(patterns)]
 
 
 # ---- the planted content ----------------------------------------------------------------------------
@@ -132,7 +121,7 @@ class Plan:
             d_bytes[torch.from_numpy(idx).cuda()] = torch.from_numpy(vals.copy()).cuda()
         torch.cuda.synchronize()
 
-    def expect(self, offsets, patterns, finder):
+    def expect(self, offsets, patterns):
         """sorted record keys of the batch `offsets` (absolute, packets numbered from 0) over this content"""
         offsets = np.asarray(offsets, dtype=np.uint64)
         off = offsets.astype(np.int64)
@@ -164,11 +153,11 @@ class Plan:
             data = np.frombuffer(b"".join(pieces[i] for i in keep), dtype=np.uint8)
             cut = np.zeros(len(keep) + 1, dtype=np.uint64)
             np.cumsum([len(pieces[i]) for i in keep], out=cut[1:])
-            r = finder.find_csr(data, cut, patterns)
+            r = finder().find_csr(data, cut, patterns)
             kk = np.array([pk[i] for i in keep], dtype=np.uint64)
             oo = np.array([po[i] for i in keep], dtype=np.uint64)
             j = r["packet"].astype(np.int64)
-            parts.append(keys_of(kk[j], oo[j] + r["offset"], r["pattern"]))
+            parts.append(keys({"packet": kk[j], "offset": oo[j] + r["offset"], "pattern": r["pattern"]}))
         # markers alone in their packet: the records of "id", shifted, unless a NUL comes before them
         m = self.markers[(self.markers >= lo) & (self.markers < hi)]
         if m.size:
@@ -179,9 +168,9 @@ class Plan:
                 nul_at[kn] = z
             alive = nul_at[k] > m
             k, m = k[alive], m[alive]
-            t = finder.find_csr(np.frombuffer(MARK, np.uint8), np.array([0, len(MARK)], np.uint64), patterns)
+            t = finder().find_csr(np.frombuffer(MARK, np.uint8), np.array([0, len(MARK)], np.uint64), patterns)
             for ro, rp in zip(t["offset"].tolist(), t["pattern"].tolist()):
-                parts.append(keys_of(k, m - off[k] + ro, np.full(k.size, rp)))
+                parts.append(keys({"packet": k, "offset": m - off[k] + ro, "pattern": np.full(k.size, rp)}))
         return np.sort(np.concatenate(parts)) if parts else np.zeros(0, dtype=np.uint64)
 
 
@@ -221,11 +210,6 @@ def with_len_at_least(off, k, step, n=200):
 # ---- fixtures -------------------------------------------------------------------------------------
 
 @pytest.fixture(scope="module")
-def finder(tmp_path_factory):
-    return RefFinder(str(tmp_path_factory.mktemp("kmp_find_ref")))
-
-
-@pytest.fixture(scope="module")
 def patterns(strings_txt):
     return pattern_set(kmp.load_patterns(strings_txt))
 
@@ -254,7 +238,7 @@ def need_device(nbytes):
         pytest.skip("needs %.1f GiB of free device memory" % (nbytes / GiB))
 
 
-def build_stream(patterns, finder):
+def build_stream(patterns):
     """The ~9.3 GiB stream's layouts over the same bytes -- A (packets straddle 2^32 and 2^33), B (A cut at exactly 2^32
     and 2^33), C (A with the packet before the one straddling 2^32 merged into it, so that a NUL 1.1 MB below 2^32 ends
     that packet's text) -- the spans checked, the planted content and the expected records (host only)."""
@@ -367,7 +351,7 @@ def build_stream(patterns, finder):
     plan = Plan(markers, islands)
 
     g = SimpleNamespace(plan=plan, layouts=layouts, spans=spans, big_packets=big_pk)
-    whole = plan.expect(off_a, patterns, finder)
+    whole = plan.expect(off_a, patterns)
     g.want = {}
     for name, (lay, s0, s1) in spans.items():
         if lay == "a":
@@ -375,46 +359,22 @@ def build_stream(patterns, finder):
             sel = whole[(pk >= s0) & (pk < s1)]
             g.want[name] = sel - (np.uint64(s0) << np.uint64(41))
         else:
-            g.want[name] = plan.expect(layouts[lay][s0:s1 + 1].astype(np.uint64), patterns, finder)
+            g.want[name] = plan.expect(layouts[lay][s0:s1 + 1].astype(np.uint64), patterns)
     return g
 
 
 @pytest.fixture(scope="module")
-def big(patterns, finder):
+def big(patterns):
     import torch
 
     need_device(13 * GiB)
-    g = build_stream(patterns, finder)
+    g = build_stream(patterns)
     g.d_bytes = torch.empty(N + 4096, dtype=torch.uint8, device="cuda:0")
     g.plan.write(g.d_bytes, SEED)
-    g.d_off = {lay: torch.from_numpy(o).cuda() for lay, o in g.layouts.items()}
+    g.batch = {lay: DeviceBatch.on_device(g.d_bytes, torch.from_numpy(o).cuda(), o) for lay, o in g.layouts.items()}
     yield g
-    del g.d_bytes, g.d_off
+    del g.d_bytes, g.batch
     torch.cuda.empty_cache()
-
-
-def device_find(m, d_bytes, d_off, k0, k1, span, capacity, sorted_, canary=64):
-    """kmpb_find_device_span over packets [k0, k1) of a device batch -> (records, total, canary intact)"""
-    import torch
-
-    d_out = torch.full(((capacity + canary) * 16,), 0xA5, dtype=torch.uint8, device="cuda:0")
-    d_n = torch.full((1,), -1, dtype=torch.int64, device="cuda:0")
-    m.find_device(d_bytes.data_ptr(), d_off.data_ptr() + 8 * k0, k1 - k0, d_out.data_ptr(), capacity, d_n.data_ptr(),
-                  span, sorted=sorted_)
-    torch.cuda.synchronize()
-    total = int(d_n.item())
-    rec = d_out[: 16 * min(total, capacity)].cpu().numpy().view(kmp.MATCH_DTYPE)
-    ok = bool((d_out[16 * capacity:] == 0xA5).all().item())
-    return rec, total, ok
-
-
-def device_counts(m, d_bytes, d_off, k0, k1, span, n_pat):
-    import torch
-
-    d_counts = torch.zeros(n_pat, dtype=torch.int64, device="cuda:0")
-    m.count_device(d_bytes.data_ptr(), d_off.data_ptr() + 8 * k0, k1 - k0, d_counts.data_ptr(), span=span)
-    torch.cuda.synchronize()
-    return d_counts.cpu().tolist()
 
 
 def diff(got, want):
@@ -423,26 +383,26 @@ def diff(got, want):
     return "%d got, %d expected; missing %s; extra %s" % (len(got), len(want), dec(w - g), dec(g - w))
 
 
-def check_all_forms(m, patterns, d_bytes, d_off, k0, k1, span, want, label, perpat=True):
+def check_all_forms(m, patterns, batch, k0, k1, want, label, perpat=True):
     """count (union, per-pattern), find unsorted, sorted, and sorted into a buffer one record short"""
     counts = key_counts(want, patterns)
     assert len(want) > 0
-    assert device_counts(m, d_bytes, d_off, k0, k1, span, len(patterns)) == counts, (label, "union counts")
+    assert batch.count(m, k0=k0, k1=k1) == [counts], (label, "union counts")
     if perpat:
         m.set_engine("perpat")
         try:
-            assert device_counts(m, d_bytes, d_off, k0, k1, span, len(patterns)) == counts, (label, "perpat counts")
+            assert batch.count(m, k0=k0, k1=k1) == [counts], (label, "perpat counts")
         finally:
             m.set_engine("union")
     total = len(want)
-    rec, n, ok = device_find(m, d_bytes, d_off, k0, k1, span, total, False)
-    got = np.sort(rec_keys(rec))
+    rec, n, ok = batch.find(m, total, False, k0, k1, canary=64)
+    got = np.sort(keys(rec))
     assert n == total and ok and np.array_equal(got, want), (label, "unsorted", diff(got, want))
-    rec, n, ok = device_find(m, d_bytes, d_off, k0, k1, span, total, True)
-    got = rec_keys(rec)
+    rec, n, ok = batch.find(m, total, True, k0, k1, canary=64)
+    got = keys(rec)
     assert n == total and ok and np.array_equal(got, want), (label, "sorted", diff(got, want))
-    rec, n, ok = device_find(m, d_bytes, d_off, k0, k1, span, total - 1, True)
-    got = np.sort(rec_keys(rec))
+    rec, n, ok = batch.find(m, total - 1, True, k0, k1, canary=64)
+    got = np.sort(keys(rec))
     at = np.minimum(np.searchsorted(want, got), total - 1)
     assert n == total and ok and len(got) == total - 1, (label, "capacity - 1", n)
     assert (np.diff(got) > 0).all() and (want[at] == got).all(), (label, "capacity - 1: not a distinct subset")
@@ -452,7 +412,7 @@ def check_all_forms(m, patterns, d_bytes, d_off, k0, k1, span, want, label, perp
 # ---- packets at the size limit (own 2 GiB buffer: runs before the big stream is built) ----------------
 
 @pytest.fixture(scope="class")
-def limit_batch(patterns, finder):
+def limit_batch(patterns):
     """~2 GiB buffer around a packet of LIMIT - 1 bytes, its host copy, and a context of its own: the host forms grow
     the context's four staging slots to the size of that packet, and closing it gives their 8 GiB back"""
     import torch
@@ -499,7 +459,7 @@ def limit_batch(patterns, finder):
 class TestPacketLimit:
     """A packet of LIMIT - 1 bytes works in every form; one of LIMIT bytes is refused (one 2 GiB buffer for both)."""
 
-    def test_packet_one_byte_under_the_limit(self, patterns, finder, limit_batch):
+    def test_packet_one_byte_under_the_limit(self, patterns, limit_batch):
         """A packet of LIMIT - 1 bytes behind ~150 KiB of small packets and before a few more, and the same packet alone:
         exact counts and records through the device forms, kmpb_count_host and kmpb_find_host, and no KMPB_ELIMIT."""
         import torch
@@ -508,15 +468,13 @@ class TestPacketLimit:
         matcher, plan, d_bytes, host, off, g = lb.m, lb.plan, lb.d_bytes, lb.host, lb.off, lb.g
         cases = {"with neighbours": off, "alone": off[g:g + 2]}
         for label, offs in cases.items():
-            want = plan.expect(offs, patterns, finder)
+            want = plan.expect(offs, patterns)
             counts = key_counts(want, patterns)
             assert len(want) > 100 and counts[patterns.index(long_patterns()[1])] >= 1, label
-            d_off = torch.from_numpy(offs.astype(np.int64)).cuda()
-            n = len(offs) - 1
-            span = (int(offs[0]), int(offs[-1]))
-            check_all_forms(matcher, patterns, d_bytes, d_off, 0, n, span, want, label, perpat=False)
+            batch = DeviceBatch.on_device(d_bytes, torch.from_numpy(offs.astype(np.int64)).cuda(), offs)
+            check_all_forms(matcher, patterns, batch, 0, len(offs) - 1, want, label, perpat=False)
             assert matcher.count_host(host, offs) == counts, label
-            got = rec_keys(matcher.find_host(host, offs))
+            got = keys(matcher.find_host(host, offs))
             assert np.array_equal(got, want), (label, "find_host", diff(got, want))
 
     def test_packet_at_the_limit_is_refused(self, limit_batch):
@@ -532,14 +490,12 @@ class TestPacketLimit:
                 with pytest.raises(kmp.KmpbError) as e:
                     call(host, offs)
                 assert e.value.code == ELIMIT and "packet %d " % (len(offs) - 2) in str(e.value), str(e.value)
-            d_off = torch.from_numpy(offs.astype(np.int64)).cuda()
-            device_counts(matcher, d_bytes, d_off, 0, len(offs) - 1, (int(offs[0]), int(offs[-1])), len(matcher.patterns))
+            DeviceBatch.on_device(d_bytes, torch.from_numpy(offs.astype(np.int64)).cuda(), offs).count(matcher)
             lib = kmp.lib()
             assert lib.kmpb_check_device_errors(matcher.handle) == ELIMIT
             assert lib.kmpb_check_device_errors(matcher.handle) == 0
         # a batch within the limits afterwards: clean
-        d_off = torch.from_numpy(off.astype(np.int64)).cuda()
-        device_counts(matcher, d_bytes, d_off, 0, len(off) - 1, (0, int(off[-1])), len(matcher.patterns))
+        DeviceBatch.on_device(d_bytes, torch.from_numpy(off.astype(np.int64)).cuda(), off).count(matcher)
         kmp.matcher.check(kmp.lib().kmpb_check_device_errors(matcher.handle))
 
 
@@ -551,8 +507,7 @@ def test_device_spans(matcher, patterns, big, name):
     first: whole (256 KiB items), 5 GiB from an odd first byte near 3.5 GiB across 2^32 and 2^33 (128 KiB items), a
     slice that starts exactly at 2^32, 1 GiB above 2^33 (high word 2 everywhere), the first 3 GiB (64 KiB items)."""
     lay, k0, k1 = big.spans[name]
-    o = big.layouts[lay]
-    check_all_forms(matcher, patterns, big.d_bytes, big.d_off[lay], k0, k1, (int(o[k0]), int(o[k1])), big.want[name], name)
+    check_all_forms(matcher, patterns, big.batch[lay], k0, k1, big.want[name], name)
 
 
 def test_plants_are_where_they_should_be(patterns, big):
@@ -562,12 +517,12 @@ def test_plants_are_where_they_should_be(patterns, big):
     ib = big.spans["from_2^32"][1:]
     oa, ob = big.layouts["a"], big.layouts["b"]
 
-    def at(layout, keys, pos, pat, k_base=0):
+    def at(layout, want, pos, pat, k_base=0):
         o = big.layouts[layout]
         k = int(np.searchsorted(o, pos, "right")) - 1
-        key = keys_of([k - k_base], [pos - int(o[k])], [patterns.index(pat)])[0]
-        i = int(np.searchsorted(keys, key))
-        return i < len(keys) and keys[i] == key
+        key = keys({"packet": [k - k_base], "offset": [pos - int(o[k])], "pattern": [patterns.index(pat)]})[0]
+        i = int(np.searchsorted(want, key))
+        return i < len(want) and want[i] == key
 
     wa, wb, wc = big.want["whole"], big.want["from_2^32"], big.want["nul_below_2^32"]
     kb, kc = ib[0], big.spans["nul_below_2^32"][1]
@@ -601,12 +556,12 @@ def test_host_forms_past_4GiB(matcher, patterns, big):
     # absolute byte 0, below the copy: the library reads a chunk from bytes + (offsets[k0] & ~511) on, never below
     ptr = host.ctypes.data - base
     assert matcher.count_host_ptr(ptr, offs.ctypes.data, k1 - k0) == key_counts(want, patterns)
-    got = rec_keys(matcher.find_host_ptr(ptr, offs.ctypes.data, k1 - k0, len(want) + 16))
+    got = keys(matcher.find_host_ptr(ptr, offs.ctypes.data, k1 - k0, len(want) + 16))
     assert np.array_equal(got, want), diff(got, want)
     del host
 
 
-def test_tables_in_global_memory(patterns, finder, big):
+def test_tables_in_global_memory(patterns, big):
     """~700 patterns (the probe tables leave shared memory), most of them cut from the planted windows, on the span
     above 2^33: counts and sorted records."""
     lay, k0, k1 = big.spans["1GiB_above_2^33"]
@@ -621,32 +576,26 @@ def test_tables_in_global_memory(patterns, finder, big):
         if b"\0" not in w[at:at + m]:
             pats.append(w[at:at + m])
     pats += pats[100:110]  # duplicates: credited to their first listing
-    want = big.plan.expect(o[k0:k1 + 1].astype(np.uint64), pats, finder)
+    want = big.plan.expect(o[k0:k1 + 1].astype(np.uint64), pats)
     with kmp.Matcher(0, engine="union") as m:
         m.set_patterns(pats)
         counts = key_counts(want, pats)
-        assert device_counts(m, big.d_bytes, big.d_off[lay], k0, k1, (int(o[k0]), int(o[k1])), len(pats)) == counts
-        rec, n, ok = device_find(m, big.d_bytes, big.d_off[lay], k0, k1, (int(o[k0]), int(o[k1])), len(want), True)
-        got = rec_keys(rec)
+        assert big.batch[lay].count(m, k0=k0, k1=k1) == [counts]
+        rec, n, ok = big.batch[lay].find(m, len(want), True, k0, k1, canary=64)
+        got = keys(rec)
         assert n == len(want) and ok and np.array_equal(got, want), diff(got, want)
-
-
-def udp_frame(payload_len, payload=b""):
-    """Ethernet + IPv4 (20 bytes) + UDP header, then `payload` and zeros up to payload_len bytes"""
-    return b"\x02" * 12 + b"\x08\x00" + bytes([0x45, 0, 0, 0, 0, 0, 0, 0, 64, 17]) + bytes(10 + 8) + \
-        payload + bytes(payload_len - len(payload))
 
 
 def test_savefile_and_stream_refuse_a_packet_at_the_limit(matcher, patterns, tmp_path):
     """The savefile forms and pushed frames check every payload before anything runs: one of LIMIT bytes (its frame's
     captured length less the headers) is refused by kmpb_count_pcap, kmpb_find_pcap and kmpb_stream_push, and the
     packets around it still count when the range leaves it out."""
-    small = [udp_frame(100, b"xx http yy ack"), udp_frame(50, b"dos udp test")]
+    small = [udp_frame(b"xx http yy ack".ljust(100, b"\0")), udp_frame(b"dos udp test".ljust(50, b"\0"))]
     path = str(tmp_path / "giant.pcap")
     with open(path, "wb") as f:  # the giant payload is a hole in a sparse file: zeros
         f.write(struct.pack("<IHHiIII", 0xA1B2C3D4, 2, 4, 0, 0, 262144, 1))
         f.write(struct.pack("<IIII", 1, 2, len(small[0]), len(small[0])) + small[0])
-        head = udp_frame(0)
+        head = udp_frame(b"")
         f.write(struct.pack("<IIII", 1, 2, len(head) + LIMIT, len(head) + LIMIT) + head)
         f.seek(LIMIT, 1)
         f.write(struct.pack("<IIII", 1, 2, len(small[1]), len(small[1])) + small[1])
@@ -663,7 +612,7 @@ def test_savefile_and_stream_refuse_a_packet_at_the_limit(matcher, patterns, tmp
     assert matcher.count_pcap_streamed(path, first=2, count=1) == [w - f for w, f in zip(want, first)]
     with matcher.stream("udp") as st:
         st.push(small[0])
-        giant = udp_frame(LIMIT)
+        giant = udp_frame(bytes(LIMIT))
         with pytest.raises(kmp.KmpbError) as e:
             st.push(giant)
         assert e.value.code == ELIMIT and "packet 1 " in str(e.value), str(e.value)

@@ -5,7 +5,7 @@ A packet is selected iff it holds at least one match the count forms count: exac
 (tests/c/kmp_find_ref.c) reports a record for.  The CPU tests check the writer on hand-built savefiles of every kind the
 reader takes, the writer on the bundled captures with the reference finder's verdicts, the entry points without a
 device, and that the existing union kernels compile to the same SASS as before the mark kernel was added.  The GPU
-tests check every select form against the reference finder (case-sensitive sets) or the find forms (nocase sets)."""
+tests check every select form against the reference finder."""
 import ctypes
 import hashlib
 import json
@@ -18,47 +18,17 @@ import numpy as np
 import pytest
 
 from conftest import DATA, GOLDEN, ROOT
-from test_find import RefFinder, csr, pcap_frames
-from test_host import _pcapng, _udp_frame, _write_pcap
+from kmpb_harness import (MATCH, PCAPS, SELECT, SELECT_FORMS, DeviceBatch, check_forms, classic_records, pcap_frames,
+                          pcapng, udp_frame, write_pcap)
+from kmpb_reference import csr, expected
 
 import multithreading_string_matching_b200 as kmp
 
 PKG = os.path.join(ROOT, "multithreading_string_matching_b200")
-SELECT = os.path.join(PKG, "bin", "kmp_select")
-MATCH = os.path.join(PKG, "bin", "kmp_match")
-PCAPS = ["udp", "udp_1000", "big_udp", "very_big_udp", "tcp"]
 EINVAL, ESTATE = -1, -7
 
 
-@pytest.fixture(scope="module")
-def finder(tmp_path_factory):
-    return RefFinder(str(tmp_path_factory.mktemp("kmp_find_ref_sel")))
-
-
-def expected_flags(finder, data, offsets, patterns):
-    """the packets with at least one record of the reference finder"""
-    n = len(offsets) - 1
-    flags = np.zeros(n, dtype=bool)
-    if patterns and n:
-        flags[finder.find_csr(data, offsets, patterns)["packet"].astype(np.int64)] = True
-    return flags
-
-
 # ---- savefile parsing for the checks --------------------------------------------------------------------
-
-def classic_records(path):
-    """(global header, [whole record bytes]) of a classic savefile, up to a cut trailing record"""
-    raw = open(path, "rb").read()
-    e = "<" if struct.unpack("<I", raw[:4])[0] in (0xA1B2C3D4, 0xA1B23C4D) else ">"
-    at, recs = 24, []
-    while len(raw) - at >= 16:
-        cap = struct.unpack(e + "I", raw[at + 8:at + 12])[0]
-        if cap > len(raw) - at - 16:
-            break
-        recs.append(raw[at:at + 16 + cap])
-        at += 16 + cap
-    return raw[:24], recs
-
 
 def pcapng_blocks(raw):
     """[(is_packet_block, block bytes)] of a well-formed pcapng file"""
@@ -91,23 +61,8 @@ def accepted_frames(path, proto="udp"):
         lib.kmpb_pcap_close(pc)
 
 
-def _pb_pcapng(frames, big_endian=False):
-    """SHB, IDB, then obsolete Packet Blocks (type 2) and an Interface Statistics Block at the end"""
-    e = ">" if big_endian else "<"
-
-    def block(btype, body):
-        body += b"\0" * (-len(body) % 4)
-        return struct.pack(e + "II", btype, len(body) + 12) + body + struct.pack(e + "I", len(body) + 12)
-
-    out = block(0x0A0D0D0A, struct.pack(e + "IHHq", 0x1A2B3C4D, 1, 0, -1))
-    out += block(1, struct.pack(e + "HHI", 1, 0, 65535))
-    for k, f in enumerate(frames):
-        out += block(2, struct.pack(e + "HHIIII", 0, 0, 0, k, len(f), len(f)) + f)
-    return out + block(5, struct.pack(e + "III", 0, 0, 0))
-
-
-FRAMES = [_udp_frame(b"hello world"), b"short", _udp_frame(b"", ihl=6), _udp_frame(b"x" * 1400), _udp_frame(b"a\0b"),
-          _udp_frame(b"ack ack"), _udp_frame(b"z" * 77)]
+FRAMES = [udp_frame(b"hello world"), b"short", udp_frame(b"", ihl=6), udp_frame(b"x" * 1400), udp_frame(b"a\0b"),
+          udp_frame(b"ack ack"), udp_frame(b"z" * 77)]
 
 
 def check_written(src, flags, tmp_path, tag):
@@ -162,7 +117,7 @@ def test_writer_classic(tmp_path, variant):
     if variant == "snaplen":  # caplen < len records are kept as they are
         caplens = [len(f) if i % 2 else min(len(f), 46) for i, f in enumerate(FRAMES)]
     src = str(tmp_path / "in.pcap")
-    _write_pcap(src, FRAMES, caplens=caplens, **kw)
+    write_pcap(src, FRAMES, caplens=caplens, **kw)
     if variant == "cut_tail":
         with open(src, "r+b") as f:
             f.truncate(os.path.getsize(src) - 20)
@@ -179,12 +134,10 @@ def test_writer_classic(tmp_path, variant):
 @pytest.mark.parametrize("variant", ["le", "be", "simple", "two_sections", "two_sections_be", "packet_blocks",
                                      "packet_blocks_be"])
 def test_writer_pcapng(tmp_path, variant):
-    if variant.startswith("packet_blocks"):
-        raw = _pb_pcapng(FRAMES, big_endian=variant.endswith("_be"))
-    else:
-        kw = {"le": {}, "be": {"big_endian": True}, "simple": {"simple_from": 2}, "two_sections": {"second_section_at": 3},
-              "two_sections_be": {"big_endian": True, "second_section_at": 2}}[variant]
-        raw = _pcapng(FRAMES, **kw)
+    kw = {"le": {}, "be": {"big_endian": True}, "simple": {"simple_from": 2}, "two_sections": {"second_section_at": 3},
+          "two_sections_be": {"big_endian": True, "second_section_at": 2}, "packet_blocks": {"packet_blocks": True},
+          "packet_blocks_be": {"packet_blocks": True, "big_endian": True}}[variant]
+    raw = pcapng(FRAMES, **kw)
     src = str(tmp_path / "in.pcapng")
     open(src, "wb").write(raw)
     n = len(accepted_frames(src))
@@ -202,7 +155,7 @@ def test_writer_section_length_is_unspecified(tmp_path):
     Every other byte of every kept block is the input's."""
     for big in (False, True):
         e = ">" if big else "<"
-        raw = bytearray(_pcapng(FRAMES, big_endian=big, second_section_at=3))
+        raw = bytearray(pcapng(FRAMES, big_endian=big, second_section_at=3))
         shbs = [at for at in range(0, len(raw), 4) if raw[at:at + 4] == b"\x0a\x0d\x0d\x0a"]
         assert len(shbs) == 2
         ends = shbs[1:] + [len(raw)]
@@ -233,7 +186,7 @@ def test_writer_section_length_is_unspecified(tmp_path):
 
 def test_writer_slices_and_refusals(tmp_path):
     src = str(tmp_path / "in.pcap")
-    _write_pcap(src, FRAMES)
+    write_pcap(src, FRAMES)
     acc = accepted_frames(src)
     _, recs = classic_records(src)
     out = str(tmp_path / "out.pcap")
@@ -262,13 +215,13 @@ def test_writer_slices_and_refusals(tmp_path):
 
 @pytest.mark.parametrize("pcap", PCAPS)
 @pytest.mark.parametrize("proto", ["udp", "tcp"])
-def test_expected_verdicts_write_the_matching_frames(oracle, finder, strings_txt, tmp_path, pcap, proto):
+def test_expected_verdicts_write_the_matching_frames(oracle, strings_txt, tmp_path, pcap, proto):
     """The reference finder's verdicts on the bundled captures, written out: the selected frames hold every match of
     the input (same counts), the others none."""
     path = os.path.join(DATA, pcap + ".pcap")
     pats = kmp.load_patterns(strings_txt)
     b = kmp.PayloadBatch(path, proto)
-    flags = expected_flags(finder, b.data, b.offsets, pats)
+    flags = expected(pats, b.data, b.offsets)[2]
     want = oracle.count_csr(b.data, b.offsets, pats)
     for inv in (False, True):
         out = str(tmp_path / ("out_%d.pcap" % inv))
@@ -354,71 +307,15 @@ def strings(strings_txt):
     return kmp.load_patterns(strings_txt)
 
 
-def device_select(m, data, offsets, k0=0, k1=None, invert=False, stream=None, sync=True, n_pat=None):
-    """kmpb_select_device_span over packets [k0, k1) of a device copy of the batch -> (flags, index list, counts);
-    the counts start at 5 each (accumulated into)."""
-    import torch
-
-    k1 = len(offsets) - 1 if k1 is None else k1
-    n = k1 - k0
-    n_pat = len(m.patterns) if n_pat is None else n_pat
-    d_bytes = torch.zeros(((len(data) + 64 + 31) // 32) * 32, dtype=torch.uint8, device="cuda:0")
-    if len(data):
-        d_bytes[: len(data)] = torch.from_numpy(np.array(data, dtype=np.uint8)).cuda()
-    d_off = torch.from_numpy(np.ascontiguousarray(offsets, dtype=np.int64)).cuda()
-    d_flags = torch.full((max(n, 1),), 7, dtype=torch.uint8, device="cuda:0")
-    d_index = torch.full((max(n, 1),), -1, dtype=torch.int64, device="cuda:0")
-    d_n = torch.full((1,), -1, dtype=torch.int64, device="cuda:0")
-    d_counts = torch.full((max(n_pat, 1),), 5, dtype=torch.int64, device="cuda:0")
-    span = (int(offsets[k0]), int(offsets[k1]))
-    m.select_device(d_bytes.data_ptr(), d_off.data_ptr() + 8 * k0, n, d_flags.data_ptr(), span, d_index.data_ptr(),
-                    d_n.data_ptr(), d_counts.data_ptr(), invert=invert, stream=stream)
-    res = lambda: (d_flags[:n].cpu().numpy().astype(bool), d_index[: int(d_n.item())].cpu().numpy(),  # noqa: E731
-                   [c - 5 for c in d_counts[:n_pat].cpu().tolist()])
-    if sync:
-        torch.cuda.synchronize()
-        return res()
-    return res, (d_bytes, d_off, d_flags, d_index, d_n, d_counts)
-
-
-def check_batch(m, data, offsets, want, label=""):
-    """host and device forms (plain and inverted) against the expected verdicts; counts against kmpb_count_host"""
-    n = len(offsets) - 1
-    flags, counts = m.select_host(data, offsets)
-    assert np.array_equal(flags, want), (label, "host", np.flatnonzero(flags != want)[:8])
-    want_counts = m.count_host(data, offsets) if m.patterns else []
-    assert counts == want_counts, (label, "host counts")
-    for inv in (False, True):
-        f, idx, c = device_select(m, data, offsets, invert=inv)
-        assert np.array_equal(f, want), (label, "device", inv, np.flatnonzero(f != want)[:8])
-        assert np.array_equal(idx, np.flatnonzero(want != inv)), (label, "index", inv)
-        assert c == want_counts, (label, "device counts")
-    assert len(want) == n
-    # *n_selected of the host form, and the form without counts_out
-    d = np.array(data, dtype=np.uint8) if len(data) else np.zeros(1, np.uint8)
-    o = np.ascontiguousarray(offsets, dtype=np.uint64)
-    fl = np.zeros(max(n, 1), dtype=np.uint8)
-    n_sel = ctypes.c_uint64(12345)
-    kmp.matcher.check(kmp.lib().kmpb_select_host(m.handle, d.ctypes.data, o.ctypes.data, n, fl.ctypes.data,
-                                                 ctypes.byref(n_sel), None))
-    assert n_sel.value == int(want.sum()) and np.array_equal(fl[:n].astype(bool), want), (label, "n_selected")
-    kmp.matcher.check(kmp.lib().kmpb_check_device_errors(m.handle))
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("pcap", PCAPS)
 @pytest.mark.parametrize("proto", ["udp", "tcp"])
 @pytest.mark.parametrize("nocase", [False, True])
-def test_bundled_captures(matcher, finder, strings, pcap, proto, nocase):
+def test_bundled_captures(matcher, strings, pcap, proto, nocase):
     path = os.path.join(DATA, pcap + ".pcap")
-    matcher.set_patterns(strings, nocase=nocase)
     b = kmp.PayloadBatch(path, proto)
-    if nocase:  # the find forms' packets (their records are checked against the reference in test_nocase.py)
-        want = np.zeros(b.n_packets, dtype=bool)
-        want[matcher.find_host(b.data, b.offsets)["packet"].astype(np.int64)] = True
-    else:
-        want = expected_flags(finder, b.data, b.offsets, strings)
-    check_batch(matcher, b.data, b.offsets, want, (pcap, proto, nocase))
+    want = check_forms((matcher,), strings, b.data, b.offsets, nocase, label=(pcap, proto, nocase),
+                       forms=SELECT_FORMS)[2]
     assert np.array_equal(matcher.select_pcap(path, proto), want)
     n = b.n_packets
     if n > 4:
@@ -444,7 +341,7 @@ def _uniform(n, size, fill):
 
 
 @pytest.mark.gpu
-def test_edge_batches(matcher, finder):
+def test_edge_batches(matcher):
     rng = np.random.default_rng(5)
     p99 = bytes(rng.integers(97, 100, 99).astype(np.uint8))
     cases = {
@@ -463,27 +360,26 @@ def test_edge_batches(matcher, finder):
         "all_empty_packets": ([b""] * 77, [b"a"]),
     }
     for label, (pkts, pats) in cases.items():
-        matcher.set_patterns(pats)
-        data, offsets = csr(pkts)
-        check_batch(matcher, data, offsets, expected_flags(finder, data, offsets, pats), label)
+        check_forms((matcher,), pats, *csr(pkts), label=label, forms=SELECT_FORMS)
 
 
 @pytest.mark.gpu
-def test_first_byte_not_a_multiple_of_32(matcher, finder):
+def test_first_byte_not_a_multiple_of_32(matcher):
     """device spans and host batches that start at every residue of 32 (offsets relative to absolute byte 0)"""
     rng = np.random.default_rng(9)
     pats = [b"ab", b"b", b"abcab", b"cc"]
     matcher.set_patterns(pats)
     pkts = [bytes(rng.integers(97, 100, int(s)).astype(np.uint8)) for s in rng.integers(0, 40, 4000)]
     data, offsets = csr(pkts)
-    want = expected_flags(finder, data, offsets, pats)
+    want = expected(pats, data, offsets)[2]
+    batch = DeviceBatch(data, offsets)
     seen = set()
     for k0 in range(0, 400):
         if int(offsets[k0]) % 32 in seen:
             continue
         seen.add(int(offsets[k0]) % 32)
         k1 = len(pkts) - int(rng.integers(0, 50))
-        f, idx, c = device_select(matcher, data, offsets, k0, k1)
+        f, idx, c = batch.select(matcher, k0, k1)
         assert np.array_equal(f, want[k0:k1]), k0
         assert np.array_equal(idx, np.flatnonzero(want[k0:k1]))
         sub = offsets[k0:k1 + 1]
@@ -493,7 +389,7 @@ def test_first_byte_not_a_multiple_of_32(matcher, finder):
 
 
 @pytest.mark.gpu
-def test_random_batches_and_global_tables(finder):
+def test_random_batches_and_global_tables():
     rng = np.random.default_rng(1234)
     with kmp.Matcher(0) as m:
         for trial in range(12):
@@ -501,9 +397,7 @@ def test_random_batches_and_global_tables(finder):
             pats = [bytes(rng.choice(list(alpha.replace(b"\0", b""))) for _ in range(int(rng.choice([1, 2, 3, 5, 9, 99]))))
                     for _ in range(int(rng.integers(1, 9)))]
             pkts = [bytes(rng.choice(list(alpha), int(s)).astype(np.uint8)) for s in rng.choice([0, 1, 3, 17, 120, 1400], 3000)]
-            m.set_patterns(pats)
-            data, offsets = csr(pkts)
-            check_batch(m, data, offsets, expected_flags(finder, data, offsets, pats), ("random", trial))
+            check_forms((m,), pats, *csr(pkts), label=("random", trial), forms=SELECT_FORMS)
         # ~800 patterns: the probe tables leave shared memory
         pkts = [bytes(rng.integers(97, 105, int(s)).astype(np.uint8)) for s in rng.integers(0, 600, 6000)]
         data, offsets = csr(pkts)
@@ -514,12 +408,11 @@ def test_random_batches_and_global_tables(finder):
             if len(p) > ln:
                 at = int(rng.integers(0, len(p) - ln))
                 pats.append(p[at:at + ln] if rng.random() < 0.3 else bytes(rng.integers(97, 105, ln).astype(np.uint8)))
-        m.set_patterns(pats)
-        check_batch(m, data, offsets, expected_flags(finder, data, offsets, pats), "global tables")
+        check_forms((m,), pats, data, offsets, label="global tables", forms=SELECT_FORMS)
 
 
 @pytest.mark.gpu
-def test_chunked_forms(monkeypatch, finder, strings):
+def test_chunked_forms(monkeypatch, strings):
     """1 MiB chunks: many chunks through every stream slot, host and savefile forms, first / count slices"""
     monkeypatch.setenv("KMPB_CHUNK_MB", "1")
     synth = kmp.Synth(seed=77, payload_len=1400, len_mode=1, plants=1, plant_patterns=strings)
@@ -527,20 +420,20 @@ def test_chunked_forms(monkeypatch, finder, strings):
     data = silence(data, offsets, 3)
     with kmp.Matcher(0) as m:
         m.set_patterns(strings)
-        want = expected_flags(finder, data, offsets, strings)
+        want = expected(strings, data, offsets)[2]
         assert 0 < want.sum() < len(want)
         flags, counts = m.select_host(data, offsets)
         assert np.array_equal(flags, want) and counts == m.count_host(data, offsets)
         path = os.path.join(DATA, "very_big_udp.pcap")
         b = kmp.PayloadBatch(path, "udp")
-        pw = expected_flags(finder, b.data, b.offsets, strings)
+        pw = expected(strings, b.data, b.offsets)[2]
         n = b.n_packets
         for first, count in ((0, n), (1, n - 1), (n // 3, n // 2), (n - 1, 1), (5, 0)):
             assert np.array_equal(m.select_pcap(path, "udp", first, count), pw[first:first + count]), (first, count)
 
 
 @pytest.mark.gpu
-def test_back_to_back_selects_are_independent(matcher, finder, strings):
+def test_back_to_back_selects_are_independent(matcher, strings):
     """a verdict pass that left bits behind would select packets of the previous batch"""
     matcher.set_patterns(strings)
     synth = kmp.Synth(seed=3, payload_len=700, plants=1, plant_patterns=strings)
@@ -548,39 +441,39 @@ def test_back_to_back_selects_are_independent(matcher, finder, strings):
     data_a = silence(data_a, off_a, 2)
     data_b, off_b = synth.fill_host(5000, 4000)
     data_b = silence(data_b, off_b, 5)
-    want_a = expected_flags(finder, data_a, off_a, strings)
-    want_b = expected_flags(finder, data_b, off_b, strings)
+    want_a = expected(strings, data_a, off_a)[2]
+    want_b = expected(strings, data_b, off_b)[2]
     assert want_a.any() and not want_a.all() and not np.array_equal(want_a[:4000], want_b)
+    batch_a, batch_b = DeviceBatch(data_a, off_a), DeviceBatch(data_b, off_b)
     for _ in range(2):
-        for data, off, want in ((data_a, off_a, want_a), (data_b, off_b, want_b), (data_a, off_a, want_a)):
-            assert np.array_equal(device_select(matcher, data, off)[0], want)
+        for data, off, batch, want in ((data_a, off_a, batch_a, want_a), (data_b, off_b, batch_b, want_b),
+                                       (data_a, off_a, batch_a, want_a)):
+            assert np.array_equal(batch.select(matcher)[0], want)
             assert np.array_equal(matcher.select_host(data, off)[0], want)
 
 
 @pytest.mark.gpu
-def test_interleaved_with_count_and_find(finder, strings):
+def test_interleaved_with_count_and_find(strings):
     """selects, counts and finds on three streams with no host sync in between give the answers each gives alone;
     KMPB_ESTATE while a frame stream is open"""
     import torch
 
     synth = kmp.Synth(seed=21, payload_len=900, len_mode=1, plants=2, plant_patterns=strings)
     data, offsets = synth.fill_host(0, 20000)
-    want = expected_flags(finder, data, offsets, strings)
+    want = expected(strings, data, offsets)[2]
     with kmp.Matcher(0) as m:
         m.set_patterns(strings)
         want_counts = m.count_host(data, offsets)
         total = distinct_total(want_counts, strings)
         streams = [torch.cuda.Stream() for _ in range(3)]
         keep, results = [], []
-        d_bytes = torch.from_numpy(np.concatenate([data, np.zeros(64, np.uint8)])).cuda()
-        d_off = torch.from_numpy(offsets.astype(np.int64)).cuda()
+        batch = DeviceBatch(data, offsets)
+        d_bytes, d_off = batch.d_bytes, batch.d_off
         torch.cuda.synchronize()
         span = (0, int(offsets[-1]))
         n = len(offsets) - 1
         for rnd in range(3):
-            res, bufs = device_select(m, data, offsets, stream=streams[0].cuda_stream, sync=False)
-            keep.append(bufs)
-            results.append(res)
+            results.append(batch.select(m, stream=streams[0].cuda_stream, wait=False))
             d_counts = torch.zeros(len(strings), dtype=torch.int64, device="cuda:0")
             m.count_device(d_bytes.data_ptr(), d_off.data_ptr(), n, d_counts.data_ptr(), span=span, stream=streams[1].cuda_stream)
             d_rec = torch.zeros(total * 16, dtype=torch.uint8, device="cuda:0")
@@ -592,13 +485,13 @@ def test_interleaved_with_count_and_find(finder, strings):
         for res in results:
             f, idx, c = res()
             assert np.array_equal(f, want) and np.array_equal(idx, np.flatnonzero(want)) and c == want_counts
-        for d_counts, d_rec, d_n in keep[1::2]:
+        for d_counts, d_rec, d_n in keep:
             assert d_counts.cpu().tolist() == want_counts and int(d_n.item()) == total
             pk = np.unique(d_rec.cpu().numpy().view(kmp.MATCH_DTYPE)["packet"].astype(np.int64))
             assert np.array_equal(pk, np.flatnonzero(want))
         with m.stream("udp") as st:
-            st.push(_udp_frame(b"x"))
-            for call in (lambda: m.select_host(data, offsets), lambda: device_select(m, data, offsets),
+            st.push(udp_frame(b"x"))
+            for call in (lambda: m.select_host(data, offsets), lambda: batch.select(m),
                          lambda: m.select_pcap(os.path.join(DATA, "udp.pcap"))):
                 with pytest.raises(kmp.KmpbError) as e:
                     call()

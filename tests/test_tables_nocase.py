@@ -1,7 +1,7 @@
 """Case-insensitive patterns without a GPU: the host tables (tests/c/test_tables_nocase.c against csrc/host/automaton.c),
-the usage text of `kmp_match -i` / `kmp_find -i`, and the derivation of the expected answers tests/test_nocase.py uses
-(a nocase pattern's matches are the case-sensitive matches of the folded pattern in the folded text), checked against a
-naive case-insensitive finder."""
+the usage text of `kmp_match -i` / `kmp_find -i`, and the derivation of the expected answers (tests/kmpb_reference.py
+`expected`: a nocase pattern's matches are the case-sensitive matches of the folded pattern in the folded text, the
+oracle's counts of each flag group alongside), checked against a naive finder."""
 import os
 import random
 import subprocess
@@ -10,11 +10,10 @@ import numpy as np
 import pytest
 
 from conftest import ROOT
-from test_find import RefFinder, csr
-from test_nocase import expected, fold, naive_nocase_find
+from kmpb_harness import BIN
+from kmpb_reference import csr, expected, firsts, fold, naive
 
 HOSTC = os.path.join(ROOT, "multithreading_string_matching_b200", "csrc", "host")
-BIN = os.path.join(ROOT, "multithreading_string_matching_b200", "bin")
 
 
 def test_host_tables_nocase_selfcheck(tmp_path):
@@ -45,8 +44,7 @@ def test_fold_is_ascii_letters_only():
     assert fold(b"@[\\]^_\x7f\xc1\xdf`{|}~") == b"@[\\]^_\x7f\xc1\xdf`{|}~"
 
 
-def test_expected_answers_against_a_naive_finder(oracle, tmp_path):
-    finder = RefFinder(str(tmp_path))
+def test_expected_answers_against_a_naive_finder(oracle):
     rng = random.Random(7)
     alpha = b"aAbBzZ@`[{^~_\x7f\xc1\xe1\0"
     for trial in range(150):
@@ -56,11 +54,9 @@ def test_expected_answers_against_a_naive_finder(oracle, tmp_path):
         nocase = [rng.random() < 0.5 for _ in pats]
         pkts = [bytes(rng.choice(alpha) for _ in range(rng.randint(0, 40))) for _ in range(rng.randint(1, 6))]
         data, offsets = csr(pkts)
-        counts, rec = expected(oracle, finder, pats, nocase, data, offsets)
-        want = naive_nocase_find(pkts, pats, nocase)
+        counts, rec, _ = expected(pats, data, offsets, nocase, oracle=oracle)
+        want = naive(pkts, pats, nocase)
         assert list(zip(rec["packet"].tolist(), rec["offset"].tolist(), rec["pattern"].tolist())) == want, trial
-        firsts = {}
-        keys = [(fold(p) if n else p, n) for p, n in zip(pats, nocase)]
-        first = [firsts.setdefault(k, i) for i, k in enumerate(keys)]
+        first = firsts(pats, nocase)
         hist = np.bincount(rec["pattern"].astype(np.int64), minlength=len(pats))
         assert counts == [int(hist[first[i]]) for i in range(len(pats))], trial

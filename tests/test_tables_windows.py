@@ -1,6 +1,7 @@
 """Position windows without a GPU: the host tables (tests/c/test_tables_windows.c against csrc/host/automaton.c), the
 `-w` option of the three command lines (malformed values, exit codes, unchanged usage texts), Matcher's argument
-checks, and the derivation of the expected answers tests/test_windows.py uses, checked against a naive finder."""
+checks, and the derivation of the expected answers (tests/kmpb_reference.py `expected`) checked against a naive
+finder."""
 import hashlib
 import json
 import os
@@ -10,14 +11,12 @@ import subprocess
 import pytest
 
 from conftest import ROOT
-from test_find import RefFinder, csr
-from test_nocase import fold
-from test_windows import expected
+from kmpb_harness import BIN
+from kmpb_reference import csr, expected, firsts, naive
 
 import multithreading_string_matching_b200 as kmp
 
 HOSTC = os.path.join(ROOT, "multithreading_string_matching_b200", "csrc", "host")
-BIN = os.path.join(ROOT, "multithreading_string_matching_b200", "bin")
 
 
 def test_host_tables_windows_selfcheck(tmp_path):
@@ -81,23 +80,7 @@ def test_matcher_window_argument_checks():
             m.set_patterns([b"a", b"b"], window=bad)
 
 
-def naive(packets, patterns, nocase, window):
-    """sorted (packet, offset, pattern) straight from the definition"""
-    seen = {}
-    firsts = [seen.setdefault((fold(p) if n else p, n, w), i) for i, (p, n, w) in enumerate(zip(patterns, nocase, window))]
-    out = []
-    for k, payload in enumerate(packets):
-        text = payload.split(b"\0", 1)[0]
-        for i, (p, n, w) in enumerate(zip(patterns, nocase, window)):
-            if firsts[i] != i:
-                continue
-            t, q = (fold(text), fold(p)) if n else (text, p)
-            out += [(k, s, i) for s in range(len(t) - len(q) + 1) if t[s:s + len(q)] == q and (w is None or w[0] <= s <= w[1])]
-    return sorted(out)
-
-
-def test_expected_answers_against_a_naive_finder(tmp_path):
-    finder = RefFinder(str(tmp_path))
+def test_expected_answers_against_a_naive_finder():
     rng = random.Random(9)
     alpha = b"aAbz\0"
     for trial in range(200):
@@ -108,10 +91,9 @@ def test_expected_answers_against_a_naive_finder(tmp_path):
         window = [None if rng.random() < 0.3 else (lambda lo: (lo, lo + rng.randint(0, 12)))(rng.randint(0, 10)) for _ in pats]
         pkts = [bytes(rng.choice(alpha) for _ in range(rng.randint(0, 30))) for _ in range(rng.randint(1, 6))]
         data, offsets = csr(pkts)
-        counts, rec, verdicts = expected(finder, pats, nocase, window, data, offsets)
+        counts, rec, verdicts = expected(pats, data, offsets, nocase, window)
         want = naive(pkts, pats, nocase, window)
         assert list(zip(rec["packet"].tolist(), rec["offset"].tolist(), rec["pattern"].tolist())) == want, trial
         assert verdicts.tolist() == [any(r[0] == k for r in want) for k in range(len(pkts))]
-        seen = {}
-        firsts = [seen.setdefault((fold(p) if n else p, n, w), i) for i, (p, n, w) in enumerate(zip(pats, nocase, window))]
-        assert counts == [sum(1 for r in want if r[2] == firsts[i]) for i in range(len(pats))]
+        first = firsts(pats, nocase, window)
+        assert counts == [sum(1 for r in want if r[2] == first[i]) for i in range(len(pats))]

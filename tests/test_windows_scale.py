@@ -2,12 +2,9 @@
 counters or its probe tables in global memory, walks runs of thousands of one-byte patterns, and compares long
 patterns at tile edges -- through both engines and every form, against an exact reference.
 
-The reference (`reference`) is numpy and costs about one table lookup per (text position, distinct (flag, length)),
-not patterns x bytes: the distinct patterns are grouped by (flag, length); a group's keys are looked up at every text
-position with room for them (for a group of windowed patterns only at offsets [min lo, max hi]); the hits of a key,
-sorted by offset, give each of its patterns its records as one slice, cut by two binary searches on lo and hi.  The CPU
-tests check it against the naive finder of tests/test_tables_windows.py and the reference-finder answers of
-tests/test_windows.py.
+The reference is the numpy one of tests/kmpb_reference.py, which costs about one table lookup per text byte and
+distinct (flag, length), not patterns x bytes.  The CPU tests check it against the naive finder and the
+reference-finder answers of the same module.
 
 The kernel's two placement decisions (`kmpb_launch_window`): the counters go to shared memory for at most 4096
 distinct windowed patterns (8 * n_win <= 32768), the probe tables for at most 16384 words (4 * wvtab_words <= 65536).
@@ -23,11 +20,8 @@ import numpy as np
 import pytest
 
 from conftest import ROOT
-from test_find import RefFinder, csr
-from test_host import _udp_frame, _write_pcap
-from test_nocase import fold
-from test_tables_windows import naive
-from test_windows import ORDER, check, expected, firsts_of
+from kmpb_harness import check_forms, engines, udp_frame, write_pcap  # noqa: F401
+from kmpb_reference import ORDER, csr, expected, firsts, fold, naive, normalise, reference
 
 import multithreading_string_matching_b200 as kmp
 
@@ -36,109 +30,8 @@ ANY = 0xFFFFFFFF
 COUNTS_SMEM_MAX = 4096  # window.cu: distinct windowed patterns whose 64-bit counters stay in shared memory
 VTAB_SMEM_MAX = 16384   # window.cu: words of probe tables that stay in shared memory
 TILE = 1024             # window.cu WN_TILE: start offsets per tile
-FOLD = np.frombuffer(fold(bytes(range(256))), dtype=np.uint8)
 LOWER = b"abcdefghijklmnopqrstuvwxyz"
 MIXED = LOWER + LOWER.upper() + b"0123456789"
-
-
-# ---- the reference --------------------------------------------------------------------------------------------------
-
-def normalised(patterns, nocase, window):
-    n = len(patterns)
-    nocase = [bool(x) for x in (nocase if isinstance(nocase, (list, tuple)) else [nocase] * n)]
-    window = list(window) if isinstance(window, list) else [window] * n
-    return [bytes(p) for p in patterns], nocase, window
-
-
-def _prefix64(text):
-    """the little-endian 64-bit word of text bytes p..p+7 for every p (zero past the end)"""
-    t = np.zeros(len(text) + 8, dtype=np.uint64)
-    t[: len(text)] = text
-    out = np.zeros(len(text), dtype=np.uint64)
-    for i in range(8):
-        out |= t[i: i + len(text)] << np.uint64(8 * i)
-    return out
-
-
-def reference(patterns, nocase, window, data, offsets):
-    """(counts in file order, records sorted by (packet, offset, pattern), verdicts) of a set with windows"""
-    patterns, nocase, window = normalised(patterns, nocase, window)
-    data = np.ascontiguousarray(data, dtype=np.uint8)
-    offsets = np.asarray(offsets, dtype=np.int64)
-    starts, n_pk = offsets[:-1], len(offsets) - 1
-    # a packet's text: its payload up to the first NUL
-    nul = np.append(np.flatnonzero(data == 0), len(data))
-    text_end = np.minimum(nul[np.searchsorted(nul, starts)], offsets[1:]) if n_pk else starts
-    texts, words = {False: data, True: FOLD[data]}, {}
-    firsts = firsts_of(patterns, nocase, window)
-    groups = {}
-    for i, (p, nc, w) in enumerate(zip(patterns, nocase, window)):
-        if firsts[i] == i:
-            groups.setdefault((nc, len(p)), []).append((fold(p) if nc else p, w, i))
-    rec_pk, rec_off, rec_pat = [], [], []
-    for (nc, m), members in groups.items():
-        windowed = all(w is not None for _, w, _ in members)
-        o_lo = min(w[0] for _, w, _ in members) if windowed else 0
-        o_hi = max(w[1] for _, w, _ in members) if windowed else 1 << 62
-        first = starts + o_lo
-        cnt = np.maximum(np.minimum(text_end - m, starts + o_hi) - first + 1, 0)
-        total = int(cnt.sum())
-        if total == 0:
-            continue
-        pk = np.repeat(np.arange(n_pk), cnt)
-        pos = np.arange(total, dtype=np.int64) + np.repeat(first - (np.cumsum(cnt) - cnt), cnt)
-        text = texts[nc]
-        if nc not in words:
-            words[nc] = _prefix64(text)
-        # the first min(m, 8) bytes as one word pick the candidates; longer keys are compared in full after that
-        mask = np.uint64((1 << (8 * min(m, 8))) - 1)
-        keys = sorted({k for k, _, _ in members})
-        kw = np.array([int.from_bytes(k[:8], "little") for k in keys], dtype=np.uint64)
-        kord = np.argsort(kw, kind="stable")
-        sw = kw[kord]
-        tw = words[nc][pos] & mask
-        j = np.minimum(np.searchsorted(sw, tw), len(sw) - 1)
-        cand = sw[j] == tw
-        pk, pos = pk[cand], pos[cand]
-        if m <= 8:
-            kid = kord[j[cand]]  # (a key of up to 8 bytes is its word)
-        else:
-            skeys = np.array(keys, dtype="S%d" % m)
-            tk = np.ascontiguousarray(np.lib.stride_tricks.sliding_window_view(text, m)[pos]).view("S%d" % m).ravel()
-            kid = np.minimum(np.searchsorted(skeys, tk), len(keys) - 1)
-            same = skeys[kid] == tk
-            kid, pk, pos = kid[same], pk[same], pos[same]
-        off = pos - starts[pk]
-        order = np.lexsort((off, kid))
-        kid, pk, off = kid[order], pk[order], off[order]
-        bounds = np.searchsorted(kid, np.arange(len(keys) + 1))
-        where = {k: x for x, k in enumerate(keys)}
-        a_s, b_s, ids = [], [], []
-        for key, w, i in members:
-            a, b = bounds[where[key]], bounds[where[key] + 1]
-            if w is not None:
-                a, b = a + np.searchsorted(off[a:b], [w[0], w[1] + 1])
-            a_s.append(a)
-            b_s.append(b)
-            ids.append(i)
-        lens = np.array(b_s, dtype=np.int64) - np.array(a_s, dtype=np.int64)
-        n = int(lens.sum())
-        if n == 0:
-            continue
-        idx = np.arange(n, dtype=np.int64) + np.repeat(np.array(a_s, dtype=np.int64) - (np.cumsum(lens) - lens), lens)
-        rec_pk.append(pk[idx])
-        rec_off.append(off[idx])
-        rec_pat.append(np.repeat(np.array(ids, dtype=np.int64), lens))
-    rec = np.zeros(sum(len(x) for x in rec_pk), dtype=kmp.MATCH_DTYPE)
-    if len(rec):
-        pk, off, pat = (np.concatenate(x) for x in (rec_pk, rec_off, rec_pat))
-        order = np.lexsort((pat, off, pk))
-        rec["packet"], rec["offset"], rec["pattern"] = pk[order], off[order], pat[order]
-    hist = np.bincount(rec["pattern"].astype(np.int64), minlength=max(len(patterns), 1))
-    counts = [int(hist[firsts[i]]) for i in range(len(patterns))]
-    verdicts = np.zeros(n_pk, dtype=bool)
-    verdicts[rec["packet"].astype(np.int64)] = True
-    return counts, rec, verdicts
 
 
 # ---- the tables' geometry -------------------------------------------------------------------------------------------
@@ -153,7 +46,7 @@ def geometry(tmp_path_factory):
                     os.path.join(HOSTC, "errors.c"), "-o", exe], check=True)
 
     def run(patterns, nocase, window):
-        patterns, nocase, window = normalised(patterns, nocase, window)
+        patterns, nocase, window = normalise(patterns, nocase, window)
         path = str(d / "set.txt")
         with open(path, "w") as f:
             for p, nc, w in zip(patterns, nocase, window):
@@ -174,7 +67,7 @@ def paths(g):
 
 def longest_run(patterns, nocase, window):
     """the most distinct windowed one-byte patterns of one byte and flag (the kernel walks down such a run)"""
-    patterns, nocase, window = normalised(patterns, nocase, window)
+    patterns, nocase, window = normalise(patterns, nocase, window)
     runs = {}
     for p, nc, w in {(fold(p) if nc else p, nc, w) for p, nc, w in zip(patterns, nocase, window)}:
         if len(p) == 1 and w is not None:
@@ -183,7 +76,7 @@ def longest_run(patterns, nocase, window):
 
 
 def distinct_windowed(patterns, nocase, window):
-    patterns, nocase, window = normalised(patterns, nocase, window)
+    patterns, nocase, window = normalise(patterns, nocase, window)
     return len({(fold(p) if nc else p, nc, w) for p, nc, w in zip(patterns, nocase, window) if w is not None})
 
 
@@ -351,7 +244,7 @@ def tile_packets():
 def planted(seed, patterns, nocase, window, n_packets, sizes, alpha, plants=24, nul=0.05):
     """packets of random bytes from alpha with patterns written in: most at offsets inside their window or one off
     its edges, nocase ones in random case; a few packets with a NUL"""
-    patterns, nocase, window = normalised(patterns, nocase, window)
+    patterns, nocase, window = normalise(patterns, nocase, window)
     rng = random.Random(seed)
     npr = np.random.default_rng(seed)
     abytes = np.frombuffer(alpha, dtype=np.uint8)
@@ -392,15 +285,13 @@ def test_reference_against_the_naive_finder():
         data, offsets = csr(pkts)
         counts, rec, verdicts = reference(pats, nocase, window, data, offsets)
         want = naive(pkts, pats, nocase, window)
-        seen = {}
-        firsts = [seen.setdefault((fold(p) if n else p, n, w), i) for i, (p, n, w) in enumerate(zip(pats, nocase, window))]
+        first = firsts(pats, nocase, window)
         assert list(zip(rec["packet"].tolist(), rec["offset"].tolist(), rec["pattern"].tolist())) == want, trial
         assert verdicts.tolist() == [any(r[0] == k for r in want) for k in range(len(pkts))], trial
-        assert counts == [sum(1 for r in want if r[2] == firsts[i]) for i in range(len(pats))], trial
+        assert counts == [sum(1 for r in want if r[2] == first[i]) for i in range(len(pats))], trial
 
 
-def test_reference_against_the_reference_finder(tmp_path):
-    finder = RefFinder(str(tmp_path))
+def test_reference_against_the_reference_finder():
     rng = random.Random(82)
     for trial in range(6):
         pats = [bytes(rng.choice(b"abcdAB") for _ in range(rng.choice([1, 2, 3, 5, 9, 14, 40]))) for _ in range(300)]
@@ -409,7 +300,7 @@ def test_reference_against_the_reference_finder(tmp_path):
         pkts = planted(trial, pats, nocase, window, 120, [0, 30, 400, 1500], b"abcdAB", plants=6, nul=0.3)
         data, offsets = csr(pkts)
         got = reference(pats, nocase, window, data, offsets)
-        want = expected(finder, pats, nocase, window, data, offsets)
+        want = expected(pats, data, offsets, nocase, window)
         assert got[0] == want[0] and np.array_equal(got[1], want[1]) and np.array_equal(got[2], want[2]), trial
         assert len(want[1]) > 1000
 
@@ -456,19 +347,11 @@ def test_tile_packets_cover_every_lead():
 
 # ---- GPU ------------------------------------------------------------------------------------------------------------
 
-@pytest.fixture(scope="module")
-def engines():
-    u, p = kmp.Matcher(0, engine="union"), kmp.Matcher(0, engine="perpat")
-    yield u, p
-    u.close()
-    p.close()
-
-
 def run_case(engines, s, pkts, label):
     data, offsets = csr(pkts)
     answers = reference(*s, data, offsets)
     assert sum(answers[0]) > 0, label
-    return check(engines, None, *s, pkts, label=label, answers=answers)
+    return check_forms(engines, s[0], data, offsets, *s[1:], label=label, answers=answers)
 
 
 @pytest.mark.gpu
@@ -499,7 +382,7 @@ def test_all_windowed_global_counters_and_tables(engines):
 @pytest.mark.gpu
 def test_mixed_at_scale(engines):
     s = mixed_scale_set()
-    want_counts, want = run_case(engines, s, planted(15, *s, 300, [0, 50, 600, 1800], b"abcdefghijklmnop"), "mixed")
+    want_counts, want, _ = run_case(engines, s, planted(15, *s, 300, [0, 50, 600, 1800], b"abcdefghijklmnop"), "mixed")
     # one text occurrence of shared bytes is a record of each kind
     pats, _, window = s
     kinds = {(int(r["packet"]), int(r["offset"]), window[int(r["pattern"])] is None) for r in want}
@@ -526,8 +409,8 @@ def test_chunked_host_and_savefile_forms(monkeypatch, which, tmp_path):
     want_counts, want, verdicts = reference(*s, data, offsets)
     assert len(want) > 1000
     path = str(tmp_path / "w.pcap")
-    frames = [_udp_frame(p) for p in pkts]
-    _write_pcap(path, frames)
+    frames = [udp_frame(p) for p in pkts]
+    write_pcap(path, frames)
     with kmp.Matcher(0, engine="union") as union, kmp.Matcher(0, engine="perpat") as perpat:
         for m in (union, perpat):
             m.set_patterns(*s)
